@@ -220,6 +220,48 @@ def cpu_model() -> str:
     return "unknown"
 
 
+DUMP_SAMPLE = 1 << 19     # candidates in the --dump-outputs sample: at most 2 + 9 float64 values each, 44 MB in all
+DUMP_SEED = 1
+
+
+def dump_outputs(out_dir: str, n: int, d_edges, d_nonedge, d_counts) -> None:
+    """Writes what a step of hc_score_batch_device handed back (hc_edge records, non-edge indices, counts) as float64 .npy
+    files of finite values, so that two builds run with the same arguments can be compared output for output: counts.npy
+    whole; for a fixed seeded sample of the step's candidates cand.npy (index) and cls.npy (0 discarded, 1 edge, 2 non-edge);
+    for the sampled candidates that are edges, in the same order, the hc_edge fields edge_cand, edge_score,
+    edge_mismatch_rate, edge_pos3, edge_pos4, edge_mean_log (0 for a window that was not scored, where the record holds NaN)
+    and edge_window_scored (1 where it was)."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    counts = d_counts.cpu()
+    ne, nn = int(counts[0]), int(counts[1])
+    pick = np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=min(n, DUMP_SAMPLE), replace=False))
+    k = torch.from_numpy(pick).to(d_edges.device)
+
+    def find(sorted_idx):      # position of each sampled candidate in an input-ordered index list, and whether it is there
+        if len(sorted_idx) == 0:
+            return torch.zeros_like(k), torch.zeros_like(k, dtype=torch.bool)
+        at = torch.searchsorted(sorted_idx, k).clamp_(max=len(sorted_idx) - 1)
+        return at, sorted_idx[at] == k
+
+    edges = d_edges[:ne]
+    at, is_edge = find(edges.view(torch.int64)[:, 0].contiguous())
+    _, is_non = find(d_nonedge[:nn])
+    rec = edges[at[is_edge]]
+    f64, i32 = rec.view(torch.float64), rec.view(torch.int32)
+    mean_log = f64[:, 4:6]
+    scored = ~torch.isnan(mean_log)
+    cls = torch.where(is_edge, 1, torch.where(is_non, 2, 0))
+    out = {"counts": counts.double().numpy(), "cand": pick.astype(np.float64), "cls": cls.double().cpu().numpy(),
+           "edge_cand": rec.view(torch.int64)[:, 0].double(), "edge_score": f64[:, 1], "edge_mismatch_rate": f64[:, 2],
+           "edge_pos3": i32[:, 6].double(), "edge_pos4": i32[:, 7].double(), "edge_mean_log": torch.where(scored, mean_log, 0.0),
+           "edge_window_scored": scored.double()}
+    for name, v in out.items():
+        v = v.cpu().numpy() if torch.is_tensor(v) else v
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(v))
+
+
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -259,7 +301,15 @@ def main() -> None:
                     help="HC_FLAG_EXACT_EDGE_SCORES: re-sum every accepted edge in the reference's order (diagnostic)")
     ap.add_argument("--position-sorted-ids", action="store_true",
                     help="diagnostic only: number the reads in genome order (cache-friendly, NOT the benchmark layout)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0: counts, the class of a fixed seeded sample of "
+                         "its candidates and the edge fields of the sampled edges) to DIR/<name>.npy as float64, to compare two builds "
+                         "output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.device_chunk):
+        ap.error("--dump-outputs writes the outputs of the device-resident step of --impl ours, without --device-chunk")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -437,6 +487,8 @@ def main() -> None:
         log("[dma-load] host->device %.1f GB/s, device->host %.1f GB/s while the kernels ran" %
             (args.steps * h_in.numel() * 4 / ci0.elapsed_time(ci1) / 1e6, args.steps * h_out.numel() * 4 / co0.elapsed_time(co1) / 1e6))
     clocks = sampler.stop(tw0, tw1) if rank == 0 else None
+    if args.dump_outputs and rank == 0:     # before the legs below reuse d_edges (the exact-scores leg writes other scores)
+        dump_outputs(args.dump_outputs, n, d_edges, d_nonedge, d_counts)
     # dominant-kernel duration, measured live with CUDA events around hc_score_kernel on its stream
     kms, stats = [], None
     for _ in range(3):
