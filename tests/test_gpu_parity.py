@@ -179,9 +179,12 @@ def test_ragged_windows_and_chunk_boundaries(built_lib):
     assert set(np.unique(per["status"][:, 0])) >= {1, 2, 5}   # scored, pos out of range, empty (all N)
 
 
-def test_long_contigs_and_wide_quality_alphabet(built_lib):
+@pytest.mark.parametrize("n_quals", [94, 63])
+def test_long_contigs_and_wide_quality_alphabet(built_lib, n_quals):
     """1-10 kb contigs (config 5): warp-cooperative path, windows far longer than one warp round,
-    94 distinct quality values (7-bit codes, the largest score table)."""
+    94 distinct quality values (7-bit codes, the largest score table) or 63 including Phred 0 and 93 (the most the
+    packed layout holds: every code bit in use)."""
+    qset = np.arange(94) if n_quals == 94 else np.array([0, 93] + list(range(2, 63)))
     rng = np.random.RandomState(9)
     genome = rng.randint(0, 4, size=30000)
     singles = []
@@ -193,7 +196,7 @@ def test_long_contigs_and_wide_quality_alphabet(built_lib):
         mut = rng.random_sample(L) < (0.0 if k % 3 else 0.004)
         seg[mut] = (seg[mut] + 1) % 4
         s = "".join("ACGT"[x] for x in seg)
-        qv = rng.randint(0, 94, size=L)
+        qv = qset[rng.randint(0, len(qset), size=L)]
         singles.append((k, s, "".join(chr(33 + x) for x in qv)))
         segs.append((st, st + L))
     rs = F.ReadSet.from_lists(singles, [])
@@ -205,7 +208,7 @@ def test_long_contigs_and_wide_quality_alphabet(built_lib):
                 cs.append(_mk_cand(a, b, segs[b][0] - segs[a][0] + 1))
     c = np.concatenate(cs)
     with capi.Store(rs) as st:
-        assert st.quality_alphabet == 94
+        assert st.quality_alphabet == n_quals
         per, ref, stats = _against_oracle(rs, F.make_params(edge_threshold=0.995, min_read_len=100), c, store=st)
     assert int(O.window_lengths(ref).max()) > 4096
     assert not per["indel_count"].any()            # the path compares gaplessly: no indels (SURVEY 8a)
