@@ -46,13 +46,11 @@ struct DevCtx {
     int sm_count = 0;
     size_t smem_per_sm = 0;
     // store planes
-    uint8_t* pk = nullptr;       // packed layout (code | base << 6): pk_alloc + HC_PLANE_GUARD (zero bytes in front), or
-    uint8_t* pk_alloc = nullptr;
+    uint8_t* pk = nullptr;       // packed layout (code | base << 6), or
     uint8_t* qual = nullptr;     // planar layout: quality codes, 2-bit bases, N mask
     uint32_t* base2 = nullptr;
     uint32_t* nmask = nullptr;
     hc_rdesc* rdesc = nullptr;
-    hc_nlist* nlist = nullptr;   // packed layout: N positions per read
     // tables
     uint32_t* fx_table = nullptr;
     double* dbl_table = nullptr;
@@ -97,7 +95,7 @@ struct DevCtx {
     cudaStream_t stream = nullptr, s_copy = nullptr, s_out = nullptr;
     cudaEvent_t ev_in[2] = {nullptr, nullptr}, ev_done[2] = {nullptr, nullptr}, ev_out[2] = {nullptr, nullptr};
     cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    hc_launch_cfg cfg{}, cfg_walk{};
+    hc_launch_cfg cfg{};
 };
 
 }  // namespace
@@ -125,7 +123,7 @@ namespace {
 void free_ctx(DevCtx& d) {
     if (d.device < 0) return;
     cudaSetDevice(d.device);
-    cudaFree(d.pk_alloc); cudaFree(d.qual); cudaFree(d.base2); cudaFree(d.nmask); cudaFree(d.rdesc); cudaFree(d.nlist);
+    cudaFree(d.pk); cudaFree(d.qual); cudaFree(d.base2); cudaFree(d.nmask); cudaFree(d.rdesc);
     cudaFree(d.fx_table); cudaFree(d.dbl_table);
     cudaFree(d.tmp); cudaFree(d.cls); cudaFree(d.flagged); cudaFree(d.blockcounts); cudaFree(d.counters);
     for (int k = 0; k < 2; k++) {
@@ -163,11 +161,9 @@ int ensure_tables(hc_store* s, DevCtx& d, double mismatch, cudaStream_t st) {
     // synchronous upload: tables change only when ps.mismatch changes (it never does in the drivers)
     CU(cudaStreamSynchronize(st));
     const std::vector<uint32_t>& fx = s->packed ? s->tables.fx_packed : s->tables.fx;
-    const std::vector<uint32_t>& fa = s->tables.fx_anchor;          // packed layout: the anchor-walk table follows
-    if (!d.fx_table) CU(cudaMalloc(&d.fx_table, (fx.size() + (s->packed ? fa.size() : 0)) * sizeof(uint32_t)));
+    if (!d.fx_table) CU(cudaMalloc(&d.fx_table, fx.size() * sizeof(uint32_t)));
     if (!d.dbl_table) CU(cudaMalloc(&d.dbl_table, s->tables.dbl.size() * sizeof(double)));
     CU(cudaMemcpy(d.fx_table, fx.data(), fx.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
-    if (s->packed) CU(cudaMemcpy(d.fx_table + fx.size(), fa.data(), fa.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
     CU(cudaMemcpy(d.dbl_table, s->tables.dbl.data(), s->tables.dbl.size() * sizeof(double), cudaMemcpyHostToDevice));
     d.tables_valid = true;
     d.tables_mismatch = mismatch;
@@ -219,7 +215,7 @@ int enqueue_batch(hc_store* s, DevCtx& d, cudaStream_t st, const hc_params* p, c
     hc_kparams P;
     memset(&P, 0, sizeof(P));
     P.qual = d.qual; P.base2 = d.base2; P.nmask = d.nmask; P.rdesc = d.rdesc;
-    P.pk = d.pk; P.packed = s->packed ? 1u : 0u; P.nlist = d.nlist;
+    P.pk = d.pk; P.packed = s->packed ? 1u : 0u;
     P.n_reads = (uint32_t)s->n_reads; P.n_single = (uint32_t)s->n_single;
     P.fx_table = d.fx_table; P.dbl_table = d.dbl_table; P.ncodes = (uint32_t)s->ncodes; P.has_void = d.has_void ? 1u : 0u;
     P.cand = d_cand; P.cand_compact = (uint32_t)compact; P.run = d_run; P.n = n; P.tmp = d.tmp; P.cls = d.cls; P.per_cand = d_per_cand; P.flagged = d.flagged;
@@ -242,20 +238,12 @@ int enqueue_batch(hc_store* s, DevCtx& d, cudaStream_t st, const hc_params* p, c
     P.zero_above_edge = 0.0 > p->edge_threshold;
     P.zero_above_ov = 0.0 > p->ov_threshold;
     P.exact_edges = (p->flags & HC_FLAG_EXACT_EDGE_SCORES) ? 1u : 0u;
-    // Anchor walk (hc_kernels.cu): an alternative schedule for lists with runs, packed layout only.  Measured on config 4
-    // it removes the bank conflicts of the table lookups but does not beat the lane-chunk rounds (per-tile set-up cost,
-    // DESIGN.md section 6), so it is opt-in: HC_ANCHOR_WALK=1 (tests, experiments); a walk is started for tiles in which
-    // at least HC_ANCHOR_WALK_MIN lanes (default 12) take part.
-    uint32_t walk_min = 12;
-    if (const char* e = getenv("HC_ANCHOR_WALK_MIN")) walk_min = (uint32_t)std::max(1l, std::min(32l, strtol(e, nullptr, 10)));
-    const char* walk_env = getenv("HC_ANCHOR_WALK");
-    P.anchor_walk = (s->packed && walk_env && atoi(walk_env) != 0) ? walk_min : 0u;
     P.void_exact = d.void_exact ? 1u : 0u;
     CU(cudaMemsetAsync(d.counters, 0, HC_CNT_N * sizeof(unsigned long long), st));
     if (k0) CU(cudaEventRecord(k0, st));
     uint32_t nl = 0;
     if (n > 0) {
-        hc_launch_cfg cfg = P.anchor_walk ? d.cfg_walk : d.cfg;
+        hc_launch_cfg cfg = d.cfg;
         const uint64_t ntiles = (n + 31) / 32;
         const uint64_t warps_per_block = cfg.threads / 32;
         const uint64_t need_blocks = (ntiles + warps_per_block - 1) / warps_per_block;
@@ -413,19 +401,9 @@ cudaError_t init_ctx(hc_store* s, DevCtx& d, int device, bool* not_sm100) {
 
 cudaError_t alloc_planes(hc_store* s, DevCtx& d, cudaStream_t st) {
     const uint64_t total = s->total_positions;
-    // The packed plane has HC_PLANE_GUARD zero bytes in front: the anchor walk of hc_score_kernel reads up to 32 bytes
-    // before a sequence (the zero padding of the slot before it; for the first slot, this guard).
-    cudaError_t e;
-    if (s->packed) {
-        e = cudaMalloc(&d.pk_alloc, total + 64 + HC_PLANE_GUARD);
-        if (e == cudaSuccess) d.pk = d.pk_alloc + HC_PLANE_GUARD;
-        if (e == cudaSuccess) e = cudaMemsetAsync(d.pk_alloc, 0, total + 64 + HC_PLANE_GUARD, st);
-    } else {
-        e = cudaMalloc(&d.qual, total + 64);
-        if (e == cudaSuccess) e = cudaMemsetAsync(d.qual, 0, total + 64, st);
-    }
-    if (e == cudaSuccess && s->packed) e = cudaMalloc(&d.nlist, s->n_reads * sizeof(hc_nlist));
-    if (e == cudaSuccess && s->packed) e = cudaMemsetAsync(d.nlist, 0xff, s->n_reads * sizeof(hc_nlist), st);
+    uint8_t** bytes = s->packed ? &d.pk : &d.qual;   // one byte per position in either layout
+    cudaError_t e = cudaMalloc(bytes, total + 64);
+    if (e == cudaSuccess) e = cudaMemsetAsync(*bytes, 0, total + 64, st);
     if (e == cudaSuccess && !s->packed) e = cudaMalloc(&d.base2, (total / 16 + 16) * 4);
     if (e == cudaSuccess && !s->packed) e = cudaMalloc(&d.nmask, (total / 32 + 16) * 4);
     if (e == cudaSuccess && !s->packed) e = cudaMemsetAsync(d.base2, 0, (total / 16 + 16) * 4, st);
@@ -471,8 +449,8 @@ int build_store(hc_store* s, std::vector<hc_rdesc>& rd, const uint8_t* d_text, c
         memset(lut, 0, sizeof(lut));
         s->ncodes = 0;
         s->code_to_q[0] = -1;
-        // quality codes ranked by frequency, the most frequent value first (ties: the smaller Phred value): the codes that
-        // share a shared-memory bank in the anchor-walk table, c and c + 32, are then the rare ones (hc_layout.h)
+        // quality codes ranked by frequency, the most frequent value first (ties: the smaller Phred value); this order
+        // decides which code each Phred value gets, and so the bytes of the stored planes
         std::vector<int> present;
         for (int c = 33; c <= 33 + 93; c++) if (h_flags[c]) present.push_back(c);
         std::stable_sort(present.begin(), present.end(), [&](int a, int b) { return h_flags[a] > h_flags[b]; });
@@ -488,7 +466,7 @@ int build_store(hc_store* s, std::vector<hc_rdesc>& rd, const uint8_t* d_text, c
         if (e == cudaSuccess) e = alloc_planes(s, d0, d0.stream);
         if (e == cudaSuccess)
             e = hc_pack_write_launch(d_text, d_src, d0.rdesc, n_reads, n_upper, d_lut, s->packed, s->packed ? d0.pk : d0.qual, d0.base2,
-                                     d0.nmask, d0.nlist, d0.stream);
+                                     d0.nmask, d0.stream);
         if (e == cudaSuccess) e = cudaStreamSynchronize(d0.stream);
     }
     cudaFree(d_flags);
@@ -498,8 +476,7 @@ int build_store(hc_store* s, std::vector<hc_rdesc>& rd, const uint8_t* d_text, c
     for (int k = 0; k < n_devices && e == cudaSuccess; k++) {
         DevCtx& d = s->devs[k];
         e = cudaSetDevice(d.device);
-        if (e == cudaSuccess) e = hc_score_occupancy((uint32_t)s->ncodes, 0, d.sm_count, d.smem_per_sm, &d.cfg);
-        if (e == cudaSuccess && s->packed) e = hc_score_occupancy((uint32_t)s->ncodes, 1, d.sm_count, d.smem_per_sm, &d.cfg_walk);
+        if (e == cudaSuccess) e = hc_score_occupancy((uint32_t)s->ncodes, d.sm_count, d.smem_per_sm, &d.cfg);
         if (k == 0 || e != cudaSuccess) continue;
         e = alloc_planes(s, d, d.stream);
         if (e == cudaSuccess) e = cudaStreamSynchronize(d.stream);
@@ -507,7 +484,6 @@ int build_store(hc_store* s, std::vector<hc_rdesc>& rd, const uint8_t* d_text, c
         if (e == cudaSuccess && !s->packed) e = cudaMemcpyPeer(d.base2, d.device, d0.base2, d0.device, total / 16 * 4);
         if (e == cudaSuccess && !s->packed) e = cudaMemcpyPeer(d.nmask, d.device, d0.nmask, d0.device, total / 32 * 4);
         if (e == cudaSuccess) e = cudaMemcpyPeer(d.rdesc, d.device, d0.rdesc, d0.device, n_reads * sizeof(hc_rdesc));
-        if (e == cudaSuccess && s->packed) e = cudaMemcpyPeer(d.nlist, d.device, d0.nlist, d0.device, n_reads * sizeof(hc_nlist));
     }
     if (e != cudaSuccess) return fail(e == cudaErrorMemoryAllocation ? HC_ERR_NOMEM : HC_ERR_CUDA, std::string("hc_store_create: ") + cudaGetErrorString(e));
     return HC_OK;

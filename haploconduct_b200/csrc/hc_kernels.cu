@@ -35,9 +35,7 @@ struct Win {
     uint32_t ypos16;  // position of B[0] / 16
     uint32_t L;       // window length (src/EdgeCalculator.cpp:88); 0 when not scored
     uint32_t status;  // HC_WIN_*
-    uint32_t hasN;    // bit 0: a read of the window contains N; bit 1: more than hc_nlist holds
-    uint32_t pos;     // start of the window in A (xpos = start of A's strand slot + pos)
-    uint32_t a_read;  // 1 / 2: the A side belongs to read 1 / read 2 of the candidate
+    uint32_t hasN;    // a read of the window contains N
 };
 
 struct CandSetup {
@@ -46,9 +44,8 @@ struct CandSetup {
     uint32_t err;
 };
 
-__device__ __forceinline__ hc_candidate load_candidate(const hc_kparams& P, u64 i, uint32_t* anchor_read = nullptr) {
+__device__ __forceinline__ hc_candidate load_candidate(const hc_kparams& P, u64 i) {
     hc_candidate c;
-    if (anchor_read) *anchor_read = 0u;   // 1 / 2: the run's shared read is ID1 / ID2 (run-encoded records only)
     if (P.cand_compact == 4u) {   // hc_candidate_entry6: 6 bytes (three 16-bit loads), run-encoded like hc_candidate_entry
         const uint16_t* hp = reinterpret_cast<const uint16_t*>(P.cand) + 3 * i;
         const uint32_t h0 = __ldg(hp), h1 = __ldg(hp + 1), h2 = __ldg(hp + 2);
@@ -57,7 +54,6 @@ __device__ __forceinline__ hc_candidate load_candidate(const hc_kparams& P, u64 
         while ((uint32_t)i >= __ldg(P.run_start + r + 1)) r++;
         const uint32_t anchor = __ldg(P.run_anchor + r), other = lo & 0x01ffffffu;
         const bool anchor_is_2 = ((lo >> 25) & 1u) != 0u;
-        if (anchor_read) *anchor_read = anchor_is_2 ? 2u : 1u;
         c.idx1 = anchor_is_2 ? other : anchor;
         c.idx2 = anchor_is_2 ? anchor : other;
         c.pos1 = (lo >> 30) | ((h2 & 0x7fu) << 2);         // bits 30-38
@@ -74,7 +70,6 @@ __device__ __forceinline__ hc_candidate load_candidate(const hc_kparams& P, u64 
         while ((uint32_t)i >= __ldg(P.run_start + r + 1)) r++;     // runs are rarely shorter than a tile
         const uint32_t anchor = __ldg(P.run_anchor + r), other = e.x & 0x7fffffffu;
         const bool anchor_is_2 = (e.x >> 31) != 0u;
-        if (anchor_read) *anchor_read = anchor_is_2 ? 2u : 1u;
         c.idx1 = anchor_is_2 ? other : anchor;
         c.idx2 = anchor_is_2 ? anchor : other;
         const uint32_t w = e.y;
@@ -122,7 +117,6 @@ __device__ __forceinline__ void make_window(const hc_kparams& P, uint32_t rawA, 
     w.xpos = 0;
     w.ypos16 = 0;
     w.hasN = 0;
-    w.pos = pos;
     if (pos >= lenA) { w.status = HC_WIN_POS_OOR; return; }
     if (lenA < P.min_read_len || lenB < P.min_read_len) { w.status = HC_WIN_SHORT; return; }
     const u64 sa = 16ull * slotA + (rcA ? hc_slot_size(lenA) : 0u);
@@ -131,7 +125,7 @@ __device__ __forceinline__ void make_window(const hc_kparams& P, uint32_t rawA, 
     w.ypos16 = (uint32_t)(sb >> 4);
     w.L = min(lenA - pos, lenB);
     w.status = HC_WIN_SCORED;
-    w.hasN = (((rawA | rawB) & HC_HASN_BIT) ? 1u : 0u) | (((rawA | rawB) & HC_MANYN_BIT) ? 2u : 0u);   // bit 1: not in hc_nlist
+    w.hasN = ((rawA | rawB) & HC_HASN_BIT) ? 1u : 0u;
 }
 
 // Window selection of EdgeCalculator::compute_overlap, src/EdgeCalculator.cpp:199-351, written
@@ -151,7 +145,6 @@ __device__ __forceinline__ void setup_windows(const hc_kparams& P, const hc_cand
     s.two = (p1 | p2) ? 1u : 0u;
     s.err = 0;
     s.w[1].L = 0; s.w[1].xpos = 0; s.w[1].ypos16 = 0; s.w[1].hasN = 0; s.w[1].status = HC_WIN_UNUSED;
-    s.w[1].pos = 0; s.w[0].a_read = 1u; s.w[1].a_read = 1u;
     if (p1 && p2) { if (c.ord != '1' && c.ord != '2') s.err = 1; }            // assert :369
     else if (P.n_single == 0) s.err = 1;                                        // :197, "Read types not recognized" :381
     make_window(P, f1 ? r1.w : r1.z, f1 ? r1.y : r1.x, rc1, f2 ? r2.w : r2.z, f2 ? r2.y : r2.x, rc2, c.pos1, s.w[0]);
@@ -161,7 +154,6 @@ __device__ __forceinline__ void setup_windows(const hc_kparams& P, const hc_cand
         const bool swapped = p1 && (!p2 || c.ord == '2');
         if (swapped) make_window(P, rb, sb, rc2, ra, sa, rc1, c.pos2, s.w[1]);
         else make_window(P, ra, sa, rc1, rb, sb, rc2, c.pos2, s.w[1]);
-        s.w[1].a_read = swapped ? 2u : 1u;
     }
     if (s.err) { s.w[0].L = s.w[1].L = 0; s.w[0].status = s.w[1].status = HC_WIN_UNUSED; }
 }
@@ -185,7 +177,6 @@ __device__ __forceinline__ bool load_and_setup(const hc_kparams& P, const hc_can
         s.err = 1; s.two = 0;
         s.w[0].L = s.w[1].L = 0; s.w[0].xpos = s.w[1].xpos = 0; s.w[0].ypos16 = s.w[1].ypos16 = 0;
         s.w[0].hasN = s.w[1].hasN = 0; s.w[0].status = s.w[1].status = HC_WIN_UNUSED;
-        s.w[0].pos = s.w[1].pos = 0; s.w[0].a_read = s.w[1].a_read = 1u;
         r1 = r2 = make_uint4(0, 0, 0, 0);
         return false;
     }
@@ -563,275 +554,20 @@ __device__ __noinline__ void write_per_cand(const hc_kparams& P, u64 i, double s
     P.per_cand[i] = r;
 }
 
-// ---- anchor walk (packed layout) ---------------------------------------------------------------------
-// An overlaps file lists the overlaps of one read one after the other, so the 32 candidates of a tile share a read --
-// the ANCHOR -- or a few of them.  The lanes (= candidates) then walk the anchor's sequence together, 32 positions per
-// step: every lane looks at the SAME anchor position at the same time, so all table lookups of one instruction fall into
-// one table row (row = anchor code) and distinct columns are distinct shared-memory banks -- no bank conflicts, where the
-// lane-chunk scheme below pays 2.9 wavefronts per lookup -- and what depends on the anchor only (row offsets, base bits)
-// is prepared once per tile in shared memory instead of once per lane and word.  Each lane streams its own other read
-// through registers (one 256-bit load per step, re-aligned to the anchor's coordinates).  The table is symmetric
-// (hc_tables.cpp), so it does not matter whether the anchor is the A or the B side of a window.
-// Windows the walk does not take (N in either read, more anchors in the tile than the staging area holds, long windows)
-// go through the lane-chunk rounds; sums are integers, so which path scored a window does not show in the result.
-#ifndef HC_AS_STAGE_WORDS
-#define HC_AS_STAGE_WORDS 256u     // staged anchor words per warp and window pass, 16 bytes each (the part[] area of the scratch)
-#endif
-#define HC_AS_MAXBLK 16u           // windows that end beyond 512 anchor positions are left to the lane-chunk rounds
-
-// staged entry of one anchor word (4 positions): .x/.y = table row offsets (bytes) of positions 0,2 / 1,3 in 16-bit halves,
-// .z = the word's base bits (0xc0 of every byte), .w = .z >> 8
-__device__ __forceinline__ uint4 as_stage_entry(uint32_t aw) {
-    uint4 e;
-    e.x = (aw & 0x003f003fu) << 10;
-    e.y = ((aw >> 8) & 0x003f003fu) << 10;
-    e.z = aw & 0xc0c0c0c0u;
-    e.w = e.z >> 8;
-    return e;
-}
-
-// (a ^ b) & c as one LOP3 the compiler does not take apart again
-__device__ __forceinline__ uint32_t xor_and(uint32_t a, uint32_t b, uint32_t c) {
-    uint32_t d;
-    asm("lop3.b32 %0, %1, %2, %3, 0x28;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
-    return d;
-}
-
-__device__ __forceinline__ uint32_t lds_byteoff(const unsigned char* base, uint32_t off) {
-    return *reinterpret_cast<const uint32_t*>(base + off);
-}
-
-// One step: the lane's other-read bytes under anchor positions [32k, 32k+32) are the 32 bytes at byte offset `off` of
-// S = {lo[8], hi[8]}.  Adds the fixed-point sum to acc and ORs the base-difference bits into mE (words 0,2,4,6) / mO.
-template <bool HAS_VOID>
-__device__ __forceinline__ void as_block(const unsigned char* __restrict__ TA, const uint4* __restrict__ stg, const uint32_t* lo,
-                                         const uint32_t* hi, uint32_t off, uint32_t& acc, uint32_t& orv, uint32_t& mE,
-                                         uint32_t& mO) {
-    const bool s4 = (off & 16u) != 0, s2 = (off & 8u) != 0, s1 = (off & 4u) != 0;
-    uint32_t V2[12], V1[10], V[9];
-#pragma unroll
-    for (int i = 0; i < 12; i++) {
-        const uint32_t a = i < 8 ? lo[i] : hi[i - 8];
-        const uint32_t b = i + 4 < 8 ? lo[i + 4] : hi[i - 4];
-        V2[i] = s4 ? b : a;
-    }
-#pragma unroll
-    for (int i = 0; i < 10; i++) V1[i] = s2 ? V2[i + 2] : V2[i];
-#pragma unroll
-    for (int i = 0; i < 9; i++) V[i] = s1 ? V1[i + 1] : V1[i];
-    const uint32_t sh = (off & 3u) * 8u;
-#pragma unroll
-    for (int j = 0; j < 8; j++) {
-        const uint32_t wo = __funnelshift_r(V[j], V[j + 1], sh);
-        const uint4 st = stg[j];
-        const uint32_t X = wo ^ st.z;                               // code of the other read | base difference << 6, per byte
-        // byte offsets into the anchor rows: (X & 0x00ff00ff) * 4 + row offsets, positions 0,2 / 1,3 -- one LOP3 + one LEA each
-        const uint32_t E2 = xor_and(wo, st.z, 0x00ff00ffu) * 4u + st.x;
-        const uint32_t O2 = xor_and(wo >> 8, st.w, 0x00ff00ffu) * 4u + st.y;
-        const uint32_t t0 = lds_byteoff(TA, E2 & 0xffffu);
-        const uint32_t t1 = lds_byteoff(TA, O2 & 0xffffu);
-        const uint32_t t2 = lds_byteoff(TA, E2 >> 16);
-        const uint32_t t3 = lds_byteoff(TA, O2 >> 16);
-        acc += (t0 + t1) + (t2 + t3);
-        if (HAS_VOID) orv |= (t0 | t1) | (t2 | t3);
-        if (j & 1) mO |= (X >> (j - 1)) & (0xc0c0c0c0u >> (j - 1));
-        else mE |= (X >> j) & (0xc0c0c0c0u >> j);
-    }
-}
-
-// Mask of the positions < n of a step in the bit order as_block leaves the mismatch flags in: position p = 4j + t sits on
-// bit 8t + 7 - j of the even-word flags (j even) resp. bit 8t + 8 - j of the odd-word flags.
-HC_HD uint2 hc_as_vmask(uint32_t n) {
-    uint2 m;
-    m.x = 0; m.y = 0;
-    for (uint32_t p = 0; p < n && p < 32u; p++) {
-        const uint32_t j = p >> 2, t = p & 3u;
-        if (j & 1u) m.y |= 1u << (8u * t + 8u - j);
-        else m.x |= 1u << (8u * t + 7u - j);
-    }
-    return m;
-}
-
-// One window of one lane in the anchor's coordinates.
-struct AsWin {
-    u64 akey;        // store position of the first base of the anchor's sequence (strand slot): equal for lanes that share it
-    long long o0;    // store position of the other read's byte that lies under anchor position 0 (other index = anchor index - delta,
-                     // delta = +pos if the anchor is the window's A side, -pos if it is the B side)
-    uint32_t jb, je; // the window [jb, je) in anchor coordinates
-    bool elig;       // scored window the walk may take (no more N than hc_nlist holds, not beyond HC_AS_MAXBLK blocks)
-};
-
-__device__ __forceinline__ AsWin as_win_of(const Win& W, uint32_t anch, bool lane_ok) {
-    AsWin a;
-    const bool a_side = W.a_read == anch;
-    const u64 sa = W.xpos - W.pos, sb = 16ull * W.ypos16;
-    a.akey = a_side ? sa : sb;
-    a.o0 = a_side ? (long long)sb - (long long)W.pos : (long long)W.xpos;
-    a.jb = a_side ? W.pos : 0u;
-    a.je = a.jb + W.L;
-    a.elig = lane_ok && W.status == HC_WIN_SCORED && W.L > 0u && !(W.hasN & 2u) && a.je <= 32u * HC_AS_MAXBLK;
-    return a;
-}
-
-// Groups of lanes with the same anchor sequence, in lane order; every group's anchor words are staged behind the
-// `running` entries already there while the staging area lasts (lanes of groups that do not fit stay with the lane-chunk
-// rounds).  Returns whether the walk takes this lane's window; goff = where its group is staged.
-__device__ __forceinline__ bool as_stage(const hc_kparams& P, uint4* stg, int lane, const AsWin& w, uint32_t& running, uint32_t& goff) {
-    const uint32_t FULL = 0xffffffffu;
-    const uint32_t nblk = w.elig ? ((w.je + 31u) >> 5) : 0u;
-    uint32_t rem = __ballot_sync(FULL, w.elig);
-    bool handled = false;
-    goff = 0;
-    for (int groups = 0; rem != 0u && groups < 6 && running + 8u <= HC_AS_STAGE_WORDS; groups++) {
-        const int L = __ffs(rem) - 1;
-        const uint32_t klo = __shfl_sync(FULL, (uint32_t)w.akey, L), khi = __shfl_sync(FULL, (uint32_t)(w.akey >> 32), L);
-        const u64 gkey = ((u64)khi << 32) | klo;
-        const bool member = w.elig && w.akey == gkey;
-        rem &= ~__ballot_sync(FULL, member);
-        uint32_t gblk = member ? nblk : 0u;
-#pragma unroll
-        for (int d = 16; d > 0; d >>= 1) gblk = max(gblk, __shfl_xor_sync(FULL, gblk, d));
-        const uint32_t words = gblk * 8u;
-        if (running + words > HC_AS_STAGE_WORDS) continue;
-        if (member) { handled = true; goff = running; }
-        const uint32_t* ap = reinterpret_cast<const uint32_t*>(P.pk + gkey);
-        for (uint32_t i = lane; i < words; i += 32) stg[running + i] = as_stage_entry(__ldg(ap + i));
-        running += words;
-    }
-    // a walk keeps the whole warp busy for as long as its longest window: not worth it for a few lanes
-    if ((uint32_t)__popc(__ballot_sync(FULL, handled)) < P.anchor_walk) handled = false;
-    return handled;
-}
-
-// The walk over one window of every lane that takes part (on).  Block b of the lane's other read = the 32 bytes at
-// ob + 32 b; step k scores anchor positions [32k, 32k+32) from blocks k and k+1 and requests block k+2.
-template <bool HAS_VOID>
-__device__ __forceinline__ void as_walk(const hc_kparams& P, const unsigned char* __restrict__ TA, const uint2* __restrict__ VMT,
-                                        const uint4* __restrict__ mystg, long long o0, uint32_t jb, uint32_t je, bool on, u64& S_out,
-                                        uint32_t& mm_out, uint32_t& vd_out) {
-    const uint32_t FULL = 0xffffffffu;
-    const int kb = on ? (int)(jb >> 5) : 0x7fffffff, ke = on ? (int)((je - 1u) >> 5) : -1;
-    int kmin = kb, kmax = ke;
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) {
-        kmin = min(kmin, __shfl_xor_sync(FULL, kmin, d));
-        kmax = max(kmax, __shfl_xor_sync(FULL, kmax, d));
-    }
-    const uint32_t off = (uint32_t)o0 & 31u;
-    // per lane, relative to step kmin: the steps in which it scores (act) and the blocks its window touches (ld); at most
-    // HC_AS_MAXBLK + 1 bits each
-    uint32_t act = 0, ld = 0;
-    if (on) {
-        const int bb = (int)((off + jb) >> 5), be = (int)((off + je - 1u) >> 5);
-        act = ((2u << (ke - kmin)) - 1u) & ~((1u << (kb - kmin)) - 1u);
-        ld = ((2u << (be - kmin)) - 1u) & ~((1u << (bb - kmin)) - 1u);
-    }
-    const uint8_t* bp = P.pk + (o0 - (long long)off) + 32ll * kmin;      // block kmin
-    const uint4* sp = mystg + 8 * kmin;
-    int sb = (int)jb - 32 * kmin, eb = (int)je - 32 * kmin;              // the window relative to the step's first position
-    uint32_t lo[8], hi[8], nx[8];
-#pragma unroll
-    for (int i = 0; i < 8; i++) { lo[i] = 0u; hi[i] = 0u; }
-    if (ld & 1u) ldg256(bp, lo);
-    if (ld & 2u) ldg256(bp + 32, hi);
-    ld >>= 2;
-    bp += 64;
-    u64 S = 0;
-    uint32_t mm = 0, vd = 0;
-#pragma unroll 1
-    for (int n = kmax - kmin + 1; n > 0; n--) {
-        // a block the window does not touch counts as zeros
-#pragma unroll
-        for (int i = 0; i < 8; i++) nx[i] = 0u;
-        if (ld & 1u) ldg256(bp, nx);
-        if (act & 1u) {
-            uint32_t acc = 0, orv = 0, mE = 0, mO = 0;
-            as_block<HAS_VOID>(TA, sp, lo, hi, off, acc, orv, mE, mO);
-            S += acc;
-            const uint2 vs = VMT[max(sb, 0)], ve = VMT[min(eb, 32)];
-            mE = (mE | (mE << 1)) & 0xaaaaaaaau & ve.x & ~vs.x;
-            mO = (mO | (mO << 1)) & 0xaaaaaaaau & ve.y & ~vs.y;
-            mm += __popc(mE) + __popc(mO);
-            if (HAS_VOID) vd |= (orv & HC_VOID_BIT) ? 1u : 0u;
-        }
-        act >>= 1; ld >>= 1;
-        bp += 32; sp += 8;
-        sb -= 32; eb -= 32;
-#pragma unroll
-        for (int i = 0; i < 8; i++) { lo[i] = hi[i]; hi[i] = nx[i]; }
-    }
-    S_out = S; mm_out = mm; vd_out = vd;
-}
-
-// N positions of a window the anchor walk scores without looking for them.  An N is a zero byte: it adds nothing to the
-// sum, but it is not a compared position (:35-39,:122-124) and the walk flags it as a mismatch iff the base across it is
-// not 'A' (base bits 0).  The window is A[pos..pos+L) over B[0..L); sides as in setup_windows.  Returns
-// (number of N positions in the window) | (wrongly flagged mismatches) << 16.  Called while the tile is set up, so that the
-// few loads it needs are long back when the walk ends.
-__device__ __forceinline__ uint32_t as_n_counts(const hc_kparams& P, const hc_candidate& c, const uint4& r1, const uint4& r2, int w,
-                                                const Win& W) {
-    const int p1 = (r1.w & HC_LEN_MASK) != 0, p2 = (r2.w & HC_LEN_MASK) != 0;
-    const int rc1 = c.ori1 ? 0 : 1, rc2 = c.ori2 ? 0 : 1;
-    const int m1 = w == 0 ? (p1 ? rc1 : 0) : (p1 ? 1 - rc1 : 0);      // mate slot of read 1 / read 2 this window uses
-    const int m2 = w == 0 ? (p2 ? rc2 : 0) : (p2 ? 1 - rc2 : 0);
-    const uint32_t l1 = (m1 ? r1.w : r1.z) & HC_LEN_MASK, l2 = (m2 ? r2.w : r2.z) & HC_LEN_MASK;
-    const bool a1 = W.a_read == 1u;
-    const uint32_t lenA = a1 ? l1 : l2, lenB = a1 ? l2 : l1;
-    const int rcA = a1 ? rc1 : rc2, rcB = a1 ? rc2 : rc1;
-    const uint2 qA = __ldg(reinterpret_cast<const uint2*>(P.nlist + (a1 ? c.idx1 : c.idx2)));
-    const uint2 qB = __ldg(reinterpret_cast<const uint2*>(P.nlist + (a1 ? c.idx2 : c.idx1)));
-    const uint32_t nA = (a1 ? m1 : m2) ? qA.y : qA.x, nB = (a1 ? m2 : m1) ? qB.y : qB.x;     // two 16-bit positions of the mate used
-    const u64 sa = W.xpos - W.pos, sb = 16ull * W.ypos16;
-    const uint32_t pos = W.pos, L = W.L;
-    uint32_t nn = 0, fix = 0;
-#pragma unroll
-    for (int k = 0; k < 2; k++) {
-        const uint32_t pf = (nA >> (16 * k)) & 0xffffu;
-        if (pf == 0xffffu) continue;
-        const uint32_t a = rcA ? lenA - 1u - pf : pf;
-        if (a < pos || a - pos >= L) continue;
-        nn++;
-        const uint32_t other = P.pk[sb + (a - pos)];
-        if ((other & 0x3fu) != 0u && (other >> 6) != 0u) fix++;
-    }
-#pragma unroll
-    for (int k = 0; k < 2; k++) {
-        const uint32_t pf = (nB >> (16 * k)) & 0xffffu;
-        if (pf == 0xffffu) continue;
-        const uint32_t b = rcB ? lenB - 1u - pf : pf;
-        if (b >= L) continue;
-        const uint32_t other = P.pk[sa + pos + b];
-        if ((other & 0x3fu) == 0u) continue;                            // N on both sides: counted above
-        nn++;
-        if ((other >> 6) != 0u) fix++;
-    }
-    return nn | (fix << 16);
-}
-
-// WALK: the instantiation with the anchor walk in front of the lane-chunk rounds (one CTA of HC_WALK_WARPS warps per SM, it
-// keeps a second table in shared memory); without it two CTAs of HC_WARPS_MAX warps.
-template <bool HAS_VOID, bool PACKED, bool WALK>
-__global__ void __launch_bounds__((WALK ? HC_WALK_WARPS : HC_WARPS_MAX) * 32, WALK ? 1 : HC_MIN_CTAS) hc_score_kernel(const hc_kparams P) {
+template <bool HAS_VOID, bool PACKED>
+__global__ void __launch_bounds__(HC_WARPS_MAX * 32, HC_MIN_CTAS) hc_score_kernel(const hc_kparams P) {
     extern __shared__ __align__(16) unsigned char smem[];
     uint32_t* T = reinterpret_cast<uint32_t*>(smem);
-    const uint32_t ntab = (P.ncodes + 1u) * 256u;                     // score table, then the tail masks,
+    const uint32_t ntab = (P.ncodes + 1u) * 256u;                     // score table, then the tail masks, then per-warp scratch
     uint32_t* VM = T + ntab;
-    uint32_t* TAw = VM + HC_VM_WORDS;                                  // then (packed layout) the anchor-walk table and its masks
-    uint2* VMT = reinterpret_cast<uint2*>(TAw + (WALK ? ntab : 0u));
-    const uint32_t tbl_entries = ntab + HC_VM_WORDS + (WALK ? ntab + HC_AS_VMT_WORDS : 0u);
     for (uint32_t i = threadIdx.x; i < ntab; i += blockDim.x) T[i] = P.fx_table[i];
     if (threadIdx.x < HC_VM_WORDS) VM[threadIdx.x] = hc_packed_vmask(threadIdx.x);
-    if (WALK) {
-        for (uint32_t i = threadIdx.x; i < ntab; i += blockDim.x) TAw[i] = P.fx_table[ntab + i];
-        if (threadIdx.x < 33u) VMT[threadIdx.x] = hc_as_vmask(threadIdx.x);
-    }
     __syncthreads();
-    const unsigned char* TA = reinterpret_cast<const unsigned char*>(TAw);
 
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
     const int nwarps = blockDim.x >> 5;
-    unsigned char* scratch = smem + (size_t)tbl_entries * 4u + (size_t)warp * HC_WARP_SCRATCH;
+    unsigned char* scratch = smem + (size_t)(ntab + HC_VM_WORDS) * 4u + (size_t)warp * HC_WARP_SCRATCH;
     uint2* part = reinterpret_cast<uint2*>(scratch);                                     // [HC_PARTMAX]
     uint4* wdA = reinterpret_cast<uint4*>(scratch + HC_PARTMAX * 8u);                    // [64] xpos lo/hi, ypos16, L
     uint2* wdB = reinterpret_cast<uint2*>(scratch + HC_PARTMAX * 8u + HC_WINSLOTS * 16u); // [64] start chunk, hasN
@@ -848,77 +584,21 @@ __global__ void __launch_bounds__((WALK ? HC_WALK_WARPS : HC_WARPS_MAX) * 32, WA
         const u64 i = (tile << 5) + lane;
         const bool valid = i < P.n;
         CandSetup s;
-        hc_candidate c;
-        uint4 r1, r2;
         s.err = 0; s.two = 0;
         s.w[0].L = s.w[1].L = 0; s.w[0].status = s.w[1].status = HC_WIN_UNUSED;
         s.w[0].xpos = s.w[1].xpos = 0; s.w[0].ypos16 = s.w[1].ypos16 = 0; s.w[0].hasN = s.w[1].hasN = 0;
-        s.w[0].pos = s.w[1].pos = 0; s.w[0].a_read = s.w[1].a_read = 1u;
-        uint32_t anch = 0, nfix0 = 0, nfix1 = 0;
         if (valid) {
-            c = load_candidate(P, i, &anch);
+            const hc_candidate c = load_candidate(P, i);
+            uint4 r1, r2;
             load_and_setup(P, c, s, r1, r2);
 #ifndef HC_NO_PREFETCH
-#ifdef HC_PREFETCH_LIGHT
-            if (WALK && P.anchor_walk) {   // the walk requests its blocks a step ahead itself: only what it needs first
-                if (s.w[0].L) { prefetch_l2(P.pk + (s.w[0].xpos & ~127ull)); prefetch_l2(P.pk + 16ull * s.w[0].ypos16); }
-                if (s.w[1].L) { prefetch_l2(P.pk + (s.w[1].xpos & ~127ull)); prefetch_l2(P.pk + 16ull * s.w[1].ypos16); }
-            } else
+            prefetch_window(P, s.w[0]);
+            prefetch_window(P, s.w[1]);
 #endif
-            {
-                prefetch_window(P, s.w[0]);
-                prefetch_window(P, s.w[1]);
-            }
-#endif
-            if (WALK && P.anchor_walk && !s.err) {   // N counts of windows the walk may take (rare: a read with one or two N)
-                if (s.w[0].hasN == 1u && s.w[0].L) nfix0 = as_n_counts(P, c, r1, r2, 0, s.w[0]);
-                if (s.w[1].hasN == 1u && s.w[1].L) nfix1 = as_n_counts(P, c, r1, r2, 1, s.w[1]);
-            }
         }
         WinAcc acc[2];
         acc[0].S = acc[1].S = 0; acc[0].mm = acc[1].mm = 0; acc[0].nn = acc[1].nn = 0; acc[0].vd = acc[1].vd = 0;
-        uint32_t c0 = (s.w[0].L + 31u) >> 5, c1 = (s.w[1].L + 31u) >> 5;     // lane-chunks left to the rounds below
-
-        // ---- anchor walk: windows of candidates that share a read with their neighbours (packed layout)
-        if (WALK && P.anchor_walk) {
-            const uint32_t id1 = valid ? c.idx1 : 0xffffffffu, id2 = valid ? c.idx2 : 0xfffffffeu;
-            const uint32_t p1 = __shfl_up_sync(0xffffffffu, id1, 1), p2 = __shfl_up_sync(0xffffffffu, id2, 1);
-            const uint32_t n1 = __shfl_down_sync(0xffffffffu, id1, 1), n2 = __shfl_down_sync(0xffffffffu, id2, 1);
-            const int up = lane > 0, dn = lane < 31;
-            const int sc1 = (up && (id1 == p1 || id1 == p2)) + (dn && (id1 == n1 || id1 == n2));
-            const int sc2 = (up && (id2 == p1 || id2 == p2)) + (dn && (id2 == n1 || id2 == n2));
-            // records without run information: the anchor is the read shared with the neighbouring candidates, else the smaller index
-            if (P.cand_compact < 3u) anch = sc1 > sc2 ? 1u : (sc2 > sc1 ? 2u : (id1 <= id2 ? 1u : 2u));
-            const bool lane_ok = valid && !s.err;
-            // lists without runs: do not even start (the lanes of a group are neighbours in a list sorted by read)
-            if ((uint32_t)__popc(__ballot_sync(0xffffffffu, lane_ok && (sc1 | sc2))) + 1u >= P.anchor_walk) {
-                uint4* stg = reinterpret_cast<uint4*>(scratch);
-                uint32_t running = 0, goff0, goff1;
-                const AsWin a0 = as_win_of(s.w[0], anch, lane_ok), a1 = as_win_of(s.w[1], anch, lane_ok);
-                const bool on0 = as_stage(P, stg, lane, a0, running, goff0);
-                const bool on1 = as_stage(P, stg, lane, a1, running, goff1);
-                // what the walks need: 4 registers per window
-                const long long o00 = a0.o0, o01 = a1.o0;
-                const uint32_t jj0 = a0.jb | (a0.je << 16), jj1 = a1.jb | (a1.je << 16);
-                __syncwarp();
-#pragma unroll 1
-                for (int w = 0; w < 2; w++) {
-                    const bool on = w ? on1 : on0;
-                    if (!__any_sync(0xffffffffu, on)) continue;
-                    const uint32_t jj = w ? jj1 : jj0;
-                    u64 S;
-                    uint32_t mm, vd;
-                    as_walk<HAS_VOID>(P, TA, VMT, stg + (w ? goff1 : goff0), w ? o01 : o00, jj & 0xffffu, jj >> 16, on, S, mm, vd);
-                    if (on) {
-                        const uint32_t nf = w ? nfix1 : nfix0;
-                        WinAcc r;
-                        r.S = S; r.mm = mm - (nf >> 16); r.nn = nf & 0xffffu; r.vd = vd;
-                        if (w) { acc[1] = r; c1 = 0u; } else { acc[0] = r; c0 = 0u; }
-                    }
-                }
-                __syncwarp();
-            }
-        }
+        const uint32_t c0 = (s.w[0].L + 31u) >> 5, c1 = (s.w[1].L + 31u) >> 5;     // lane-chunks per window
         const uint32_t ct = c0 + c1;
 
         // ---- big candidates (>= 64 lane-chunks): the whole warp walks one window at a time
@@ -1643,12 +1323,11 @@ static unsigned hc_grid_cap() {
     return (unsigned)sms[dev] * 8u;
 }
 
-cudaError_t hc_score_occupancy(uint32_t ncodes, int walk, int sm_count, size_t smem_per_sm, hc_launch_cfg* cfg) {
-    // score table + tail masks (+ the anchor-walk table and its masks), per CTA
-    const size_t table = (size_t)(ncodes + 1u) * 1024u * (walk ? 2u : 1u) + HC_VM_WORDS * 4u + (walk ? HC_AS_VMT_WORDS * 4u : 0u);
-    const int max_ctas = walk ? 1 : HC_MIN_CTAS;                                 // what the register allocation allows
+cudaError_t hc_score_occupancy(uint32_t ncodes, int sm_count, size_t smem_per_sm, hc_launch_cfg* cfg) {
+    const size_t table = (size_t)(ncodes + 1u) * 1024u + HC_VM_WORDS * 4u;    // score table + tail masks, per CTA
+    const int max_ctas = HC_MIN_CTAS;                                            // what the register allocation allows
     int best_warps = 0, best_nw = 0, best_ctas = 0;
-    for (int nw = walk ? HC_WALK_WARPS : HC_WARPS_MAX; nw >= 4; nw -= 4) {       // the tables are per CTA: prefer large CTAs
+    for (int nw = HC_WARPS_MAX; nw >= 4; nw -= 4) {                              // the table is per CTA: prefer large CTAs
         const size_t per_cta = table + (size_t)nw * HC_WARP_SCRATCH + 1024u;   // +1 KB the driver reserves per CTA
         if (per_cta > 227u * 1024u) continue;
         int ctas = (int)(smem_per_sm / per_cta);
@@ -1666,9 +1345,8 @@ cudaError_t hc_score_occupancy(uint32_t ncodes, int walk, int sm_count, size_t s
 
 cudaError_t hc_launch_score(const hc_kparams& P, const hc_launch_cfg& cfg, cudaStream_t st) {
     void (*fn)(const hc_kparams);
-    if (P.packed && P.anchor_walk) fn = P.has_void ? hc_score_kernel<true, true, true> : hc_score_kernel<false, true, true>;
-    else if (P.packed) fn = P.has_void ? hc_score_kernel<true, true, false> : hc_score_kernel<false, true, false>;
-    else fn = P.has_void ? hc_score_kernel<true, false, false> : hc_score_kernel<false, false, false>;
+    if (P.packed) fn = P.has_void ? hc_score_kernel<true, true> : hc_score_kernel<false, true>;
+    else fn = P.has_void ? hc_score_kernel<true, false> : hc_score_kernel<false, false>;
     cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cfg.smem);
     if (e != cudaSuccess) return e;
     fn<<<cfg.blocks, cfg.threads, cfg.smem, st>>>(P);

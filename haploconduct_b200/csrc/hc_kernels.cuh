@@ -13,9 +13,6 @@
 #ifndef HC_MIN_CTAS
 #define HC_MIN_CTAS 2             // ... and resident CTAs per SM the register allocation aims at
 #endif
-#ifndef HC_WALK_WARPS
-#define HC_WALK_WARPS 20         // anchor-walk instantiation: one CTA per SM (two tables in shared memory), 96 registers per thread
-#endif
 #define HC_LANE_CHUNK 32u        // positions one lane handles per step (two 16-position halves)
 #ifndef HC_PARTMAX
 #define HC_PARTMAX 512u
@@ -23,7 +20,6 @@
 //                            // lane-chunk partials per warp round (x 8 B = 4 KB of shared memory)
 #define HC_BIG_CHUNKS 64u        // candidates with >= this many lane-chunks are scored warp-cooperatively
 #define HC_WINSLOTS 64u          // 2 windows x 32 candidates
-#define HC_AS_VMT_WORDS 72u      // anchor walk: 33 x 2 words of position masks (hc_as_vmask), padded
 #define HC_VM_WORDS 64u          // tail-mask table of the packed layout (33 used), kept behind the score table
 // per-warp scratch: partials + window descriptors (16 B + 8 B per slot) + head bitmap
 #define HC_WARP_SCRATCH (HC_PARTMAX * 8u + HC_WINSLOTS * 16u + HC_WINSLOTS * 8u + (HC_PARTMAX / 32u) * 4u)
@@ -47,7 +43,6 @@ struct hc_kparams {
     const uint32_t* nmask;
     const uint8_t* pk;          // packed layout: code | base << 6 per position (qual/base2/nmask are NULL then)
     const hc_rdesc* rdesc;
-    const hc_nlist* nlist;      // packed layout
     uint32_t packed;
     uint32_t n_reads;
     uint32_t n_single;
@@ -82,8 +77,6 @@ struct hc_kparams {
     uint32_t never_edge;        // t_edge > 0: a mean (<= 0) can never reach it
     uint32_t never_ov;
     uint32_t exact_edges;       // HC_FLAG_EXACT_EDGE_SCORES
-    uint32_t anchor_walk;       // packed layout: candidates that share a read walk it together (fx_table holds both tables);
-                                // 0 = off, else the least number of lanes of a tile a walk is started for
     uint32_t void_exact;        // hc_tables::void_asymmetric: void hits are decided by the reference-order pass
 };
 
@@ -114,7 +107,7 @@ cudaError_t hc_launch_tile_runs(const uint32_t* run_start, uint32_t n_runs, uint
 cudaError_t hc_launch_compact(const hc_kparams& P, hc_edge* d_edges, uint64_t edges_cap, uint64_t* d_nonedge,
                               uint64_t nonedge_cap, uint32_t* d_blockcounts, uint64_t cand_offset, unsigned long long* d_run,
                               cudaStream_t st, int small_out = 0, uint32_t* d_bits = nullptr);
-cudaError_t hc_score_occupancy(uint32_t ncodes, int walk, int sm_count, size_t smem_per_sm, hc_launch_cfg* cfg);
+cudaError_t hc_score_occupancy(uint32_t ncodes, int sm_count, size_t smem_per_sm, hc_launch_cfg* cfg);
 uint32_t hc_compact_blocks(uint64_t n);
 
 #endif

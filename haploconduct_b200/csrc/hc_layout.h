@@ -26,7 +26,6 @@
 
 #define HC_SLOT_ALIGN 64u
 #define HC_SLOT_PAD 32u
-#define HC_PLANE_GUARD 128u      // zero bytes in front of the packed plane (a multiple of 128 keeps the plane's alignment)
 #define HC_CHUNK 16u            // positions per lane-chunk
 #define HC_MAX_CODES 127        // quality codes 1..127 (7 bits), 0 = null
 #define HC_FX_SHIFT 22          // fixed point: entry = round(-log(p) * 2^22)
@@ -37,7 +36,6 @@
 #define HC_LEN_MASK 0x3fffffffu  // sequence lengths are below 2^30
 #define HC_LEN_MAX 0x3fffffffu
 #define HC_HASN_BIT 0x80000000u  // the sequence contains an N
-#define HC_MANYN_BIT 0x40000000u // ... more than two of them (or it is too long for 16-bit positions): not in hc_nlist
 
 #if defined(__CUDACC__)
 #define HC_HD __host__ __device__ __forceinline__
@@ -47,14 +45,7 @@
 
 struct hc_rdesc {          // device read descriptor
     uint32_t slot16[2];    // forward-slot start / 16 for mate 0 / 1
-    uint32_t len[2];       // length | HC_HASN_BIT | HC_MANYN_BIT ; len[1] == 0 <=> single-end read
-};
-
-// Packed layout: where the (at most two) N of a sequence are, forward-strand positions, 0xffff = none.  The anchor walk
-// of hc_score_kernel scores windows without looking for N (an N is a zero byte: it adds nothing) and corrects the
-// compared-length and mismatch counts afterwards from this list.
-struct alignas(8) hc_nlist {
-    uint16_t pos[2][2];    // [mate][k]
+    uint32_t len[2];       // length | HC_HASN_BIT ; len[1] == 0 <=> single-end read
 };
 
 HC_HD uint32_t hc_slot_size(uint32_t len) {
@@ -85,12 +76,6 @@ HC_HD uint32_t hc_swz1_packed(uint32_t cb) { return ((cb << 1) & 0x3eu) | (cb & 
 #endif
 HC_HD uint32_t hc_fx_index_packed(uint32_t ca, uint32_t cb, uint32_t bx) {
     return (cb << 8) | ((ca ^ hc_swz1_packed(cb)) & 0x3fu) | (bx << 6);
-}
-// Anchor-walk table (hc_score_kernel, anchor-synchronous path): row = code of the read the lanes of a warp share, column =
-// code of the other read | base difference << 6.  All lanes of a warp read the same row, so distinct columns fall
-// into distinct banks (codes are ranked by frequency: the codes that share a bank, c and c + 32, are the rare ones).
-HC_HD uint32_t hc_fx_index_anchor(uint32_t c_anchor, uint32_t c_other, uint32_t bx) {
-    return (c_anchor << 8) | (c_other & 0x3fu) | (bx << 6);
 }
 // Mismatch flags of a 32-position lane-chunk are gathered as OR_j (flags(word j) >> j): position
 // p = 4j + t lands on bit 8t + 7 - j.  Mask of the first n positions in that bit order:

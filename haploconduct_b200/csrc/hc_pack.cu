@@ -26,7 +26,7 @@ __device__ __forceinline__ int dev_base_code(unsigned char c) {
 
 __device__ __forceinline__ unsigned char dev_upper(unsigned char c) { return (c >= 'a' && c <= 'z') ? (unsigned char)(c - 32) : c; }
 
-// hist[128]: how often every quality character occurs (quality codes are ranked by frequency, see hc_layout.h);
+// hist[128]: how often every quality character occurs (quality codes are ranked by frequency, see build_store in hc_api.cu);
 // err: 1 invalid nucleotide, 2 quality out of range
 __global__ void __launch_bounds__(256) pack_validate(const uint8_t* __restrict__ text, const hc_pack_src* __restrict__ src,
                                                      const hc_rdesc* __restrict__ rd, u64 n_reads, u64 n_upper,
@@ -62,7 +62,7 @@ __global__ void __launch_bounds__(256) pack_validate(const uint8_t* __restrict__
 template <bool PACKED>
 __global__ void __launch_bounds__(256) pack_write(const uint8_t* __restrict__ text, const hc_pack_src* __restrict__ src, hc_rdesc* rd,
                                                   u64 n_reads, u64 n_upper, const uint8_t* __restrict__ q2code, uint8_t* qplane,
-                                                  uint32_t* base2, uint32_t* nmask, hc_nlist* nlist) {
+                                                  uint32_t* base2, uint32_t* nmask) {
     __shared__ uint8_t lut[256];
     lut[threadIdx.x] = q2code[threadIdx.x];
     __syncthreads();
@@ -78,17 +78,10 @@ __global__ void __launch_bounds__(256) pack_write(const uint8_t* __restrict__ te
         const bool up = r < n_upper;
         const u64 fwd = 16ull * rd[r].slot16[m], rev = fwd + hc_slot_size(len);
         bool hasN = false;
-        uint32_t n_cnt = 0, n_pos[2] = {0xffffu, 0xffffu};      // warp-uniform: the first two N of the sequence
         for (uint32_t i0 = 0; i0 < len; i0 += 32) {
             const uint32_t i = i0 + lane;
-            const int bc = i < len ? dev_base_code(up ? dev_upper(b[i]) : b[i]) : -1;
-            uint32_t nm = __ballot_sync(0xffffffffu, bc == 4);
-            while (nm) {
-                if (n_cnt < 2) n_pos[n_cnt] = i0 + (uint32_t)__ffs(nm) - 1u;
-                n_cnt++;
-                nm &= nm - 1;
-            }
             if (i >= len) continue;
+            const int bc = dev_base_code(up ? dev_upper(b[i]) : b[i]);
             const u64 pf = fwd + i, pr = rev + (len - 1 - i);
             if (bc == 4) {
                 hasN = true;          // N: quality code 0 (contributes nothing), base bits 0, mask bit set
@@ -109,12 +102,7 @@ __global__ void __launch_bounds__(256) pack_write(const uint8_t* __restrict__ te
                 }
             }
         }
-        const bool many = n_cnt > 2 || len > 0xfff0u;
-        if (__any_sync(0xffffffffu, hasN) && lane == 0) rd[r].len[m] |= HC_HASN_BIT | (many ? HC_MANYN_BIT : 0u);
-        if (PACKED && lane == 0) {
-            nlist[r].pos[m][0] = (uint16_t)(many ? 0xffffu : n_pos[0]);
-            nlist[r].pos[m][1] = (uint16_t)(many ? 0xffffu : n_pos[1]);
-        }
+        if (__any_sync(0xffffffffu, hasN) && lane == 0) rd[r].len[m] |= HC_HASN_BIT;
     }
 }
 
@@ -172,11 +160,11 @@ cudaError_t hc_pack_validate_launch(const uint8_t* d_text, const hc_pack_src* d_
 
 cudaError_t hc_pack_write_launch(const uint8_t* d_text, const hc_pack_src* d_src, hc_rdesc* d_rd, uint64_t n_reads, uint64_t n_upper,
                                  const uint8_t* d_q2code, int packed, uint8_t* qplane, uint32_t* base2, uint32_t* nmask,
-                                 hc_nlist* nlist, cudaStream_t stream) {
+                                 cudaStream_t stream) {
     const u64 warps = 2 * n_reads;
     const unsigned blocks = (unsigned)std::min<u64>((warps + 7) / 8, 148ull * 32);
-    if (packed) pack_write<true><<<blocks ? blocks : 1, 256, 0, stream>>>(d_text, d_src, d_rd, n_reads, n_upper, d_q2code, qplane, base2, nmask, nlist);
-    else pack_write<false><<<blocks ? blocks : 1, 256, 0, stream>>>(d_text, d_src, d_rd, n_reads, n_upper, d_q2code, qplane, base2, nmask, nlist);
+    if (packed) pack_write<true><<<blocks ? blocks : 1, 256, 0, stream>>>(d_text, d_src, d_rd, n_reads, n_upper, d_q2code, qplane, base2, nmask);
+    else pack_write<false><<<blocks ? blocks : 1, 256, 0, stream>>>(d_text, d_src, d_rd, n_reads, n_upper, d_q2code, qplane, base2, nmask);
     return cudaGetLastError();
 }
 

@@ -35,7 +35,6 @@ void hc_build_tables(const int* code_to_q, int ncodes, double mismatch_param, hc
     out->fx.assign((size_t)n1 * 256, 0u);
     const bool packed = ncodes <= HC_PACKED_MAX_CODES;
     out->fx_packed.assign(packed ? (size_t)n1 * 256 : 0, 0u);
-    out->fx_anchor.assign(packed ? (size_t)n1 * 256 : 0, 0u);
     out->has_void = false;
     out->void_asymmetric = false;
     for (int ca = 1; ca <= ncodes; ca++) {
@@ -66,15 +65,8 @@ void hc_build_tables(const int* code_to_q, int ncodes, double mismatch_param, hc
                 out->dbl[hc_dbl_index(ca, cb, mm, n1)] = lp;
                 out->fx[hc_fx_index(ca, cb, mm)] = fx;
                 if (packed) {
-                    if (!mm) {
-                        out->fx_packed[hc_fx_index_packed(ca, cb, 0)] = fx;
-                        out->fx_anchor[hc_fx_index_anchor(ca, cb, 0)] = fx;
-                    } else {
-                        for (uint32_t bx = 1; bx < 4; bx++) {
-                            out->fx_packed[hc_fx_index_packed(ca, cb, bx)] = fx;
-                            out->fx_anchor[hc_fx_index_anchor(ca, cb, bx)] = fx;
-                        }
-                    }
+                    if (!mm) out->fx_packed[hc_fx_index_packed(ca, cb, 0)] = fx;
+                    else for (uint32_t bx = 1; bx < 4; bx++) out->fx_packed[hc_fx_index_packed(ca, cb, bx)] = fx;
                 }
             }
         }

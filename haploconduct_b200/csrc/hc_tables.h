@@ -11,8 +11,6 @@ struct hc_tables {
     std::vector<double> dbl;     // [(K+1)*(K+1)*2] log(p), exact reference addends (2.0 = void sentinel)
     std::vector<uint32_t> fx;    // [(K+1)*256] round(-log(p)*2^22), swizzled layout of hc_fx_index()
     std::vector<uint32_t> fx_packed;  // same values in the hc_fx_index_packed() layout (K <= 63 only, else empty)
-    std::vector<uint32_t> fx_anchor;  // same values, row = code of the anchor side, column = other code | base difference << 6
-                                      // (hc_fx_index_anchor(), no bank swizzle: a warp reads one row at a time)
     bool void_asymmetric;        // some (qa,qb) is void in one order only: void hits are decided by the reference-order pass
 };
 

@@ -6,7 +6,8 @@
 * void decided differently in the two orders of a quality pair (the reference-order pass decides);
 * the switch between the packed (<= 63 quality values) and the three-plane layout;
 * the 16-bit counts of the small edge records (HC_EDGE_OVERFLOW);
-* both modes of the reference-order pass and the anchor walk on long windows.
+* both modes of the reference-order pass on long windows;
+* the cases in the order of an overlaps file (sorted by read), as plain and as run-encoded records.
 
 Every read set is cut from a seeded random genome, so each window's length and content is known by construction.
 test_cases_hit_their_shapes (no GPU) checks from geometry and oracle output alone that every case still reaches the
@@ -25,7 +26,6 @@ from oracle import oracle as O
 from util import assert_results_match
 
 BIG_CHUNKS, PARTMAX = 64, 512          # HC_BIG_CHUNKS, HC_PARTMAX (hc_kernels.cuh)
-WALK_END = 16 * 32                     # HC_AS_MAXBLK * 32: the anchor walk takes windows that end at or before it
 FX_SCALE = 2.0 ** 22                   # HC_FX_SCALE
 # reference-order pass on a B200 (148 SMs): queued candidates below which every launch configuration of hc_exact_kernel
 # gives each one a warp, and above which every one gives each a thread
@@ -408,35 +408,6 @@ def case_exact_modes():
     return b.finish("exact_modes", [F.make_params(edge_threshold=0.9, ov_threshold=0.5, flags=F.FLAG_EXACT_EDGE_SCORES)])
 
 
-@functools.lru_cache(maxsize=None)
-def case_walk_ends():
-    """One anchor read of 700 bases and 48 partners whose windows end at anchor positions 511, 512 and 513 (the walk takes
-    windows that end at or before 512), with the anchor on the A and on the B side, on both strands, some with one or two
-    N (the walk corrects its counts for them) or three (left to the rounds)."""
-    b = _Builder(909, 10000)
-    s0 = 2000
-    X = b.cut(s0, 700)
-    qx = b.qual(700)
-    hx = b.single(X, qx)
-    for k in range(48):
-        end = (511, 512, 513)[k % 3]
-        rc = k % 4 >= 2
-        ns = ((), (), (7,), (7, 300), (1, 2, 3))[k % 5]
-        if k % 2 == 0:                                          # anchor = A side: the window is X[pos:end]
-            pos = int(b.rng.randint(0, 200))
-            B = b.cut(s0 + pos, end - pos, 0.003)
-            for p in ns:
-                B[p] = 4
-            b.cand(hx, b.single(B, b.qual(end - pos), rc), pos)
-        else:                                                   # anchor = B side: the window is X[0:end]
-            pos = int(b.rng.randint(1, 200))
-            A = b.cut(s0 - pos, pos + end, 0.003)
-            for p in ns:
-                A[pos + p] = 4
-            b.cand(b.single(A, b.qual(pos + end), rc), hx, pos)
-    return b.finish("walk_ends", [F.make_params(edge_threshold=0.98)])
-
-
 # ---- checks ------------------------------------------------------------------------------------------------
 _REF = {}
 
@@ -581,16 +552,18 @@ def test_reference_order_pass_modes_on_long_windows(built_lib):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("name", ["walk_ends"] + sorted(CORE))
-def test_anchor_walk_against_oracle(built_lib, monkeypatch, name):
-    """The opt-in anchor walk (packed layout; a no-op in the three-plane one) on lists sorted by read, started in every
-    tile (HC_ANCHOR_WALK_MIN=1), with the records with and without run information."""
-    case = case_walk_ends() if name == "walk_ends" else CORE[name]()
+@pytest.mark.parametrize("exact", [False, True])
+@pytest.mark.parametrize("name", sorted(CORE))
+def test_by_read_order_against_oracle(built_lib, name, exact):
+    """The cases sorted by read, as an overlaps file lists them, against the oracle, with the records with and without run
+    information; with exact, every accepted edge is also re-added in the reference's order."""
+    case = CORE[name]()
     order = _by_read(case.cands)
-    monkeypatch.setenv("HC_ANCHOR_WALK", "1")
-    monkeypatch.setenv("HC_ANCHOR_WALK_MIN", "1")
     with capi.Store(case.rs) as st:
         for p in case.params:
+            if exact:                  # set here so that the run-encoded call below scores under the same flags
+                p = p.copy()
+                p["flags"] |= F.FLAG_EXACT_EDGE_SCORES
             per, _, _ = _against(st, case, p, order=order)
             _, _, per_runs, _ = st.score_batch(p, case.cands[order], compact="runs")
             assert per_runs.tobytes() == per.tobytes()
@@ -675,8 +648,3 @@ def test_cases_hit_their_shapes():
     rh = _oracle(h, h.params[0])
     assert (rh["cls"] == 1).sum() > THREAD_MODE_MIN and 0 < (rh["cls"][:500] == 1).sum() < WARP_MODE_MAX - 100
     assert O.window_lengths(rh).max() > 2500
-    # i. windows that end at anchor positions 511, 512, 513, some with the anchor on the B side
-    w = case_walk_ends()
-    wl = _window_lengths(w.rs, w.cands)[:, 0]
-    ends = np.where(w.cands["idx1"] == 0, w.cands["pos1"] + wl, wl)
-    assert set(ends.tolist()) == {WALK_END - 1, WALK_END, WALK_END + 1} and (w.cands["idx2"] == 0).sum() == 24

@@ -1,7 +1,7 @@
 """GPU suite: the small-output entry points (hc_score_batch_runs_small / hc_score_batch_short_small) against the full
 outputs of hc_score_batch on the same candidates -- same accepted edges in the same order, the same non-edge set,
-scores / mean logs / counts bit for bit -- and the opt-in anchor walk of hc_score_kernel against the lane-chunk rounds
-(the two schedules add the same integers: every per-candidate field must be identical)."""
+scores / mean logs / counts bit for bit -- and, on lists sorted by read, the run-encoded records of hc_score_batch_runs
+against the plain hc_candidate records (every output must be byte-identical)."""
 import ctypes
 
 import numpy as np
@@ -72,21 +72,17 @@ def test_small_outputs_capacity_and_empty(built_lib):
 
 
 @pytest.mark.parametrize("seed", [11, 12, 13])
-@pytest.mark.parametrize("walk_min", ["1", "12"])
-def test_anchor_walk_equals_lane_chunk_rounds(built_lib, monkeypatch, seed, walk_min):
+@pytest.mark.parametrize("exact", [False, True])
+def test_run_records_equal_candidate_records(built_lib, seed, exact):
     rng = np.random.RandomState(seed)
     ss = W.synth_readset(int(rng.randint(20, 120)), int(rng.randint(20, 120)), genome_len=int(rng.randint(800, 4000)), read_len=(60, 400),
                          qmax=41, q_lo=int(rng.choice([2, 20])), seed=seed, n_rate=float(rng.choice([0.0, 0.002])), flip_fraction=0.3)
     c = W.geometry_candidates(ss, 6000, seed=seed + 1, junk_fraction=0.1, min_ov=20)
     c = c[(c["pos1"] < (1 << 14)) & (c["pos2"] < (1 << 14))]                                   # (junk candidates carry any position)
     c = c[np.lexsort((np.maximum(c["idx1"], c["idx2"]), np.minimum(c["idx1"], c["idx2"])))]     # sorted by read, like an overlaps file
-    p = F.make_params(edge_threshold=0.95, ov_threshold=0.9, mismatch=float(rng.choice([0.0, 0.05])))
+    p = F.make_params(edge_threshold=0.95, ov_threshold=0.9, mismatch=float(rng.choice([0.0, 0.05])),
+                      flags=F.FLAG_EXACT_EDGE_SCORES if exact else 0)
     with capi.Store(ss.rs) as st:
-        monkeypatch.delenv("HC_ANCHOR_WALK", raising=False)
         e0, n0, p0, _ = st.score_batch(p, c)
-        monkeypatch.setenv("HC_ANCHOR_WALK", "1")
-        monkeypatch.setenv("HC_ANCHOR_WALK_MIN", walk_min)
-        e1, n1, p1, _ = st.score_batch(p, c)
-        e2, n2, p2, _ = st.score_batch(p, c, compact="runs")
+        e1, n1, p1, _ = st.score_batch(p, c, compact="runs")
     assert p1.tobytes() == p0.tobytes() and e1.tobytes() == e0.tobytes() and np.array_equal(n1, n0)
-    assert p2.tobytes() == p0.tobytes() and e2.tobytes() == e0.tobytes() and np.array_equal(n2, n0)
