@@ -753,7 +753,8 @@ int hc_consensus(hc_store* s, const hc_cons_problem* problems, uint64_t n_proble
     if (e == cudaSuccess) {
         hc_cons_dev D;
         D.pk = d.pk; D.qual = d.qual; D.base2 = d.base2; D.nmask = d.nmask; D.rdesc = d.rdesc; D.packed = s->packed ? 1 : 0;
-        // (a NaN threshold never compares: with HC_CONS_HOST_ALL the min_qual closeness test is replaced by marking everything)
+        // (with HC_CONS_HOST_ALL the kernel gets a list of capacity 0: it still counts its marks but stores none, and the
+        // host decides every column from the sums, all_cols below)
         e = hc_launch_cons_sums(D, d_prob, n_problems, d_seqs, d_toff, n_tiles, d_add, d_c2q, min_qual, d_sums, d_cnt, d_base, d_qual,
                                 d_marked, mark_all ? 0 : marked_cap, d_nmarked, d.stream);
         if (e == cudaSuccess && n_seqs) {
