@@ -24,6 +24,7 @@ EXPORTED = [
     "hc_overlap_score", "hc_overlap_score_multi",
     "hc_phred_to_prob", "hc_exp_threshold", "hc_device_count", "hc_warm_up", "hc_last_error", "hc_version", "hc_fno1", "hc_fno3", "hc_fno1_small", "hc_fno3_small", "hc_build_adjacency", "hc_subread_info", "hc_host_alloc", "hc_host_free",
     "hc_store_create_fastq", "hc_store_create_fastq_files", "hc_store_read_ids", "hc_consensus", "hc_dedup_edges", "hc_idmap_create", "hc_idmap_destroy", "hc_ingest_overlaps", "hc_ingest_overlaps_device",
+    "hc_ingest_score_overlaps",
 ]
 
 _lib: Optional[ctypes.CDLL] = None
@@ -118,6 +119,8 @@ def lib() -> ctypes.CDLL:
         L.hc_ingest_overlaps.argtypes = [vp, vp, u64, vp, vp, vp, u64, vp, vp, u64, vp]
         L.hc_ingest_overlaps_device.restype = i32
         L.hc_ingest_overlaps_device.argtypes = [vp, vp, vp, u64, vp, vp, vp, u64, vp, vp, u64, vp]
+        L.hc_ingest_score_overlaps.restype = i32
+        L.hc_ingest_score_overlaps.argtypes = [vp, vp, vp, u64, vp, vp, vp, vp, vp, u64, vp, u64, vp, vp, u64, vp]
         L.hc_last_error.restype = ctypes.c_char_p
         L.hc_version.restype = ctypes.c_char_p
         _lib = L
@@ -310,6 +313,36 @@ class Store:
         flags = np.unpackbits(bits[: (n + 63) // 64].view(np.uint8), bitorder="little")[:n].astype(bool)
         assert int(flags.sum()) == int(nn.value)
         return edges[: ne.value], flags, stats[0]
+
+    def ingest_score(self, idmap: "IdMap", text, ingest_params: np.ndarray, params: np.ndarray, kept_cap: Optional[int] = None,
+                     edges_cap: Optional[int] = None, filtered_cap: Optional[int] = None):
+        """hc_ingest_score_overlaps: overlaps-file text (bytes or a uint8 array, e.g. from host_alloc) parsed and scored on
+        the id map's device.  Returns (kept CANDIDATE records, their line numbers, their classes, edges as EDGE_SMALL or
+        EDGE_SMALL_EXACT records whose `cand` indexes kept, filtered OVERLAP_REC records, their line numbers, stats)."""
+        buf = text if isinstance(text, np.ndarray) else (np.frombuffer(text, dtype=np.uint8) if len(text) else np.zeros(0, dtype=np.uint8))
+        exact = bool(int(params["flags"][0]) & F.FLAG_EXACT_EDGE_SCORES)
+        guess = int(np.count_nonzero(buf == 10)) + 1
+        kcap = guess if kept_cap is None else kept_cap
+        ecap = guess if edges_cap is None else edges_cap
+        fcap = guess if filtered_cap is None else filtered_cap
+        kept = np.zeros(max(kcap, 1), dtype=F.CANDIDATE)
+        kl = np.zeros(max(kcap, 1), dtype=np.uint64)
+        kc = np.zeros(max(kcap, 1), dtype=np.uint8)
+        edges = np.zeros(max(ecap, 1), dtype=F.EDGE_SMALL_EXACT if exact else F.EDGE_SMALL)
+        filt = np.zeros(max(fcap, 1), dtype=F.OVERLAP_REC)
+        fl = np.zeros(max(fcap, 1), dtype=np.uint64)
+        st = np.zeros(1, dtype=F.INGEST_SCORE_STATS)
+        rc = lib().hc_ingest_score_overlaps(self._h, idmap.handle, buf.ctypes.data if len(buf) else None, len(buf),
+                                            ingest_params.ctypes.data, params.ctypes.data, kept.ctypes.data, kl.ctypes.data,
+                                            kc.ctypes.data, kcap, edges.ctypes.data, ecap, filt.ctypes.data, fl.ctypes.data, fcap,
+                                            st.ctypes.data)
+        s = st[0]
+        if rc != 0:
+            err = HcError(rc, last_error())
+            err.required = (int(s["n_kept"]), int(s["score"]["n_edges"]), int(s["ingest"]["n_filtered"]))
+            raise err
+        nk, ne, nf = int(s["n_kept"]), int(s["score"]["n_edges"]), int(s["ingest"]["n_filtered"])
+        return kept[:nk], kl[:nk], kc[:nk], edges[:ne], filt[:nf], fl[:nf], s
 
     def score_batch_device(self, device: int, stream: int, params: np.ndarray, d_cand: int, n: int, d_per_cand: int,
                            d_edges: int, edges_cap: int, d_nonedge: int, nonedge_cap: int, d_counts: int, want_stats: bool):

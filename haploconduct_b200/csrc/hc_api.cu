@@ -23,6 +23,7 @@
 #include "hc_pack.cuh"
 #include "hc_consensus.cuh"
 #include "hc_cons_final.h"
+#include "hc_ingest.h"
 
 namespace {
 
@@ -90,6 +91,9 @@ struct DevCtx {
     uint64_t acc_b_cap = 0;                // small outputs: one bit per candidate of the shard (32-bit words)
     uint32_t* d_acc_bits = nullptr;
     unsigned long long* d_run = nullptr;   // {edges, non-edges} emitted so far in this call
+    // hc_ingest_score_overlaps: per slot the kept outputs of a piece ([cand][line][edge records][edge_kept][class], kept_cap each)
+    uint64_t kept_cap = 0;
+    unsigned char* d_kept[2] = {nullptr, nullptr};
     unsigned long long* h_cnt = nullptr;   // pinned: [2][HC_CNT_N] counter snapshots per slot
     uint64_t* d_counts = nullptr;
     cudaStream_t stream = nullptr, s_copy = nullptr, s_out = nullptr;
@@ -136,6 +140,7 @@ void free_ctx(DevCtx& d) {
     }
     cudaFree(d.d_acc_edges); cudaFree(d.d_acc_nonedge); cudaFree(d.d_acc_bits); cudaFree(d.d_run); cudaFree(d.d_counts);
     cudaFree(d.d_whole); cudaFree(d.d_runs_all);
+    cudaFree(d.d_kept[0]); cudaFree(d.d_kept[1]);
     if (d.h_runs_all) cudaFreeHost(d.h_runs_all);
     for (cudaEvent_t e : d.ev_step) cudaEventDestroy(e);
     if (d.h_cnt) cudaFreeHost(d.h_cnt);
@@ -204,7 +209,8 @@ struct RunDev {                 // device-side run arrays of one batch of hc_can
 int enqueue_batch(hc_store* s, DevCtx& d, cudaStream_t st, const hc_params* p, const void* d_cand, int compact, uint64_t n,
                   hc_result* d_per_cand, hc_edge* d_edges, uint64_t edges_cap, uint64_t* d_nonedge, uint64_t nonedge_cap,
                   uint64_t* d_counts, uint64_t cand_offset, unsigned long long* d_run, cudaEvent_t k0, cudaEvent_t k1,
-                  uint32_t* launches, const RunDev* runs = nullptr, int small_out = 0, uint32_t* d_bits = nullptr) {
+                  uint32_t* launches, const RunDev* runs = nullptr, int small_out = 0, uint32_t* d_bits = nullptr,
+                  const hc_kept_dev* kept = nullptr) {
     if (n > 0xffffffffull) return fail(HC_ERR_ARG, "more than 2^32-1 candidates in one device batch");
     if (compact >= 3 && !runs) return fail(HC_ERR_ARG, "run-encoded candidates without run arrays");
     int rc = ensure_tables(s, d, p->mismatch, st);
@@ -255,7 +261,7 @@ int enqueue_batch(hc_store* s, DevCtx& d, cudaStream_t st, const hc_params* p, c
         CU(hc_launch_exact(P, st));
         nl += 2;
     }
-    CU(hc_launch_compact(P, d_edges, edges_cap, d_nonedge, nonedge_cap, d.blockcounts, cand_offset, d_run, st, small_out, d_bits));
+    CU(hc_launch_compact(P, d_edges, edges_cap, d_nonedge, nonedge_cap, d.blockcounts, cand_offset, d_run, st, small_out, d_bits, kept));
     nl += (n > 0 ? 4 : 1) + (d_run ? 1 : 0) + ((n > 0 && small_out && d_bits) ? 1 : 0);   // count, scan, scatter, emit_edges (+ advance, + bit map)
     if (k1) CU(cudaEventRecord(k1, st));
     if (d_counts) {   // {n_edges, n_nonedges, n_exact} are contiguous in the counter block; [3] = invalid candidates
@@ -1241,6 +1247,147 @@ int hc_score_batch_short_small(hc_store* s, const hc_params* p, const hc_candida
     if (n && !nonedge_bits) return fail(HC_ERR_ARG, "hc_score_batch_short_small: NULL bit map");
     if (n > 0xffffffffull) return fail(HC_ERR_ARG, "hc_score_batch_short_small: a call takes fewer than 2^32 candidates");
     return score_host(s, p, cand, 2, n, nullptr, reinterpret_cast<hc_edge*>(edges), edges_cap, n_edges, nonedge_bits, 0, n_nonedges, stats, nullptr, 1);
+}
+
+// Text in, kept candidates and edges out.  The buffer is cut into pieces as hc_ingest_overlaps cuts it; on the id map's
+// main stream every piece is parsed (hc_ingest_device) and scored (enqueue_batch in kept mode, running totals in d.d_run),
+// and only what the host needs leaves the device.  The copy in of piece i + 1 runs on the copy stream and the copy out
+// of piece i - 1 on the output stream while piece i is processed (two buffer sets).
+int hc_ingest_score_overlaps(hc_store* s, const hc_idmap* cm, const char* text, uint64_t n_bytes, const hc_ingest_params* ip,
+                             const hc_params* p, hc_candidate* kept, uint64_t* kept_line, uint8_t* kept_class, uint64_t kept_cap,
+                             void* edges, uint64_t edges_cap, hc_overlap_rec* filtered, uint64_t* filtered_line, uint64_t filtered_cap,
+                             hc_ingest_score_stats* stats) {
+    if (!s || !cm || !ip || !p || !stats || (n_bytes && !text) || (kept_cap && (!kept || !kept_class)) || (edges_cap && !edges) ||
+        (filtered_cap && !filtered))
+        return fail(HC_ERR_ARG, "hc_ingest_score_overlaps: NULL argument");
+    hc_idmap* m = const_cast<hc_idmap*>(cm);
+    memset(stats, 0, sizeof(*stats));
+    stats->ingest.first_error_line = ~0ull;
+    DevCtx* dp = find_ctx(s, m->device);
+    if (!dp) return fail(HC_ERR_ARG, "hc_ingest_score_overlaps: the store has no replica on the id map's device");
+    if (n_bytes == 0) return HC_OK;
+    DevCtx& d = *dp;
+    CU(cudaSetDevice(d.device));
+    const std::vector<uint64_t> cut = hc_ingest_cuts(text, n_bytes, hc_ingest_piece_bytes());
+    const size_t n_pieces = cut.size() - 1;
+    uint64_t max_piece = 0;
+    for (size_t i = 0; i < n_pieces; i++) max_piece = std::max(max_piece, cut[i + 1] - cut[i]);
+    const uint64_t cap = hc_ingest_rec_cap(max_piece);           // records of any kind one piece can produce
+    const uint64_t tbytes = (max_piece + 16 + 255) & ~255ull;
+    const size_t erec = (p->flags & HC_FLAG_EXACT_EDGE_SCORES) ? sizeof(hc_edge_small_exact) : sizeof(hc_edge_small);
+    // a kept slot: [cand 32][line 8][edge record <= 32][edge_kept 4][class 1] bytes per record
+    const uint64_t o_line = cap * sizeof(hc_candidate), o_edge = o_line + cap * sizeof(uint64_t);
+    const uint64_t o_src = o_edge + cap * sizeof(hc_edge_small_exact), o_cls = o_src + cap * sizeof(uint32_t);
+    if (cap > d.kept_cap) {
+        for (int k = 0; k < 2; k++) { cudaFree(d.d_kept[k]); d.d_kept[k] = nullptr; }
+        d.kept_cap = 0;
+        for (int k = 0; k < 2; k++) CU(cudaMalloc(&d.d_kept[k], o_cls + cap));
+        d.kept_cap = cap;
+    }
+    {
+        const int rcw = ensure_workspace(d, cap);
+        if (rcw != HC_OK) return rcw;
+    }
+    char* d_text = nullptr;
+    hc_candidate* d_cand = nullptr;
+    hc_overlap_rec* d_filt = nullptr;
+    uint64_t *d_cl = nullptr, *d_fl = nullptr;
+    CU(hc_idmap_ws(m, 11, 2 * tbytes, (void**)&d_text));
+    CU(hc_idmap_ws(m, 12, 2 * cap * sizeof(hc_candidate), (void**)&d_cand));
+    CU(hc_idmap_ws(m, 13, 2 * cap * sizeof(hc_overlap_rec), (void**)&d_filt));
+    if (kept_line) CU(hc_idmap_ws(m, 14, 2 * cap * sizeof(uint64_t), (void**)&d_cl));
+    if (filtered_line) CU(hc_idmap_ws(m, 15, 2 * cap * sizeof(uint64_t), (void**)&d_fl));
+    hc_ingest_stats& is = stats->ingest;
+    hc_batch_stats& bs = stats->score;
+    bool overflow = false;
+    uint64_t lines = 0, nk = 0, ne = 0, nf = 0;
+    struct Out { int b; bool copy; uint64_t nk, pk, ne, pe, nf, pf; };   // a piece whose outputs wait to be copied out
+    Out pend{};
+    bool have_pend = false;
+    auto copy_out = [&](const Out& o) -> int {
+        const unsigned char* kb = d.d_kept[o.b];
+        if (o.copy && o.pk) {
+            CU(hc_copy_d2h_on(kept + o.nk, kb, o.pk * sizeof(hc_candidate), m->s_out, nullptr));
+            if (kept_line) CU(hc_copy_d2h_on(kept_line + o.nk, kb + o_line, o.pk * sizeof(uint64_t), m->s_out, nullptr));
+            CU(hc_copy_d2h_on(kept_class + o.nk, kb + o_cls, o.pk, m->s_out, nullptr));
+        }
+        if (o.copy && o.pe) CU(hc_copy_d2h_on(static_cast<char*>(edges) + o.ne * erec, kb + o_edge, o.pe * erec, m->s_out, nullptr));
+        if (o.copy && o.pf) {
+            CU(hc_copy_d2h_on(filtered + o.nf, d_filt + (size_t)o.b * cap, o.pf * sizeof(hc_overlap_rec), m->s_out, nullptr));
+            if (filtered_line) CU(hc_copy_d2h_on(filtered_line + o.nf, d_fl + (size_t)o.b * cap, o.pf * sizeof(uint64_t), m->s_out, nullptr));
+        }
+        CU(cudaEventRecord(m->ev_out[o.b], m->s_out));
+        return HC_OK;
+    };
+    auto run = [&]() -> int {
+        hc_ingest_params pp = *ip;
+        CU(cudaMemsetAsync(d.d_run, 0, 2 * sizeof(unsigned long long), m->s_main));
+        CU(cudaEventRecord(d.ev[2], m->s_main));
+        CU(hc_copy_h2d_on(d_text, text, cut[1] - cut[0], m->s_copy));
+        CU(cudaEventRecord(m->ev_in[0], m->s_copy));
+        for (size_t i = 0; i < n_pieces && lines < ip->max_overlaps; i++) {
+            const int b = (int)(i & 1);
+            if (i + 1 < n_pieces) {   // text buffer b ^ 1 was read by piece i - 1, which has completed
+                CU(hc_copy_h2d_on(d_text + (size_t)(b ^ 1) * tbytes, text + cut[i + 1], cut[i + 2] - cut[i + 1], m->s_copy));
+                CU(cudaEventRecord(m->ev_in[b ^ 1], m->s_copy));
+            }
+            CU(cudaStreamWaitEvent(m->s_main, m->ev_in[b], 0));
+            if (i >= 2) CU(cudaEventSynchronize(m->ev_out[b]));          // buffer set b has been copied out
+            hc_candidate* dc = d_cand + (size_t)b * cap;
+            uint64_t* dcl = d_cl ? d_cl + (size_t)b * cap : nullptr;
+            hc_ingest_stats st;
+            pp.max_overlaps = ip->max_overlaps - lines;
+            int rc = hc_ingest_device(m, d_text + (size_t)b * tbytes, cut[i + 1] - cut[i], &pp, dc, dcl, cap, d_filt + (size_t)b * cap,
+                                      d_fl ? d_fl + (size_t)b * cap : nullptr, cap, &st, m->s_main, lines);
+            if (rc != HC_OK) return rc;
+            if (st.first_error_line != ~0ull && is.first_error_line == ~0ull) {
+                is.first_error_line = lines + st.first_error_line;
+                is.first_error_offset = cut[i] + st.first_error_offset;
+                is.first_error_length = st.first_error_length;
+                is.first_error_status = st.first_error_status;
+            }
+            unsigned char* kb = d.d_kept[b];
+            const hc_kept_dev K{reinterpret_cast<hc_candidate*>(kb), kept_line ? reinterpret_cast<uint64_t*>(kb + o_line) : nullptr, kb + o_cls,
+                                dcl, reinterpret_cast<uint32_t*>(kb + o_src)};
+            uint32_t nl = 0;
+            rc = enqueue_batch(s, d, m->s_main, p, dc, 0, st.n_scored, nullptr, reinterpret_cast<hc_edge*>(kb + o_edge), cap, nullptr, 0,
+                               nullptr, 0, d.d_run, d.ev[0], d.ev[1], &nl, nullptr, 1, nullptr, &K);
+            if (rc != HC_OK) return rc;
+            CU(cudaMemcpyAsync(d.h_cnt, d.counters, HC_CNT_N * sizeof(unsigned long long), cudaMemcpyDeviceToHost, m->s_main));
+            if (have_pend) { rc = copy_out(pend); have_pend = false; if (rc != HC_OK) return rc; }   // overlaps this piece's kernels
+            CU(cudaStreamSynchronize(m->s_main));
+            const unsigned long long* h = d.h_cnt;
+            rc = add_stats(d, h, st.n_scored, &bs, nullptr, nullptr);     // the message of hc_score_batch* for rejected candidates
+            if (rc != HC_OK) return rc;
+            float ms = 0;
+            if (cudaEventElapsedTime(&ms, d.ev[0], d.ev[1]) == cudaSuccess) bs.kernel_ms += ms;
+            if (st.n_scored && cudaEventElapsedTime(&ms, d.ev[4], d.ev[5]) == cudaSuccess) bs.score_kernel_ms += ms;
+            bs.kernel_launches += nl;
+            const uint64_t pe = h[HC_CNT_EDGES], pk = pe + h[HC_CNT_NONEDGES];
+            if (nk + pk > 0xffffffffull)
+                return fail(HC_ERR_ARG, "hc_ingest_score_overlaps: 2^32 or more kept candidates (hc_edge_small.cand is 32 bits)");
+            overflow = overflow || nk + pk > kept_cap || ne + pe > edges_cap || nf + st.n_filtered > filtered_cap;
+            pend = Out{b, !overflow, nk, pk, ne, pe, nf, st.n_filtered};
+            have_pend = true;
+            lines += st.n_lines; nk += pk; ne += pe; nf += st.n_filtered;
+            is.n_scored += st.n_scored; is.n_skipped += st.n_skipped; is.n_dropped += st.n_dropped; is.device_ms += st.device_ms;
+        }
+        if (have_pend) { have_pend = false; return copy_out(pend); }
+        return HC_OK;
+    };
+    int rc = run();
+    const cudaError_t e1 = cudaStreamSynchronize(m->s_out), e2 = cudaStreamSynchronize(m->s_copy);
+    if (rc != HC_OK) return rc;
+    CU(e1);
+    CU(e2);
+    CU(cudaEventRecord(d.ev[3], m->s_main));
+    CU(cudaEventSynchronize(d.ev[3]));
+    float ms = 0;
+    if (cudaEventElapsedTime(&ms, d.ev[2], d.ev[3]) == cudaSuccess) bs.total_ms = ms;
+    is.n_lines = lines; is.n_filtered = nf;
+    stats->n_kept = nk;
+    if (overflow) return fail(HC_ERR_CAPACITY, "hc_ingest_score_overlaps: output buffer too small (required sizes returned in stats)");
+    return HC_OK;
 }
 
 int hc_overlap_score_multi(const char* seq1, uint32_t len1, const char* seq2, uint32_t len2, const char* qual1,

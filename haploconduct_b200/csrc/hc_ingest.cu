@@ -11,26 +11,11 @@
 #include <vector>
 #include <cuda_runtime.h>
 #include "../../include/hc_b200.h"
+#include "hc_ingest.h"
 
 void hc_set_last_error(const char* msg);   // hc_api.cu
 
-struct hc_idmap {
-    int device;
-    uint64_t n;        // reads
-    uint64_t mask;     // hash table size - 1 (open addressing, one 16-byte slot {id, index} per entry)
-    ulonglong2* slots;
-    uint64_t direct_n; // > 0: ids are dense, direct[id] = index for id < direct_n (fits L2 for 1e7 reads)
-    uint32_t* direct;
-    // grow-only workspace of hc_ingest_overlaps* (one call at a time per handle)
-    void* ws[16];
-    size_t ws_cap[16];
-    cudaEvent_t e0, e1;
-    // piece pipeline of the host-buffer entry point: copies in / kernels / copies out on three streams
-    cudaStream_t s_main, s_copy, s_out;
-    cudaEvent_t ev_in[2], ev_out[2];
-};
-
-static cudaError_t ws_get(hc_idmap* m, int k, size_t bytes, void** out) {
+cudaError_t hc_idmap_ws(hc_idmap* m, int k, size_t bytes, void** out) {
     if (bytes > m->ws_cap[k]) {
         cudaFree(m->ws[k]);
         m->ws[k] = nullptr;
@@ -364,9 +349,9 @@ extern "C" void hc_idmap_destroy(hc_idmap* m) {
 }
 
 // Device-side core: text already on the device.  Outputs are device buffers; counts[0..1] land in host memory.
-static int ingest_device(const hc_idmap* cm, const char* d_text, u64 n_bytes, const hc_ingest_params* p, hc_candidate* d_cand,
-                         uint64_t* d_cand_line, u64 cand_cap, hc_overlap_rec* d_filt, uint64_t* d_filt_line, u64 filt_cap,
-                         hc_ingest_stats* st, cudaStream_t stream, u64 line_base = 0) {
+int hc_ingest_device(const hc_idmap* cm, const char* d_text, uint64_t n_bytes, const hc_ingest_params* p, hc_candidate* d_cand,
+                     uint64_t* d_cand_line, uint64_t cand_cap, hc_overlap_rec* d_filt, uint64_t* d_filt_line, uint64_t filt_cap,
+                     hc_ingest_stats* st, cudaStream_t stream, uint64_t line_base) {
     hc_idmap* m = const_cast<hc_idmap*>(cm);     // the workspace is the only thing a call changes
     int rc = HC_OK;
     const u64 n_tiles = (n_bytes + TILE - 1) / TILE;
@@ -381,9 +366,9 @@ static int ingest_device(const hc_idmap* cm, const char* d_text, u64 n_bytes, co
     memset(st, 0, sizeof(*st));
     st->first_error_line = EMPTY;
     if (n_bytes == 0) return HC_OK;
-    ICU(ws_get(m, 0, n_tiles * sizeof(uint32_t), (void**)&d_tcnt));
-    ICU(ws_get(m, 1, n_tiles * sizeof(u64), (void**)&d_toff));
-    ICU(ws_get(m, 2, (8 + hc_scan::blocks_for(n_tiles)) * sizeof(u64), (void**)&d_tot));
+    ICU(hc_idmap_ws(m, 0, n_tiles * sizeof(uint32_t), (void**)&d_tcnt));
+    ICU(hc_idmap_ws(m, 1, n_tiles * sizeof(u64), (void**)&d_toff));
+    ICU(hc_idmap_ws(m, 2, (8 + hc_scan::blocks_for(n_tiles)) * sizeof(u64), (void**)&d_tot));
     d_misc = d_tot + 2;
     ICU(cudaEventRecord(m->e0, stream));
     nl_count<<<(unsigned)n_tiles, 256, 0, stream>>>(d_text, n_bytes, d_tcnt);
@@ -392,20 +377,20 @@ static int ingest_device(const hc_idmap* cm, const char* d_text, u64 n_bytes, co
     ICU(cudaMemcpyAsync(&last, d_text + n_bytes - 1, 1, cudaMemcpyDeviceToHost, stream));
     ICU(cudaStreamSynchronize(stream));
     n_lines = n_nl + (last != '\n' ? 1 : 0);          // getline also returns an unterminated last line
-    ICU(ws_get(m, 3, (n_nl + 2) * sizeof(u64), (void**)&d_ls));
+    ICU(hc_idmap_ws(m, 3, (n_nl + 2) * sizeof(u64), (void**)&d_ls));
     ICU(cudaMemsetAsync(d_ls, 0, sizeof(u64), stream));
     nl_mark<<<(unsigned)n_tiles, 256, 0, stream>>>(d_text, n_bytes, d_toff, d_ls);
     if (n_lines > p->max_overlaps) n_lines = p->max_overlaps;   // while (getline(...) && i < max_overlaps), :581
     st->n_lines = n_lines;
     if (n_lines == 0) { ICU(cudaStreamSynchronize(stream)); goto done; }
     n_blocks = (n_lines + LINES_PER_BLOCK - 1) / LINES_PER_BLOCK;
-    ICU(ws_get(m, 4, n_lines * sizeof(hc_candidate), (void**)&d_tmp_c));
-    ICU(ws_get(m, 5, n_lines * sizeof(hc_overlap_rec), (void**)&d_tmp_f));
-    ICU(ws_get(m, 6, n_lines, (void**)&d_status));
-    ICU(ws_get(m, 7, n_blocks * sizeof(uint32_t), (void**)&d_cs));
-    ICU(ws_get(m, 8, n_blocks * sizeof(uint32_t), (void**)&d_cf));
-    ICU(ws_get(m, 9, n_blocks * sizeof(u64), (void**)&d_os));
-    ICU(ws_get(m, 10, n_blocks * sizeof(u64), (void**)&d_of));
+    ICU(hc_idmap_ws(m, 4, n_lines * sizeof(hc_candidate), (void**)&d_tmp_c));
+    ICU(hc_idmap_ws(m, 5, n_lines * sizeof(hc_overlap_rec), (void**)&d_tmp_f));
+    ICU(hc_idmap_ws(m, 6, n_lines, (void**)&d_status));
+    ICU(hc_idmap_ws(m, 7, n_blocks * sizeof(uint32_t), (void**)&d_cs));
+    ICU(hc_idmap_ws(m, 8, n_blocks * sizeof(uint32_t), (void**)&d_cf));
+    ICU(hc_idmap_ws(m, 9, n_blocks * sizeof(u64), (void**)&d_os));
+    ICU(hc_idmap_ws(m, 10, n_blocks * sizeof(u64), (void**)&d_of));
     ICU(cudaMemcpyAsync(d_misc, misc, sizeof(misc), cudaMemcpyHostToDevice, stream));
     D.text = d_text; D.n_bytes = n_bytes; D.line_start = d_ls; D.n_lines = n_lines; D.n_newlines = n_nl;
     D.ids.slots = m->slots; D.ids.mask = m->mask; D.ids.direct = m->direct; D.ids.direct_n = m->direct_n;
@@ -452,18 +437,19 @@ extern "C" int hc_ingest_overlaps_device(const hc_idmap* m, void* stream, const 
                                          hc_ingest_stats* stats) {
     if (!m || !p || !stats || (n_bytes && !d_text)) { hc_set_last_error("hc_ingest_overlaps_device: NULL argument"); return HC_ERR_ARG; }
     if (cudaSetDevice(m->device) != cudaSuccess) { hc_set_last_error("hc_ingest_overlaps_device: cudaSetDevice failed"); return HC_ERR_CUDA; }
-    return ingest_device(m, d_text, n_bytes, p, d_cand, d_cand_line, cand_cap, d_filtered, d_filtered_line, filtered_cap, stats,
+    return hc_ingest_device(m, d_text, n_bytes, p, d_cand, d_cand_line, cand_cap, d_filtered, d_filtered_line, filtered_cap, stats,
                          (cudaStream_t)stream);
 }
 
-// Large buffers are cut into pieces that end at a line end; the copy in of piece i + 1 and the copy out of piece i - 1
-// overlap the kernels of piece i (three streams, two buffer sets).  A line that reaches an output has 13 fields, i.e.
-// at least 26 bytes with its newline, which bounds the records a piece can produce without counting its lines first.
-static int ingest_pipelined(hc_idmap* m, const char* text, u64 n_bytes, const hc_ingest_params* p, hc_candidate* cand,
-                            uint64_t* cand_line, u64 cand_cap, hc_overlap_rec* filtered, uint64_t* filtered_line, u64 filtered_cap,
-                            hc_ingest_stats* stats, u64 piece) {
-    int rc = HC_OK;
-    std::vector<u64> cut(1, 0);
+uint64_t hc_ingest_piece_bytes() {
+    u64 piece = 32ull << 20;
+    if (const char* e = getenv("HC_INGEST_PIECE")) { const u64 v = strtoull(e, nullptr, 10); if (v) piece = v; }   // tests
+    return piece;
+}
+
+std::vector<uint64_t> hc_ingest_cuts(const char* text, uint64_t n_bytes, uint64_t piece) {
+    std::vector<uint64_t> cut(1, 0);
+    if (n_bytes <= piece + piece / 2) { if (n_bytes) cut.push_back(n_bytes); return cut; }
     while (cut.back() < n_bytes) {
         u64 end = cut.back() + piece;
         if (end >= n_bytes) end = n_bytes;
@@ -477,10 +463,21 @@ static int ingest_pipelined(hc_idmap* m, const char* text, u64 n_bytes, const hc
         }
         cut.push_back(end);
     }
+    return cut;
+}
+
+// Large buffers are cut into pieces that end at a line end; the copy in of piece i + 1 and the copy out of piece i - 1
+// overlap the kernels of piece i (three streams, two buffer sets).  hc_ingest_rec_cap bounds the records a piece can
+// produce without counting its lines first.
+static int ingest_pipelined(hc_idmap* m, const char* text, u64 n_bytes, const hc_ingest_params* p, hc_candidate* cand,
+                            uint64_t* cand_line, u64 cand_cap, hc_overlap_rec* filtered, uint64_t* filtered_line, u64 filtered_cap,
+                            hc_ingest_stats* stats, u64 piece) {
+    int rc = HC_OK;
+    const std::vector<uint64_t> cut = hc_ingest_cuts(text, n_bytes, piece);
     const size_t n_pieces = cut.size() - 1;
     u64 max_piece = 0;
-    for (size_t i = 0; i < n_pieces; i++) max_piece = std::max(max_piece, cut[i + 1] - cut[i]);
-    const u64 rec_cap = max_piece / 26 + 2;
+    for (size_t i = 0; i < n_pieces; i++) max_piece = std::max<u64>(max_piece, cut[i + 1] - cut[i]);
+    const u64 rec_cap = hc_ingest_rec_cap(max_piece);
     const u64 tbytes = (max_piece + 16 + 255) & ~255ull;
     char* d_text = nullptr;
     hc_candidate* d_cand = nullptr;
@@ -489,11 +486,11 @@ static int ingest_pipelined(hc_idmap* m, const char* text, u64 n_bytes, const hc
     u64 lines = 0, ns = 0, nf = 0;
     bool overflow = false;
     hc_ingest_params pp = *p;
-    ICU(ws_get(m, 11, 2 * tbytes, (void**)&d_text));
-    ICU(ws_get(m, 12, 2 * rec_cap * sizeof(hc_candidate), (void**)&d_cand));
-    ICU(ws_get(m, 13, 2 * rec_cap * sizeof(hc_overlap_rec), (void**)&d_filt));
-    if (cand_line) ICU(ws_get(m, 14, 2 * rec_cap * sizeof(u64), (void**)&d_cl));
-    if (filtered_line) ICU(ws_get(m, 15, 2 * rec_cap * sizeof(u64), (void**)&d_fl));
+    ICU(hc_idmap_ws(m, 11, 2 * tbytes, (void**)&d_text));
+    ICU(hc_idmap_ws(m, 12, 2 * rec_cap * sizeof(hc_candidate), (void**)&d_cand));
+    ICU(hc_idmap_ws(m, 13, 2 * rec_cap * sizeof(hc_overlap_rec), (void**)&d_filt));
+    if (cand_line) ICU(hc_idmap_ws(m, 14, 2 * rec_cap * sizeof(u64), (void**)&d_cl));
+    if (filtered_line) ICU(hc_idmap_ws(m, 15, 2 * rec_cap * sizeof(u64), (void**)&d_fl));
     // pageable text / result buffers (a file read into memory, a std::vector) go through the pinned ring of hc_stage.cu,
     // copied by several host threads; pinned ones are handed to the copy engine as they are
     ICU(hc_copy_h2d_on(d_text, text, cut[1] - cut[0], m->s_copy));
@@ -509,7 +506,7 @@ static int ingest_pipelined(hc_idmap* m, const char* text, u64 n_bytes, const hc
         hc_ingest_stats st;
         pp.max_overlaps = p->max_overlaps - lines;
         const u64 room_s = overflow ? 0 : std::min<u64>(rec_cap, cand_cap - ns), room_f = overflow ? 0 : std::min<u64>(rec_cap, filtered_cap - nf);
-        int prc = ingest_device(m, d_text + (size_t)b * tbytes, cut[i + 1] - cut[i], &pp, d_cand + (size_t)b * rec_cap,
+        int prc = hc_ingest_device(m, d_text + (size_t)b * tbytes, cut[i + 1] - cut[i], &pp, d_cand + (size_t)b * rec_cap,
                                 d_cl ? d_cl + (size_t)b * rec_cap : nullptr, room_s, d_filt + (size_t)b * rec_cap,
                                 d_fl ? d_fl + (size_t)b * rec_cap : nullptr, room_f, &st, m->s_main, lines);
         if (prc == HC_ERR_CAPACITY) { overflow = true; prc = HC_OK; }   // keep counting: the caller gets the required sizes
@@ -561,16 +558,15 @@ extern "C" int hc_ingest_overlaps(const hc_idmap* cm, const char* text, uint64_t
     if (n_bytes == 0) return HC_OK;
     ICU(cudaSetDevice(m->device));
     {
-        u64 piece = 32ull << 20;
-        if (const char* e = getenv("HC_INGEST_PIECE")) { const u64 v = strtoull(e, nullptr, 10); if (v) piece = v; }   // tests
+        const u64 piece = hc_ingest_piece_bytes();
         if (n_bytes > piece + piece / 2)
             return ingest_pipelined(m, text, n_bytes, p, cand, cand_line, cand_cap, filtered, filtered_line, filtered_cap, stats, piece);
     }
-    ICU(ws_get(m, 11, n_bytes + 16, (void**)&d_text));
+    ICU(hc_idmap_ws(m, 11, n_bytes + 16, (void**)&d_text));
     ICU(hc_copy_h2d(d_text, text, n_bytes));
-    if (cand_cap) { ICU(ws_get(m, 12, cand_cap * sizeof(hc_candidate), (void**)&d_cand)); if (cand_line) ICU(ws_get(m, 14, cand_cap * sizeof(u64), (void**)&d_cl)); }
-    if (filtered_cap) { ICU(ws_get(m, 13, filtered_cap * sizeof(hc_overlap_rec), (void**)&d_filt)); if (filtered_line) ICU(ws_get(m, 15, filtered_cap * sizeof(u64), (void**)&d_fl)); }
-    rc = ingest_device(m, d_text, n_bytes, p, d_cand, d_cl, cand_cap, d_filt, d_fl, filtered_cap, stats, m->s_main);
+    if (cand_cap) { ICU(hc_idmap_ws(m, 12, cand_cap * sizeof(hc_candidate), (void**)&d_cand)); if (cand_line) ICU(hc_idmap_ws(m, 14, cand_cap * sizeof(u64), (void**)&d_cl)); }
+    if (filtered_cap) { ICU(hc_idmap_ws(m, 13, filtered_cap * sizeof(hc_overlap_rec), (void**)&d_filt)); if (filtered_line) ICU(hc_idmap_ws(m, 15, filtered_cap * sizeof(u64), (void**)&d_fl)); }
+    rc = hc_ingest_device(m, d_text, n_bytes, p, d_cand, d_cl, cand_cap, d_filt, d_fl, filtered_cap, stats, m->s_main);
     if (rc != HC_OK) goto done;
     if (stats->n_scored) {
         ICU(hc_copy_d2h(cand, d_cand, stats->n_scored * sizeof(hc_candidate)));

@@ -1249,6 +1249,66 @@ __global__ void __launch_bounds__(HC_CB_THREADS) hc_compact_scatter(const hc_kpa
     }
 }
 
+// Kept mode of hc_compact_scatter (the same ranks; that kernel stays as it is): a kept candidate's index is its rank
+// among the edges plus its rank among the non-edges.  The candidate, its line and its class are written at that index
+// relative to the batch (the running totals P.run taken off), and an edge's absolute kept index goes to K.edge_kept for
+// hc_emit_edges_kept.
+__global__ void __launch_bounds__(HC_CB_THREADS) hc_compact_scatter_kept(const hc_kparams P, const u64* __restrict__ blockoffs,
+                                                                        uint32_t* edge_src, const hc_kept_dev K) {
+    __shared__ uint32_t wtot[HC_CB_THREADS / 32];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const u64 base = (u64)blockIdx.x * HC_CB_ITEMS;
+    const u64 run_e = P.run ? P.run[0] : 0ull, run_n = P.run ? P.run[1] : 0ull;
+    u64 eoff = blockoffs[2 * blockIdx.x] + run_e, ooff = blockoffs[2 * blockIdx.x + 1] + run_n;
+    const hc_candidate* cand = reinterpret_cast<const hc_candidate*>(P.cand);
+    for (uint32_t k0 = 0; k0 < HC_CB_ITEMS; k0 += 4 * HC_CB_THREADS) {
+        const u64 i0 = base + k0 + 4ull * threadIdx.x;
+        uint32_t w4 = 0;
+        if (i0 + 4 <= P.n) w4 = __ldg(reinterpret_cast<const uint32_t*>(P.cls + i0));
+        else for (int j = 0; j < 4; j++) if (i0 + j < P.n) w4 |= (uint32_t)P.cls[i0 + j] << (8 * j);
+        uint32_t ce = 0, co = 0;
+        count_classes4(w4, ce, co);
+        const uint32_t mine = ce | (co << 16);
+        uint32_t inc = mine;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const uint32_t t = __shfl_up_sync(0xffffffffu, inc, d);
+            if (lane >= d) inc += t;
+        }
+        if (lane == 31) wtot[warp] = inc;
+        __syncthreads();
+        uint32_t before = 0, total = 0;
+#pragma unroll
+        for (int w = 0; w < HC_CB_THREADS / 32; w++) {
+            if (w < warp) before += wtot[w];
+            total += wtot[w];
+        }
+        const uint32_t ex = before + inc - mine;
+        u64 de = eoff + (ex & 0xffffu), dn = ooff + (ex >> 16);
+        if (mine) {
+#pragma unroll
+            for (int j = 0; j < 4; j++) {
+                const uint32_t c = (w4 >> (8 * j)) & HC_CLS_MASK;
+                if (c != HC_CLASS_EDGE && c != HC_CLASS_NONEDGE) continue;
+                const u64 r = (de - run_e) + (dn - run_n);
+                K.cand[r] = cand[i0 + j];
+                if (K.line) K.line[r] = K.line_in[i0 + j];
+                K.cls[r] = (uint8_t)c;
+                if (c == HC_CLASS_EDGE) {
+                    edge_src[de - run_e] = (uint32_t)(i0 + j);
+                    K.edge_kept[de - run_e] = (uint32_t)(de + dn);
+                    de++;
+                } else {
+                    dn++;
+                }
+            }
+        }
+        eoff += total & 0xffffu;
+        ooff += total >> 16;
+        __syncthreads();
+    }
+}
+
 // One thread per accepted edge of the batch (dense: no idle lanes next to the exp() and the random loads)
 __global__ void __launch_bounds__(256) hc_emit_edges(const hc_kparams P, const uint32_t* __restrict__ edge_src, hc_edge* edges,
                                                      u64 edges_cap, u64 cand_offset) {
@@ -1270,6 +1330,18 @@ __global__ void __launch_bounds__(256) hc_emit_edges_small(const hc_kparams P, c
         if (run_e + k >= edges_cap) break;
         const u64 i = edge_src[k];
         emit_edge_small<EXACT>(P, i, P.cls[i], cand_offset, edges, run_e + k);
+    }
+}
+
+// Kept mode: the batch's k-th edge goes to edges[k] and names its kept index as `cand` (emit_edge_small writes
+// i + cand_offset, so the offset is the kept index minus i, modulo 2^64)
+template <bool EXACT>
+__global__ void __launch_bounds__(256) hc_emit_edges_kept(const hc_kparams P, const uint32_t* __restrict__ edge_src,
+                                                          const uint32_t* __restrict__ edge_kept, void* edges) {
+    const u64 n_edges = P.counters[HC_CNT_EDGES];
+    for (u64 k = (u64)blockIdx.x * blockDim.x + threadIdx.x; k < n_edges; k += (u64)gridDim.x * blockDim.x) {
+        const u64 i = edge_src[k];
+        emit_edge_small<EXACT>(P, i, P.cls[i], (u64)edge_kept[k] - i, edges, k);
     }
 }
 
@@ -1391,14 +1463,20 @@ uint32_t hc_compact_blocks(uint64_t n) { return (uint32_t)((n + HC_CB_ITEMS - 1)
 // d_blockcounts: uint32[2*nblocks] followed (8-byte aligned) by uint64[2*nblocks] block offsets
 cudaError_t hc_launch_compact(const hc_kparams& P, hc_edge* d_edges, uint64_t edges_cap, uint64_t* d_nonedge,
                               uint64_t nonedge_cap, uint32_t* d_blockcounts, uint64_t cand_offset, unsigned long long* d_run,
-                              cudaStream_t st, int small_out, uint32_t* d_bits) {
+                              cudaStream_t st, int small_out, uint32_t* d_bits, const hc_kept_dev* kept) {
     const uint32_t nb = hc_compact_blocks(P.n);
     u64* offs = reinterpret_cast<u64*>(d_blockcounts + 2ull * nb + (2ull * nb & 1ull));
     if (nb > 0) {
         hc_compact_count<<<nb, HC_CB_THREADS, 0, st>>>(P.cls, P.n, d_blockcounts);
     }
     hc_compact_scan<<<1, 1024, 0, st>>>(d_blockcounts, nb, offs, P.counters);
-    if (nb > 0) {
+    if (nb > 0 && kept) {
+        hc_compact_scatter_kept<<<nb, HC_CB_THREADS, 0, st>>>(P, offs, P.flagged, *kept);
+        const u64 want = (P.n + 255) / 256;
+        const unsigned eb = (unsigned)(want < (unsigned long long)hc_grid_cap() ? want : (unsigned long long)hc_grid_cap());
+        if (P.exact_edges) hc_emit_edges_kept<true><<<eb, 256, 0, st>>>(P, P.flagged, kept->edge_kept, d_edges);
+        else hc_emit_edges_kept<false><<<eb, 256, 0, st>>>(P, P.flagged, kept->edge_kept, d_edges);
+    } else if (nb > 0) {
         // P.flagged has been consumed by the reference-order pass; it now carries the source index of every edge
         hc_compact_scatter<<<nb, HC_CB_THREADS, 0, st>>>(P, offs, P.flagged, d_nonedge, nonedge_cap, cand_offset);
         const u64 want = (P.n + 255) / 256;

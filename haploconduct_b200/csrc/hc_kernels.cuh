@@ -98,15 +98,26 @@ struct hc_launch_cfg {
     size_t smem;
 };
 
+// Kept mode of the compaction (hc_ingest_score_overlaps): the candidates classified edge or non-edge are written out
+// themselves, in batch order, and every edge names its kept index (plus the running totals P.run) as `cand`.
+struct hc_kept_dev {
+    hc_candidate* cand;          // [n] kept candidates of the batch
+    uint64_t* line;              // nullable: their line numbers, taken from line_in
+    uint8_t* cls;                // [n] their classes (HC_CLASS_EDGE / HC_CLASS_NONEDGE)
+    const uint64_t* line_in;     // nullable: line number of every candidate of the batch
+    uint32_t* edge_kept;         // [n] scratch: kept index of the batch's k-th edge
+};
+
 // host-callable launchers (hc_kernels.cu)
 cudaError_t hc_launch_score(const hc_kparams& P, const hc_launch_cfg& cfg, cudaStream_t st);
 cudaError_t hc_launch_exact(const hc_kparams& P, cudaStream_t st);
 cudaError_t hc_launch_tile_runs(const uint32_t* run_start, uint32_t n_runs, uint32_t* tile_run, cudaStream_t st);
 // small_out: d_edges receives hc_edge_small (hc_edge_small_exact with P.exact_edges) records and d_bits one bit per candidate
-// of the batch (1 = non-edge overlap) instead of the index list
+// of the batch (1 = non-edge overlap) instead of the index list.  kept != NULL (small_out, P.cand holds hc_candidate): kept
+// mode, d_edges receives the batch's edges from index 0 and no non-edge list or bit map is written
 cudaError_t hc_launch_compact(const hc_kparams& P, hc_edge* d_edges, uint64_t edges_cap, uint64_t* d_nonedge,
                               uint64_t nonedge_cap, uint32_t* d_blockcounts, uint64_t cand_offset, unsigned long long* d_run,
-                              cudaStream_t st, int small_out = 0, uint32_t* d_bits = nullptr);
+                              cudaStream_t st, int small_out = 0, uint32_t* d_bits = nullptr, const hc_kept_dev* kept = nullptr);
 cudaError_t hc_score_occupancy(uint32_t ncodes, int sm_count, size_t smem_per_sm, hc_launch_cfg* cfg);
 uint32_t hc_compact_blocks(uint64_t n);
 

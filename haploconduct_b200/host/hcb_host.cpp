@@ -879,7 +879,11 @@ inline void put_rec_line(std::string& b, const hc_overlap_rec& r) {
 }  // namespace
 
 bool EdgeCalculator::construct_edges_arrays() {
-    if (fastq_->max_read_len >= (1u << 14) || fastq_->m_read_vec.size() >= (1ull << 31)) return false;   // needs the 8-byte records
+    // one device: parse and score in one call, no limit on read lengths; more devices: the 8-byte run records, which
+    // hc_score_batch_runs_small shards over the devices
+    hc_store* const store = fastq_->device_store();
+    const bool one_call = hc_store_n_devices(store) == 1;
+    if (!one_call && (fastq_->max_read_len >= (1u << 14) || fastq_->m_read_vec.size() >= (1ull << 31))) return false;   // needs the 8-byte records
     const int T = std::max(1, omp_get_max_threads());
     // HC_MIRROR_TIMING=1: wall clock of every step of this function on stderr
     const bool timing = getenv("HC_MIRROR_TIMING") != nullptr;
@@ -903,10 +907,6 @@ bool EdgeCalculator::construct_edges_arrays() {
     for (long long i = 0; i < (long long)got; i++) lines += text[i] == '\n';
     (void)t0r;
     mark("file read + line count");
-    // ---- parse + pre-filter + id lookup on the device
-    std::unique_ptr<hc_candidate[]> cand(new hc_candidate[lines]);
-    size_t filt_cap = std::max<size_t>(lines / 8, 4096);
-    std::unique_ptr<hc_overlap_rec[]> filt(new hc_overlap_rec[filt_cap]);
     hc_ingest_params ip;
     memset(&ip, 0, sizeof(ip));
     ip.max_overlaps = ps_.max_overlaps;
@@ -914,73 +914,127 @@ bool EdgeCalculator::construct_edges_arrays() {
     ip.relax_PE_edges = ps_.relax_PE_edges; ip.allow_spaces = ps_.allow_spaces;
     hc_ingest_stats st;
     hc_idmap* idmap = fastq_->device_idmap();
-    int rc = hc_ingest_overlaps(idmap, text.get(), got, &ip, cand.get(), nullptr, lines, filt.get(), nullptr, filt_cap, &st);
-    if (rc == HC_ERR_CAPACITY) {
-        filt_cap = st.n_filtered + 1;
-        filt.reset(new hc_overlap_rec[filt_cap]);
-        rc = hc_ingest_overlaps(idmap, text.get(), got, &ip, cand.get(), nullptr, lines, filt.get(), nullptr, filt_cap, &st);
-    }
-    if (rc != HC_OK) die(std::string("hc_ingest_overlaps: ") + hc_last_error());
-    parse_device_ms += st.device_ms;
-    if (st.first_error_line != ~0ull) return false;      // the line-by-line path reproduces what the reference does up to that line
-    const size_t n = st.n_scored;
-    mark("hc_ingest_overlaps");
-    const double t1 = wall_s();
-    t_ingest_s += t1 - t0;
-    bool fits = true;
-#pragma omp parallel for schedule(static) reduction(&& : fits)
-    for (long long i = 0; i < (long long)n; i++) fits = fits && cand[i].pos1 < (1u << 14) && cand[i].pos2 < (1u << 14);
-    if (!fits) return false;
-    for (uint64_t k = 0; k < st.n_skipped; k++) std::cout << "incorrect overlap; skipping" << std::endl;   // :600-603
-    // ---- run-encoded records: a run = a stretch of candidates with the same smaller read index (an overlaps file sorted by
-    // read gives long runs; any list gives valid ones), cut by every thread in its own share
-    std::unique_ptr<hc_candidate_entry[]> en(new hc_candidate_entry[n ? n : 1]);
-    std::vector<std::vector<uint64_t>> t_start(T);
-    std::vector<uint32_t> anchor;
-    std::vector<uint64_t> start;
-#pragma omp parallel num_threads(T)
-    {
-        const int t = omp_get_thread_num();
-        const size_t lo = n * (size_t)t / (size_t)T, hi = n * (size_t)(t + 1) / (size_t)T;
-        std::vector<uint64_t>& mine = t_start[t];
-        for (size_t i = lo; i < hi; i++) {
-            const hc_candidate& c = cand[i];
-            const uint32_t key = std::min(c.idx1, c.idx2);
-            if (i == 0 || key != std::min(cand[i - 1].idx1, cand[i - 1].idx2)) mine.push_back(i);
-            const uint32_t o = c.ord == '1' ? 1u : (c.ord == '2' ? 2u : 0u);
-            en[i].other = c.idx1 == key ? c.idx2 : (c.idx1 | 0x80000000u);
-            en[i].pos = c.pos1 | (c.pos2 << 14) | ((uint32_t)(c.ori1 != 0) << 28) | ((uint32_t)(c.ori2 != 0) << 29) | (o << 30);
-        }
-    }
-    for (int t = 0; t < T; t++) start.insert(start.end(), t_start[t].begin(), t_start[t].end());
-    anchor.resize(start.size());
-#pragma omp parallel for schedule(static)
-    for (long long r = 0; r < (long long)start.size(); r++) anchor[r] = std::min(cand[start[r]].idx1, cand[start[r]].idx2);
-    start.push_back(n);
-    mark("run-encoded records");
-    // ---- scoring: small outputs
+    size_t filt_cap = std::max<size_t>(lines / 8, 4096);
+    std::unique_ptr<hc_overlap_rec[]> filt(new hc_overlap_rec[filt_cap]);
     const hc_params p = to_params(ps_);
     const size_t erec = ps_.exact_scores ? sizeof(hc_edge_small_exact) : sizeof(hc_edge_small);
-    size_t ecap = std::max<size_t>(n / 4, 1024);
-    std::unique_ptr<char[]> ebuf(new char[ecap * erec]);
-    std::unique_ptr<uint64_t[]> bits(new uint64_t[n / 64 + 2]);
+    // what the rest works on: candidates (the edge records' `cand` indexes them), the non-edge bit map over them, edges
+    std::unique_ptr<hc_candidate[]> cand;
+    std::unique_ptr<uint64_t[]> bits;
+    std::unique_ptr<char[]> ebuf;
+    size_t n = 0;
     uint64_t ne = 0, nn = 0;
-    hc_batch_stats bst;
-    memset(&bst, 0, sizeof(bst));
-    if (n) {
-        rc = hc_score_batch_runs_small(fastq_->device_store(), &p, anchor.data(), start.data(), anchor.size(), en.get(), n, ebuf.get(), ecap, &ne,
-                                       bits.get(), &nn, &bst);
+    int rc = HC_OK;
+    double t1 = 0;
+    if (one_call) {
+        // ---- parse + pre-filter + id lookup + scoring on the device; only the candidates scored as edges or non-edges
+        // come back (with their class), and the edge records name them
+        t_ingest_s += wall_s() - t0;
+        t1 = wall_s();
+        size_t kcap = std::max<size_t>(lines / 2, 4096), ecap = std::max<size_t>(lines / 8, 1024);
+        std::unique_ptr<uint8_t[]> kcls(new uint8_t[kcap]);
+        cand.reset(new hc_candidate[kcap]);
+        ebuf.reset(new char[ecap * erec]);
+        hc_ingest_score_stats ss;
+        rc = hc_ingest_score_overlaps(store, idmap, text.get(), got, &ip, &p, cand.get(), nullptr, kcls.get(), kcap, ebuf.get(), ecap,
+                                      filt.get(), nullptr, filt_cap, &ss);
         if (rc == HC_ERR_CAPACITY) {
-            ecap = ne;
-            ebuf.reset(new char[ecap * erec]);
-            rc = hc_score_batch_runs_small(fastq_->device_store(), &p, anchor.data(), start.data(), anchor.size(), en.get(), n, ebuf.get(), ecap,
-                                           &ne, bits.get(), &nn, &bst);
+            if (ss.n_kept > kcap) { kcap = ss.n_kept; kcls.reset(new uint8_t[kcap]); cand.reset(new hc_candidate[kcap]); }
+            if (ss.score.n_edges > ecap) { ecap = ss.score.n_edges; ebuf.reset(new char[ecap * erec]); }
+            if (ss.ingest.n_filtered > filt_cap) { filt_cap = ss.ingest.n_filtered; filt.reset(new hc_overlap_rec[filt_cap]); }
+            rc = hc_ingest_score_overlaps(store, idmap, text.get(), got, &ip, &p, cand.get(), nullptr, kcls.get(), kcap, ebuf.get(), ecap,
+                                          filt.get(), nullptr, filt_cap, &ss);
         }
-        if (rc != HC_OK) die(std::string("hc_score_batch_runs_small: ") + hc_last_error());
+        if (rc != HC_OK) die(std::string("hc_ingest_score_overlaps: ") + hc_last_error());
+        st = ss.ingest;
+        parse_device_ms += st.device_ms;
+        if (st.first_error_line != ~0ull) return false;      // the line-by-line path reproduces what the reference does up to that line
+        n = ss.n_kept;
+        ne = ss.score.n_edges;
+        nn = ss.score.n_nonedges;
+        bool overflow = false;
+#pragma omp parallel for schedule(static) reduction(|| : overflow)
+        for (long long k = 0; k < (long long)ne; k++) overflow = overflow || (reinterpret_cast<const hc_edge_small*>(ebuf.get() + (size_t)k * erec)->flags & HC_EDGE_OVERFLOW);
+        if (overflow) return false;                          // a window of 65536+ positions: the batch path scores it
+        const size_t words = (n + 63) / 64;
+        bits.reset(new uint64_t[words + 1]);
+#pragma omp parallel for schedule(static)
+        for (long long w = 0; w < (long long)words; w++) {
+            uint64_t b = 0;
+            for (size_t i = (size_t)w * 64; i < std::min(n, (size_t)w * 64 + 64); i++) b |= (uint64_t)(kcls[i] == HC_CLASS_NONEDGE) << (i & 63);
+            bits[w] = b;
+        }
+        scored_candidates += st.n_scored;
+        device_ms += ss.score.total_ms;
+        for (uint64_t k = 0; k < st.n_skipped; k++) std::cout << "incorrect overlap; skipping" << std::endl;   // :600-603
+        mark("hc_ingest_score_overlaps");
+    } else {
+        cand.reset(new hc_candidate[lines]);
+        rc = hc_ingest_overlaps(idmap, text.get(), got, &ip, cand.get(), nullptr, lines, filt.get(), nullptr, filt_cap, &st);
+        if (rc == HC_ERR_CAPACITY) {
+            filt_cap = st.n_filtered + 1;
+            filt.reset(new hc_overlap_rec[filt_cap]);
+            rc = hc_ingest_overlaps(idmap, text.get(), got, &ip, cand.get(), nullptr, lines, filt.get(), nullptr, filt_cap, &st);
+        }
+        if (rc != HC_OK) die(std::string("hc_ingest_overlaps: ") + hc_last_error());
+        parse_device_ms += st.device_ms;
+        if (st.first_error_line != ~0ull) return false;      // the line-by-line path reproduces what the reference does up to that line
+        n = st.n_scored;
+        mark("hc_ingest_overlaps");
+        t1 = wall_s();
+        t_ingest_s += t1 - t0;
+        bool fits = true;
+#pragma omp parallel for schedule(static) reduction(&& : fits)
+        for (long long i = 0; i < (long long)n; i++) fits = fits && cand[i].pos1 < (1u << 14) && cand[i].pos2 < (1u << 14);
+        if (!fits) return false;
+        for (uint64_t k = 0; k < st.n_skipped; k++) std::cout << "incorrect overlap; skipping" << std::endl;   // :600-603
+        // ---- run-encoded records: a run = a stretch of candidates with the same smaller read index (an overlaps file sorted by
+        // read gives long runs; any list gives valid ones), cut by every thread in its own share
+        std::unique_ptr<hc_candidate_entry[]> en(new hc_candidate_entry[n ? n : 1]);
+        std::vector<std::vector<uint64_t>> t_start(T);
+        std::vector<uint32_t> anchor;
+        std::vector<uint64_t> start;
+#pragma omp parallel num_threads(T)
+        {
+            const int t = omp_get_thread_num();
+            const size_t lo = n * (size_t)t / (size_t)T, hi = n * (size_t)(t + 1) / (size_t)T;
+            std::vector<uint64_t>& mine = t_start[t];
+            for (size_t i = lo; i < hi; i++) {
+                const hc_candidate& c = cand[i];
+                const uint32_t key = std::min(c.idx1, c.idx2);
+                if (i == 0 || key != std::min(cand[i - 1].idx1, cand[i - 1].idx2)) mine.push_back(i);
+                const uint32_t o = c.ord == '1' ? 1u : (c.ord == '2' ? 2u : 0u);
+                en[i].other = c.idx1 == key ? c.idx2 : (c.idx1 | 0x80000000u);
+                en[i].pos = c.pos1 | (c.pos2 << 14) | ((uint32_t)(c.ori1 != 0) << 28) | ((uint32_t)(c.ori2 != 0) << 29) | (o << 30);
+            }
+        }
+        for (int t = 0; t < T; t++) start.insert(start.end(), t_start[t].begin(), t_start[t].end());
+        anchor.resize(start.size());
+#pragma omp parallel for schedule(static)
+        for (long long r = 0; r < (long long)start.size(); r++) anchor[r] = std::min(cand[start[r]].idx1, cand[start[r]].idx2);
+        start.push_back(n);
+        mark("run-encoded records");
+        // ---- scoring: small outputs
+        size_t ecap = std::max<size_t>(n / 4, 1024);
+        ebuf.reset(new char[ecap * erec]);
+        bits.reset(new uint64_t[n / 64 + 2]);
+        hc_batch_stats bst;
+        memset(&bst, 0, sizeof(bst));
+        if (n) {
+            rc = hc_score_batch_runs_small(store, &p, anchor.data(), start.data(), anchor.size(), en.get(), n, ebuf.get(), ecap, &ne,
+                                           bits.get(), &nn, &bst);
+            if (rc == HC_ERR_CAPACITY) {
+                ecap = ne;
+                ebuf.reset(new char[ecap * erec]);
+                rc = hc_score_batch_runs_small(store, &p, anchor.data(), start.data(), anchor.size(), en.get(), n, ebuf.get(), ecap,
+                                               &ne, bits.get(), &nn, &bst);
+            }
+            if (rc != HC_OK) die(std::string("hc_score_batch_runs_small: ") + hc_last_error());
+        }
+        scored_candidates += n;
+        device_ms += bst.total_ms;
+        mark("hc_score_batch_runs_small");
     }
-    scored_candidates += n;
-    device_ms += bst.total_ms;
-    mark("hc_score_batch_runs_small");
     const double t2 = wall_s();
     t_score_s += t2 - t1;
     // ---- nonedge_overlaps.txt: the scored non-edges (bit map) in file order, then the pre-filtered lines (:546-555, :654-660);

@@ -573,6 +573,44 @@ int hc_ingest_overlaps_device(const hc_idmap* m, void* stream, const char* d_tex
                               hc_overlap_rec* d_filtered, uint64_t* d_filtered_line, uint64_t filtered_cap,
                               hc_ingest_stats* stats);
 
+/* Ingestion and scoring in one call: the text goes to the device, is parsed there and its candidates are scored there;
+ * only the candidates scored as edges or non-edges, their edge records and the pre-filtered overlaps come back.  This is
+ * EdgeCalculator::construct_edges (src/EdgeCalculator.cpp:561-666) up to the graph insert, for a host that keeps no
+ * candidate list of its own.
+ * Inputs
+ *   text          host memory (pageable or pinned) holding complete lines, as for hc_ingest_overlaps.  Parsing, the
+ *                 pre-filter, max_overlaps and the id lookup are those of hc_ingest_overlaps with `ip`; scoring is that of
+ *                 hc_score_batch* with `p`, applied to the candidates the parser passes on.  Full hc_candidate records are
+ *                 scored: no limit on read lengths or on the number of reads beyond the store's own.
+ *   The work runs on the id map's device, where the store must have a replica (else HC_ERR_ARG).
+ * Outputs, all in file order
+ *   kept[k], kept_line[k], kept_class[k]   the scored candidates classified HC_CLASS_EDGE or HC_CLASS_NONEDGE, their 0-based
+ *                 line in the text and their class.  Candidates classified HC_CLASS_DISCARD never leave the device.
+ *   edges         hc_edge_small records (hc_edge_small_exact under HC_FLAG_EXACT_EDGE_SCORES); `cand` is the index of the
+ *                 edge's candidate in kept[].  Every other field equals what hc_score_batch_short_small returns for the same
+ *                 candidate, HC_EDGE_OVERFLOW included, so an Edge follows from kept[cand] as described above hc_edge_small.
+ *   filtered, filtered_line   as from hc_ingest_overlaps.
+ *   kept_line and filtered_line may be NULL; an output pointer may be NULL when its capacity is 0.
+ * Errors
+ *   Lines after the first error line are still classified and scored; stats->ingest.first_error_* reports that line and the
+ *   caller decides (as for hc_ingest_overlaps).  A candidate the scorer rejects (e.g. a P-P candidate with ORD '-', an index
+ *   outside the store) gives HC_ERR_ARG with the message of hc_score_batch*.  2^32 or more kept candidates give HC_ERR_ARG
+ *   (cand is 32 bits).  A capacity that is too small gives HC_ERR_CAPACITY with the required sizes in stats->n_kept,
+ *   stats->score.n_edges and stats->ingest.n_filtered. */
+typedef struct {
+    hc_ingest_stats ingest;    /* what hc_ingest_overlaps reports for the same text and parameters                      */
+    hc_batch_stats  score;     /* what hc_score_batch* reports for the candidates the ingestion passed on (times: summed
+                                  over the pieces the text is cut into; total_ms: the whole call)                          */
+    uint64_t        n_kept;    /* scored candidates classified edge or non-edge (score.n_edges + score.n_nonedges)         */
+} hc_ingest_score_stats;       /* 152 bytes */
+
+int hc_ingest_score_overlaps(hc_store* s, const hc_idmap* m, const char* text, uint64_t n_bytes,
+                             const hc_ingest_params* ip, const hc_params* p,
+                             hc_candidate* kept, uint64_t* kept_line /* nullable */, uint8_t* kept_class, uint64_t kept_cap,
+                             void* edges, uint64_t edges_cap,
+                             hc_overlap_rec* filtered, uint64_t* filtered_line /* nullable */, uint64_t filtered_cap,
+                             hc_ingest_score_stats* stats);
+
 /* ------------------------------------------------------------------------------------------
  * Super-read consensus (third "next" row, SURVEY 8f): SRBuilder::consensus + consensus_pos,
  * src/SRBuilder.cpp:297-522, for many pile-ups at once.
