@@ -12,7 +12,7 @@ LIB = os.path.join(LIBDIR, "libhc_b200.so")
 NVCC = os.environ.get("HC_NVCC", "/usr/local/cuda/bin/nvcc")
 HOST_CXX = "/usr/bin/g++"
 
-CU_SOURCES = ["hc_kernels.cu", "hc_api.cu", "hc_fno.cu", "hc_dedup.cu", "hc_ingest.cu", "hc_pack.cu", "hc_consensus.cu", "hc_stage.cu", "hc_adjacency.cu"]
+CU_SOURCES = ["hc_kernels.cu", "hc_api.cu", "hc_fno.cu", "hc_fno_text.cu", "hc_dedup.cu", "hc_ingest.cu", "hc_pack.cu", "hc_consensus.cu", "hc_stage.cu", "hc_adjacency.cu"]
 CPP_SOURCES = ["hc_tables.cpp", "hc_cons_final.cpp"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 

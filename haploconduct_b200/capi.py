@@ -22,7 +22,7 @@ EXPORTED = [
     "hc_store_create", "hc_store_destroy", "hc_store_n_reads", "hc_store_n_single", "hc_store_n_devices",
     "hc_store_device_bytes", "hc_store_quality_alphabet", "hc_score_batch", "hc_score_batch_compact", "hc_score_batch_short", "hc_score_batch_runs", "hc_score_batch_runs_small", "hc_score_batch_runs6_small", "hc_score_batch_short_small", "hc_edge_extra_pos", "hc_score_batch_device",
     "hc_overlap_score", "hc_overlap_score_multi",
-    "hc_phred_to_prob", "hc_exp_threshold", "hc_device_count", "hc_warm_up", "hc_last_error", "hc_version", "hc_fno1", "hc_fno3", "hc_fno1_small", "hc_fno3_small", "hc_build_adjacency", "hc_subread_info", "hc_host_alloc", "hc_host_free",
+    "hc_phred_to_prob", "hc_exp_threshold", "hc_device_count", "hc_warm_up", "hc_last_error", "hc_version", "hc_fno1", "hc_fno3", "hc_fno1_small", "hc_fno3_small", "hc_fno1_text", "hc_fno3_text", "hc_build_adjacency", "hc_subread_info", "hc_host_alloc", "hc_host_free",
     "hc_store_create_fastq", "hc_store_create_fastq_files", "hc_store_read_ids", "hc_consensus", "hc_dedup_edges", "hc_idmap_create", "hc_idmap_destroy", "hc_ingest_overlaps", "hc_ingest_overlaps_device",
     "hc_ingest_score_overlaps",
 ]
@@ -109,6 +109,10 @@ def lib() -> ctypes.CDLL:
         L.hc_fno1_small.argtypes = L.hc_fno1.argtypes
         L.hc_fno3_small.restype = i32
         L.hc_fno3_small.argtypes = L.hc_fno3.argtypes
+        L.hc_fno1_text.restype = i32
+        L.hc_fno1_text.argtypes = [vp, vp, u64, vp, u64, ctypes.POINTER(u64), ctypes.POINTER(u64), ctypes.POINTER(u64), i32]
+        L.hc_fno3_text.restype = i32
+        L.hc_fno3_text.argtypes = [u64, vp, vp, vp, u64, vp, i32, vp, u64, ctypes.POINTER(u64), ctypes.POINTER(u64), i32]
         L.hc_dedup_edges.restype = i32
         L.hc_dedup_edges.argtypes = [vp, u64, i32, vp, vp, u64, vp, i32]
         L.hc_idmap_create.restype = vp
@@ -412,13 +416,19 @@ def fno_small_to_overlaps(r: np.ndarray) -> np.ndarray:
     return o
 
 
-def fno1(fi: "F.FnoInput", device: int = 0, small: bool = False) -> np.ndarray:
-    """hc_fno1 (small: hc_fno1_small, decoded): next-iteration overlaps derived on the GPU, in processing order
-    (formats.FNO_OVERLAP)."""
+def _fno_input_c(fi: "F.FnoInput"):
+    """hc_fno_input for fi, and the arrays it points into (keep them alive while it is used)."""
     keep = [np.ascontiguousarray(a) for a in (fi.visited, fi.label, fi.vertex_read, fi.sr_off, fi.sr_idx, fi.sr_sub, fi.superread)]
     st = _FnoInputC(len(fi.visited), keep[0].ctypes.data, keep[1].ctypes.data, keep[2].ctypes.data, keep[3].ctypes.data,
                     keep[4].ctypes.data, keep[5].ctypes.data, len(fi.superread), keep[6].ctypes.data, fi.resolve_orientations,
                     fi.no_inclusions)
+    return st, keep
+
+
+def fno1(fi: "F.FnoInput", device: int = 0, small: bool = False) -> np.ndarray:
+    """hc_fno1 (small: hc_fno1_small, decoded): next-iteration overlaps derived on the GPU, in processing order
+    (formats.FNO_OVERLAP)."""
+    st, keep = _fno_input_c(fi)
     edges = np.ascontiguousarray(fi.edges)
     cap = max(2 * len(edges), 1024)
     fn = lib().hc_fno1_small if small else lib().hc_fno1
@@ -448,6 +458,34 @@ def fno3(fi: "F.Fno3Input", device: int = 0, small: bool = False) -> np.ndarray:
         if rc != -5:
             raise HcError(rc, last_error())
         cap = int(n.value)
+
+
+def _text_call(call, cap: int) -> bytes:
+    while True:
+        out = np.empty(max(cap, 1), dtype=np.uint8)
+        nb, nl = ctypes.c_uint64(0), ctypes.c_uint64(0)
+        rc = call(out.ctypes.data, cap, ctypes.byref(nb), ctypes.byref(nl))
+        if rc == 0:
+            return out[: nb.value].tobytes()
+        if rc != -5:
+            raise HcError(rc, last_error())
+        cap = int(nb.value)
+
+
+def fno1_text(fi: "F.FnoInput", device: int = 0) -> bytes:
+    """hc_fno1_text: the reference's overlaps.txt (unique lines in byte order, each ending in a newline), built on the GPU."""
+    st, keep = _fno_input_c(fi)
+    edges = np.ascontiguousarray(fi.edges)
+    return _text_call(lambda p, cap, nb, nl: lib().hc_fno1_text(ctypes.byref(st), edges.ctypes.data if len(edges) else None, len(edges),
+                                                                 p, cap, nb, nl, None, device), max(96 * len(edges), 4096))
+
+
+def fno3_text(fi: "F.Fno3Input", device: int = 0) -> bytes:
+    """hc_fno3_text: the lines of hc_fno3's overlaps in discovery order, each ending in a newline, built on the GPU."""
+    off, idx, pos, reads = (np.ascontiguousarray(a) for a in (fi.off, fi.sr_idx, fi.sr_pos, fi.reads))
+    return _text_call(lambda p, cap, nb, nl: lib().hc_fno3_text(len(off) - 1, off.ctypes.data, idx.ctypes.data, pos.ctypes.data,
+                                                                 len(reads), reads.ctypes.data, fi.no_inclusions, p, cap, nb, nl,
+                                                                 device), 1 << 16)
 
 
 ADJ_EDGE = np.dtype([("vertex1", "<u4"), ("vertex2", "<u4"), ("nonoverlap_len", "<u4"), ("reserved", "<u4")])   # hc_adj_edge

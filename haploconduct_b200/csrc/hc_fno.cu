@@ -30,6 +30,7 @@
 #include <string>
 #include <cuda_runtime.h>
 #include "../../include/hc_b200.h"
+#include "hc_fno_text.h"
 #include "hc_scan.cuh"
 #include "hc_stage.h"
 
@@ -602,47 +603,19 @@ thread_local std::string g_fno_err;
 
 }  // namespace
 
-extern "C" const char* hc_last_error(void);
-void hc_set_last_error(const char* msg);   // hc_api.cu
-
-#define FCU(call)                                                                         \
-    do {                                                                                  \
-        cudaError_t _e = (call);                                                          \
-        if (_e != cudaSuccess) {                                                          \
-            hc_set_last_error((std::string(#call) + ": " + cudaGetErrorString(_e)).c_str()); \
-            rc = HC_ERR_CUDA;                                                             \
-            goto done;                                                                    \
-        }                                                                                 \
-    } while (0)
-
-// HC_FNO_TIMING=1: phase times on stderr (synchronises the device at every mark)
-struct FnoPhase {
-    bool on;
-    double t0;
-    const char* who;
-    static double now() { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6; }
-    explicit FnoPhase(const char* w) : on(getenv("HC_FNO_TIMING") != nullptr), t0(0), who(w) { if (on) t0 = now(); }
-    void mark(const char* what) {
-        if (!on) return;
-        cudaDeviceSynchronize();
-        const double t = now();
-        fprintf(stderr, "[%s] %-28s %8.2f ms\n", who, what, t - t0);
-        t0 = t;
-    }
-};
-
 static bool fno_force_big() { const char* v = getenv("HC_FNO_STAGE48"); return v && *v && *v != '0'; }
 
 // Winners are known (d_win); stage the successful attempts, rank them, move them to the output.  `resolve(small)` launches
-// the resolve kernel with the given staging format.  out48 / out24: exactly one is non-null.
+// the resolve kernel with the given staging format.  Exactly one of out48 / out24 / txt is non-null; with txt the compacted
+// records stay on the device (24-byte ones unless a value needed 48-byte staging) and fno_text turns them into the file.
 template <class Resolve>
-static int fno_finish(Resolve resolve, u64 attempts, hc_fno_overlap* out48, hc_fno_overlap_small* out24, u64 out_cap, uint64_t* n_out,
-                      FnoPhase& ph, const char* who) {
+static int fno_finish(Resolve resolve, u64 attempts, hc_fno_overlap* out48, hc_fno_overlap_small* out24, const FnoText* txt,
+                      u64 out_cap, uint64_t* n_out, FnoPhase& ph, const char* who) {
     int rc = HC_OK;
     uint32_t *d_flags = nullptr, *d_ovf = nullptr, ovf = 0;
     u64 *d_outpos = nullptr, *d_total = nullptr, *d_bsum = nullptr, produced = 0;
     void *d_rec = nullptr, *d_out = nullptr;
-    bool small = !fno_force_big();
+    bool small = !fno_force_big(), out_small;
     FCU(hc_scratch_alloc((void**)&d_flags, attempts * sizeof(uint32_t))); FCU(hc_scratch_alloc((void**)&d_outpos, attempts * sizeof(u64)));
     FCU(hc_scratch_alloc((void**)&d_ovf, sizeof(uint32_t))); FCU(hc_scratch_alloc((void**)&d_total, sizeof(u64)));
     FCU(hc_scratch_alloc((void**)&d_bsum, hc_scan::blocks_for(attempts) * sizeof(u64)));
@@ -667,19 +640,30 @@ static int fno_finish(Resolve resolve, u64 attempts, hc_fno_overlap* out48, hc_f
     hc_scan::exclusive_u32(d_flags, attempts, d_outpos, d_total, d_bsum, 0);
     FCU(cudaMemcpy(&produced, d_total, sizeof(u64), cudaMemcpyDeviceToHost));
     *n_out = produced;
-    if (produced > out_cap) {
+    if (!txt && produced > out_cap) {
         hc_set_last_error((std::string(who) + ": output buffer too small (required size returned in n_out)").c_str());
         rc = HC_ERR_CAPACITY;
         goto done;
     }
-    if (produced == 0) goto done;
-    FCU(hc_scratch_alloc(&d_out, produced * (out24 ? sizeof(Rec24) : sizeof(hc_fno_overlap))));
+    if (produced == 0) {
+        if (txt) rc = fno_text((const hc_fno_overlap_small*)nullptr, 0, *txt, ph, who);
+        goto done;
+    }
+    out_small = out24 || (txt && small);
+    FCU(hc_scratch_alloc(&d_out, produced * (out_small ? sizeof(Rec24) : sizeof(hc_fno_overlap))));
     ph.mark("scan of flags");
-    if (out24) fno_compact<true, true><<<148 * 16, 256>>>(d_flags, d_outpos, d_rec, attempts, d_out, produced);
+    if (out_small) fno_compact<true, true><<<148 * 16, 256>>>(d_flags, d_outpos, d_rec, attempts, d_out, produced);
     else if (small) fno_compact<true, false><<<148 * 16, 256>>>(d_flags, d_outpos, d_rec, attempts, d_out, produced);
     else fno_compact<false, false><<<148 * 16, 256>>>(d_flags, d_outpos, d_rec, attempts, d_out, produced);
     FCU(cudaGetLastError());
     ph.mark("fno_compact");
+    if (txt) {
+        hc_scratch_free(d_flags); hc_scratch_free(d_outpos); hc_scratch_free(d_rec);   // the text stage needs the room
+        d_flags = nullptr; d_outpos = nullptr; d_rec = nullptr;
+        if (out_small) rc = fno_text(static_cast<const hc_fno_overlap_small*>(d_out), produced, *txt, ph, who);
+        else rc = fno_text(static_cast<const hc_fno_overlap*>(d_out), produced, *txt, ph, who);
+        goto done;
+    }
     if (out24) FCU(hc_copy_d2h(out24, d_out, produced * sizeof(Rec24)));
     else FCU(hc_copy_d2h(out48, d_out, produced * sizeof(hc_fno_overlap)));
     ph.mark("copy out");
@@ -690,8 +674,8 @@ done:
 }
 
 static int fno1_impl(const hc_fno_input* in, const hc_fno_edge* edges, uint64_t n_edges, hc_fno_overlap* out48,
-                     hc_fno_overlap_small* out24, uint64_t out_cap, uint64_t* n_out, int device) {
-    const char* who = out24 ? "hc_fno1_small" : "hc_fno1";
+                     hc_fno_overlap_small* out24, const FnoText* txt, uint64_t out_cap, uint64_t* n_out, int device) {
+    const char* who = txt ? "hc_fno1_text" : (out24 ? "hc_fno1_small" : "hc_fno1");
     if (!in || !n_out || (n_edges && !edges) || (out_cap && !out48 && !out24)) { hc_set_last_error((std::string(who) + ": NULL argument").c_str()); return HC_ERR_ARG; }
     *n_out = 0;
     const u64 V = in->n_vertices, NS = in->n_superreads;
@@ -766,7 +750,7 @@ static int fno1_impl(const hc_fno_input* in, const hc_fno_edge* edges, uint64_t 
     rc = fno_finish([&](bool small, uint32_t* d_flags, void* d_rec, uint32_t* d_ovf) {
         if (small) fno_resolve<true><<<blocks, threads>>>(D, d_edges, n_edges, d_off, d_win, d_flags, d_rec, d_ovf);
         else fno_resolve<false><<<blocks, threads>>>(D, d_edges, n_edges, d_off, d_win, d_flags, d_rec, d_ovf);
-    }, attempts, out48, out24, out_cap, n_out, ph, who);
+    }, attempts, out48, out24, txt, out_cap, n_out, ph, who);
 done:
     hc_scratch_free(d_vis); hc_scratch_free(d_lab); hc_scratch_free(d_vr); hc_scratch_free(d_sr); hc_scratch_free(d_sroff); hc_scratch_free(d_sridx); hc_scratch_free(d_sub);
     hc_scratch_free(d_edges); hc_scratch_free(d_cnt); hc_scratch_free(d_off); hc_scratch_free(d_total); hc_scratch_free(d_keys);
@@ -776,18 +760,18 @@ done:
 
 extern "C" int hc_fno1(const hc_fno_input* in, const hc_fno_edge* edges, uint64_t n_edges, hc_fno_overlap* out, uint64_t out_cap,
                        uint64_t* n_out, int device) {
-    return fno1_impl(in, edges, n_edges, out, nullptr, out_cap, n_out, device);
+    return fno1_impl(in, edges, n_edges, out, nullptr, nullptr, out_cap, n_out, device);
 }
 
 extern "C" int hc_fno1_small(const hc_fno_input* in, const hc_fno_edge* edges, uint64_t n_edges, hc_fno_overlap_small* out,
                              uint64_t out_cap, uint64_t* n_out, int device) {
-    return fno1_impl(in, edges, n_edges, nullptr, out, out_cap, n_out, device);
+    return fno1_impl(in, edges, n_edges, nullptr, out, nullptr, out_cap, n_out, device);
 }
 
 static int fno3_impl(uint64_t n_originals, const uint64_t* off, const uint32_t* sr_idx, const hc_fno3_pos* sr_pos, uint64_t n_reads,
-                     const hc_fno_read* reads, int no_inclusions, hc_fno_overlap* out48, hc_fno_overlap_small* out24, uint64_t out_cap,
-                     uint64_t* n_out, int device) {
-    const char* who = out24 ? "hc_fno3_small" : "hc_fno3";
+                     const hc_fno_read* reads, int no_inclusions, hc_fno_overlap* out48, hc_fno_overlap_small* out24, const FnoText* txt,
+                     uint64_t out_cap, uint64_t* n_out, int device) {
+    const char* who = txt ? "hc_fno3_text" : (out24 ? "hc_fno3_small" : "hc_fno3");
     if (!n_out || (n_originals && (!off || !sr_idx || !sr_pos || !reads)) || (out_cap && !out48 && !out24)) {
         hc_set_last_error((std::string(who) + ": NULL argument").c_str());
         return HC_ERR_ARG;
@@ -837,7 +821,7 @@ static int fno3_impl(uint64_t n_originals, const uint64_t* off, const uint32_t* 
     rc = fno_finish([&](bool small, uint32_t* d_flags, void* d_rec, uint32_t* d_ovf) {
         if (small) fno3_resolve<true><<<blocks, threads>>>(d_off, n_originals, d_idx, d_pos, d_reads, (uint32_t)no_inclusions, d_seq, d_win, d_flags, d_rec, d_ovf);
         else fno3_resolve<false><<<blocks, threads>>>(d_off, n_originals, d_idx, d_pos, d_reads, (uint32_t)no_inclusions, d_seq, d_win, d_flags, d_rec, d_ovf);
-    }, attempts, out48, out24, out_cap, n_out, ph, who);
+    }, attempts, out48, out24, txt, out_cap, n_out, ph, who);
 done:
     hc_scratch_free(d_off); hc_scratch_free(d_idx); hc_scratch_free(d_pos); hc_scratch_free(d_reads); hc_scratch_free(d_cnt); hc_scratch_free(d_seq); hc_scratch_free(d_total);
     hc_scratch_free(d_keys); hc_scratch_free(d_bsum); hc_scratch_free(d_win);
@@ -847,11 +831,38 @@ done:
 extern "C" int hc_fno3(uint64_t n_originals, const uint64_t* off, const uint32_t* sr_idx, const hc_fno3_pos* sr_pos, uint64_t n_reads,
                        const hc_fno_read* reads, int no_inclusions, hc_fno_overlap* out, uint64_t out_cap, uint64_t* n_out,
                        int device) {
-    return fno3_impl(n_originals, off, sr_idx, sr_pos, n_reads, reads, no_inclusions, out, nullptr, out_cap, n_out, device);
+    return fno3_impl(n_originals, off, sr_idx, sr_pos, n_reads, reads, no_inclusions, out, nullptr, nullptr, out_cap, n_out, device);
 }
 
 extern "C" int hc_fno3_small(uint64_t n_originals, const uint64_t* off, const uint32_t* sr_idx, const hc_fno3_pos* sr_pos, uint64_t n_reads,
                              const hc_fno_read* reads, int no_inclusions, hc_fno_overlap_small* out, uint64_t out_cap, uint64_t* n_out,
                              int device) {
-    return fno3_impl(n_originals, off, sr_idx, sr_pos, n_reads, reads, no_inclusions, nullptr, out, out_cap, n_out, device);
+    return fno3_impl(n_originals, off, sr_idx, sr_pos, n_reads, reads, no_inclusions, nullptr, out, nullptr, out_cap, n_out, device);
+}
+
+// ---- overlaps.txt itself (hc_fno_text.cu) --------------------------------------------------------------------------------
+static bool text_args_ok(const char* who, const char* text, uint64_t text_cap, uint64_t* n_bytes, uint64_t* n_lines) {
+    if (!n_bytes || !n_lines || (text_cap && !text)) { hc_set_last_error((std::string(who) + ": NULL argument").c_str()); return false; }
+    *n_bytes = 0;
+    *n_lines = 0;
+    return true;
+}
+
+extern "C" int hc_fno1_text(const hc_fno_input* in, const hc_fno_edge* edges, uint64_t n_edges, char* text, uint64_t text_cap,
+                            uint64_t* n_bytes, uint64_t* n_lines, uint64_t* n_records, int device) {
+    if (!text_args_ok("hc_fno1_text", text, text_cap, n_bytes, n_lines)) return HC_ERR_ARG;
+    const FnoText t = {text, text_cap, n_bytes, n_lines, true};
+    uint64_t records = 0;
+    const int rc = fno1_impl(in, edges, n_edges, nullptr, nullptr, &t, 0, &records, device);
+    if (n_records) *n_records = records;
+    return rc;
+}
+
+extern "C" int hc_fno3_text(uint64_t n_originals, const uint64_t* off, const uint32_t* sr_idx, const hc_fno3_pos* sr_pos, uint64_t n_reads,
+                            const hc_fno_read* reads, int no_inclusions, char* text, uint64_t text_cap, uint64_t* n_bytes,
+                            uint64_t* n_lines, int device) {
+    if (!text_args_ok("hc_fno3_text", text, text_cap, n_bytes, n_lines)) return HC_ERR_ARG;
+    const FnoText t = {text, text_cap, n_bytes, n_lines, false};
+    uint64_t records = 0;
+    return fno3_impl(n_originals, off, sr_idx, sr_pos, n_reads, reads, no_inclusions, nullptr, nullptr, &t, 0, &records, device);
 }

@@ -356,7 +356,8 @@ double hc_exp_threshold(double threshold);
  * super-read containing u resp. v, by index arithmetic on the sub-read positions.  Per unordered
  * pair of new reads the FIRST derivation in processing order wins, even if it then fails
  * (:84-97 precede :115-118).  The host keeps the graph walk that produces the edge stream
- * (:605-631, :635-697, :816-887) and the sorted, de-duplicated text output (:937-953).
+ * (:605-631, :635-697, :816-887); hc_fno1_text / hc_fno3_text below also build the text of
+ * overlaps.txt on the device.
  * ------------------------------------------------------------------------------------------ */
 typedef struct {
     uint32_t u, v;            /* old vertices                                                      */
@@ -434,6 +435,21 @@ int hc_fno3(uint64_t n_originals, const uint64_t* off /* [n_originals+1] */, con
 int hc_fno3_small(uint64_t n_originals, const uint64_t* off, const uint32_t* sr_idx, const hc_fno3_pos* sr_pos,
                   uint64_t n_reads, const hc_fno_read* reads, int no_inclusions,
                   hc_fno_overlap_small* out, uint64_t out_cap, uint64_t* n_out, int device);
+
+/* The reference's overlaps.txt itself: the lines of the records hc_fno1 derives, formatted as
+ * "%lu\t%lu\t%d\t%d\t%c\t%c\t%c\t%d\t%d\t%d\t%d\t%c\t%c" (src/FindNextOverlaps.cpp:122-148), unique and in
+ * std::string (byte) order like the reference's std::set<std::string> (:918,:946-948); every line ends in '\n'.
+ * *n_bytes / *n_lines receive the size of the file and its line count, *n_records (nullable) the records before
+ * de-duplication.  HC_ERR_CAPACITY (sizes still written) if text_cap < *n_bytes; text may be NULL when text_cap is 0.
+ * The arguments are checked as by hc_fno1; HC_ERR_ARG also for 2^32 or more records.  Sorting, de-duplication and
+ * formatting run on the device; the text is the only thing copied back. */
+int hc_fno1_text(const hc_fno_input* in, const hc_fno_edge* edges, uint64_t n_edges,
+                 char* text, uint64_t text_cap, uint64_t* n_bytes, uint64_t* n_lines, uint64_t* n_records, int device);
+
+/* The same for hc_fno3: the lines in discovery order, not sorted, not de-duplicated (src/FindNextOverlaps3.cpp:139-166). */
+int hc_fno3_text(uint64_t n_originals, const uint64_t* off, const uint32_t* sr_idx, const hc_fno3_pos* sr_pos,
+                 uint64_t n_reads, const hc_fno_read* reads, int no_inclusions,
+                 char* text, uint64_t text_cap, uint64_t* n_bytes, uint64_t* n_lines, int device);
 
 /* ------------------------------------------------------------------------------------------
  * Duplicate-edge resolution of the graph insert (first "next" row, SURVEY 8f):

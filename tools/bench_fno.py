@@ -2,12 +2,20 @@
 """Throughput of FindNextOverlaps 1 on one B200 (hc_fno1, host buffers in and out) next to the pinned C restatement
 of the reference's sequential walk (oracle/fno_oracle.c, one host core) on the same input.
 
+The "text" leg times hc_fno1_text (overlaps.txt formatted, sorted and de-duplicated on the device) into a pinned and
+into a pageable buffer, checks its bytes once against the Python statement of the reference's std::set<std::string>,
+and times, on the same records, the host step it replaces (snprintf + std::set<std::string> + concatenation, as the
+C++ binding did it), compiled here with the build's host compiler.
+
     python tools/bench_fno.py [--edges 10000000] [--vertices 1000000] [--steps 5]
 Prints one JSON line."""
 import argparse
 import json
 import os
+import statistics
+import subprocess
 import sys
+import tempfile
 import time
 
 import numpy as np
@@ -15,7 +23,92 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
-from haploconduct_b200 import capi, formats as F  # noqa: E402
+from haploconduct_b200 import build as B, capi, formats as F  # noqa: E402
+
+HOST_FORMAT = r"""
+#include <chrono>
+#include <cstdio>
+#include <set>
+#include <string>
+#include "hc_b200.h"
+// the host step of the C++ binding before hc_fno1_text: one snprintf per record into a std::set<std::string>, then the
+// set's lines concatenated with '\n'
+extern "C" double host_format(const hc_fno_overlap* o, unsigned long long n, unsigned long long* bytes, unsigned long long* lines) {
+    const auto t0 = std::chrono::steady_clock::now();
+    std::set<std::string> set;
+    std::string line;
+    char buf[160];
+    for (unsigned long long k = 0; k < n; k++) {
+        const int m = std::snprintf(buf, sizeof(buf), "%lu\t%lu\t%d\t%d\t%c\t%c\t%c\t%d\t%d\t%d\t%d\t%c\t%c", (unsigned long)o[k].id1,
+                                    (unsigned long)o[k].id2, o[k].pos1, o[k].pos2, o[k].ord, o[k].ori1, o[k].ori2, o[k].perc, o[k].perc2,
+                                    o[k].len1, o[k].len2, o[k].type1, o[k].type2);
+        line.assign(buf, (size_t)m);
+        set.insert(line);
+    }
+    std::string out;
+    for (const std::string& l : set) { out.append(l); out.push_back('\n'); }
+    *bytes = out.size();
+    *lines = set.size();
+    return std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+}
+"""
+
+
+def gpu_info():
+    try:
+        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader", "-i", "0"],
+                             check=True, stdout=subprocess.PIPE, text=True).stdout.strip()
+        name, power, clock = [x.strip() for x in out.split(",")]
+        return {"name": name, "power_limit": power, "max_sm_clock": clock}
+    except Exception as e:          # the numbers are only worth something with the card they were taken on
+        return {"error": str(e)}
+
+
+def host_format_seconds(records: np.ndarray):
+    """(seconds, bytes, lines) of the replaced host step on `records` (formats.FNO_OVERLAP), built in a temporary directory."""
+    import ctypes
+    with tempfile.TemporaryDirectory() as d:
+        src, so = os.path.join(d, "host_format.cpp"), os.path.join(d, "host_format.so")
+        with open(src, "w") as f:
+            f.write(HOST_FORMAT)
+        subprocess.check_call([B.HOST_CXX, "-O2", "-std=c++14", "-shared", "-fPIC", "-I" + os.path.join(ROOT, "include"), src, "-o", so])
+        L = ctypes.CDLL(so)
+    L.host_format.restype = ctypes.c_double
+    L.host_format.argtypes = [ctypes.c_void_p, ctypes.c_uint64, ctypes.POINTER(ctypes.c_uint64), ctypes.POINTER(ctypes.c_uint64)]
+    rec = np.ascontiguousarray(records)
+    nb, nl = ctypes.c_uint64(0), ctypes.c_uint64(0)
+    dt = L.host_format(rec.ctypes.data, len(rec), ctypes.byref(nb), ctypes.byref(nl))
+    return dt, nb.value, nl.value
+
+
+def text_leg(fi: F.FnoInput, records: np.ndarray, steps: int) -> dict:
+    import ctypes
+    L = capi.lib()
+    st, keep = capi._fno_input_c(fi)
+    edges = np.ascontiguousarray(fi.edges)
+    text = capi.fno1_text(fi)                                      # warm-up; sizes the buffers
+    n = len(text)
+    pinned = capi.host_alloc(n)
+    pageable = np.empty(n, dtype=np.uint8)
+    pageable[:] = 0                                                # touched once: no page faults inside the timed calls
+    nb, nl, nr = ctypes.c_uint64(0), ctypes.c_uint64(0), ctypes.c_uint64(0)
+    t = {"pinned": [], "pageable": []}
+    for _ in range(steps):
+        for kind, buf in (("pinned", pinned), ("pageable", pageable)):
+            t0 = time.perf_counter()
+            rc = L.hc_fno1_text(ctypes.byref(st), edges.ctypes.data, len(edges), buf.ctypes.data, n, ctypes.byref(nb), ctypes.byref(nl),
+                                ctypes.byref(nr), 0)
+            t[kind].append(time.perf_counter() - t0)
+            assert rc == 0 and nb.value == n
+    assert pinned[:n].tobytes() == text and pageable.tobytes() == text
+    ref = sorted(set(F.fno_lines(records)), key=lambda s: s.encode())
+    identical = text == "".join(l + "\n" for l in ref).encode()
+    del ref
+    host_s, host_bytes, host_lines = host_format_seconds(records)
+    return {"ms_pinned": statistics.median(t["pinned"]) * 1e3, "ms_pageable": statistics.median(t["pageable"]) * 1e3,
+            "bytes": n, "lines": int(nl.value), "records": int(nr.value), "identical_to_sorted_set_of_lines": bool(identical),
+            "host_step_replaced": {"what": "snprintf + std::set<std::string> + concatenation, one host core, same records",
+                                   "s": host_s, "bytes": int(host_bytes), "lines": int(host_lines)}}
 
 
 def make_input(V: int, n_sr: int, n_edges: int, seed: int = 3, paired_fraction: float = 0.4) -> F.FnoInput:
@@ -65,6 +158,7 @@ def main():
     ap.add_argument("--vertices", type=int, default=1_000_000)
     ap.add_argument("--steps", type=int, default=5)
     ap.add_argument("--cpu-edges", type=int, default=2_000_000)
+    ap.add_argument("--no-text", action="store_true", help="skip the text leg")
     a = ap.parse_args()
     fi = make_input(a.vertices, a.vertices // 3, a.edges)
     import ctypes
@@ -95,7 +189,9 @@ def main():
            "records": "hc_fno1_small: 24-byte result records (the call of the C++ binding hcb::SRBuilder)",
            "ms_48_byte_records": min(t) * 1e3,
            "bytes_in": int(fi.edges.nbytes + fi.sr_sub.nbytes + fi.sr_idx.nbytes + fi.vertex_read.nbytes + fi.superread.nbytes),
-           "bytes_out": int(len(out) * 24), "bytes_out_48": int(out.nbytes)}
+           "bytes_out": int(len(out) * 24), "bytes_out_48": int(out.nbytes), "gpu": gpu_info()}
+    if not a.no_text:
+        res["text"] = text_leg(fi, out, a.steps)
     try:
         from oracle import oracle as O
         import copy
