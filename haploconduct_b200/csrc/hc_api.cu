@@ -99,6 +99,9 @@ struct DevCtx {
     cudaStream_t stream = nullptr, s_copy = nullptr, s_out = nullptr;
     cudaEvent_t ev_in[2] = {nullptr, nullptr}, ev_done[2] = {nullptr, nullptr}, ev_out[2] = {nullptr, nullptr};
     cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    // recorded at the end of every enqueue_batch: the next call waits for it (on its own stream, or on the host before it
+    // frees the workspace or rewrites the tables), so calls on different streams do not share the workspace at once
+    cudaEvent_t ws_event = nullptr;
     hc_launch_cfg cfg{};
 };
 
@@ -145,6 +148,7 @@ void free_ctx(DevCtx& d) {
     for (cudaEvent_t e : d.ev_step) cudaEventDestroy(e);
     if (d.h_cnt) cudaFreeHost(d.h_cnt);
     for (int k = 0; k < 6; k++) if (d.ev[k]) cudaEventDestroy(d.ev[k]);
+    if (d.ws_event) cudaEventDestroy(d.ws_event);
     if (d.stream) cudaStreamDestroy(d.stream);
     if (d.s_copy) cudaStreamDestroy(d.s_copy);
     if (d.s_out) cudaStreamDestroy(d.s_out);
@@ -163,13 +167,16 @@ int ensure_tables(hc_store* s, DevCtx& d, double mismatch, cudaStream_t st) {
         }
     }
     if (d.tables_valid && d.tables_mismatch == mismatch) return HC_OK;
-    // synchronous upload: tables change only when ps.mismatch changes (it never does in the drivers)
+    // tables change only when ps.mismatch changes (it never does in the drivers): wait on the host for every earlier call,
+    // whatever its stream, then upload on this call's stream, ahead of its kernels (a pageable source is staged before
+    // the copy returns, so the host tables may be rebuilt afterwards)
+    CU(cudaEventSynchronize(d.ws_event));
     CU(cudaStreamSynchronize(st));
     const std::vector<uint32_t>& fx = s->packed ? s->tables.fx_packed : s->tables.fx;
     if (!d.fx_table) CU(cudaMalloc(&d.fx_table, fx.size() * sizeof(uint32_t)));
     if (!d.dbl_table) CU(cudaMalloc(&d.dbl_table, s->tables.dbl.size() * sizeof(double)));
-    CU(cudaMemcpy(d.fx_table, fx.data(), fx.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(d.dbl_table, s->tables.dbl.data(), s->tables.dbl.size() * sizeof(double), cudaMemcpyHostToDevice));
+    CU(cudaMemcpyAsync(d.fx_table, fx.data(), fx.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d.dbl_table, s->tables.dbl.data(), s->tables.dbl.size() * sizeof(double), cudaMemcpyHostToDevice, st));
     d.tables_valid = true;
     d.tables_mismatch = mismatch;
     d.has_void = s->tables.has_void;
@@ -180,6 +187,7 @@ int ensure_tables(hc_store* s, DevCtx& d, double mismatch, cudaStream_t st) {
 int ensure_workspace(DevCtx& d, uint64_t n) {
     if (n <= d.ws_cap && d.counters) return HC_OK;
     uint64_t cap = std::max<uint64_t>(n, 1024);
+    CU(cudaEventSynchronize(d.ws_event));   // an earlier call on another stream may still be using the buffers
     cudaFree(d.tmp); cudaFree(d.cls); cudaFree(d.flagged); cudaFree(d.blockcounts);
     d.tmp = nullptr; d.cls = nullptr; d.flagged = nullptr; d.blockcounts = nullptr;
     d.ws_cap = 0;
@@ -213,6 +221,7 @@ int enqueue_batch(hc_store* s, DevCtx& d, cudaStream_t st, const hc_params* p, c
                   const hc_kept_dev* kept = nullptr) {
     if (n > 0xffffffffull) return fail(HC_ERR_ARG, "more than 2^32-1 candidates in one device batch");
     if (compact >= 3 && !runs) return fail(HC_ERR_ARG, "run-encoded candidates without run arrays");
+    CU(cudaStreamWaitEvent(st, d.ws_event, 0));   // the previous call's use of the workspace, whatever its stream
     int rc = ensure_tables(s, d, p->mismatch, st);
     if (rc != HC_OK) return rc;
     rc = ensure_workspace(d, n);
@@ -268,6 +277,7 @@ int enqueue_batch(hc_store* s, DevCtx& d, cudaStream_t st, const hc_params* p, c
         CU(cudaMemcpyAsync(d_counts, d.counters + HC_CNT_EDGES, 3 * sizeof(uint64_t), cudaMemcpyDeviceToDevice, st));
         CU(cudaMemcpyAsync(d_counts + 3, d.counters + HC_CNT_ERRORS, sizeof(uint64_t), cudaMemcpyDeviceToDevice, st));
     }
+    CU(cudaEventRecord(d.ws_event, st));
     if (launches) *launches = nl;
     return HC_OK;
 }
@@ -400,6 +410,7 @@ cudaError_t init_ctx(hc_store* s, DevCtx& d, int device, bool* not_sm100) {
     if (e == cudaSuccess) e = cudaMalloc(&d.d_run, 2 * sizeof(unsigned long long));
     if (e == cudaSuccess) e = cudaMallocHost(&d.h_cnt, 2 * HC_CNT_N * sizeof(unsigned long long));
     for (int j = 0; j < 6 && e == cudaSuccess; j++) e = cudaEventCreate(&d.ev[j]);
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&d.ws_event, cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaMalloc(&d.rdesc, s->n_reads * sizeof(hc_rdesc));
     if (e == cudaSuccess) e = cudaMalloc(&d.d_counts, 4 * sizeof(uint64_t));
     return e;
@@ -830,6 +841,10 @@ int hc_score_batch_device(hc_store* s, int device, void* stream, const hc_params
                           hc_result* d_per_cand, hc_edge* d_edges, uint64_t edges_cap, uint64_t* d_nonedge_idx,
                           uint64_t nonedge_cap, uint64_t* d_counts, hc_batch_stats* stats) {
     if (!s || !p || !d_counts || (n && !d_cand)) return fail(HC_ERR_ARG, "hc_score_batch_device: NULL argument");
+    // the kernels read a candidate as two 16-byte loads and store 8-byte aligned records: a misaligned pointer would fault
+    if (((uintptr_t)d_cand & 15u) || (((uintptr_t)d_per_cand | (uintptr_t)d_edges | (uintptr_t)d_nonedge_idx | (uintptr_t)d_counts) & 7u))
+        return fail(HC_ERR_ARG, "hc_score_batch_device: d_cand must be 16-byte aligned; d_per_cand, d_edges, d_nonedge_idx and "
+                                "d_counts 8-byte aligned");
     DevCtx* d = find_ctx(s, device);
     if (!d) return fail(HC_ERR_ARG, "hc_score_batch_device: the store has no replica on this device");
     CU(cudaSetDevice(device));

@@ -300,7 +300,21 @@ int hc_score_batch_short_small(hc_store* s, const hc_params* p,
 
 /* Same, but every buffer is DEVICE memory on device `device` (one of the store's devices) and the
  * work is enqueued on `stream` (a cudaStream_t passed as void*; NULL = default stream).
- * d_counts receives {n_edges, n_nonedges, n_exact, 0} as uint64_t[4].  Asynchronous unless stats != NULL.
+ * d_counts receives {n_edges, n_nonedges, n_exact, n_invalid} as uint64_t[4], where n_invalid counts the
+ * candidates with an invalid read index, a self overlap, or a P-P candidate whose ORD is not '1' or '2'
+ * (they are classified HC_CLASS_DISCARD).  With stats == NULL such a batch still returns HC_OK, so
+ * d_counts[3] is the caller's only sign of them; with stats != NULL the call returns HC_ERR_ARG.
+ * Asynchronous unless stats != NULL.
+ * Capacities: when edges_cap or nonedge_cap is smaller than the list, the first edges_cap / nonedge_cap
+ * records are written and the rest dropped; d_counts still holds the full counts and the call returns
+ * HC_OK (unlike the host-buffer calls, which return HC_ERR_CAPACITY).  An output pointer may be NULL when
+ * its capacity is 0.
+ * Alignment: d_cand must be 16-byte aligned; d_per_cand, d_edges, d_nonedge_idx and d_counts 8-byte
+ * aligned (cudaMalloc'ed buffers and whole records inside them are).  Anything else returns HC_ERR_ARG.
+ * Ordering: calls on one store (this one, hc_score_batch* and hc_ingest_score_overlaps) share a device
+ * workspace; each call's device work waits for the previous call's, whatever streams they use, so a
+ * caller needs no synchronisation between them.  This holds for calls made from one host thread;
+ * concurrent calls on one store from several host threads are not supported.
  * This is what the throughput benchmark times with inputs resident in HBM, and what a
  * device-side consumer (NCCL gather, GPU FindNextOverlaps) calls. */
 int hc_score_batch_device(hc_store* s, int device, void* stream, const hc_params* p,
@@ -582,8 +596,8 @@ int hc_ingest_overlaps(const hc_idmap* m, const char* text, uint64_t n_bytes, co
                        hc_candidate* cand, uint64_t* cand_line, uint64_t cand_cap,
                        hc_overlap_rec* filtered, uint64_t* filtered_line, uint64_t filtered_cap,
                        hc_ingest_stats* stats);
-/* The same on DEVICE buffers of the id map's device (d_text 16-byte aligned is fastest); the
- * candidates can be handed to hc_score_batch_device without leaving HBM. */
+/* The same on DEVICE buffers of the id map's device; d_text may have any alignment (16-byte aligned
+ * is fastest).  The candidates can be handed to hc_score_batch_device without leaving HBM. */
 int hc_ingest_overlaps_device(const hc_idmap* m, void* stream, const char* d_text, uint64_t n_bytes,
                               const hc_ingest_params* p, hc_candidate* d_cand, uint64_t* d_cand_line, uint64_t cand_cap,
                               hc_overlap_rec* d_filtered, uint64_t* d_filtered_line, uint64_t filtered_cap,
