@@ -24,7 +24,7 @@ EXPORTED = [
     "hc_overlap_score", "hc_overlap_score_multi",
     "hc_phred_to_prob", "hc_exp_threshold", "hc_device_count", "hc_warm_up", "hc_last_error", "hc_version", "hc_fno1", "hc_fno3", "hc_fno1_small", "hc_fno3_small", "hc_fno1_text", "hc_fno3_text", "hc_build_adjacency", "hc_subread_info", "hc_host_alloc", "hc_host_free",
     "hc_store_create_fastq", "hc_store_create_fastq_files", "hc_store_read_ids", "hc_consensus", "hc_dedup_edges", "hc_idmap_create", "hc_idmap_destroy", "hc_ingest_overlaps", "hc_ingest_overlaps_device",
-    "hc_ingest_score_overlaps",
+    "hc_ingest_score_overlaps", "hc_fno1_text_nonedges",
 ]
 
 _lib: Optional[ctypes.CDLL] = None
@@ -125,6 +125,9 @@ def lib() -> ctypes.CDLL:
         L.hc_ingest_overlaps_device.argtypes = [vp, vp, vp, u64, vp, vp, vp, u64, vp, vp, u64, vp]
         L.hc_ingest_score_overlaps.restype = i32
         L.hc_ingest_score_overlaps.argtypes = [vp, vp, vp, u64, vp, vp, vp, vp, vp, u64, vp, u64, vp, vp, u64, vp]
+        L.hc_fno1_text_nonedges.restype = i32
+        L.hc_fno1_text_nonedges.argtypes = [vp, vp, vp, u64, u64, vp, u64, vp, u64, vp, u64, ctypes.POINTER(u64), ctypes.POINTER(u64),
+                                            ctypes.POINTER(u64), vp, i32]
         L.hc_last_error.restype = ctypes.c_char_p
         L.hc_version.restype = ctypes.c_char_p
         _lib = L
@@ -478,6 +481,32 @@ def fno1_text(fi: "F.FnoInput", device: int = 0) -> bytes:
     edges = np.ascontiguousarray(fi.edges)
     return _text_call(lambda p, cap, nb, nl: lib().hc_fno1_text(ctypes.byref(st), edges.ctypes.data if len(edges) else None, len(edges),
                                                                  p, cap, nb, nl, None, device), max(96 * len(edges), 4096))
+
+
+def fno1_text_nonedges(fi: "F.FnoInput", idmap: "IdMap", head: np.ndarray, n_adjacency: int, nonedge_text, tail: np.ndarray,
+                       device: int = 0, text_cap: Optional[int] = None):
+    """hc_fno1_text_nonedges: overlaps.txt of the stream head ++ (lines of nonedge_text that are not an edge of
+    head[:n_adjacency]) ++ tail, the non-edge lines parsed on the GPU (fi.edges is not read).  nonedge_text: bytes or a
+    uint8 array (e.g. a slice of host_alloc memory).  Returns (rc, text, n_lines, n_records, stats of formats.FNO_NONEDGE_STATS);
+    with text_cap one call with that capacity (rc may be HC_ERR_CAPACITY), else the capacity is grown until the text fits.
+    Argument and input errors are returned in rc, not raised."""
+    st, keep = _fno_input_c(fi)
+    head = np.ascontiguousarray(head, dtype=F.FNO_EDGE)
+    tail = np.ascontiguousarray(tail, dtype=F.FNO_EDGE)
+    buf = np.frombuffer(nonedge_text, dtype=np.uint8) if isinstance(nonedge_text, (bytes, bytearray)) else nonedge_text
+    cap = max(96 * (len(head) + len(tail) + len(buf) // 40), 4096) if text_cap is None else text_cap
+    stats = np.zeros(1, dtype=F.FNO_NONEDGE_STATS)
+    while True:
+        out = np.empty(max(cap, 1), dtype=np.uint8)
+        nb, nl, nr = ctypes.c_uint64(0), ctypes.c_uint64(0), ctypes.c_uint64(0)
+        rc = lib().hc_fno1_text_nonedges(ctypes.byref(st), idmap.handle, head.ctypes.data if len(head) else None, len(head), n_adjacency,
+                                         buf.ctypes.data if len(buf) else None, len(buf), tail.ctypes.data if len(tail) else None,
+                                         len(tail), out.ctypes.data if cap else None, cap, ctypes.byref(nb), ctypes.byref(nl),
+                                         ctypes.byref(nr), stats.ctypes.data, device)
+        if rc == -5 and text_cap is None:
+            cap = int(nb.value)
+            continue
+        return rc, out[: nb.value].tobytes() if rc == 0 else b"", int(nl.value), int(nr.value), stats[0]
 
 
 def fno3_text(fi: "F.Fno3Input", device: int = 0) -> bytes:

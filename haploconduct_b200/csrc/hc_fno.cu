@@ -31,6 +31,7 @@
 #include <cuda_runtime.h>
 #include "../../include/hc_b200.h"
 #include "hc_fno_text.h"
+#include "hc_ingest.h"
 #include "hc_scan.cuh"
 #include "hc_stage.h"
 
@@ -599,6 +600,62 @@ __global__ void fno3_resolve(const u64* __restrict__ off, u64 n, const uint32_t*
     }
 }
 
+// ---- the non-edge segment of the FNO1 stream (hc_fno1_text_nonedges) -----------------------------------------------------
+// First position of every ordered vertex pair (u, v) of the adjacency segment: the claim of ffw_claim, keyed by u << 32 | v.
+__global__ void adj_claim(const hc_fno_edge* __restrict__ adj, u64 n, Cell* __restrict__ tab, uint32_t mask) {
+    for (u64 t = (u64)blockIdx.x * blockDim.x + threadIdx.x; t < n; t += (u64)gridDim.x * blockDim.x) {
+        const uint2 uv = __ldg(reinterpret_cast<const uint2*>(adj + t));
+        const u64 key = ((u64)uv.x << 32) | uv.y;
+        uint32_t s = key_slot(mix64(key), mask);
+        while (true) {
+            const u64 prev = atomicCAS(&tab[s].key, ~0ull, key);
+            if (prev == ~0ull || prev == key) break;
+            s = (s + 1) & mask;
+        }
+        atomicMin(&tab[s].min, t);
+    }
+}
+
+__device__ __forceinline__ u64 adj_first(const Cell* __restrict__ tab, uint32_t mask, u64 key) {   // ~0: no such pair
+    uint32_t s = key_slot(mix64(key), mask);
+    while (true) {
+        const u64 k = tab[s].key;
+        if (k == key) return tab[s].min;
+        if (k == ~0ull) return ~0ull;
+        s = (s + 1) & mask;
+    }
+}
+
+// keep[i] = !(checkEdge(v1, v2, true) > 0), src/FindNextOverlaps.cpp:694-696 with OverlapGraph::checkEdge
+// (src/OverlapGraph.cpp:233-259): the first adjacency entry v1 -> v2 decides, and only if there is none the first
+// v2 -> v1; its score is > 0 exactly when it is not a non-edge overlap (adjacency scores are never negative).
+__global__ void nonedge_probe(const hc_candidate* __restrict__ c, u64 n, const Cell* __restrict__ tab, uint32_t mask,
+                              const hc_fno_edge* __restrict__ adj, uint32_t* __restrict__ keep) {
+    for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x) {
+        const uint2 uv = __ldg(reinterpret_cast<const uint2*>(c + i));
+        u64 p = adj_first(tab, mask, ((u64)uv.x << 32) | uv.y);
+        if (p == ~0ull) p = adj_first(tab, mask, ((u64)uv.y << 32) | uv.x);
+        keep[i] = p == ~0ull || __ldg(&adj[p].nonedge) != 0;
+    }
+}
+
+// the kept lines as stream edges, in file order: the Edge of :640-690 (score 0, fields of the Overlap) as to_fno_edge
+// of hcb_fno.cpp makes it
+__global__ void nonedge_scatter(const hc_candidate* __restrict__ c, const uint32_t* __restrict__ keep, const u64* __restrict__ pos,
+                                u64 n, hc_fno_edge* __restrict__ out) {
+    for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x) {
+        if (!keep[i]) continue;
+        const hc_candidate a = c[i];
+        hc_fno_edge e;
+        e.u = a.idx1; e.v = a.idx2;
+        e.pos1 = (int32_t)a.pos1; e.pos2 = (int32_t)a.pos2;
+        e.perc = a.perc2 > 0 ? (int32_t)(uint32_t)(0.5 * (double)((uint32_t)a.perc1 + (uint32_t)a.perc2)) : (int32_t)a.perc1;   // Overlap::get_perc
+        e.len1 = (int32_t)a.len1; e.len2 = (int32_t)a.len2;
+        e.ord = a.ord; e.ori1 = a.ori1; e.ori2 = a.ori2; e.nonedge = 1;
+        out[pos[i]] = e;
+    }
+}
+
 thread_local std::string g_fno_err;
 
 }  // namespace
@@ -673,16 +730,18 @@ done:
     return rc;
 }
 
-static int fno1_impl(const hc_fno_input* in, const hc_fno_edge* edges, uint64_t n_edges, hc_fno_overlap* out48,
-                     hc_fno_overlap_small* out24, const FnoText* txt, uint64_t out_cap, uint64_t* n_out, int device) {
-    const char* who = txt ? "hc_fno1_text" : (out24 ? "hc_fno1_small" : "hc_fno1");
-    if (!in || !n_out || (n_edges && !edges) || (out_cap && !out48 && !out24)) { hc_set_last_error((std::string(who) + ": NULL argument").c_str()); return HC_ERR_ARG; }
-    *n_out = 0;
-    const u64 V = in->n_vertices, NS = in->n_superreads;
+static bool fno_edges_in_range(const hc_fno_edge* edges, uint64_t n_edges, u64 V, const char* who) {
     int bad = 0;
 #pragma omp parallel for schedule(static) reduction(| : bad)
     for (long long i = 0; i < (long long)n_edges; i++) bad |= (edges[i].u >= V || edges[i].v >= V);
-    if (bad) { hc_set_last_error((std::string(who) + ": edge vertex out of range").c_str()); return HC_ERR_ARG; }
+    if (bad) hc_set_last_error((std::string(who) + ": edge vertex out of range").c_str());
+    return !bad;
+}
+
+// The checks of hc_fno_input (the edges are checked by the caller)
+static int fno1_check_input(const hc_fno_input* in, const char* who) {
+    const u64 V = in->n_vertices, NS = in->n_superreads;
+    int bad = 0;
     const u64 nsr = V ? in->sr_off[V] : 0;
     if (nsr >> 32) { hc_set_last_error((std::string(who) + ": more than 2^32 super-read list entries").c_str()); return HC_ERR_ARG; }
 #pragma omp parallel for schedule(static) reduction(| : bad)
@@ -696,7 +755,24 @@ static int fno1_impl(const hc_fno_input* in, const hc_fno_edge* edges, uint64_t 
 #pragma omp parallel for schedule(static) reduction(| : bad)
     for (long long v = 0; v < (long long)V; v++) bad |= (!in->visited[v] && in->vertex_read[v].id != ~0ull && (in->vertex_read[v].id >> 32) != 0);
     if (bad) { hc_set_last_error((std::string(who) + ": a new read id does not fit 32 bits (ids of new reads must be below 2^32)").c_str()); return HC_ERR_ARG; }
+    return HC_OK;
+}
+
+// FNO1 on `device`.  The edge stream is either the host array `edges` (checked, with `in`, and copied here) or, with
+// d_edges_in, already in HBM -- then the caller has checked the edges and `in` (fno1_check_input).
+static int fno1_impl(const hc_fno_input* in, const hc_fno_edge* edges, uint64_t n_edges, const hc_fno_edge* d_edges_in,
+                     hc_fno_overlap* out48, hc_fno_overlap_small* out24, const FnoText* txt, uint64_t out_cap, uint64_t* n_out,
+                     int device, const char* who = nullptr) {
+    if (!who) who = txt ? "hc_fno1_text" : (out24 ? "hc_fno1_small" : "hc_fno1");
+    if (!in || !n_out || (n_edges && !edges && !d_edges_in) || (out_cap && !out48 && !out24)) { hc_set_last_error((std::string(who) + ": NULL argument").c_str()); return HC_ERR_ARG; }
+    *n_out = 0;
+    const u64 V = in->n_vertices, NS = in->n_superreads;
     int rc = HC_OK;
+    if (!d_edges_in) {                                          // device edges: the caller has checked them and `in`
+        if (!fno_edges_in_range(edges, n_edges, V, who)) return HC_ERR_ARG;
+        if ((rc = fno1_check_input(in, who)) != HC_OK) return rc;
+    }
+    const u64 nsr = V ? in->sr_off[V] : 0;
     FnoPhase ph(who);
     ph.mark("argument checks");
     uint8_t *d_vis = nullptr, *d_lab = nullptr, *d_win = nullptr;
@@ -704,7 +780,8 @@ static int fno1_impl(const hc_fno_input* in, const hc_fno_edge* edges, uint64_t 
     u64 *d_sroff = nullptr, *d_off = nullptr, *d_total = nullptr, *d_keys = nullptr, *d_bsum = nullptr;
     uint32_t *d_sridx = nullptr, *d_cnt = nullptr;
     hc_fno_subread* d_sub = nullptr;
-    hc_fno_edge* d_edges = nullptr;
+    hc_fno_edge* d_edges_own = nullptr;
+    const hc_fno_edge* d_edges = d_edges_in;
     VDesc* d_vd = nullptr;
     EDesc* d_en = nullptr;
     u64 attempts = 0;
@@ -720,7 +797,8 @@ static int fno1_impl(const hc_fno_input* in, const hc_fno_edge* edges, uint64_t 
     FCU(hc_scratch_alloc((void**)&d_sroff, (V + 1) * sizeof(u64))); FCU(hc_scratch_alloc((void**)&d_sridx, (nsr ? nsr : 1) * sizeof(uint32_t)));
     FCU(hc_scratch_alloc((void**)&d_sub, (nsr ? nsr : 1) * sizeof(hc_fno_subread)));
     FCU(hc_scratch_alloc((void**)&d_vd, (V ? V : 1) * sizeof(VDesc))); FCU(hc_scratch_alloc((void**)&d_en, (nsr ? nsr : 1) * sizeof(EDesc)));
-    FCU(hc_scratch_alloc((void**)&d_edges, n_edges * sizeof(hc_fno_edge))); FCU(hc_scratch_alloc((void**)&d_cnt, n_edges * sizeof(uint32_t)));
+    if (!d_edges_in) FCU(hc_scratch_alloc((void**)&d_edges_own, n_edges * sizeof(hc_fno_edge)));
+    FCU(hc_scratch_alloc((void**)&d_cnt, n_edges * sizeof(uint32_t)));
     FCU(hc_scratch_alloc((void**)&d_off, n_edges * sizeof(u64))); FCU(hc_scratch_alloc((void**)&d_total, sizeof(u64)));
     FCU(hc_copy_h2d(d_vis, in->visited, V)); FCU(hc_copy_h2d(d_lab, in->label, V));
     FCU(hc_copy_h2d(d_vr, in->vertex_read, V * sizeof(hc_fno_read)));
@@ -731,7 +809,10 @@ static int fno1_impl(const hc_fno_input* in, const hc_fno_edge* edges, uint64_t 
     // the packed per-vertex / per-entry records are built while the edges (the bulk of the input) are still being copied
     fno_prep_vertices<<<vblocks, threads>>>(V, d_vis, d_lab, d_vr, d_sroff, d_vd);
     fno_prep_entries<<<vblocks, threads>>>(V, d_vr, d_sroff, d_sridx, d_sub, d_sr, d_en);
-    FCU(hc_copy_h2d(d_edges, edges, n_edges * sizeof(hc_fno_edge)));
+    if (!d_edges_in) {
+        FCU(hc_copy_h2d(d_edges_own, edges, n_edges * sizeof(hc_fno_edge)));
+        d_edges = d_edges_own;
+    }
     ph.mark("allocations + copies in");
     D.vd = d_vd; D.en = d_en; D.resolve_orientations = in->resolve_orientations; D.no_inclusions = in->no_inclusions;
     fno_count<<<blocks, threads>>>(D, d_edges, n_edges, d_cnt);
@@ -753,19 +834,19 @@ static int fno1_impl(const hc_fno_input* in, const hc_fno_edge* edges, uint64_t 
     }, attempts, out48, out24, txt, out_cap, n_out, ph, who);
 done:
     hc_scratch_free(d_vis); hc_scratch_free(d_lab); hc_scratch_free(d_vr); hc_scratch_free(d_sr); hc_scratch_free(d_sroff); hc_scratch_free(d_sridx); hc_scratch_free(d_sub);
-    hc_scratch_free(d_edges); hc_scratch_free(d_cnt); hc_scratch_free(d_off); hc_scratch_free(d_total); hc_scratch_free(d_keys);
+    hc_scratch_free(d_edges_own); hc_scratch_free(d_cnt); hc_scratch_free(d_off); hc_scratch_free(d_total); hc_scratch_free(d_keys);
     hc_scratch_free(d_bsum); hc_scratch_free(d_win); hc_scratch_free(d_vd); hc_scratch_free(d_en);
     return rc;
 }
 
 extern "C" int hc_fno1(const hc_fno_input* in, const hc_fno_edge* edges, uint64_t n_edges, hc_fno_overlap* out, uint64_t out_cap,
                        uint64_t* n_out, int device) {
-    return fno1_impl(in, edges, n_edges, out, nullptr, nullptr, out_cap, n_out, device);
+    return fno1_impl(in, edges, n_edges, nullptr, out, nullptr, nullptr, out_cap, n_out, device);
 }
 
 extern "C" int hc_fno1_small(const hc_fno_input* in, const hc_fno_edge* edges, uint64_t n_edges, hc_fno_overlap_small* out,
                              uint64_t out_cap, uint64_t* n_out, int device) {
-    return fno1_impl(in, edges, n_edges, nullptr, out, nullptr, out_cap, n_out, device);
+    return fno1_impl(in, edges, n_edges, nullptr, nullptr, out, nullptr, out_cap, n_out, device);
 }
 
 static int fno3_impl(uint64_t n_originals, const uint64_t* off, const uint32_t* sr_idx, const hc_fno3_pos* sr_pos, uint64_t n_reads,
@@ -853,8 +934,152 @@ extern "C" int hc_fno1_text(const hc_fno_input* in, const hc_fno_edge* edges, ui
     if (!text_args_ok("hc_fno1_text", text, text_cap, n_bytes, n_lines)) return HC_ERR_ARG;
     const FnoText t = {text, text_cap, n_bytes, n_lines, true};
     uint64_t records = 0;
-    const int rc = fno1_impl(in, edges, n_edges, nullptr, nullptr, &t, 0, &records, device);
+    const int rc = fno1_impl(in, edges, n_edges, nullptr, nullptr, nullptr, &t, 0, &records, device);
     if (n_records) *n_records = records;
+    return rc;
+}
+
+// head ++ (the lines of nonedge_text that are not an edge of the adjacency segment) ++ tail, built in HBM.  The text goes
+// through the pieces of hc_ingest_cuts (two device buffers, the copy of piece i + 1 overlapping the work on piece i); every
+// piece is parsed by the ingestion parser in all-lines mode, probed against the adjacency pairs and compacted in file order
+// behind what the earlier pieces kept.  No line is kept past an error line: on HC_ERR_INPUT the stream is discarded.
+static int fno1_nonedge_stream(const hc_idmap* m, const hc_fno_edge* head, uint64_t n_head, uint64_t n_adjacency,
+                               const char* text, uint64_t n_bytes, const hc_fno_edge* tail, uint64_t n_tail,
+                               hc_fno_edge** d_stream_out, hc_fno_nonedge_stats* stats, const char* who) {
+    int rc = HC_OK;
+    const std::vector<uint64_t> cut = hc_ingest_cuts(text, n_bytes, hc_ingest_piece_bytes());
+    const size_t n_pieces = cut.size() - 1;
+    u64 max_piece = 0, bound = n_head + n_tail;
+    for (size_t i = 0; i < n_pieces; i++) {
+        max_piece = std::max<u64>(max_piece, cut[i + 1] - cut[i]);
+        bound += hc_ingest_all_cap(cut[i + 1] - cut[i]);
+    }
+    const u64 tbytes = (max_piece + 16 + 255) & ~255ull, cap = hc_ingest_all_cap(max_piece);
+    u64 slots = 1024, kept = 0, lines = 0, total = 0;
+    while (slots < 2 * n_adjacency + 2) slots <<= 1;
+    hc_fno_edge* d_stream = nullptr;
+    char* d_text = nullptr;
+    hc_candidate* d_cand = nullptr;
+    uint32_t* d_keep = nullptr;
+    u64 *d_pos = nullptr, *d_total = nullptr, *d_bsum = nullptr;
+    Cell* d_tab = nullptr;
+    cudaStream_t s_copy = nullptr;
+    cudaEvent_t ev_in[2] = {nullptr, nullptr}, t0 = nullptr, t1 = nullptr;
+    hc_ingest_params ip;
+    memset(&ip, 0, sizeof(ip));
+    ip.max_overlaps = ~0ull;                                     // the loop reads the whole file; ORD / ORI / TYPE split on tabs only
+    FCU(cudaStreamCreateWithFlags(&s_copy, cudaStreamNonBlocking));
+    for (int k = 0; k < 2; k++) FCU(cudaEventCreateWithFlags(&ev_in[k], cudaEventDisableTiming));
+    FCU(cudaEventCreate(&t0)); FCU(cudaEventCreate(&t1));
+    FCU(cudaEventRecord(t0, 0));
+    FCU(hc_scratch_alloc((void**)&d_stream, (bound ? bound : 1) * sizeof(hc_fno_edge)));
+    FCU(hc_copy_h2d(d_stream, head, n_head * sizeof(hc_fno_edge)));
+    if (n_pieces) {
+        FCU(hc_scratch_alloc((void**)&d_text, 2 * tbytes));
+        FCU(hc_scratch_alloc((void**)&d_cand, cap * sizeof(hc_candidate)));
+        FCU(hc_scratch_alloc((void**)&d_keep, cap * sizeof(uint32_t))); FCU(hc_scratch_alloc((void**)&d_pos, cap * sizeof(u64)));
+        FCU(hc_scratch_alloc((void**)&d_total, sizeof(u64))); FCU(hc_scratch_alloc((void**)&d_bsum, hc_scan::blocks_for(cap) * sizeof(u64)));
+        FCU(hc_scratch_alloc((void**)&d_tab, slots * sizeof(Cell)));
+        FCU(cudaMemsetAsync(d_tab, 0xff, slots * sizeof(Cell)));
+        if (n_adjacency) {
+            const int ab = (int)std::min<u64>((n_adjacency + 255) / 256, 148 * 16);
+            adj_claim<<<ab, 256>>>(d_stream, n_adjacency, d_tab, (uint32_t)(slots - 1));
+            FCU(cudaGetLastError());
+        }
+        FCU(hc_copy_h2d_on(d_text, text, cut[1] - cut[0], s_copy));
+        FCU(cudaEventRecord(ev_in[0], s_copy));
+    }
+    for (size_t i = 0; i < n_pieces; i++) {
+        const int b = (int)(i & 1);
+        if (i + 1 < n_pieces) {   // buffer b ^ 1 held piece i - 1, whose work has completed (the kept count below is read back)
+            FCU(hc_copy_h2d_on(d_text + (size_t)(b ^ 1) * tbytes, text + cut[i + 1], cut[i + 2] - cut[i + 1], s_copy));
+            FCU(cudaEventRecord(ev_in[b ^ 1], s_copy));
+        }
+        FCU(cudaStreamWaitEvent(0, ev_in[b], 0));
+        hc_ingest_stats st;
+        rc = hc_ingest_device(m, d_text + (size_t)b * tbytes, cut[i + 1] - cut[i], &ip, d_cand, nullptr, cap, nullptr, nullptr, 0,
+                              &st, 0, 0, true);
+        if (rc != HC_OK) goto done;
+        if (st.first_error_line != ~0ull) {
+            stats->first_error_line = lines + st.first_error_line;
+            stats->first_error_offset = cut[i] + st.first_error_offset;
+            stats->first_error_length = st.first_error_length;
+            stats->first_error_status = st.first_error_status;
+            const char* what = st.first_error_status == HC_LINE_SKIPPED ? "not 13 tab-separated fields"
+                               : st.first_error_status == HC_LINE_UNKNOWN_ID ? "a read id that is not in the id map"
+                                                                             : "fields the Overlap constructor rejects";
+            hc_set_last_error((std::string(who) + ": line " + std::to_string(stats->first_error_line) + " of the non-edge text has " + what).c_str());
+            rc = HC_ERR_INPUT;
+            goto done;
+        }
+        lines += st.n_lines;
+        if (st.n_scored) {
+            const int pb = (int)std::min<u64>((st.n_scored + 255) / 256, 148 * 16);
+            nonedge_probe<<<pb, 256>>>(d_cand, st.n_scored, d_tab, (uint32_t)(slots - 1), d_stream, d_keep);
+            hc_scan::exclusive_u32(d_keep, st.n_scored, d_pos, d_total, d_bsum, 0);
+            nonedge_scatter<<<pb, 256>>>(d_cand, d_keep, d_pos, st.n_scored, d_stream + n_head + kept);
+            FCU(cudaGetLastError());
+            FCU(cudaMemcpy(&total, d_total, sizeof(u64), cudaMemcpyDeviceToHost));
+            kept += total;
+        }
+    }
+    FCU(hc_copy_h2d(d_stream + n_head + kept, tail, n_tail * sizeof(hc_fno_edge)));
+    FCU(cudaEventRecord(t1, 0));
+    FCU(cudaEventSynchronize(t1));
+    FCU(cudaEventElapsedTime(&stats->device_ms, t0, t1));
+    stats->n_lines = lines;
+    stats->n_nonedges = kept;
+    stats->n_stream = n_head + kept + n_tail;
+    *d_stream_out = d_stream;
+    d_stream = nullptr;
+done:
+    if (s_copy) { cudaStreamSynchronize(s_copy); cudaStreamDestroy(s_copy); }
+    for (int k = 0; k < 2; k++) if (ev_in[k]) cudaEventDestroy(ev_in[k]);
+    if (t0) cudaEventDestroy(t0);
+    if (t1) cudaEventDestroy(t1);
+    hc_scratch_free(d_stream); hc_scratch_free(d_text); hc_scratch_free(d_cand); hc_scratch_free(d_keep); hc_scratch_free(d_pos);
+    hc_scratch_free(d_total); hc_scratch_free(d_bsum); hc_scratch_free(d_tab);
+    return rc;
+}
+
+extern "C" int hc_fno1_text_nonedges(const hc_fno_input* in, const hc_idmap* m, const hc_fno_edge* head, uint64_t n_head,
+                                     uint64_t n_adjacency, const char* nonedge_text, uint64_t nonedge_bytes, const hc_fno_edge* tail,
+                                     uint64_t n_tail, char* text, uint64_t text_cap, uint64_t* n_bytes, uint64_t* n_lines,
+                                     uint64_t* n_records, hc_fno_nonedge_stats* stats, int device) {
+    const char* who = "hc_fno1_text_nonedges";
+    if (!text_args_ok(who, text, text_cap, n_bytes, n_lines)) return HC_ERR_ARG;
+    if (!in || !m || !stats || (n_head && !head) || (n_tail && !tail) || (nonedge_bytes && !nonedge_text)) {
+        hc_set_last_error((std::string(who) + ": NULL argument").c_str());
+        return HC_ERR_ARG;
+    }
+    memset(stats, 0, sizeof(*stats));
+    stats->first_error_line = ~0ull;
+    if (n_records) *n_records = 0;
+    const u64 V = in->n_vertices;
+    if (m->device != device) { hc_set_last_error((std::string(who) + ": the id map is on another device").c_str()); return HC_ERR_ARG; }
+    if (m->n != V) { hc_set_last_error((std::string(who) + ": the id map does not hold one read per vertex (vertex i is read i)").c_str()); return HC_ERR_ARG; }
+    if (n_adjacency > n_head) { hc_set_last_error((std::string(who) + ": n_adjacency > n_head").c_str()); return HC_ERR_ARG; }
+    for (u64 i = 1; i < n_adjacency; i++)
+        if (head[i].u < head[i - 1].u) { hc_set_last_error((std::string(who) + ": the adjacency lists are not in vertex order").c_str()); return HC_ERR_ARG; }
+    if (!fno_edges_in_range(head, n_head, V, who) || !fno_edges_in_range(tail, n_tail, V, who)) return HC_ERR_ARG;
+    int rc = fno1_check_input(in, who);
+    if (rc != HC_OK) return rc;
+    hc_fno_edge* d_stream = nullptr;
+    FCU(cudaSetDevice(device));
+    {
+        FnoPhase ph(who);
+        rc = fno1_nonedge_stream(m, head, n_head, n_adjacency, nonedge_text, nonedge_bytes, tail, n_tail, &d_stream, stats, who);
+        if (rc != HC_OK) goto done;
+        ph.mark("stream with non-edge lines");
+    }
+    {
+        const FnoText t = {text, text_cap, n_bytes, n_lines, true};
+        uint64_t records = 0;
+        rc = fno1_impl(in, nullptr, stats->n_stream, d_stream, nullptr, nullptr, &t, 0, &records, device, who);
+        if (n_records) *n_records = records;
+    }
+done:
+    hc_scratch_free(d_stream);
     return rc;
 }
 

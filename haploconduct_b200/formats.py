@@ -154,6 +154,10 @@ INGEST_STATS = np.dtype([("n_lines", "<u8"), ("n_scored", "<u8"), ("n_filtered",
 assert INGEST_PARAMS.itemsize == 24 and OVERLAP_REC.itemsize == 48 and INGEST_STATS.itemsize == 72
 INGEST_SCORE_STATS = np.dtype([("ingest", INGEST_STATS), ("score", BATCH_STATS), ("n_kept", "<u8")])   # hc_ingest_score_stats
 assert INGEST_SCORE_STATS.itemsize == 152
+FNO_NONEDGE_STATS = np.dtype([("n_lines", "<u8"), ("n_nonedges", "<u8"), ("n_stream", "<u8"), ("first_error_line", "<u8"),
+                              ("first_error_offset", "<u8"), ("first_error_length", "<u8"), ("first_error_status", "<u4"),
+                              ("device_ms", "<f4")])   # hc_fno_nonedge_stats
+assert FNO_NONEDGE_STATS.itemsize == 56
 CONS_SEQ = np.dtype([("read", "<u4"), ("mate", "u1"), ("rc", "u1"), ("reserved", "<u2"), ("pos", "<i4")])
 CONS_PROBLEM = np.dtype([("seq_begin", "<u8"), ("seq_end", "<u8"), ("out_offset", "<u8"), ("total_len", "<i4"),
                          ("subreads_needed", "u1"), ("error_correction", "u1"), ("reserved", "u1", (2,))])

@@ -9,6 +9,7 @@
 //   S  s|p|t  read_id  len1  len2  node:index1:index2:startpos1:startpos2 ...      a super-read (single / paired / trivial)
 //   O  original_id:index1:index2 ...                                              its original reads, reference map order
 // nonedge_overlaps.txt is read from, overlaps.txt written to, the output directory.  Prints one JSON summary line.
+// --gpu_parse=true (FNO1): nonedge_overlaps.txt is parsed and checked against the adjacency lists on the device.
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -43,6 +44,7 @@ int main(int argc, char** argv) {
         else if (a == "--state") state = v;
         else if (a == "--FNO") fno = atoi(v.c_str());
         else if (a == "--gpu_fastq") ps.gpu_fastq = v == "true" || v == "1";
+        else if (a == "--gpu_parse") ps.gpu_parse = v == "true" || v == "1";     // FNO1: nonedge_overlaps.txt parsed on the device
         else { fprintf(stderr, "unknown option %s\n", a.c_str()); return 2; }
     }
     if (state.empty()) { fprintf(stderr, "No state file provided.\n"); return 1; }
@@ -128,7 +130,9 @@ int main(int argc, char** argv) {
     unsigned long lines = 0;
     if (fno == 3) { srb->findNextOverlaps3(); lines = srb->next_overlaps_count; }
     else lines = srb->findNextOverlaps();
-    printf("{\"fno\": %d, \"lines\": %lu, \"stream\": %lu, \"device_overlaps\": %lu, \"t_stream_s\": %.6f, \"t_device_s\": %.6f, \"t_format_s\": %.6f}\n",
-           fno, lines, srb->n_stream_edges, srb->n_device_overlaps, srb->t_stream_s, srb->t_device_s, srb->t_format_s);
+    printf("{\"fno\": %d, \"lines\": %lu, \"stream\": %lu, \"device_overlaps\": %lu, \"t_stream_s\": %.6f, \"t_device_s\": %.6f, \"t_format_s\": %.6f, "
+           "\"nonedge_lines\": %lu, \"nonedge_kept\": %lu, \"nonedge_on_device\": %d, \"nonedge_device_ms\": %.3f}\n",
+           fno, lines, srb->n_stream_edges, srb->n_device_overlaps, srb->t_stream_s, srb->t_device_s, srb->t_format_s,
+           srb->nonedge_lines, srb->nonedge_kept, srb->nonedge_on_device ? 1 : 0, srb->nonedge_device_ms);
     return 0;
 }

@@ -21,8 +21,9 @@ double now_s() { return std::chrono::duration<double>(std::chrono::steady_clock:
 // Calls `call(buf, cap, &n_bytes, &n_lines)` into a buffer sized from `guess` lines and, if the text does not fit, once more
 // with the exact size; writes the text to `filename` with one write.  Returns the line count; `t_text` is when the text
 // had arrived in host memory.
+// With input_error, HC_ERR_INPUT sets it and returns 0 without writing the file (the caller takes another path).
 template <class Call>
-uint64_t write_text(Call call, uint64_t guess, const std::string& filename, const char* what, double& t_text) {
+uint64_t write_text(Call call, uint64_t guess, const std::string& filename, const char* what, double& t_text, bool* input_error = nullptr) {
     uint64_t cap = std::min<uint64_t>(guess, 1ull << 24) * 128 + 4096, n_bytes = 0, n_lines = 0;
     std::unique_ptr<char[]> buf(new char[cap]);            // not touched here: only the written pages are committed
     int rc = call(buf.get(), cap, &n_bytes, &n_lines);
@@ -31,6 +32,7 @@ uint64_t write_text(Call call, uint64_t guess, const std::string& filename, cons
         buf.reset(new char[cap]);
         rc = call(buf.get(), cap, &n_bytes, &n_lines);
     }
+    if (rc == HC_ERR_INPUT && input_error) { *input_error = true; return 0; }
     if (rc != HC_OK) die(std::string(what) + ": " + hc_last_error());
     t_text = now_s();
     std::ofstream outfile(filename.c_str(), std::ios::binary);
@@ -87,6 +89,58 @@ void SRBuilder::read_lengths(node_id_t index, unsigned long& l1, unsigned long& 
     l2 = r.is_paired ? r.seq2.size() : 0;
 }
 
+// The loop of :635-697 over nonedge_overlaps.txt: every overlap that is not an edge of the graph joins the stream as a
+// non-edge (score 0)
+void SRBuilder::append_nonedges(std::vector<hc_fno_edge>& stream) {
+    const std::string path = ps_.output_dir + "nonedge_overlaps.txt";
+    std::ifstream f(path.c_str());
+    if (!f.is_open()) die("Unable to open non-edge overlaps file");
+    if (fastq_->m_ID_to_index.empty())      // --gpu_fastq with --gpu_parse leaves the host map empty (FastqStorage)
+        for (unsigned int i = 0; i < fastq_->m_read_vec.size(); i++) fastq_->m_ID_to_index.insert(std::make_pair(fastq_->m_read_vec[i].read_id, i));
+    std::string line, tmp;
+    std::vector<std::string> fields;
+    unsigned long lines = 0, kept = 0;
+    while (std::getline(f, line)) {
+        lines++;
+        const size_t b = line.find_first_not_of("\t "), e2 = line.find_last_not_of("\t ");
+        line = b == std::string::npos ? std::string() : line.substr(b, e2 - b + 1);                          // boost::trim_if, :650
+        fields.clear();
+        std::stringstream ss(line);
+        while (std::getline(ss, tmp, '\t')) fields.push_back(tmp);
+        const Overlap ov = Overlap::from_fields(fields);
+        const Read& r1 = fastq_->m_read_vec.at(fastq_->m_ID_to_index.at(ov.id1));
+        const Read& r2 = fastq_->m_read_vec.at(fastq_->m_ID_to_index.at(ov.id2));
+        Edge e;
+        e.score = 0;
+        e.pos1 = (int)ov.pos1;
+        e.pos2 = (int)ov.pos2;
+        e.ori1 = ov.ori1 == '+';
+        e.ori2 = ov.ori2 == '+';
+        e.ord = ov.ord;
+        e.overlap_perc = (int)ov.get_perc();
+        e.overlap_len1 = (int)ov.len1;
+        e.overlap_len2 = (int)ov.len2;
+        e.vertex1 = r1.vertex_id;
+        e.vertex2 = r2.vertex_id;
+        if (checkEdge(e.vertex1, e.vertex2, true) > 0) continue;                                               // :694-696
+        stream.push_back(to_fno_edge(e));
+        kept++;
+    }
+    nonedge_lines = lines;
+    nonedge_kept = kept;
+}
+
+// What hc_fno1_text_nonedges assumes of the graph: vertex i is read i, list v holds the edges out of v (its (u, v) pairs are
+// what checkEdge looks up) and every edge score is 0 (non-edge) or positive (edge)
+bool SRBuilder::nonedge_device_ok() const {
+    const auto& reads = fastq_->m_read_vec;
+    if (graph_->adj_out.size() != reads.size()) return false;
+    for (size_t i = 0; i < reads.size(); i++) if (reads[i].vertex_id != i) return false;
+    for (size_t v = 0; v < graph_->adj_out.size(); v++)
+        for (const Edge& e : graph_->adj_out[v]) if (e.vertex1 != v || !(e.score == 0 || e.score > 0)) return false;
+    return true;
+}
+
 unsigned long SRBuilder::findNextOverlaps() {
     if (ps_.add_duplicates) die("findNextOverlaps: --add_duplicates=true is not supported by the GPU path");
     const size_t V = graph_->getVertexCount();
@@ -134,41 +188,20 @@ unsigned long SRBuilder::findNextOverlaps() {
         vertex_read[v].len1 = (uint32_t)l1;
         vertex_read[v].len2 = (uint32_t)l2;
     }
-    // ---- the edge stream in processing order
+    // ---- the edge stream in processing order: head (adjacency lists, branching edges), non-edge lines, tail
     std::vector<hc_fno_edge> stream;
     for (const auto& lst : graph_->adj_out) for (const Edge& e : lst) stream.push_back(to_fno_edge(e));       // :610-623
+    const uint64_t n_adjacency = stream.size();
     for (const Edge& e : graph_state.branching_edges) stream.push_back(to_fno_edge(e));                        // :624-630
-    if (!optimize) {                                                                                           // :635-697
-        const std::string path = ps_.output_dir + "nonedge_overlaps.txt";
-        std::ifstream f(path.c_str());
-        if (!f.is_open()) die("Unable to open non-edge overlaps file");
-        std::string line, tmp;
-        std::vector<std::string> fields;
-        while (std::getline(f, line)) {
-            const size_t b = line.find_first_not_of("\t "), e2 = line.find_last_not_of("\t ");
-            line = b == std::string::npos ? std::string() : line.substr(b, e2 - b + 1);                      // boost::trim_if, :650
-            fields.clear();
-            std::stringstream ss(line);
-            while (std::getline(ss, tmp, '\t')) fields.push_back(tmp);
-            const Overlap ov = Overlap::from_fields(fields);
-            const Read& r1 = fastq_->m_read_vec.at(fastq_->m_ID_to_index.at(ov.id1));
-            const Read& r2 = fastq_->m_read_vec.at(fastq_->m_ID_to_index.at(ov.id2));
-            Edge e;
-            e.score = 0;
-            e.pos1 = (int)ov.pos1;
-            e.pos2 = (int)ov.pos2;
-            e.ori1 = ov.ori1 == '+';
-            e.ori2 = ov.ori2 == '+';
-            e.ord = ov.ord;
-            e.overlap_perc = (int)ov.get_perc();
-            e.overlap_len1 = (int)ov.len1;
-            e.overlap_len2 = (int)ov.len2;
-            e.vertex1 = r1.vertex_id;
-            e.vertex2 = r2.vertex_id;
-            if (checkEdge(e.vertex1, e.vertex2, true) > 0) continue;                                           // :694-696
-            stream.push_back(to_fno_edge(e));
-        }
+    const uint64_t n_head = stream.size();
+    FileBuf nonedge_text;
+    const bool nonedges_on_device = !optimize && ps_.gpu_parse && nonedge_device_ok();
+    if (nonedges_on_device) {
+        if (!read_whole_file(ps_.output_dir + "nonedge_overlaps.txt", nonedge_text)) die("Unable to open non-edge overlaps file");
+    } else if (!optimize) {
+        append_nonedges(stream);                                                                               // :635-697
     }
+    std::vector<hc_fno_edge> tail;
     for (const auto& edge_list : graph_state.inclusion_edges) {                                                // :816-887
         const size_t l = edge_list.size();
         for (size_t i = 0; i < l; i++) {
@@ -200,11 +233,11 @@ unsigned long SRBuilder::findNextOverlaps() {
                 ne.overlap_perc = perc;
                 ne.overlap_len1 = len;
                 ne.overlap_len2 = 0;
-                if (checkEdge(n1, n2, true) == -1) stream.push_back(to_fno_edge(ne));
+                if (checkEdge(n1, n2, true) == -1) tail.push_back(to_fno_edge(ne));
             }
         }
     }
-    n_stream_edges = stream.size();
+    if (!nonedges_on_device) stream.insert(stream.end(), tail.begin(), tail.end());
     const double t1 = now_s();
     // ---- the derivations, on the device
     hc_fno_input in;
@@ -222,14 +255,44 @@ unsigned long SRBuilder::findNextOverlaps() {
     in.no_inclusions = no_inclusions ? 1 : 0;
     // ---- overlaps.txt, formatted, sorted and de-duplicated on the device (the reference's std::set<std::string>, :918,:946-948)
     const int dev = ps_.first_device;
-    uint64_t n_records = 0;
-    double t2 = 0;
-    const uint64_t n_lines = write_text([&](char* text, uint64_t cap, uint64_t* n_bytes, uint64_t* n_lines) {
-        return hc_fno1_text(&in, stream.data(), stream.size(), text, cap, n_bytes, n_lines, &n_records, dev); },
-        stream.size(), ps_.output_dir + "overlaps.txt", "hc_fno1_text", t2);
+    uint64_t n_records = 0, n_lines = 0;
+    double t2 = 0, t_host = t1 - t0, t_call = t1;
+    nonedge_on_device = false;
+    nonedge_device_ms = 0;
+    bool input_error = false;
+    if (nonedges_on_device) {
+        // the non-edge file is parsed, checked against the adjacency lists and put into the stream on the device; a line the
+        // loop below would die on sends the whole file there, so that the messages stay the reference's.  If the guessed
+        // text size is too small, write_text's second call repeats the whole device job (copy, parse, probe, derivations):
+        // the guess of 128 bytes per stream edge and non-edge line makes that rare
+        hc_idmap* idmap = fastq_->device_idmap();
+        hc_fno_nonedge_stats st;
+        n_lines = write_text([&](char* text, uint64_t cap, uint64_t* n_bytes, uint64_t* n_lines) {
+            return hc_fno1_text_nonedges(&in, idmap, stream.data(), n_head, n_adjacency, nonedge_text.data, nonedge_text.size,
+                                         tail.data(), tail.size(), text, cap, n_bytes, n_lines, &n_records, &st, dev); },
+            n_head + tail.size() + nonedge_text.size / 40, ps_.output_dir + "overlaps.txt", "hc_fno1_text_nonedges", t2, &input_error);
+        if (!input_error) {
+            nonedge_on_device = true;
+            n_stream_edges = st.n_stream;
+            nonedge_lines = st.n_lines;
+            nonedge_kept = st.n_nonedges;
+            nonedge_device_ms = st.device_ms;
+        } else {
+            append_nonedges(stream);
+            stream.insert(stream.end(), tail.begin(), tail.end());
+        }
+    }
+    if (!nonedges_on_device || input_error) {
+        t_call = now_s();
+        t_host += t_call - t1;       // after an HC_ERR_INPUT: the device attempt and the loop count as stream time
+        n_stream_edges = stream.size();
+        n_lines = write_text([&](char* text, uint64_t cap, uint64_t* n_bytes, uint64_t* n_lines) {
+            return hc_fno1_text(&in, stream.data(), stream.size(), text, cap, n_bytes, n_lines, &n_records, dev); },
+            stream.size(), ps_.output_dir + "overlaps.txt", "hc_fno1_text", t2);
+    }
     n_device_overlaps = n_records;
-    t_stream_s = t1 - t0;
-    t_device_s = t2 - t1;
+    t_stream_s = t_host;
+    t_device_s = t2 - t_call;
     t_format_s = now_s() - t2;
     next_overlaps_count = n_lines;
     return n_lines;

@@ -10,7 +10,9 @@
 // the reference's std::unordered_map (FindNextOverlaps3.cpp:101, same container, same insertions).  The derivations
 // themselves (updateOverlap / computeOverlapData, deduceOverlap) run on the device, and so does the text of
 // overlaps.txt: formatted there and, for FNO1, sorted and de-duplicated like the reference's std::set<std::string>
-// (:918,:946-948); the host writes the bytes it gets back.
+// (:918,:946-948); the host writes the bytes it gets back.  With ps.gpu_parse the non-edge file is parsed on the device as
+// well (hc_fno1_text_nonedges): the host reads it into memory and hands over the adjacency and inclusion segments of the
+// stream; a line the reference would die on sends the file back to the host loop, for the reference's message.
 //
 // The merging step that fills the super-read vectors (mergeAlongEdges / cliquesToSuperreads) and the graph algorithms
 // that fill branching_edges / inclusion_edges are not part of this path: a host that links this class keeps its own and
@@ -74,11 +76,17 @@ public:
     // t_device_s = device call up to the text in host memory, t_format_s = writing overlaps.txt
     unsigned long n_stream_edges = 0, n_device_overlaps = 0;
     double t_stream_s = 0, t_device_s = 0, t_format_s = 0;
+    // the non-edge file: lines read, lines that joined the stream, and (ps.gpu_parse) the device time of building the stream
+    unsigned long nonedge_lines = 0, nonedge_kept = 0;
+    double nonedge_device_ms = 0;
+    bool nonedge_on_device = false;        // the last call put the non-edge lines into the stream on the device
 
 private:
     double checkEdge(node_id_t v, node_id_t w, bool reverse_allowed) const;        // src/OverlapGraph.cpp:233-259
     bool orientation(node_id_t v) const;                                           // OverlapGraph::getOrientation
     void read_lengths(node_id_t index, unsigned long& l1, unsigned long& l2) const;
+    void append_nonedges(std::vector<hc_fno_edge>& stream);                          // :635-697 on the host
+    bool nonedge_device_ok() const;                                                 // the graph hc_fno1_text_nonedges assumes
     ProgramSettings ps_;
     std::shared_ptr<FastqStorage> fastq_;
     std::shared_ptr<OverlapGraph> graph_;

@@ -460,6 +460,44 @@ int hc_fno3_small(uint64_t n_originals, const uint64_t* off, const uint32_t* sr_
 int hc_fno1_text(const hc_fno_input* in, const hc_fno_edge* edges, uint64_t n_edges,
                  char* text, uint64_t text_cap, uint64_t* n_bytes, uint64_t* n_lines, uint64_t* n_records, int device);
 
+/* hc_fno1_text for the stream head ++ N ++ tail, where N -- the non-edge overlaps the reference re-reads from
+ * nonedge_overlaps.txt (reconsiderNonedgeOverlaps, src/FindNextOverlaps.cpp:635-697, --optimize=false) -- is parsed
+ * from nonedge_text on m's device and never leaves it.  Same text, *n_bytes, *n_lines, *n_records and HC_ERR_CAPACITY
+ * protocol as hc_fno1_text on that stream (text may be NULL with text_cap 0).
+ *   head          head[0 .. n_adjacency) = the adj_out lists in vertex order (u non-decreasing), then branching_edges
+ *   nonedge_text  host memory (pageable or pinned, any alignment): lines trimmed of outer tabs / spaces, split on tabs,
+ *                 put through the Overlap constructor (src/Overlap.h:39-73) -- no self-overlap test, no pre-filter.
+ *                 Line k becomes {u, v} = the store indices of ID1 / ID2 in m (vertex i is read i), POS1, POS2, ORD,
+ *                 ORI1/2 == '+', perc = Overlap::get_perc(), LEN1, LEN2, nonedge = 1; an unterminated last line counts.
+ *                 The line is dropped when checkEdge(v1, v2, true) > 0 (:694-696): the first adjacency entry (v1, v2),
+ *                 or only if there is none the first (v2, v1), has nonedge == 0.  This reads a non-edge flag as
+ *                 "score == 0" and any other entry as "score > 0": no adjacency edge may have a negative score.
+ *                 Branching and tail edges are not in the graph and are not consulted.
+ *   tail          the edges derived through removed inclusion vertices (:816-887)
+ * A line the reference's loop would die on or leave undefined -- not 13 fields (an empty line too), a field the
+ * constructor rejects, a trailing '\r', an id not in m -- gives HC_ERR_INPUT with the first such line in
+ * stats->first_error_* and nothing written; the caller runs its own loop for the reference's message.
+ * A call after HC_ERR_CAPACITY does all the work again, the parse of nonedge_text included: size text generously.
+ * HC_ERR_ARG (checked before any device work): m on another device or m's read count != in->n_vertices,
+ * n_adjacency > n_head, adjacency u decreasing, and every check of hc_fno1_text on head and tail. */
+typedef struct {
+    uint64_t n_lines;             /* lines of nonedge_text                                                  */
+    uint64_t n_nonedges;          /* of them, lines whose pair is not an edge: the stream's middle segment   */
+    uint64_t n_stream;            /* n_head + n_nonedges + n_tail                                           */
+    uint64_t first_error_line;    /* 0-based, ~0 if none; and its byte offset / length in nonedge_text      */
+    uint64_t first_error_offset, first_error_length;
+    uint32_t first_error_status;  /* HC_LINE_SKIPPED (not 13 fields, empty), HC_LINE_ERROR, HC_LINE_UNKNOWN_ID */
+    float    device_ms;           /* the stream built in HBM: head copy, pieces copied / parsed / probed / compacted, tail */
+} hc_fno_nonedge_stats;           /* 56 bytes */
+
+struct hc_idmap;                  /* hc_idmap_create, below */
+int hc_fno1_text_nonedges(const hc_fno_input* in, const struct hc_idmap* m,
+                          const hc_fno_edge* head, uint64_t n_head, uint64_t n_adjacency,
+                          const char* nonedge_text, uint64_t nonedge_bytes,
+                          const hc_fno_edge* tail, uint64_t n_tail,
+                          char* text, uint64_t text_cap, uint64_t* n_bytes, uint64_t* n_lines, uint64_t* n_records,
+                          hc_fno_nonedge_stats* stats, int device);
+
 /* The same for hc_fno3: the lines in discovery order, not sorted, not de-duplicated (src/FindNextOverlaps3.cpp:139-166). */
 int hc_fno3_text(uint64_t n_originals, const uint64_t* off, const uint32_t* sr_idx, const hc_fno3_pos* sr_pos,
                  uint64_t n_reads, const hc_fno_read* reads, int no_inclusions,
