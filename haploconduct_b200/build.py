@@ -9,6 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libhc_b200.so")
+PRIMS_SHIM = os.path.join(LIBDIR, "libhc_prims_shim.so")
 NVCC = os.environ.get("HC_NVCC", "/usr/local/cuda/bin/nvcc")
 HOST_CXX = "/usr/bin/g++"
 
@@ -30,6 +31,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
     deps = ([os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(hostdir, f) for f in os.listdir(hostdir)]
             + [os.path.join(HERE, "..", "include", "hc_b200.h")])
     if not force and not _newer(LIB, deps):
+        build_prims_shim(verbose=verbose)
         return LIB
     objs = []
     for src in CPP_SOURCES:
@@ -53,7 +55,23 @@ def build(force: bool = False, verbose: bool = False) -> str:
         print(" ".join(cmd))
     subprocess.check_call(cmd)
     build_host(verbose)
+    build_prims_shim(force=True, verbose=verbose)
     return LIB
+
+
+def build_prims_shim(force: bool = False, verbose: bool = False) -> str:
+    """libhc_prims_shim.so: C entry points over the header-only scan, radix-sort and newline-index primitives, for
+    tests/test_gpu_prims.py.  Lives beside libhc_b200.so, which it links against."""
+    src = os.path.join(HERE, "..", "tests", "cuda", "hc_prims_shim.cu")
+    deps = [src, LIB] + [os.path.join(CSRC, f) for f in ("hc_scan.cuh", "hc_radix.cuh", "hc_text.cuh", "hc_stage.h")]
+    if not force and not _newer(PRIMS_SHIM, deps):
+        return PRIMS_SHIM
+    cmd = [NVCC, "-ccbin", HOST_CXX, "-O3", "-std=c++14", "-lineinfo", *ARCH, "-shared", "-Xcompiler", "-fPIC", "-I" + CSRC,
+           "-o", PRIMS_SHIM, src, "-L" + LIBDIR, "-lhc_b200", "-Xlinker", "-rpath,$ORIGIN"]
+    if verbose:
+        print(" ".join(cmd))
+    subprocess.check_call(cmd)
+    return PRIMS_SHIM
 
 
 def build_host(verbose: bool = False) -> str:
