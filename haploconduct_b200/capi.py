@@ -24,7 +24,7 @@ EXPORTED = [
     "hc_overlap_score", "hc_overlap_score_multi",
     "hc_phred_to_prob", "hc_exp_threshold", "hc_device_count", "hc_warm_up", "hc_last_error", "hc_version", "hc_fno1", "hc_fno3", "hc_fno1_small", "hc_fno3_small", "hc_fno1_text", "hc_fno3_text", "hc_build_adjacency", "hc_subread_info", "hc_host_alloc", "hc_host_free",
     "hc_store_create_fastq", "hc_store_create_fastq_files", "hc_store_read_ids", "hc_consensus", "hc_dedup_edges", "hc_idmap_create", "hc_idmap_destroy", "hc_ingest_overlaps", "hc_ingest_overlaps_device",
-    "hc_ingest_score_overlaps", "hc_fno1_text_nonedges",
+    "hc_ingest_score_overlaps", "hc_fno1_text_nonedges", "hc_sfo2overlaps",
 ]
 
 _lib: Optional[ctypes.CDLL] = None
@@ -128,6 +128,8 @@ def lib() -> ctypes.CDLL:
         L.hc_fno1_text_nonedges.restype = i32
         L.hc_fno1_text_nonedges.argtypes = [vp, vp, vp, u64, u64, vp, u64, vp, u64, vp, u64, ctypes.POINTER(u64), ctypes.POINTER(u64),
                                             ctypes.POINTER(u64), vp, i32]
+        L.hc_sfo2overlaps.restype = i32
+        L.hc_sfo2overlaps.argtypes = [vp, u64, ctypes.c_int64, ctypes.c_int64, vp, u64, ctypes.POINTER(u64), vp, i32]
         L.hc_last_error.restype = ctypes.c_char_p
         L.hc_version.restype = ctypes.c_char_p
         _lib = L
@@ -507,6 +509,22 @@ def fno1_text_nonedges(fi: "F.FnoInput", idmap: "IdMap", head: np.ndarray, n_adj
             cap = int(nb.value)
             continue
         return rc, out[: nb.value].tobytes() if rc == 0 else b"", int(nl.value), int(nr.value), stats[0]
+
+
+def sfo2overlaps(text, num_singles: int, num_pairs: int, device: int = 0):
+    """hc_sfo2overlaps: the overlaps file lib/hc_sfo2overlaps writes for the SFO text (bytes or a uint8 array), built on
+    the GPU.  Returns (bytes, stats of formats.SFO_STATS).  Input the device path does not take raises HcError with code
+    HC_ERR_INPUT (-4); stats.first_error_* then name the line."""
+    buf = np.frombuffer(text, dtype=np.uint8) if isinstance(text, (bytes, bytearray)) else text
+    stats = np.zeros(1, dtype=F.SFO_STATS)
+    try:
+        out = _text_call(lambda p, cap, nb, nl: lib().hc_sfo2overlaps(buf.ctypes.data if len(buf) else None, len(buf), num_singles,
+                                                                       num_pairs, p, cap, nb, stats.ctypes.data, device),
+                         max(2 * len(buf), 4096))
+    except HcError as e:
+        e.stats = stats[0]
+        raise
+    return out, stats[0]
 
 
 def fno3_text(fi: "F.Fno3Input", device: int = 0) -> bytes:

@@ -158,6 +158,11 @@ FNO_NONEDGE_STATS = np.dtype([("n_lines", "<u8"), ("n_nonedges", "<u8"), ("n_str
                               ("first_error_offset", "<u8"), ("first_error_length", "<u8"), ("first_error_status", "<u4"),
                               ("device_ms", "<f4")])   # hc_fno_nonedge_stats
 assert FNO_NONEDGE_STATS.itemsize == 56
+SFO_STATS = np.dtype([("n_lines", "<u8"), ("n_unique", "<u8"), ("s_s_count", "<u8"), ("p_count", "<u8"), ("n_out_lines", "<u8"),
+                      ("first_error_line", "<u8"), ("first_error_offset", "<u8"), ("first_error_length", "<u8"),
+                      ("first_error_status", "<u4"), ("h2d_ms", "<f4"), ("device_ms", "<f4"), ("d2h_ms", "<f4")])   # hc_sfo_stats
+assert SFO_STATS.itemsize == 80
+SFO_DIES, SFO_DECLINED = 1, 2
 CONS_SEQ = np.dtype([("read", "<u4"), ("mate", "u1"), ("rc", "u1"), ("reserved", "<u2"), ("pos", "<i4")])
 CONS_PROBLEM = np.dtype([("seq_begin", "<u8"), ("seq_end", "<u8"), ("out_offset", "<u8"), ("total_len", "<i4"),
                          ("subreads_needed", "u1"), ("error_correction", "u1"), ("reserved", "u1", (2,))])

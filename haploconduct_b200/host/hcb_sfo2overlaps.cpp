@@ -14,7 +14,12 @@
 // The script spends its time in the Python loop and two external sorts; here parsing, flipping, sorting (parallel merge
 // sort) and the per-line / per-pair work run on all host threads and the results are stitched in the script's order.
 // SURVEY 8f rank 2 (the converter half).  Reference: scripts/sfo2overlaps.py.
+// --gpu=true: the same bytes from one hc_sfo2overlaps call (include/hc_b200.h; all of 1-4 on the device).  Input the
+// device path does not take (a line this program dies on, or one outside the device's ranges) or a working set that does
+// not fit the device is said on stderr and converted here as without the flag; no usable device is an error.
 #include <omp.h>
+
+#include "../../include/hc_b200.h"
 
 #include <algorithm>
 #include <cmath>
@@ -213,6 +218,7 @@ int main(int argc, char** argv) {
     auto mark = [&](const char* what) { if (timing) { const double t = now_s(); std::fprintf(stderr, "[hc_sfo2overlaps] %-28s %8.1f ms\n", what, (t - t_mark) * 1e3); t_mark = t; } };
     std::string in, out;
     long ns = -1, np = -1;
+    bool gpu = false;
     for (int i = 1; i < argc; i++) {
         std::string a = argv[i], v;
         const size_t eq = a.find('=');
@@ -222,10 +228,11 @@ int main(int argc, char** argv) {
         else if (a == "--out") out = v;
         else if (a == "--num_singles") ns = std::atol(v.c_str());
         else if (a == "--num_pairs") np = std::atol(v.c_str());
+        else if (a == "--gpu") gpu = v == "true" || v == "1";
         else { std::fprintf(stderr, "unknown option %s\n", a.c_str()); return 2; }
     }
     if (in.empty() || out.empty() || ns < 0 || np < 0) {
-        std::fprintf(stderr, "usage: hc_sfo2overlaps --in SFO --out OVERLAPS --num_singles N --num_pairs N\n");
+        std::fprintf(stderr, "usage: hc_sfo2overlaps --in SFO --out OVERLAPS --num_singles N --num_pairs N [--gpu=true]\n");
         return 2;
     }
     // ---- the file
@@ -249,6 +256,38 @@ int main(int argc, char** argv) {
     }
     close(fd);
     mark("file read");
+    if (gpu) {
+        // the output is rarely more than twice the input; a larger one costs a second call with the exact size
+        uint64_t cap = 2 * (uint64_t)text.size() + 4096, n_out = 0;
+        hc_sfo_stats st;
+        char* buf = (char*)std::malloc(cap);
+        if (!buf) die("hc_sfo2overlaps: out of host memory");
+        int rc = hc_sfo2overlaps(text.data(), text.size(), ns, np, buf, cap, &n_out, &st, 0);
+        if (rc == HC_ERR_CAPACITY) {
+            std::free(buf);
+            cap = n_out;
+            buf = (char*)std::malloc(cap ? cap : 1);
+            if (!buf) die("hc_sfo2overlaps: out of host memory");
+            rc = hc_sfo2overlaps(text.data(), text.size(), ns, np, buf, cap, &n_out, &st, 0);
+        }
+        if (rc == HC_OK) {
+            mark("device call");
+            if (timing)
+                std::fprintf(stderr, "[hc_sfo2overlaps]   copy in %.1f ms, device %.1f ms, copy out %.1f ms\n", st.h2d_ms, st.device_ms, st.d2h_ms);
+            FILE* fo = std::fopen(out.c_str(), "w");
+            if (!fo) die("IOError: cannot write " + out);
+            if (std::fwrite(buf, 1, n_out, fo) != n_out || std::fclose(fo) != 0) die("IOError: cannot write " + out);
+            std::free(buf);
+            mark("write");
+            std::printf("total overlap count: %lu\nof which single-single: %lu\n", (unsigned long)(st.s_s_count + st.p_count),
+                        (unsigned long)st.s_s_count);
+            return 0;
+        }
+        std::free(buf);
+        if (rc != HC_ERR_INPUT && rc != HC_ERR_NOMEM) die(hc_last_error());
+        std::fprintf(stderr, "%s; converting on the host\n", hc_last_error());
+        mark("device call (not taken)");
+    }
     std::vector<size_t> ls(1, 0);                               // line starts
     for (size_t i = 0; i < text.size(); i++) if (text[i] == '\n' && i + 1 < text.size()) ls.push_back(i + 1);
     if (text.empty()) ls.clear();

@@ -538,3 +538,110 @@ def consensus_problem_text(rs, problems) -> str:
                 s, q = revcomp(s), q[::-1]
             out.append("%d %s %s" % (pos, s, q))
     return "\n".join(out) + "\n"
+
+
+def _render_int(v: np.ndarray, zeros: np.ndarray, plus: np.ndarray) -> np.ndarray:
+    """Decimal text of v, right-aligned in a uint8 matrix (one row per value, 0 = no byte): `zeros` leading zeros and a
+    '+' before non-negative values where `plus` is set."""
+    mag = np.abs(v).astype(np.int64)
+    nd = np.ones(len(v), dtype=np.int64)
+    t = mag // 10
+    while t.any():
+        nd += t > 0
+        t //= 10
+    shown = nd + zeros
+    width = int(shown.max(initial=1)) + 1
+    m = np.zeros((len(v), width), dtype=np.uint8)
+    p10 = np.ones(len(v), dtype=np.int64)
+    for j in range(width):                                # j = position from the right
+        col = width - 1 - j
+        m[:, col] = np.where(j < shown, ord("0") + (mag // p10) % 10, 0)
+        sign = np.where(v < 0, ord("-"), np.where(plus, ord("+"), 0))
+        m[:, col] = np.where(j == shown, sign, m[:, col])
+        if j < 18:
+            p10 = p10 * 10
+    return m
+
+
+def make_sfo_text(seed: int, num_singles: int, num_pairs: int, n_lines: int, irregular: bool = False,
+                  dup_fraction: float = 0.05, chunk: int = 1 << 20) -> bytes:
+    """Seeded SFO text ("idA idB ori OHA OHB OLA OLB K" per line, the overlapper's output that lib/hc_sfo2overlaps reads),
+    built with numpy a chunk of lines at a time (oracle/make_golden_sfo.make_sfo writes one line at a time and is meant
+    for small fixtures).  Per chunk: overlaps of two paired-end reads as the two lines of their ends (consistent, so that
+    the converter matches most of them), single-paired and single-single overlaps (num_singles > 0), a few
+    self-overlaps; both orientations, overhangs of either sign, either id first (flipped lines); dup_fraction of the
+    lines repeated elsewhere in the chunk.  irregular: separators of spaces and tabs, leading whitespace, '+' signs,
+    leading zeros and CRLF line ends, chosen per line."""
+    ss = np.random.SeedSequence(seed)
+    parts = []
+    left = n_lines
+    for child in ss.spawn(max(1, (n_lines + chunk - 1) // chunk)):
+        if left <= 0:
+            break
+        c = min(chunk, left)
+        left -= c
+        parts.append(_sfo_chunk(np.random.default_rng(child), num_singles, num_pairs, c, irregular, dup_fraction))
+    return b"".join(parts)
+
+
+def _sfo_chunk(rng, ns: int, npairs: int, n: int, irregular: bool, dup_fraction: float) -> bytes:
+    m = max(1, int(round(n * (1 - dup_fraction))))
+    ev = (m + 1) // 2                                      # overlap events of two lines each
+    kind = rng.random(ev)
+    if npairs == 0:
+        kind[:] = 0.95
+    elif ns == 0:
+        kind[:] = 0.0
+    a = rng.integers(0, max(npairs, 1), ev)
+    b = (a + 1 + rng.integers(0, max(min(npairs, 200) - 1, 1), ev)) % max(npairs, 1)
+    s1 = rng.integers(0, max(ns, 1), ev)
+    s2 = (s1 + 1 + rng.integers(0, max(min(ns, 200) - 1, 1), ev)) % max(ns, 1)
+    isN = rng.random(ev) < 0.6
+    end = np.stack([np.zeros(ev, np.int64), np.ones(ev, np.int64)], 1)                 # (ev, 2): the two lines
+    mateB = np.where(isN[:, None], end, 1 - end)
+    pp = (ns + a[:, None] + end * npairs, ns + b[:, None] + mateB * npairs)
+    sp = (np.repeat(s1[:, None], 2, 1), ns + a[:, None] + end * npairs)
+    s_s = (np.stack([s1, s2], 1), np.stack([s2, s1], 1))
+    self_ = (np.repeat((ns + a)[:, None], 2, 1), ns + a[:, None] + end * npairs)
+    sel = np.select([kind < 0.7, kind < 0.85, kind < 0.99], [0, 1, 2], 3)[:, None]
+    idA = np.choose(sel, [pp[0], sp[0], s_s[0], self_[0]]).ravel()[:m]
+    idB = np.choose(sel, [pp[1], sp[1], s_s[1], self_[1]]).ravel()[:m]
+    if npairs == 0:
+        idA, idB = np.stack([s1, s2], 1).ravel()[:m], np.stack([s2, s1], 1).ravel()[:m]
+    ori = np.repeat(np.where(isN, ord("N"), ord("I")), 2)[:m].astype(np.uint8)
+    oha = rng.integers(-60, 61, m)
+    ohb = rng.integers(-60, 61, m)
+    ola = rng.integers(20, 151, m)
+    olb = ola + rng.integers(-3, 4, m)
+    k = rng.integers(0, 4, m)
+    swap = rng.random(m) < 0.5                             # the same overlap seen from the other read
+    isI = ori == ord("I")
+    idA, idB = np.where(swap, idB, idA), np.where(swap, idA, idB)
+    oha, ohb = np.where(swap, np.where(isI, ohb, -oha), oha), np.where(swap, np.where(isI, oha, -ohb), ohb)
+    ola, olb = np.where(swap, olb, ola), np.where(swap, ola, olb)
+    idx = np.concatenate([np.arange(m), rng.integers(0, m, n - m)])
+    idx = idx[rng.permutation(n)]
+    f = [a_[idx] for a_ in (idA, idB, ori, oha, ohb, ola, olb, k)]
+    nf = len(f)
+    if irregular:
+        zeros = rng.integers(0, 3, (nf, n)) * (rng.random((nf, n)) < 0.1)
+        plus = rng.random((nf, n)) < 0.1
+        sep_kind = rng.integers(0, 4, (nf, n)) * (rng.random((nf, n)) < 0.3)     # 0 tab, 1 space, 2 two spaces, 3 space tab
+        lead = np.where(rng.random(n) < 0.05, ord(" "), 0).astype(np.uint8)
+        crlf = rng.random(n) < 0.2
+    else:
+        zeros = np.zeros((nf, n), np.int64)
+        plus = np.zeros((nf, n), bool)
+        sep_kind = np.zeros((nf, n), np.int64)
+        lead = np.zeros(n, np.uint8)
+        crlf = np.zeros(n, bool)
+    sep_tab = np.array([[9, 0], [32, 0], [32, 32], [32, 9]], dtype=np.uint8)
+    cols = [lead[:, None]]
+    for j in range(nf):
+        if j:
+            cols.append(sep_tab[sep_kind[j]])
+        cols.append(f[j][:, None] if j == 2 else _render_int(f[j], zeros[j], plus[j]))
+    cols.append(np.where(crlf, 13, 0).astype(np.uint8)[:, None])
+    cols.append(np.full((n, 1), 10, np.uint8))
+    mat = np.concatenate(cols, axis=1).ravel()
+    return mat[mat != 0].tobytes()

@@ -721,6 +721,48 @@ int hc_consensus(hc_store* s, const hc_cons_problem* problems, uint64_t n_proble
                  uint32_t min_clique_size, double min_qual, char* cons_seq, char* cons_qual, uint64_t out_bytes,
                  hc_cons_result* results);
 
+/* ------------------------------------------------------------------------------------------
+ * Overlapper output -> overlaps file (the converter half of SURVEY 8f rank 2): what
+ * lib/hc_sfo2overlaps --in SFO --num_singles NS --num_pairs NP writes (scripts/sfo2overlaps.py of the
+ * reference, haploconduct_b200/host/hcb_sfo2overlaps.cpp), built on the device.
+ *
+ * sfo is host memory (pageable or pinned): the lines "idA idB ori OHA OHB OLA OLB K" the overlapper wrote; an
+ * unterminated last line counts.  On HC_OK text[0 .. *n_text_bytes) holds the bytes the host converter writes for the
+ * same text, and stats its counts ("total overlap count" = s_s_count + p_count).  Parsing, flipping, the sort, both
+ * uniq steps, the pair matching and the formatting run on the device; the only copies are the text in and the file out.
+ * Capacity as for hc_fno1_text: HC_ERR_CAPACITY with the exact size in *n_text_bytes when text_cap is too small (text
+ * may be NULL when text_cap is 0); a repeated call does all the work again.
+ * HC_ERR_INPUT, nothing written, with the first such line (0-based, file order) in stats->first_error_*:
+ *   HC_SFO_DIES      the host converter exits 1 on this input: a line without 8 whitespace-separated fields (an empty
+ *                    line too), a numeric field its parse_long rejects, an sfo id outside [0, NS + 2 NP) when NP > 0, or
+ *                    min(lenA, lenB) <= 0 in s_s_overlap of a single-single line or of a pair that is matched;
+ *   HC_SFO_DECLINED  outside what the device path covers: an original or sfo id outside [0, 2^32) (NP == 0 only), a
+ *                    numeric field of more than 18 digits, |OHA|, |OHB|, |OLA| or |OLB| >= 2^40, 2^32 lines or more.
+ * The caller then runs the host converter, which writes the file or dies with its own message.
+ * HC_ERR_NOMEM when the working set does not fit the device: about 2 x n_bytes + 220 bytes per SFO line for the sort,
+ * plus 2 x the output size and 12 bytes per output line before the final uniq.
+ * HC_ERR_ARG for NULL pointers, NS < 0 or NP < 0.  HC_ERR_CUDA when no sm_100 device is usable.
+ * ------------------------------------------------------------------------------------------ */
+#define HC_SFO_DIES      1
+#define HC_SFO_DECLINED  2
+
+typedef struct {
+    uint64_t n_lines;             /* SFO lines in the text                                                  */
+    uint64_t n_unique;            /* after `sort -k1,1n -k2,2n -k3,3n -k4,4n | uniq`                        */
+    uint64_t s_s_count;           /* single-single overlaps written ("of which single-single")               */
+    uint64_t p_count;             /* matched paired overlaps                                                 */
+    uint64_t n_out_lines;         /* lines of the overlaps file (after the final uniq)                      */
+    uint64_t first_error_line;    /* 0-based in file order, ~0 if none; its byte offset / length            */
+    uint64_t first_error_offset, first_error_length;
+    uint32_t first_error_status;  /* HC_SFO_DIES / HC_SFO_DECLINED                                           */
+    float    h2d_ms;              /* host clock: the text to the device                                     */
+    float    device_ms;           /* host clock: every kernel, from the text on the device to the file there */
+    float    d2h_ms;              /* host clock: the file to `text`                                         */
+} hc_sfo_stats;                   /* 80 bytes */
+
+int hc_sfo2overlaps(const char* sfo, uint64_t n_bytes, int64_t num_singles, int64_t num_pairs,
+                    char* text, uint64_t text_cap, uint64_t* n_text_bytes, hc_sfo_stats* stats, int device);
+
 int         hc_device_count(void);
 const char* hc_last_error(void);
 const char* hc_version(void);
