@@ -13,7 +13,7 @@ PRIMS_SHIM = os.path.join(LIBDIR, "libhc_prims_shim.so")
 NVCC = os.environ.get("HC_NVCC", "/usr/local/cuda/bin/nvcc")
 HOST_CXX = "/usr/bin/g++"
 
-CU_SOURCES = ["hc_kernels.cu", "hc_api.cu", "hc_fno.cu", "hc_fno_text.cu", "hc_sfo.cu", "hc_dedup.cu", "hc_ingest.cu", "hc_pack.cu", "hc_consensus.cu", "hc_stage.cu", "hc_adjacency.cu"]
+CU_SOURCES = ["hc_kernels.cu", "hc_api.cu", "hc_fno.cu", "hc_fno_text.cu", "hc_sfo.cu", "hc_sam.cu", "hc_dedup.cu", "hc_ingest.cu", "hc_pack.cu", "hc_consensus.cu", "hc_stage.cu", "hc_adjacency.cu"]
 CPP_SOURCES = ["hc_tables.cpp", "hc_cons_final.cpp"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 
@@ -97,9 +97,10 @@ def build_host(verbose: bool = False) -> str:
     if verbose:
         print(" ".join(cmd))
     subprocess.check_call(cmd)
-    # hc_sam2overlaps: scripts/sam2overlaps.py of the reference in C++ (host only)
+    # hc_sam2overlaps: scripts/sam2overlaps.py of the reference in C++; --gpu=true through hc_sam2overlaps of the C ABI
     conv = os.path.join(LIBDIR, "hc_sam2overlaps")
-    cmd = [HOST_CXX, "-O2", "-std=c++14", "-Wall", "-fopenmp", "-o", conv, os.path.join(host, "hcb_sam2overlaps.cpp")]
+    cmd = [HOST_CXX, "-O2", "-std=c++14", "-Wall", "-fopenmp", "-o", conv, os.path.join(host, "hcb_sam2overlaps.cpp"), "-L" + LIBDIR,
+           "-lhc_b200", "-lpthread", "-Wl,-rpath,$ORIGIN"]
     if verbose:
         print(" ".join(cmd))
     subprocess.check_call(cmd)

@@ -24,7 +24,7 @@ EXPORTED = [
     "hc_overlap_score", "hc_overlap_score_multi",
     "hc_phred_to_prob", "hc_exp_threshold", "hc_device_count", "hc_warm_up", "hc_last_error", "hc_version", "hc_fno1", "hc_fno3", "hc_fno1_small", "hc_fno3_small", "hc_fno1_text", "hc_fno3_text", "hc_build_adjacency", "hc_subread_info", "hc_host_alloc", "hc_host_free",
     "hc_store_create_fastq", "hc_store_create_fastq_files", "hc_store_read_ids", "hc_consensus", "hc_dedup_edges", "hc_idmap_create", "hc_idmap_destroy", "hc_ingest_overlaps", "hc_ingest_overlaps_device",
-    "hc_ingest_score_overlaps", "hc_fno1_text_nonedges", "hc_sfo2overlaps",
+    "hc_ingest_score_overlaps", "hc_fno1_text_nonedges", "hc_sfo2overlaps", "hc_sam2overlaps",
 ]
 
 _lib: Optional[ctypes.CDLL] = None
@@ -130,6 +130,9 @@ def lib() -> ctypes.CDLL:
                                             ctypes.POINTER(u64), vp, i32]
         L.hc_sfo2overlaps.restype = i32
         L.hc_sfo2overlaps.argtypes = [vp, u64, ctypes.c_int64, ctypes.c_int64, vp, u64, ctypes.POINTER(u64), vp, i32]
+        L.hc_sam2overlaps.restype = i32
+        L.hc_sam2overlaps.argtypes = [vp, u64, vp, u64, vp, vp, vp, ctypes.c_uint32, vp, ctypes.c_uint32, ctypes.c_int64, vp, u64,
+                                      ctypes.POINTER(u64), vp, vp, i32]
         L.hc_last_error.restype = ctypes.c_char_p
         L.hc_version.restype = ctypes.c_char_p
         _lib = L
@@ -525,6 +528,36 @@ def sfo2overlaps(text, num_singles: int, num_pairs: int, device: int = 0):
         e.stats = stats[0]
         raise
     return out, stats[0]
+
+
+def sam2overlaps(sam_s, sam_p, ref_names, ref_len, min_overlap_len: int, device: int = 0):
+    """hc_sam2overlaps: the overlaps file lib/hc_sam2overlaps writes for the single-end and paired-end SAM texts (bytes
+    or uint8 arrays; None = absent), built on the GPU.  ref_names: the FASTA's name -> reference index map (a dict), or a
+    sequence whose entry r names reference r; names are str or bytes.  ref_len[r]: the length of reference r.  Returns
+    (bytes, stats of formats.SAM_STATS, per-reference stats of formats.SAM_REF_STATS).  Input the device path does not
+    take raises HcError with code HC_ERR_INPUT (-4); stats.first_error_* then name the line."""
+    def as_buf(t):
+        if t is None:
+            return np.zeros(0, dtype=np.uint8)
+        return np.frombuffer(t, dtype=np.uint8) if isinstance(t, (bytes, bytearray)) else t
+    bs, bp = as_buf(sam_s), as_buf(sam_p)
+    items = list(ref_names.items()) if isinstance(ref_names, dict) else list((n, r) for r, n in enumerate(ref_names))
+    enc = [n.encode() if isinstance(n, str) else bytes(n) for n, _ in items]
+    names = np.frombuffer(b"".join(enc) + b"\0", dtype=np.uint8)
+    off = np.concatenate([[0], np.cumsum([len(n) for n in enc], dtype=np.uint64)]).astype(np.uint64)
+    idx = np.array([r for _, r in items], dtype=np.uint32)
+    rlen = np.ascontiguousarray(ref_len, dtype=np.int64)
+    stats = np.zeros(1, dtype=F.SAM_STATS)
+    rstats = np.zeros(len(rlen), dtype=F.SAM_REF_STATS)
+    try:
+        out = _text_call(lambda p, cap, nb, nl: lib().hc_sam2overlaps(
+            bs.ctypes.data if len(bs) else None, len(bs), bp.ctypes.data if len(bp) else None, len(bp), names.ctypes.data,
+            off.ctypes.data, idx.ctypes.data, len(idx), rlen.ctypes.data, len(rlen), min_overlap_len, p, cap, nb,
+            rstats.ctypes.data, stats.ctypes.data, device), max(16 * (len(bs) + len(bp)), 4096))
+    except HcError as e:
+        e.stats = stats[0]
+        raise
+    return out, stats[0], rstats
 
 
 def fno3_text(fi: "F.Fno3Input", device: int = 0) -> bytes:

@@ -163,6 +163,15 @@ SFO_STATS = np.dtype([("n_lines", "<u8"), ("n_unique", "<u8"), ("s_s_count", "<u
                       ("first_error_status", "<u4"), ("h2d_ms", "<f4"), ("device_ms", "<f4"), ("d2h_ms", "<f4")])   # hc_sfo_stats
 assert SFO_STATS.itemsize == 80
 SFO_DIES, SFO_DECLINED = 1, 2
+SAM_STATS = np.dtype([("unmapped_s", "<u8"), ("reverse_s", "<u8"), ("discarded", "<u8"), ("unmapped_p", "<u8"), ("reverse_p", "<u8"),
+                      ("total_alns", "<u8"), ("n_out_lines", "<u8"), ("first_error_line", "<u8"), ("first_error_offset", "<u8"),
+                      ("first_error_length", "<u8"), ("first_error_file", "<u4"), ("first_error_status", "<u4"), ("h2d_ms", "<f4"),
+                      ("device_ms", "<f4"), ("d2h_ms", "<f4"), ("reserved", "<u4")])   # hc_sam_stats
+assert SAM_STATS.itemsize == 104
+SAM_REF_STATS = np.dtype([("n_alignments", "<u8"), ("n_singles", "<u8"), ("n_paired", "<u8"), ("problems", "<u8"), ("n_overlaps", "<u8"),
+                          ("types", "<u8", (4,))])   # hc_sam_ref_stats
+assert SAM_REF_STATS.itemsize == 72
+SAM_DIES, SAM_DECLINED = 1, 2
 CONS_SEQ = np.dtype([("read", "<u4"), ("mate", "u1"), ("rc", "u1"), ("reserved", "<u2"), ("pos", "<i4")])
 CONS_PROBLEM = np.dtype([("seq_begin", "<u8"), ("seq_end", "<u8"), ("out_offset", "<u8"), ("total_len", "<i4"),
                          ("subreads_needed", "u1"), ("error_correction", "u1"), ("reserved", "u1", (2,))])

@@ -9,7 +9,13 @@
 // sorted, so "read j is active when read i arrives" is  i == j + 1  or  len_j - (POS_{i-1} - POS_j) >= min_overlap_len :
 // every read i finds its partners by itself and all reads are processed in parallel, the lines stitched in the script's order.
 // SURVEY 8f rank 2 (the converter half).  Reference: scripts/sam2overlaps.py.
+// --gpu=true: the same bytes and stdout from one hc_sam2overlaps call (include/hc_b200.h; pairing, sort and sweep on the
+// device; the FASTA is read here as without the flag).  Input the device path does not take (a line this program dies
+// on, or one outside the device's ranges) or a working set that does not fit the device is said on stderr and
+// converted here as without the flag; no usable device is an error.
 #include <omp.h>
+
+#include "../../include/hc_b200.h"
 
 #include <algorithm>
 #include <cmath>
@@ -17,6 +23,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <fstream>
+#include <iterator>
 #include <map>
 #include <string>
 #include <vector>
@@ -236,7 +243,7 @@ std::vector<std::string> read_lines(const std::string& path) {
 int main(int argc, char** argv) {
     std::string sam_s, sam_p, ref_path, out;
     long min_ov = 0;
-    bool verbose = false;
+    bool verbose = false, gpu = false;
     for (int i = 1; i < argc; i++) {
         std::string a = argv[i], v;
         const size_t eq = a.find('=');
@@ -248,10 +255,11 @@ int main(int argc, char** argv) {
         else if (a == "--ref") ref_path = v;
         else if (a == "--out") out = v;
         else if (a == "--min_overlap_len") min_ov = std::atol(v.c_str());
+        else if (a == "--gpu") gpu = v == "true" || v == "1";
         else { std::fprintf(stderr, "unknown option %s\n", a.c_str()); return 2; }
     }
     if ((sam_s.empty() && sam_p.empty()) || out.empty() || ref_path.empty()) {
-        std::fprintf(stderr, "usage: hc_sam2overlaps [--sam_s S.sam] [--sam_p P.sam] --ref REF.fasta --out OVERLAPS [--min_overlap_len N] [--verbose]\n");
+        std::fprintf(stderr, "usage: hc_sam2overlaps [--sam_s S.sam] [--sam_p P.sam] --ref REF.fasta --out OVERLAPS [--min_overlap_len N] [--verbose] [--gpu=true]\n");
         return 2;
     }
     std::remove(out.c_str());
@@ -280,6 +288,77 @@ int main(int argc, char** argv) {
         if (!have_seq) { std::printf("invalid fasta file... exiting\n"); return 1; }
         ref_len.push_back(seq);
         ref_idx[id] = ref_len.size() - 1;
+    }
+    if (gpu) {
+        std::string text_s, text_p;
+        auto slurp = [](const std::string& path, std::string& t) {
+            std::ifstream f(path.c_str(), std::ios::binary);
+            if (!f.is_open()) return false;
+            t.assign(std::istreambuf_iterator<char>(f), std::istreambuf_iterator<char>());
+            return true;
+        };
+        // a file that cannot be read is left to the host path, which says so as without the flag
+        if ((sam_s.empty() || slurp(sam_s, text_s)) && (sam_p.empty() || slurp(sam_p, text_p))) {
+            std::string names;
+            std::vector<uint64_t> name_off(1, 0);
+            std::vector<uint32_t> name_idx;
+            for (const auto& e : ref_idx) {
+                names += e.first;
+                name_off.push_back(names.size());
+                name_idx.push_back((uint32_t)e.second);
+            }
+            const uint32_t n_refs = (uint32_t)ref_len.size();
+            std::vector<int64_t> rlen(ref_len.begin(), ref_len.end());
+            std::vector<hc_sam_ref_stats> rs(n_refs);
+            hc_sam_stats st;
+            // the file is typically several times the SAM text (tens of lines per alignment); a larger one costs a
+            // second call with the exact size
+            uint64_t cap = 16 * (uint64_t)(text_s.size() + text_p.size()) + (1u << 20), n_out = 0;
+            auto call = [&](char* buf) {
+                return hc_sam2overlaps(text_s.data(), text_s.size(), text_p.data(), text_p.size(), names.data(), name_off.data(),
+                                       name_idx.data(), (uint32_t)name_idx.size(), rlen.data(), n_refs, min_ov, buf, cap, &n_out,
+                                       rs.data(), &st, 0);
+            };
+            char* buf = (char*)std::malloc(cap);
+            if (!buf) die("hc_sam2overlaps: out of host memory");
+            int rc = call(buf);
+            if (rc == HC_ERR_CAPACITY) {
+                std::free(buf);
+                cap = n_out;
+                buf = (char*)std::malloc(cap ? cap : 1);
+                if (!buf) die("hc_sam2overlaps: out of host memory");
+                rc = call(buf);
+            }
+            if (rc == HC_OK) {
+                if (std::getenv("HC_TIMING"))
+                    std::fprintf(stderr, "[hc_sam2overlaps]   copy in %.1f ms, device %.1f ms, copy out %.1f ms\n", st.h2d_ms, st.device_ms, st.d2h_ms);
+                FILE* fo = std::fopen(out.c_str(), "w");
+                if (!fo) die("IOError: cannot write " + out);
+                if (std::fwrite(buf, 1, n_out, fo) != n_out || std::fclose(fo) != 0) die("IOError: cannot write " + out);
+                std::free(buf);
+                if (verbose && !sam_s.empty())
+                    std::printf("Number of singles unmapped:  %lu\nNumber of singles reversed:  %lu\n", (unsigned long)st.unmapped_s,
+                                (unsigned long)st.reverse_s);
+                if (verbose && !sam_p.empty())
+                    std::printf("Number of read ends discarded:  %lu\nNumber of read ends unmapped:  %lu\nNumber of reverse complements considered:  %lu\n",
+                                (unsigned long)st.discarded, (unsigned long)st.unmapped_p, (unsigned long)st.reverse_p);
+                for (uint32_t r = 0; r < n_refs && verbose; r++) {
+                    const hc_sam_ref_stats& x = rs[r];
+                    if (x.n_alignments == 0) continue;
+                    std::printf("Total number of alignments:  %lu\n... of which singles:  %lu\n... of which paired:  %lu\n", (unsigned long)x.n_alignments,
+                                (unsigned long)x.n_singles, (unsigned long)x.n_paired);
+                    if (x.problems > 0) std::printf("# cases where overlap_pos2 < 0:  %lu\n", (unsigned long)x.problems);
+                    std::printf("Total number of overlaps found:  %lu\n... of which ++:  %lu\n... of which +-:  %lu\n... of which -+:  %lu\n... of which --:  %lu\n",
+                                (unsigned long)x.n_overlaps, (unsigned long)x.types[0], (unsigned long)x.types[1], (unsigned long)x.types[2],
+                                (unsigned long)x.types[3]);
+                }
+                if (st.total_alns == 0) { std::printf("\n\nERROR: No reads could be aligned to reference. Exiting.\n"); return 1; }
+                return 0;
+            }
+            std::free(buf);
+            if (rc != HC_ERR_INPUT && rc != HC_ERR_NOMEM) die(hc_last_error());
+            std::fprintf(stderr, "%s; converting on the host\n", hc_last_error());
+        }
     }
     // ---- alignments (the header is skipped while lines start with '@'; parsing in parallel, pairing in file order)
     auto parse_file = [&](const std::string& path, std::vector<Aln>& alns, std::vector<char>& mapped) {

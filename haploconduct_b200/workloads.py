@@ -645,3 +645,113 @@ def _sfo_chunk(rng, ns: int, npairs: int, n: int, irregular: bool, dup_fraction:
     cols.append(np.full((n, 1), 10, np.uint8))
     mat = np.concatenate(cols, axis=1).ravel()
     return mat[mat != 0].tobytes()
+
+
+def make_sam_text(seed: int, n_single: int, n_pairs: int, refs: Sequence[Tuple[str, int]], irregular: bool = False,
+                  chunk: int = 1 << 18) -> Tuple[bytes, bytes, bytes]:
+    """Seeded (FASTA, single-end SAM, interleaved paired-end SAM) text of alignments to `refs` ((name, length) pairs),
+    what lib/hc_sam2overlaps reads, built with numpy a chunk of lines at a time (oracle/make_golden_sam.make_case writes
+    one line at a time and is meant for small fixtures).  The same cases as make_case: soft and hard clips, insertions,
+    deletions, reverse strands, unmapped singles and unmapped first ends, pair ends of different orientation, mismatched
+    pair ids (q<i>), several references, single-end positions up to 40 past the reference end.  irregular: CRLF line ends,
+    multi-character CIGAR operations ("MM", "SS", "=" runs) and alignments further past the reference end, chosen per line.
+    (A doubled hard clip, "HH", would count as reference bases but not as read length: overlaps of negative length, on
+    which the converter exits.)  Both SAM texts start with an @SQ / @PG header."""
+    ss = np.random.SeedSequence(seed)
+    r_fa, r_s, r_p = (np.random.default_rng(c) for c in ss.spawn(3))
+    fasta = b"".join(b">%s description\n" % n.encode() + _fasta_seq(r_fa, L) for n, L in refs)
+    header = b"".join(b"@SQ\tSN:%s\tLN:%d\n" % (n.encode(), L) for n, L in refs) + b"@PG\tID:x\n"
+    names = [n.encode() for n, _ in refs]
+    lens = np.array([L for _, L in refs], dtype=np.int64)
+    out_s, out_p = [header], [header]
+    for c0 in range(0, n_single, chunk):
+        c = min(chunk, n_single - c0)
+        ref = r_s.integers(0, len(refs), c)
+        flag = np.array([0, 16, 4])[r_s.choice(3, c, p=[0.55, 0.35, 0.1])]
+        pos = r_s.integers(1, lens[ref] + 40)
+        if irregular:
+            pos = np.where(r_s.random(c) < 0.02, lens[ref] + r_s.integers(0, 400, c), pos)
+        out_s.append(_sam_lines(r_s, b"s", np.arange(c0, c0 + c), np.zeros(c, bool), flag, ref, pos, names, irregular))
+    for c0 in range(0, n_pairs, chunk):
+        c = min(chunk, n_pairs - c0)
+        ref = r_p.integers(0, len(refs), c)
+        p1 = r_p.integers(1, lens[ref])
+        p2 = p1 + r_p.integers(-20, 200, c)
+        r = r_p.random(c)
+        both_rev = (r >= 0.45) & (r < 0.8)
+        f1 = np.select([r < 0.45, r < 0.8, r < 0.9], [0, 16, 0], 4)
+        f2 = np.select([r < 0.45, r < 0.8, r < 0.9], [0, 16, 16], 0)
+        p1, p2 = np.where(both_rev, np.maximum(p1, p2), p1), np.where(both_rev, np.minimum(p1, p2), p2)
+        q = r_p.random(c) <= 0.03
+        num = np.repeat(np.arange(c0, c0 + c), 2)
+        mism = np.stack([np.zeros(c, bool), q], 1).ravel()
+        flag = np.stack([f1, f2], 1).ravel()
+        pos = np.maximum(np.stack([p1, p2], 1).ravel(), 1)
+        out_p.append(_sam_lines(r_p, b"p", num, mism, flag, np.repeat(ref, 2), pos, names, irregular))
+    return fasta, b"".join(out_s), b"".join(out_p)
+
+
+def _fasta_seq(rng, L: int) -> bytes:
+    seq = np.frombuffer(b"ACGT", dtype=np.uint8)[rng.integers(0, 4, L)]
+    rows = [seq[o:o + 70].tobytes() for o in range(0, L, 70)]
+    return b"\n".join(rows) + b"\n"
+
+
+def _text_col(words: Sequence[bytes], pick: np.ndarray) -> np.ndarray:
+    """Rows of a uint8 matrix spelling words[pick[i]], 0 = no byte."""
+    w = max(1, max(len(x) for x in words))
+    tab = np.zeros((len(words), w), dtype=np.uint8)
+    for i, x in enumerate(words):
+        tab[i, :len(x)] = np.frombuffer(x, dtype=np.uint8)
+    return tab[pick]
+
+
+def _sam_lines(rng, prefix: bytes, num: np.ndarray, mism: np.ndarray, flag: np.ndarray, ref: np.ndarray, pos: np.ndarray,
+               names: List[bytes], irregular: bool) -> bytes:
+    n = len(num)
+    qlen = rng.integers(60, 151, n)
+    kind = rng.integers(0, 8, n)
+    clip = rng.integers(1, 8, n)
+    pre_s, pre_h, post_h = kind == 1, kind == 2, kind == 3
+    core = qlen - np.where(pre_s, clip, 0)
+    ins = (np.isin(kind, (4, 6)) & (core > 30))
+    dl = (np.isin(kind, (5, 7)) & (core > 30))
+    a = rng.integers(5, np.maximum(core - 10, 6))
+    k_id = np.where(ins, rng.integers(1, 4, n), rng.integers(1, 5, n))
+    rest = np.where(ins, core - a - k_id, core - a)
+    first = np.where(ins | dl, a, core)
+    none = np.zeros(n, np.int64)
+
+    def num_col(v, keep):
+        m = _render_int(v, none, np.zeros(n, bool))
+        m[~keep] = 0
+        return m
+
+    op_m = np.zeros(n, np.int64)                     # 0 "M", 1 "MM", 2 "=", indices into the words below
+    op_clip = np.zeros(n, np.int64)                  # 1: a soft clip spelled "SS"
+    crlf = np.zeros(n, bool)
+    if irregular:
+        op_m = np.where(rng.random(n) < 0.05, rng.integers(1, 3, n), 0)
+        op_clip = (rng.random(n) < 0.2).astype(np.int64)
+        crlf = rng.random(n) < 0.2
+    mid = np.where(ins, 0, np.where(dl, 1, 2))       # "I", "D", none
+    cols = [
+        np.full((n, 1), prefix[0], np.uint8), _text_col([b"", b"q"], mism.astype(np.int64)), num_col(num, np.ones(n, bool)),
+        np.full((n, 1), 9, np.uint8), num_col(flag, np.ones(n, bool)), np.full((n, 1), 9, np.uint8),
+        _text_col(names, ref), np.full((n, 1), 9, np.uint8), num_col(pos, np.ones(n, bool)), _text_col([b"\t60\t"], none),
+        num_col(clip, pre_s | pre_h), _text_col([b"", b"S", b"H", b"SS"], np.where(pre_s, 1 + 2 * op_clip, np.where(pre_h, 2, 0))),
+        num_col(first, np.ones(n, bool)), _text_col([b"M", b"MM", b"="], op_m),
+        num_col(k_id, ins | dl), _text_col([b"I", b"D", b""], mid),
+        num_col(rest, ins | dl), _text_col([b"M", b"MM", b"="], np.where(ins | dl, op_m, 0)) * (ins | dl)[:, None],
+        num_col(clip, post_h), _text_col([b"", b"H"], post_h.astype(np.int64)),
+        _text_col([b"\t=\t0\t0\t"], none),
+    ]
+    seq = np.frombuffer(b"ACGT", dtype=np.uint8)[rng.integers(0, 4, (n, 150), dtype=np.uint8)]
+    inside = np.arange(150)[None, :] < qlen[:, None]
+    cols.append(np.where(inside, seq, 0).astype(np.uint8))
+    cols.append(np.full((n, 1), 9, np.uint8))
+    cols.append(np.where(inside, ord("I"), 0).astype(np.uint8))
+    cols.append(np.where(crlf, 13, 0).astype(np.uint8)[:, None])
+    cols.append(np.full((n, 1), 10, np.uint8))
+    mat = np.concatenate(cols, axis=1).ravel()
+    return mat[mat != 0].tobytes()

@@ -763,6 +763,65 @@ typedef struct {
 int hc_sfo2overlaps(const char* sfo, uint64_t n_bytes, int64_t num_singles, int64_t num_pairs,
                     char* text, uint64_t text_cap, uint64_t* n_text_bytes, hc_sfo_stats* stats, int device);
 
+/* ------------------------------------------------------------------------------------------
+ * Alignments to a reference -> overlaps file (the other converter of SURVEY 8f rank 2): what
+ * lib/hc_sam2overlaps --sam_s S --sam_p P --ref REF --min_overlap_len N writes (scripts/sam2overlaps.py of the
+ * reference, haploconduct_b200/host/hcb_sam2overlaps.cpp), built on the device.
+ *
+ * sam_s / sam_p are host memory: the single-end SAM text and the interleaved paired-end SAM text (NULL / 0 = absent);
+ * an unterminated last line counts.  The names table is the converter's map from FASTA id to reference index: entry e
+ * is the name ref_names[ref_name_off[e] .. ref_name_off[e + 1]) (bytes) of reference ref_name_idx[e] < n_refs; names are
+ * unique (the FASTA's "last duplicate wins" is the caller's).  ref_len[r] is the length of reference r.
+ * On HC_OK text[0 .. *n_text_bytes) holds the bytes the host converter writes, stats its file-level counts and, when
+ * ref_stats is not NULL, ref_stats[r] what --verbose prints for reference r.  Pairing, the sort, the sweep and the
+ * formatting run on the device; the only copies are the two texts in and the file out.  Capacity as for
+ * hc_sfo2overlaps: HC_ERR_CAPACITY with the exact size in *n_text_bytes (text may be NULL when text_cap is 0).
+ * HC_ERR_INPUT, nothing written, with the first such line (file 0 = single-end, 1 = paired-end; 0-based line) in
+ * stats->first_error_*:
+ *   HC_SAM_DIES      the host converter exits 1 on this input: fewer than 11 fields, a FLAG / POS / MAPQ / PNEXT /
+ *                    TLEN its to_long rejects (only FLAG on an unmapped line), a CIGAR of fewer than 2 runs, a REF
+ *                    absent from the names table (singles; the first end of an accepted pair), or, where the sweep
+ *                    walks an alignment, an odd CIGAR run count, a CIGAR starting with a non-digit, a zero-length run
+ *                    (back walk only), a zero length or a percentage outside [0, 100]; sweep errors name one of the
+ *                    alignments involved;
+ *   HC_SAM_DECLINED  outside what the device path covers: a numeric field of more than 18 digits, |POS|, a clip or a
+ *                    CIGAR run of 2^40 or more, 2^32 lines or more in the two texts.
+ * The caller then runs the host converter, which writes the file or dies with its own message.
+ * HC_ERR_NOMEM when the working set does not fit the device (about the texts + 200 bytes per line + the output)
+ * or one alignment's lines reach 2^32 bytes.  HC_ERR_ARG for NULL pointers, decreasing name offsets, an index >= n_refs
+ * or a name given twice.  HC_ERR_CUDA when no sm_100 device is usable.
+ * ------------------------------------------------------------------------------------------ */
+#define HC_SAM_DIES      1
+#define HC_SAM_DECLINED  2
+
+typedef struct {
+    uint64_t unmapped_s, reverse_s;           /* "Number of singles unmapped / reversed"                        */
+    uint64_t discarded, unmapped_p, reverse_p; /* "Number of read ends discarded / unmapped", "reverse complements" */
+    uint64_t total_alns;                      /* records over all references (0: the converter's ERROR exit 1)  */
+    uint64_t n_out_lines;                     /* lines of the overlaps file                                     */
+    uint64_t first_error_line;                /* 0-based in its file, ~0 if none; its byte offset / length there */
+    uint64_t first_error_offset, first_error_length;
+    uint32_t first_error_file;                /* 0 single-end, 1 paired-end                                     */
+    uint32_t first_error_status;              /* HC_SAM_DIES / HC_SAM_DECLINED                                  */
+    float    h2d_ms;                          /* host clock: the texts to the device                            */
+    float    device_ms;                       /* host clock: every kernel, to the file in HBM                   */
+    float    d2h_ms;                          /* host clock: the file to `text`                                 */
+    uint32_t reserved;
+} hc_sam_stats;                               /* 104 bytes */
+
+typedef struct {                              /* what --verbose prints for one reference                        */
+    uint64_t n_alignments, n_singles, n_paired; /* "Total number of alignments", "... of which singles / paired" */
+    uint64_t problems;                        /* "# cases where overlap_pos2 < 0"                               */
+    uint64_t n_overlaps;                      /* "Total number of overlaps found"                               */
+    uint64_t types[4];                        /* ++, +-, -+, --                                                  */
+} hc_sam_ref_stats;                           /* 72 bytes */
+
+int hc_sam2overlaps(const char* sam_s, uint64_t n_s, const char* sam_p, uint64_t n_p,
+                    const char* ref_names, const uint64_t* ref_name_off, const uint32_t* ref_name_idx, uint32_t n_names,
+                    const int64_t* ref_len, uint32_t n_refs, int64_t min_overlap_len,
+                    char* text, uint64_t text_cap, uint64_t* n_text_bytes,
+                    hc_sam_ref_stats* ref_stats, hc_sam_stats* stats, int device);
+
 int         hc_device_count(void);
 const char* hc_last_error(void);
 const char* hc_version(void);
