@@ -5,14 +5,15 @@
 //
 // One primitive, used twice: "group items by bucket and order every group by a 64-bit key, ties by item index":
 //   count per bucket (atomicAdd) -> exclusive scan -> scatter with a per-bucket cursor (arbitrary order inside a group)
-//   -> one thread per bucket sorts its group in place (insertion sort up to 32 items, heap sort beyond; the order is total,
-//   so any sorting algorithm gives the same list).
+//   -> one thread per bucket sorts its group in place (hc_radix::sort_run; the order is total, so any sorting algorithm
+//   gives the same list).
 // adj_out: bucket = vertex1, key = item index (insertion order) or non-overlap length << 32 | vertex2 (sortEdges);
 // adj_in:  bucket = vertex2, key = position of the edge in the adj_out order.
 #include <cstring>
 #include <string>
 #include <cuda_runtime.h>
 #include "../../include/hc_b200.h"
+#include "hc_radix.cuh"
 #include "hc_scan.cuh"
 #include "hc_stage.h"
 
@@ -22,7 +23,9 @@ typedef unsigned long long u64;
 
 struct Item { u64 key; uint32_t idx; uint32_t pad; };     // 16 bytes
 
-__device__ __forceinline__ bool item_less(const Item& a, const Item& b) { return a.key != b.key ? a.key < b.key : a.idx < b.idx; }
+struct ItemLess {
+    __device__ bool operator()(const Item& a, const Item& b) const { return a.key != b.key ? a.key < b.key : a.idx < b.idx; }
+};
 
 __global__ void adj_count(const hc_adj_edge* __restrict__ e, const uint8_t* __restrict__ keep, u64 n, int by_v2, uint32_t* cnt) {
     for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x)
@@ -58,18 +61,6 @@ __global__ void adj_scatter_in(const hc_adj_edge* __restrict__ e, const uint32_t
     }
 }
 
-__device__ void sift_down(Item* a, uint32_t start, uint32_t end) {
-    uint32_t root = start;
-    while (2 * root + 1 <= end) {
-        uint32_t child = 2 * root + 1, sw = root;
-        if (item_less(a[sw], a[child])) sw = child;
-        if (child + 1 <= end && item_less(a[sw], a[child + 1])) sw = child + 1;
-        if (sw == root) return;
-        const Item t = a[root]; a[root] = a[sw]; a[sw] = t;
-        root = sw;
-    }
-}
-
 // one thread per bucket; out[p] = idx of the p-th item; tie[v] = 1 if two items of a group of more than 16 share a key
 // (std::sort leaves their order to its implementation: the host part settles those lists with std::sort itself)
 __global__ void adj_sort_groups(u64 V, const u64* __restrict__ off, Item* items, uint32_t* __restrict__ out, uint8_t* __restrict__ tie) {
@@ -77,20 +68,7 @@ __global__ void adj_sort_groups(u64 V, const u64* __restrict__ off, Item* items,
         const u64 a = off[v], b = off[v + 1];
         const uint32_t m = (uint32_t)(b - a);
         Item* g = items + a;
-        if (m > 1 && m <= 32) {
-            for (uint32_t i = 1; i < m; i++) {
-                const Item x = g[i];
-                uint32_t j = i;
-                while (j > 0 && item_less(x, g[j - 1])) { g[j] = g[j - 1]; j--; }
-                g[j] = x;
-            }
-        } else if (m > 32) {
-            for (int s = (int)(m - 2) / 2; s >= 0; s--) sift_down(g, (uint32_t)s, m - 1);
-            for (uint32_t end = m - 1; end > 0; end--) {
-                const Item t = g[end]; g[end] = g[0]; g[0] = t;
-                sift_down(g, 0, end - 1);
-            }
-        }
+        hc_radix::sort_run(g, m, ItemLess());
         bool t = false;
         for (uint32_t i = 0; i < m; i++) {
             out[a + i] = g[i].idx;
@@ -101,18 +79,6 @@ __global__ void adj_sort_groups(u64 V, const u64* __restrict__ off, Item* items,
 }
 
 }  // namespace
-
-void hc_set_last_error(const char* msg);   // hc_api.cu
-
-#define ACU(call)                                                                            \
-    do {                                                                                     \
-        cudaError_t _e = (call);                                                             \
-        if (_e != cudaSuccess) {                                                             \
-            hc_set_last_error((std::string(#call) + ": " + cudaGetErrorString(_e)).c_str()); \
-            rc = HC_ERR_CUDA;                                                                \
-            goto done;                                                                       \
-        }                                                                                    \
-    } while (0)
 
 extern "C" int hc_build_adjacency(const hc_adj_edge* edges, uint64_t n, const uint8_t* keep, uint64_t n_vertices, int sort,
                                   uint64_t* out_off, uint32_t* out_perm, uint64_t* in_off, uint32_t* in_src, uint8_t* ties,
@@ -126,58 +92,56 @@ extern "C" int hc_build_adjacency(const hc_adj_edge* edges, uint64_t n, const ui
     *n_kept = 0;
     const u64 V = n_vertices;
     int rc = HC_OK;
-    hc_adj_edge* d_e = nullptr;
-    uint8_t *d_keep = nullptr, *d_tie = nullptr;
-    uint32_t *d_cnt = nullptr, *d_perm = nullptr, *d_src = nullptr;
-    u64 *d_off = nullptr, *d_total = nullptr, *d_bsum = nullptr, kept = 0;
-    Item* d_items = nullptr;
-    const int threads = 256;
-    const int eb = (int)((n + threads - 1) / threads < 148 * 16 ? (n + threads - 1) / threads : 148 * 16);
-    const int vb = (int)((V + threads - 1) / threads < 148 * 16 ? (V + threads - 1) / threads : 148 * 16);
-    ACU(cudaSetDevice(device));
+    const char* who = "hc_build_adjacency";
+    ScratchBuf<hc_adj_edge> d_e;
+    ScratchBuf<uint8_t> d_keep, d_tie;
+    ScratchBuf<uint32_t> d_cnt, d_perm, d_src;
+    ScratchBuf<u64> d_off, d_total, d_bsum;
+    ScratchBuf<Item> d_items;
+    u64 kept = 0;
+    const int threads = 256, eb = grid_for(n, threads), vb = grid_for(V, threads);
+    HC_CU(cudaSetDevice(device));
     if (V == 0) goto done;
-    ACU(hc_scratch_alloc((void**)&d_cnt, (V + 1) * sizeof(uint32_t))); ACU(hc_scratch_alloc((void**)&d_off, (V + 1) * sizeof(u64)));
-    ACU(hc_scratch_alloc((void**)&d_total, sizeof(u64))); ACU(hc_scratch_alloc((void**)&d_bsum, hc_scan::blocks_for(V + 1) * sizeof(u64)));
-    ACU(cudaMemsetAsync(d_cnt, 0, (V + 1) * sizeof(uint32_t)));
+    HC_CU(d_cnt.alloc(V + 1)); HC_CU(d_off.alloc(V + 1));
+    HC_CU(d_total.alloc(1)); HC_CU(d_bsum.alloc(hc_scan::blocks_for(V + 1)));
+    HC_CU(cudaMemsetAsync(d_cnt, 0, (V + 1) * sizeof(uint32_t)));
     if (n) {
-        ACU(hc_scratch_alloc((void**)&d_e, n * sizeof(hc_adj_edge)));
-        ACU(hc_copy_h2d(d_e, edges, n * sizeof(hc_adj_edge)));
-        if (keep) { ACU(hc_scratch_alloc((void**)&d_keep, n)); ACU(hc_copy_h2d(d_keep, keep, n)); }
-        adj_count<<<eb ? eb : 1, threads>>>(d_e, d_keep, n, 0, d_cnt);
+        HC_CU(d_e.alloc(n));
+        HC_CU(hc_copy_h2d(d_e, edges, n * sizeof(hc_adj_edge)));
+        if (keep) { HC_CU(d_keep.alloc(n)); HC_CU(hc_copy_h2d(d_keep, keep, n)); }
+        adj_count<<<eb, threads>>>(d_e, d_keep, n, 0, d_cnt);
     }
     hc_scan::exclusive_u32(d_cnt, V + 1, d_off, d_total, d_bsum, 0);
-    ACU(cudaMemcpy(&kept, d_total, sizeof(u64), cudaMemcpyDeviceToHost));
+    HC_CU(cudaMemcpy(&kept, d_total, sizeof(u64), cudaMemcpyDeviceToHost));
     *n_kept = kept;
-    ACU(hc_copy_d2h(out_off, d_off, (V + 1) * sizeof(u64)));
+    HC_CU(hc_copy_d2h(out_off, d_off, (V + 1) * sizeof(u64)));
     if (kept) {
-        ACU(hc_scratch_alloc((void**)&d_items, kept * sizeof(Item))); ACU(hc_scratch_alloc((void**)&d_perm, kept * sizeof(uint32_t)));
-        if (ties) ACU(hc_scratch_alloc((void**)&d_tie, V));
-        ACU(cudaMemsetAsync(d_cnt, 0, (V + 1) * sizeof(uint32_t)));
+        HC_CU(d_items.alloc(kept)); HC_CU(d_perm.alloc(kept));
+        if (ties) HC_CU(d_tie.alloc(V));
+        HC_CU(cudaMemsetAsync(d_cnt, 0, (V + 1) * sizeof(uint32_t)));
         adj_scatter_out<<<eb, threads>>>(d_e, d_keep, n, sort, d_off, d_cnt, d_items);
-        adj_sort_groups<<<vb, threads>>>(V, d_off, d_items, d_perm, sort ? d_tie : nullptr);
-        ACU(cudaGetLastError());
-        ACU(hc_copy_d2h(out_perm, d_perm, kept * sizeof(uint32_t)));
-        if (ties) { if (sort) ACU(hc_copy_d2h(ties, d_tie, V)); else memset(ties, 0, V); }
+        adj_sort_groups<<<vb, threads>>>(V, d_off, d_items, d_perm, sort ? d_tie.get() : nullptr);
+        HC_CU(cudaGetLastError());
+        HC_CU(hc_copy_d2h(out_perm, d_perm, kept * sizeof(uint32_t)));
+        if (ties) { if (sort) HC_CU(hc_copy_d2h(ties, d_tie, V)); else memset(ties, 0, V); }
     } else if (ties) {
         memset(ties, 0, V);
     }
     if (in_off) {
-        ACU(cudaMemsetAsync(d_cnt, 0, (V + 1) * sizeof(uint32_t)));
-        if (n) adj_count<<<eb ? eb : 1, threads>>>(d_e, d_keep, n, 1, d_cnt);
+        HC_CU(cudaMemsetAsync(d_cnt, 0, (V + 1) * sizeof(uint32_t)));
+        if (n) adj_count<<<eb, threads>>>(d_e, d_keep, n, 1, d_cnt);
         hc_scan::exclusive_u32(d_cnt, V + 1, d_off, d_total, d_bsum, 0);
-        ACU(hc_copy_d2h(in_off, d_off, (V + 1) * sizeof(u64)));
+        HC_CU(hc_copy_d2h(in_off, d_off, (V + 1) * sizeof(u64)));
         if (kept) {
-            ACU(hc_scratch_alloc((void**)&d_src, kept * sizeof(uint32_t)));
-            ACU(cudaMemsetAsync(d_cnt, 0, (V + 1) * sizeof(uint32_t)));
-            adj_scatter_in<<<(int)((kept + threads - 1) / threads < 148 * 16 ? (kept + threads - 1) / threads : 148 * 16), threads>>>(d_e, d_perm, kept, d_off, d_cnt, d_items);
+            HC_CU(d_src.alloc(kept));
+            HC_CU(cudaMemsetAsync(d_cnt, 0, (V + 1) * sizeof(uint32_t)));
+            adj_scatter_in<<<grid_for(kept, threads), threads>>>(d_e, d_perm, kept, d_off, d_cnt, d_items);
             adj_sort_groups<<<vb, threads>>>(V, d_off, d_items, d_src, nullptr);
-            ACU(cudaGetLastError());
-            ACU(hc_copy_d2h(in_src, d_src, kept * sizeof(uint32_t)));
+            HC_CU(cudaGetLastError());
+            HC_CU(hc_copy_d2h(in_src, d_src, kept * sizeof(uint32_t)));
         }
     }
 done:
-    hc_scratch_free(d_e); hc_scratch_free(d_keep); hc_scratch_free(d_tie); hc_scratch_free(d_cnt); hc_scratch_free(d_perm); hc_scratch_free(d_src);
-    hc_scratch_free(d_off); hc_scratch_free(d_total); hc_scratch_free(d_bsum); hc_scratch_free(d_items);
     return rc;
 }
 
@@ -249,26 +213,26 @@ extern "C" int hc_subread_info(const hc_subread_problem* problems, uint64_t n_pr
         }
     }
     int rc = HC_OK;
-    hc_subread_problem* d_prob = nullptr;
-    uint32_t *d_ep = nullptr, *d_v = nullptr;
-    int32_t* d_pos = nullptr;
-    hc_fno_subread* d_info = nullptr;
-    uint8_t* d_first = nullptr;
+    const char* who = "hc_subread_info";
+    ScratchBuf<hc_subread_problem> d_prob;
+    ScratchBuf<uint32_t> d_ep, d_v;
+    ScratchBuf<int32_t> d_pos;
+    ScratchBuf<hc_fno_subread> d_info;
+    ScratchBuf<uint8_t> d_first;
     if (!err.empty()) { hc_set_last_error(err.c_str()); free(h_ep); return HC_ERR_ARG; }
-    ACU(cudaSetDevice(device));
-    ACU(hc_scratch_alloc((void**)&d_prob, (n_problems ? n_problems : 1) * sizeof(hc_subread_problem))); ACU(hc_scratch_alloc((void**)&d_ep, n_entries * sizeof(uint32_t)));
-    ACU(hc_scratch_alloc((void**)&d_v, n_entries * sizeof(uint32_t))); ACU(hc_scratch_alloc((void**)&d_pos, n_entries * sizeof(int32_t)));
-    ACU(hc_scratch_alloc((void**)&d_info, n_entries * sizeof(hc_fno_subread))); ACU(hc_scratch_alloc((void**)&d_first, n_entries));
-    ACU(hc_copy_h2d(d_prob, problems, n_problems * sizeof(hc_subread_problem)));
-    ACU(hc_copy_h2d(d_ep, h_ep, n_entries * sizeof(uint32_t)));
-    ACU(hc_copy_h2d(d_v, vertex, n_entries * sizeof(uint32_t)));
-    ACU(hc_copy_h2d(d_pos, pos, n_entries * sizeof(int32_t)));
-    subread_info_kernel<<<(unsigned)((n_entries + 255) / 256 < 148 * 16 ? (n_entries + 255) / 256 : 148 * 16), 256>>>(d_prob, d_ep, n_entries, d_pos, d_v, d_info, d_first);
-    ACU(cudaGetLastError());
-    ACU(hc_copy_d2h(info, d_info, n_entries * sizeof(hc_fno_subread)));
-    ACU(hc_copy_d2h(first, d_first, n_entries));
+    HC_CU(cudaSetDevice(device));
+    HC_CU(d_prob.alloc(n_problems ? n_problems : 1)); HC_CU(d_ep.alloc(n_entries));
+    HC_CU(d_v.alloc(n_entries)); HC_CU(d_pos.alloc(n_entries));
+    HC_CU(d_info.alloc(n_entries)); HC_CU(d_first.alloc(n_entries));
+    HC_CU(hc_copy_h2d(d_prob, problems, n_problems * sizeof(hc_subread_problem)));
+    HC_CU(hc_copy_h2d(d_ep, h_ep, n_entries * sizeof(uint32_t)));
+    HC_CU(hc_copy_h2d(d_v, vertex, n_entries * sizeof(uint32_t)));
+    HC_CU(hc_copy_h2d(d_pos, pos, n_entries * sizeof(int32_t)));
+    subread_info_kernel<<<grid_for(n_entries, 256), 256>>>(d_prob, d_ep, n_entries, d_pos, d_v, d_info, d_first);
+    HC_CU(cudaGetLastError());
+    HC_CU(hc_copy_d2h(info, d_info, n_entries * sizeof(hc_fno_subread)));
+    HC_CU(hc_copy_d2h(first, d_first, n_entries));
 done:
     free(h_ep);
-    hc_scratch_free(d_prob); hc_scratch_free(d_ep); hc_scratch_free(d_v); hc_scratch_free(d_pos); hc_scratch_free(d_info); hc_scratch_free(d_first);
     return rc;
 }

@@ -1,12 +1,8 @@
 // hc_dedup.cu -- duplicate-edge resolution of the graph insert on the device
 // (EdgeCalculator::process_overlaps, serial section, src/EdgeCalculator.cpp:429-545); see hc_b200.h.
-#include <algorithm>
-#include <string>
 #include <cuda_runtime.h>
 #include "../../include/hc_b200.h"
 #include "hc_stage.h"
-
-void hc_set_last_error(const char* msg);   // hc_api.cu
 
 namespace {
 
@@ -83,16 +79,6 @@ __global__ void dd_resolve(const hc_dedup_edge* e, u64 n, const u64* keys, const
 
 }  // namespace
 
-#define DCU(call)                                                                            \
-    do {                                                                                     \
-        cudaError_t _e = (call);                                                             \
-        if (_e != cudaSuccess) {                                                             \
-            hc_set_last_error((std::string(#call) + ": " + cudaGetErrorString(_e)).c_str()); \
-            rc = HC_ERR_CUDA;                                                                \
-            goto done;                                                                       \
-        }                                                                                    \
-    } while (0)
-
 extern "C" int hc_dedup_edges(const hc_dedup_edge* edges, uint64_t n, int ignore_inclusions, uint8_t* winner,
                               uint8_t* inclusions, uint64_t n_vertices, uint64_t counts[2], int device) {
     if ((n && (!edges || !winner)) || !counts) { hc_set_last_error("hc_dedup_edges: NULL argument"); return HC_ERR_ARG; }
@@ -104,28 +90,27 @@ extern "C" int hc_dedup_edges(const hc_dedup_edge* edges, uint64_t n, int ignore
             return HC_ERR_ARG;
         }
     int rc = HC_OK;
-    hc_dedup_edge* d_e = nullptr;
-    u64 *d_keys = nullptr, *d_best = nullptr, *d_first = nullptr, *d_counts = nullptr;
-    uint8_t *d_win = nullptr, *d_inc = nullptr;
+    const char* who = "hc_dedup_edges";
+    ScratchBuf<hc_dedup_edge> d_e;
+    ScratchBuf<u64> d_keys, d_best, d_first, d_counts;
+    ScratchBuf<uint8_t> d_win, d_inc;
     u64 cap = 64;
-    const int threads = 256;
-    const int blocks = (int)std::min<u64>((n + threads - 1) / threads, 148 * 16);
+    const int threads = 256, blocks = grid_for(n, threads);
     while (cap < 2 * n + 2) cap <<= 1;
-    DCU(cudaSetDevice(device));
-    DCU(hc_scratch_alloc((void**)&d_e, n * sizeof(hc_dedup_edge)));
-    DCU(hc_scratch_alloc((void**)&d_keys, cap * sizeof(u64))); DCU(hc_scratch_alloc((void**)&d_best, cap * sizeof(u64))); DCU(hc_scratch_alloc((void**)&d_first, cap * sizeof(u64)));
-    DCU(hc_scratch_alloc((void**)&d_counts, 2 * sizeof(u64))); DCU(hc_scratch_alloc((void**)&d_win, n));
-    DCU(cudaMemset(d_keys, 0xff, cap * sizeof(u64))); DCU(cudaMemset(d_best, 0xff, cap * sizeof(u64)));
-    DCU(cudaMemset(d_first, 0xff, cap * sizeof(u64))); DCU(cudaMemset(d_counts, 0, 2 * sizeof(u64)));
-    if (inclusions && n_vertices) { DCU(hc_scratch_alloc((void**)&d_inc, n_vertices)); DCU(cudaMemcpy(d_inc, inclusions, n_vertices, cudaMemcpyHostToDevice)); }
-    DCU(hc_copy_h2d(d_e, edges, n * sizeof(hc_dedup_edge)));
+    HC_CU(cudaSetDevice(device));
+    HC_CU(d_e.alloc(n));
+    HC_CU(d_keys.alloc(cap)); HC_CU(d_best.alloc(cap)); HC_CU(d_first.alloc(cap));
+    HC_CU(d_counts.alloc(2)); HC_CU(d_win.alloc(n));
+    HC_CU(cudaMemset(d_keys, 0xff, cap * sizeof(u64))); HC_CU(cudaMemset(d_best, 0xff, cap * sizeof(u64)));
+    HC_CU(cudaMemset(d_first, 0xff, cap * sizeof(u64))); HC_CU(cudaMemset(d_counts, 0, 2 * sizeof(u64)));
+    if (inclusions && n_vertices) { HC_CU(d_inc.alloc(n_vertices)); HC_CU(cudaMemcpy(d_inc, inclusions, n_vertices, cudaMemcpyHostToDevice)); }
+    HC_CU(hc_copy_h2d(d_e, edges, n * sizeof(hc_dedup_edge)));
     dd_claim<<<blocks, threads>>>(d_e, n, d_keys, d_best, d_first, cap - 1, d_counts);
     dd_resolve<<<blocks, threads>>>(d_e, n, d_keys, d_best, d_first, cap - 1, ignore_inclusions, d_win, d_inc, d_counts);
-    DCU(cudaGetLastError());
-    DCU(hc_copy_d2h(winner, d_win, n));
-    DCU(cudaMemcpy(counts, d_counts, 2 * sizeof(u64), cudaMemcpyDeviceToHost));
-    if (d_inc) DCU(cudaMemcpy(inclusions, d_inc, n_vertices, cudaMemcpyDeviceToHost));
+    HC_CU(cudaGetLastError());
+    HC_CU(hc_copy_d2h(winner, d_win, n));
+    HC_CU(cudaMemcpy(counts, d_counts, 2 * sizeof(u64), cudaMemcpyDeviceToHost));
+    if (d_inc) HC_CU(cudaMemcpy(inclusions, d_inc, n_vertices, cudaMemcpyDeviceToHost));
 done:
-    hc_scratch_free(d_e); hc_scratch_free(d_keys); hc_scratch_free(d_best); hc_scratch_free(d_first); hc_scratch_free(d_counts); hc_scratch_free(d_win); hc_scratch_free(d_inc);
     return rc;
 }

@@ -25,7 +25,6 @@
 // floor, :375,:429,:487,:549).
 #include <cstdio>
 #include <cstdlib>
-#include <time.h>
 #include <cstring>
 #include <string>
 #include <cuda_runtime.h>
@@ -259,14 +258,16 @@ cudaError_t ffw_winners(const u64* d_keys, u64 n, uint8_t* d_win) {
     if (P < 1) P = 1;
     if (P > 2048) P = 2048;                                    // beyond 1.8e9 attempts the tables simply grow
     const int threads = 256, blocks = 148 * 8;
-    unsigned long long *h_hist = (unsigned long long*)malloc(2 * P * sizeof(unsigned long long)), *d_hist = nullptr, *d_cursor = nullptr;
-    u64 *d_pkey = nullptr, *d_pseq = nullptr, mx = 0, total = 0, slots = 1024;
-    Cell* d_tab = nullptr;
+    unsigned long long* h_hist = (unsigned long long*)malloc(2 * P * sizeof(unsigned long long));
+    ScratchBuf<unsigned long long> d_hist, d_cursor;
+    ScratchBuf<u64> d_pkey, d_pseq;
+    ScratchBuf<Cell> d_tab;
+    u64 mx = 0, total = 0, slots = 1024;
     uint32_t mask;
     if (!h_hist) return cudaErrorMemoryAllocation;
     unsigned long long* h_start = h_hist + P;
-    if ((e = hc_scratch_alloc((void**)&d_hist, P * sizeof(unsigned long long))) != cudaSuccess) goto done;
-    if ((e = hc_scratch_alloc((void**)&d_cursor, P * sizeof(unsigned long long))) != cudaSuccess) goto done;
+    if ((e = d_hist.alloc(P)) != cudaSuccess) goto done;
+    if ((e = d_cursor.alloc(P)) != cudaSuccess) goto done;
     if ((e = cudaMemsetAsync(d_hist, 0, P * sizeof(unsigned long long))) != cudaSuccess) goto done;
     ffw_histogram<<<blocks, threads, P * sizeof(uint32_t)>>>(d_keys, n, (uint32_t)P, d_hist);
     if ((e = cudaMemcpy(h_hist, d_hist, P * sizeof(unsigned long long), cudaMemcpyDeviceToHost)) != cudaSuccess) goto done;
@@ -274,15 +275,15 @@ cudaError_t ffw_winners(const u64* d_keys, u64 n, uint8_t* d_win) {
     if (total == 0) goto done;                                 // no keyed attempt at all
     while (slots < 2 * mx + 2) slots <<= 1;                    // load <= 0.5: a partition can never fill its table
     mask = (uint32_t)(slots - 1);
-    if ((e = hc_scratch_alloc((void**)&d_pkey, total * sizeof(u64))) != cudaSuccess) goto done;
-    if ((e = hc_scratch_alloc((void**)&d_pseq, total * sizeof(u64))) != cudaSuccess) goto done;
-    if ((e = hc_scratch_alloc((void**)&d_tab, slots * sizeof(Cell))) != cudaSuccess) goto done;
+    if ((e = d_pkey.alloc(total)) != cudaSuccess) goto done;
+    if ((e = d_pseq.alloc(total)) != cudaSuccess) goto done;
+    if ((e = d_tab.alloc(slots)) != cudaSuccess) goto done;
     if ((e = cudaMemcpyAsync(d_cursor, h_start, P * sizeof(unsigned long long), cudaMemcpyHostToDevice)) != cudaSuccess) goto done;
     ffw_split<<<blocks, threads, P * (sizeof(unsigned long long) + sizeof(uint32_t))>>>(d_keys, n, (uint32_t)P, d_cursor, d_pkey, d_pseq);
     for (u64 p = 0; p < P; p++) {
         const u64 c = h_hist[p];
         if (c == 0) continue;
-        const int pb = (int)((c + threads - 1) / threads < (u64)(148 * 16) ? (c + threads - 1) / threads : 148 * 16);
+        const int pb = grid_for(c, threads);
         if ((e = cudaMemsetAsync(d_tab, 0xff, slots * sizeof(Cell))) != cudaSuccess) goto done;
         ffw_claim<<<pb, threads>>>(d_pkey + h_start[p], d_pseq + h_start[p], c, d_tab, mask);
         ffw_check<<<pb, threads>>>(d_pkey + h_start[p], d_pseq + h_start[p], c, d_tab, mask, d_win);
@@ -291,7 +292,6 @@ cudaError_t ffw_winners(const u64* d_keys, u64 n, uint8_t* d_win) {
 done:
     if (e == cudaSuccess) e = cudaStreamSynchronize(0);        // h_start / h_hist are read by the copies above
     free(h_hist);
-    hc_scratch_free(d_hist); hc_scratch_free(d_cursor); hc_scratch_free(d_pkey); hc_scratch_free(d_pseq); hc_scratch_free(d_tab);
     return e;
 }
 
@@ -669,21 +669,23 @@ template <class Resolve>
 static int fno_finish(Resolve resolve, u64 attempts, hc_fno_overlap* out48, hc_fno_overlap_small* out24, const FnoText* txt,
                       u64 out_cap, uint64_t* n_out, FnoPhase& ph, const char* who) {
     int rc = HC_OK;
-    uint32_t *d_flags = nullptr, *d_ovf = nullptr, ovf = 0;
-    u64 *d_outpos = nullptr, *d_total = nullptr, *d_bsum = nullptr, produced = 0;
-    void *d_rec = nullptr, *d_out = nullptr;
+    ScratchBuf<uint32_t> d_flags, d_ovf;
+    ScratchBuf<u64> d_outpos, d_total, d_bsum;
+    ScratchBuf<char> d_rec, d_out;                 // Rec24 or hc_fno_overlap records
+    uint32_t ovf = 0;
+    u64 produced = 0;
     bool small = !fno_force_big(), out_small;
-    FCU(hc_scratch_alloc((void**)&d_flags, attempts * sizeof(uint32_t))); FCU(hc_scratch_alloc((void**)&d_outpos, attempts * sizeof(u64)));
-    FCU(hc_scratch_alloc((void**)&d_ovf, sizeof(uint32_t))); FCU(hc_scratch_alloc((void**)&d_total, sizeof(u64)));
-    FCU(hc_scratch_alloc((void**)&d_bsum, hc_scan::blocks_for(attempts) * sizeof(u64)));
+    HC_CU(d_flags.alloc(attempts)); HC_CU(d_outpos.alloc(attempts));
+    HC_CU(d_ovf.alloc(1)); HC_CU(d_total.alloc(1));
+    HC_CU(d_bsum.alloc(hc_scan::blocks_for(attempts)));
     for (int attempt = 0; attempt < 2; attempt++) {
-        FCU(cudaMemsetAsync(d_ovf, 0, sizeof(uint32_t)));
-        FCU(hc_scratch_alloc(&d_rec, attempts * (small ? sizeof(Rec24) : sizeof(hc_fno_overlap))));
+        HC_CU(cudaMemsetAsync(d_ovf, 0, sizeof(uint32_t)));
+        HC_CU(d_rec.alloc(attempts * (small ? sizeof(Rec24) : sizeof(hc_fno_overlap))));
         resolve(small, d_flags, d_rec, d_ovf);
-        FCU(cudaGetLastError());
+        HC_CU(cudaGetLastError());
         ph.mark(small ? "resolve (24-byte staging)" : "resolve (48-byte staging)");
         if (!small) break;
-        FCU(cudaMemcpy(&ovf, d_ovf, sizeof(uint32_t), cudaMemcpyDeviceToHost));
+        HC_CU(cudaMemcpy(&ovf, d_ovf, sizeof(uint32_t), cudaMemcpyDeviceToHost));
         if (!ovf) break;
         if (out24) {
             hc_set_last_error((std::string(who) + ": a value does not fit the 24-byte record (ids below 2^32, positions and lengths "
@@ -691,11 +693,11 @@ static int fno_finish(Resolve resolve, u64 attempts, hc_fno_overlap* out48, hc_f
             rc = HC_ERR_ARG;
             goto done;
         }
-        hc_scratch_free(d_rec); d_rec = nullptr;
+        d_rec.reset();
         small = false;
     }
     hc_scan::exclusive_u32(d_flags, attempts, d_outpos, d_total, d_bsum, 0);
-    FCU(cudaMemcpy(&produced, d_total, sizeof(u64), cudaMemcpyDeviceToHost));
+    HC_CU(cudaMemcpy(&produced, d_total, sizeof(u64), cudaMemcpyDeviceToHost));
     *n_out = produced;
     if (!txt && produced > out_cap) {
         hc_set_last_error((std::string(who) + ": output buffer too small (required size returned in n_out)").c_str());
@@ -707,26 +709,23 @@ static int fno_finish(Resolve resolve, u64 attempts, hc_fno_overlap* out48, hc_f
         goto done;
     }
     out_small = out24 || (txt && small);
-    FCU(hc_scratch_alloc(&d_out, produced * (out_small ? sizeof(Rec24) : sizeof(hc_fno_overlap))));
+    HC_CU(d_out.alloc(produced * (out_small ? sizeof(Rec24) : sizeof(hc_fno_overlap))));
     ph.mark("scan of flags");
     if (out_small) fno_compact<true, true><<<148 * 16, 256>>>(d_flags, d_outpos, d_rec, attempts, d_out, produced);
     else if (small) fno_compact<true, false><<<148 * 16, 256>>>(d_flags, d_outpos, d_rec, attempts, d_out, produced);
     else fno_compact<false, false><<<148 * 16, 256>>>(d_flags, d_outpos, d_rec, attempts, d_out, produced);
-    FCU(cudaGetLastError());
+    HC_CU(cudaGetLastError());
     ph.mark("fno_compact");
     if (txt) {
-        hc_scratch_free(d_flags); hc_scratch_free(d_outpos); hc_scratch_free(d_rec);   // the text stage needs the room
-        d_flags = nullptr; d_outpos = nullptr; d_rec = nullptr;
-        if (out_small) rc = fno_text(static_cast<const hc_fno_overlap_small*>(d_out), produced, *txt, ph, who);
-        else rc = fno_text(static_cast<const hc_fno_overlap*>(d_out), produced, *txt, ph, who);
+        d_flags.reset(); d_outpos.reset(); d_rec.reset();   // the text stage needs the room
+        if (out_small) rc = fno_text(reinterpret_cast<const hc_fno_overlap_small*>(d_out.get()), produced, *txt, ph, who);
+        else rc = fno_text(reinterpret_cast<const hc_fno_overlap*>(d_out.get()), produced, *txt, ph, who);
         goto done;
     }
-    if (out24) FCU(hc_copy_d2h(out24, d_out, produced * sizeof(Rec24)));
-    else FCU(hc_copy_d2h(out48, d_out, produced * sizeof(hc_fno_overlap)));
+    if (out24) HC_CU(hc_copy_d2h(out24, d_out, produced * sizeof(Rec24)));
+    else HC_CU(hc_copy_d2h(out48, d_out, produced * sizeof(hc_fno_overlap)));
     ph.mark("copy out");
 done:
-    hc_scratch_free(d_flags); hc_scratch_free(d_outpos); hc_scratch_free(d_ovf); hc_scratch_free(d_total); hc_scratch_free(d_bsum);
-    hc_scratch_free(d_rec); hc_scratch_free(d_out);
     return rc;
 }
 
@@ -775,67 +774,64 @@ static int fno1_impl(const hc_fno_input* in, const hc_fno_edge* edges, uint64_t 
     const u64 nsr = V ? in->sr_off[V] : 0;
     FnoPhase ph(who);
     ph.mark("argument checks");
-    uint8_t *d_vis = nullptr, *d_lab = nullptr, *d_win = nullptr;
-    hc_fno_read *d_vr = nullptr, *d_sr = nullptr;
-    u64 *d_sroff = nullptr, *d_off = nullptr, *d_total = nullptr, *d_keys = nullptr, *d_bsum = nullptr;
-    uint32_t *d_sridx = nullptr, *d_cnt = nullptr;
-    hc_fno_subread* d_sub = nullptr;
-    hc_fno_edge* d_edges_own = nullptr;
+    ScratchBuf<uint8_t> d_vis, d_lab, d_win;
+    ScratchBuf<hc_fno_read> d_vr, d_sr;
+    ScratchBuf<u64> d_sroff, d_off, d_total, d_keys, d_bsum;
+    ScratchBuf<uint32_t> d_sridx, d_cnt;
+    ScratchBuf<hc_fno_subread> d_sub;
+    ScratchBuf<hc_fno_edge> d_edges_own;
     const hc_fno_edge* d_edges = d_edges_in;
-    VDesc* d_vd = nullptr;
-    EDesc* d_en = nullptr;
+    ScratchBuf<VDesc> d_vd;
+    ScratchBuf<EDesc> d_en;
     u64 attempts = 0;
     DevIn D;
     const int threads = 256;
     int blocks, vblocks;
-    FCU(cudaSetDevice(device));
+    HC_CU(cudaSetDevice(device));
     if (n_edges == 0) goto done;
     blocks = (int)((n_edges + threads - 1) / threads < 8192 ? (n_edges + threads - 1) / threads : 8192);
     vblocks = (int)((V + threads - 1) / threads < 4096 ? (V + threads - 1) / threads : 4096);
-    FCU(hc_scratch_alloc((void**)&d_vis, V ? V : 1)); FCU(hc_scratch_alloc((void**)&d_lab, V ? V : 1));
-    FCU(hc_scratch_alloc((void**)&d_vr, (V ? V : 1) * sizeof(hc_fno_read))); FCU(hc_scratch_alloc((void**)&d_sr, (NS ? NS : 1) * sizeof(hc_fno_read)));
-    FCU(hc_scratch_alloc((void**)&d_sroff, (V + 1) * sizeof(u64))); FCU(hc_scratch_alloc((void**)&d_sridx, (nsr ? nsr : 1) * sizeof(uint32_t)));
-    FCU(hc_scratch_alloc((void**)&d_sub, (nsr ? nsr : 1) * sizeof(hc_fno_subread)));
-    FCU(hc_scratch_alloc((void**)&d_vd, (V ? V : 1) * sizeof(VDesc))); FCU(hc_scratch_alloc((void**)&d_en, (nsr ? nsr : 1) * sizeof(EDesc)));
-    if (!d_edges_in) FCU(hc_scratch_alloc((void**)&d_edges_own, n_edges * sizeof(hc_fno_edge)));
-    FCU(hc_scratch_alloc((void**)&d_cnt, n_edges * sizeof(uint32_t)));
-    FCU(hc_scratch_alloc((void**)&d_off, n_edges * sizeof(u64))); FCU(hc_scratch_alloc((void**)&d_total, sizeof(u64)));
-    FCU(hc_copy_h2d(d_vis, in->visited, V)); FCU(hc_copy_h2d(d_lab, in->label, V));
-    FCU(hc_copy_h2d(d_vr, in->vertex_read, V * sizeof(hc_fno_read)));
-    FCU(hc_copy_h2d(d_sr, in->superread, NS * sizeof(hc_fno_read)));
-    FCU(hc_copy_h2d(d_sroff, in->sr_off, (V + 1) * sizeof(u64)));
-    FCU(hc_copy_h2d(d_sridx, in->sr_idx, nsr * sizeof(uint32_t)));
-    FCU(hc_copy_h2d(d_sub, in->sr_sub, nsr * sizeof(hc_fno_subread)));
+    HC_CU(d_vis.alloc(V ? V : 1)); HC_CU(d_lab.alloc(V ? V : 1));
+    HC_CU(d_vr.alloc(V ? V : 1)); HC_CU(d_sr.alloc(NS ? NS : 1));
+    HC_CU(d_sroff.alloc(V + 1)); HC_CU(d_sridx.alloc(nsr ? nsr : 1));
+    HC_CU(d_sub.alloc(nsr ? nsr : 1));
+    HC_CU(d_vd.alloc(V ? V : 1)); HC_CU(d_en.alloc(nsr ? nsr : 1));
+    if (!d_edges_in) HC_CU(d_edges_own.alloc(n_edges));
+    HC_CU(d_cnt.alloc(n_edges));
+    HC_CU(d_off.alloc(n_edges)); HC_CU(d_total.alloc(1));
+    HC_CU(hc_copy_h2d(d_vis, in->visited, V)); HC_CU(hc_copy_h2d(d_lab, in->label, V));
+    HC_CU(hc_copy_h2d(d_vr, in->vertex_read, V * sizeof(hc_fno_read)));
+    HC_CU(hc_copy_h2d(d_sr, in->superread, NS * sizeof(hc_fno_read)));
+    HC_CU(hc_copy_h2d(d_sroff, in->sr_off, (V + 1) * sizeof(u64)));
+    HC_CU(hc_copy_h2d(d_sridx, in->sr_idx, nsr * sizeof(uint32_t)));
+    HC_CU(hc_copy_h2d(d_sub, in->sr_sub, nsr * sizeof(hc_fno_subread)));
     // the packed per-vertex / per-entry records are built while the edges (the bulk of the input) are still being copied
     fno_prep_vertices<<<vblocks, threads>>>(V, d_vis, d_lab, d_vr, d_sroff, d_vd);
     fno_prep_entries<<<vblocks, threads>>>(V, d_vr, d_sroff, d_sridx, d_sub, d_sr, d_en);
     if (!d_edges_in) {
-        FCU(hc_copy_h2d(d_edges_own, edges, n_edges * sizeof(hc_fno_edge)));
+        HC_CU(hc_copy_h2d(d_edges_own, edges, n_edges * sizeof(hc_fno_edge)));
         d_edges = d_edges_own;
     }
     ph.mark("allocations + copies in");
     D.vd = d_vd; D.en = d_en; D.resolve_orientations = in->resolve_orientations; D.no_inclusions = in->no_inclusions;
     fno_count<<<blocks, threads>>>(D, d_edges, n_edges, d_cnt);
-    FCU(hc_scratch_alloc((void**)&d_bsum, hc_scan::blocks_for(n_edges) * sizeof(u64)));
+    HC_CU(d_bsum.alloc(hc_scan::blocks_for(n_edges)));
     hc_scan::exclusive_u32(d_cnt, n_edges, d_off, d_total, d_bsum, 0);
-    FCU(cudaMemcpy(&attempts, d_total, sizeof(u64), cudaMemcpyDeviceToHost));
+    HC_CU(cudaMemcpy(&attempts, d_total, sizeof(u64), cudaMemcpyDeviceToHost));
     ph.mark("count + scan");
     if (attempts == 0) goto done;
-    FCU(hc_scratch_alloc((void**)&d_keys, attempts * sizeof(u64))); FCU(hc_scratch_alloc((void**)&d_win, attempts));
-    FCU(cudaMemsetAsync(d_win, 0, attempts));
+    HC_CU(d_keys.alloc(attempts)); HC_CU(d_win.alloc(attempts));
+    HC_CU(cudaMemsetAsync(d_win, 0, attempts));
     fno_keys<<<blocks, threads>>>(D, d_edges, n_edges, d_off, d_keys);
     ph.mark("fno_keys");
-    FCU(ffw_winners(d_keys, attempts, d_win));
+    HC_CU(ffw_winners(d_keys, attempts, d_win));
     ph.mark("first-found-wins passes");
-    hc_scratch_free(d_keys); d_keys = nullptr;
+    d_keys.reset();
     rc = fno_finish([&](bool small, uint32_t* d_flags, void* d_rec, uint32_t* d_ovf) {
         if (small) fno_resolve<true><<<blocks, threads>>>(D, d_edges, n_edges, d_off, d_win, d_flags, d_rec, d_ovf);
         else fno_resolve<false><<<blocks, threads>>>(D, d_edges, n_edges, d_off, d_win, d_flags, d_rec, d_ovf);
     }, attempts, out48, out24, txt, out_cap, n_out, ph, who);
 done:
-    hc_scratch_free(d_vis); hc_scratch_free(d_lab); hc_scratch_free(d_vr); hc_scratch_free(d_sr); hc_scratch_free(d_sroff); hc_scratch_free(d_sridx); hc_scratch_free(d_sub);
-    hc_scratch_free(d_edges_own); hc_scratch_free(d_cnt); hc_scratch_free(d_off); hc_scratch_free(d_total); hc_scratch_free(d_keys);
-    hc_scratch_free(d_bsum); hc_scratch_free(d_win); hc_scratch_free(d_vd); hc_scratch_free(d_en);
     return rc;
 }
 
@@ -869,43 +865,41 @@ static int fno3_impl(uint64_t n_originals, const uint64_t* off, const uint32_t* 
     if (bad) { hc_set_last_error((std::string(who) + ": a new read id does not fit 32 bits (ids of new reads must be below 2^32)").c_str()); return HC_ERR_ARG; }
     int rc = HC_OK;
     FnoPhase ph(who);
-    u64 *d_off = nullptr, *d_seq = nullptr, *d_total = nullptr, *d_keys = nullptr, *d_bsum = nullptr;
-    uint32_t *d_idx = nullptr, *d_cnt = nullptr;
-    uint8_t* d_win = nullptr;
-    hc_fno3_pos* d_pos = nullptr;
-    hc_fno_read* d_reads = nullptr;
+    ScratchBuf<u64> d_off, d_seq, d_total, d_keys, d_bsum;
+    ScratchBuf<uint32_t> d_idx, d_cnt;
+    ScratchBuf<uint8_t> d_win;
+    ScratchBuf<hc_fno3_pos> d_pos;
+    ScratchBuf<hc_fno_read> d_reads;
     u64 attempts = 0;
     const int threads = 128;
     const int blocks = (int)((n_originals + threads - 1) / threads < 8192 ? (n_originals + threads - 1) / threads : 8192);
-    FCU(cudaSetDevice(device));
-    FCU(hc_scratch_alloc((void**)&d_off, (n_originals + 1) * sizeof(u64))); FCU(hc_scratch_alloc((void**)&d_idx, (nent ? nent : 1) * sizeof(uint32_t)));
-    FCU(hc_scratch_alloc((void**)&d_pos, (nent ? nent : 1) * sizeof(hc_fno3_pos))); FCU(hc_scratch_alloc((void**)&d_reads, (n_reads ? n_reads : 1) * sizeof(hc_fno_read)));
-    FCU(hc_scratch_alloc((void**)&d_cnt, n_originals * sizeof(uint32_t))); FCU(hc_scratch_alloc((void**)&d_seq, n_originals * sizeof(u64)));
-    FCU(hc_scratch_alloc((void**)&d_total, sizeof(u64)));
-    FCU(hc_copy_h2d(d_off, off, (n_originals + 1) * sizeof(u64)));
-    FCU(hc_copy_h2d(d_idx, sr_idx, nent * sizeof(uint32_t)));
-    FCU(hc_copy_h2d(d_pos, sr_pos, nent * sizeof(hc_fno3_pos)));
-    FCU(hc_copy_h2d(d_reads, reads, n_reads * sizeof(hc_fno_read)));
+    HC_CU(cudaSetDevice(device));
+    HC_CU(d_off.alloc(n_originals + 1)); HC_CU(d_idx.alloc(nent ? nent : 1));
+    HC_CU(d_pos.alloc(nent ? nent : 1)); HC_CU(d_reads.alloc(n_reads ? n_reads : 1));
+    HC_CU(d_cnt.alloc(n_originals)); HC_CU(d_seq.alloc(n_originals));
+    HC_CU(d_total.alloc(1));
+    HC_CU(hc_copy_h2d(d_off, off, (n_originals + 1) * sizeof(u64)));
+    HC_CU(hc_copy_h2d(d_idx, sr_idx, nent * sizeof(uint32_t)));
+    HC_CU(hc_copy_h2d(d_pos, sr_pos, nent * sizeof(hc_fno3_pos)));
+    HC_CU(hc_copy_h2d(d_reads, reads, n_reads * sizeof(hc_fno_read)));
     ph.mark("allocations + copies in");
     fno3_count<<<blocks, threads>>>(d_off, n_originals, d_cnt);
-    FCU(hc_scratch_alloc((void**)&d_bsum, hc_scan::blocks_for(n_originals) * sizeof(u64)));
+    HC_CU(d_bsum.alloc(hc_scan::blocks_for(n_originals)));
     hc_scan::exclusive_u32(d_cnt, n_originals, d_seq, d_total, d_bsum, 0);
-    FCU(cudaMemcpy(&attempts, d_total, sizeof(u64), cudaMemcpyDeviceToHost));
+    HC_CU(cudaMemcpy(&attempts, d_total, sizeof(u64), cudaMemcpyDeviceToHost));
     if (attempts == 0) goto done;
-    FCU(hc_scratch_alloc((void**)&d_keys, attempts * sizeof(u64))); FCU(hc_scratch_alloc((void**)&d_win, attempts));
-    FCU(cudaMemsetAsync(d_win, 0, attempts));
+    HC_CU(d_keys.alloc(attempts)); HC_CU(d_win.alloc(attempts));
+    HC_CU(cudaMemsetAsync(d_win, 0, attempts));
     fno3_keys<<<blocks, threads>>>(d_off, n_originals, d_idx, d_reads, d_seq, d_keys);
     ph.mark("count + scan + keys");
-    FCU(ffw_winners(d_keys, attempts, d_win));
+    HC_CU(ffw_winners(d_keys, attempts, d_win));
     ph.mark("first-found-wins passes");
-    hc_scratch_free(d_keys); d_keys = nullptr;
+    d_keys.reset();
     rc = fno_finish([&](bool small, uint32_t* d_flags, void* d_rec, uint32_t* d_ovf) {
         if (small) fno3_resolve<true><<<blocks, threads>>>(d_off, n_originals, d_idx, d_pos, d_reads, (uint32_t)no_inclusions, d_seq, d_win, d_flags, d_rec, d_ovf);
         else fno3_resolve<false><<<blocks, threads>>>(d_off, n_originals, d_idx, d_pos, d_reads, (uint32_t)no_inclusions, d_seq, d_win, d_flags, d_rec, d_ovf);
     }, attempts, out48, out24, txt, out_cap, n_out, ph, who);
 done:
-    hc_scratch_free(d_off); hc_scratch_free(d_idx); hc_scratch_free(d_pos); hc_scratch_free(d_reads); hc_scratch_free(d_cnt); hc_scratch_free(d_seq); hc_scratch_free(d_total);
-    hc_scratch_free(d_keys); hc_scratch_free(d_bsum); hc_scratch_free(d_win);
     return rc;
 }
 
@@ -945,7 +939,7 @@ extern "C" int hc_fno1_text(const hc_fno_input* in, const hc_fno_edge* edges, ui
 // behind what the earlier pieces kept.  No line is kept past an error line: on HC_ERR_INPUT the stream is discarded.
 static int fno1_nonedge_stream(const hc_idmap* m, const hc_fno_edge* head, uint64_t n_head, uint64_t n_adjacency,
                                const char* text, uint64_t n_bytes, const hc_fno_edge* tail, uint64_t n_tail,
-                               hc_fno_edge** d_stream_out, hc_fno_nonedge_stats* stats, const char* who) {
+                               ScratchBuf<hc_fno_edge>& d_stream, hc_fno_nonedge_stats* stats, const char* who) {
     int rc = HC_OK;
     const std::vector<uint64_t> cut = hc_ingest_cuts(text, n_bytes, hc_ingest_piece_bytes());
     const size_t n_pieces = cut.size() - 1;
@@ -957,45 +951,43 @@ static int fno1_nonedge_stream(const hc_idmap* m, const hc_fno_edge* head, uint6
     const u64 tbytes = (max_piece + 16 + 255) & ~255ull, cap = hc_ingest_all_cap(max_piece);
     u64 slots = 1024, kept = 0, lines = 0, total = 0;
     while (slots < 2 * n_adjacency + 2) slots <<= 1;
-    hc_fno_edge* d_stream = nullptr;
-    char* d_text = nullptr;
-    hc_candidate* d_cand = nullptr;
-    uint32_t* d_keep = nullptr;
-    u64 *d_pos = nullptr, *d_total = nullptr, *d_bsum = nullptr;
-    Cell* d_tab = nullptr;
+    ScratchBuf<char> d_text;
+    ScratchBuf<hc_candidate> d_cand;
+    ScratchBuf<uint32_t> d_keep;
+    ScratchBuf<u64> d_pos, d_total, d_bsum;
+    ScratchBuf<Cell> d_tab;
     cudaStream_t s_copy = nullptr;
     cudaEvent_t ev_in[2] = {nullptr, nullptr}, t0 = nullptr, t1 = nullptr;
     hc_ingest_params ip;
     memset(&ip, 0, sizeof(ip));
     ip.max_overlaps = ~0ull;                                     // the loop reads the whole file; ORD / ORI / TYPE split on tabs only
-    FCU(cudaStreamCreateWithFlags(&s_copy, cudaStreamNonBlocking));
-    for (int k = 0; k < 2; k++) FCU(cudaEventCreateWithFlags(&ev_in[k], cudaEventDisableTiming));
-    FCU(cudaEventCreate(&t0)); FCU(cudaEventCreate(&t1));
-    FCU(cudaEventRecord(t0, 0));
-    FCU(hc_scratch_alloc((void**)&d_stream, (bound ? bound : 1) * sizeof(hc_fno_edge)));
-    FCU(hc_copy_h2d(d_stream, head, n_head * sizeof(hc_fno_edge)));
+    HC_CU(cudaStreamCreateWithFlags(&s_copy, cudaStreamNonBlocking));
+    for (int k = 0; k < 2; k++) HC_CU(cudaEventCreateWithFlags(&ev_in[k], cudaEventDisableTiming));
+    HC_CU(cudaEventCreate(&t0)); HC_CU(cudaEventCreate(&t1));
+    HC_CU(cudaEventRecord(t0, 0));
+    HC_CU(d_stream.alloc(bound ? bound : 1));
+    HC_CU(hc_copy_h2d(d_stream, head, n_head * sizeof(hc_fno_edge)));
     if (n_pieces) {
-        FCU(hc_scratch_alloc((void**)&d_text, 2 * tbytes));
-        FCU(hc_scratch_alloc((void**)&d_cand, cap * sizeof(hc_candidate)));
-        FCU(hc_scratch_alloc((void**)&d_keep, cap * sizeof(uint32_t))); FCU(hc_scratch_alloc((void**)&d_pos, cap * sizeof(u64)));
-        FCU(hc_scratch_alloc((void**)&d_total, sizeof(u64))); FCU(hc_scratch_alloc((void**)&d_bsum, hc_scan::blocks_for(cap) * sizeof(u64)));
-        FCU(hc_scratch_alloc((void**)&d_tab, slots * sizeof(Cell)));
-        FCU(cudaMemsetAsync(d_tab, 0xff, slots * sizeof(Cell)));
+        HC_CU(d_text.alloc(2 * tbytes));
+        HC_CU(d_cand.alloc(cap));
+        HC_CU(d_keep.alloc(cap)); HC_CU(d_pos.alloc(cap));
+        HC_CU(d_total.alloc(1)); HC_CU(d_bsum.alloc(hc_scan::blocks_for(cap)));
+        HC_CU(d_tab.alloc(slots));
+        HC_CU(cudaMemsetAsync(d_tab, 0xff, slots * sizeof(Cell)));
         if (n_adjacency) {
-            const int ab = (int)std::min<u64>((n_adjacency + 255) / 256, 148 * 16);
-            adj_claim<<<ab, 256>>>(d_stream, n_adjacency, d_tab, (uint32_t)(slots - 1));
-            FCU(cudaGetLastError());
+            adj_claim<<<grid_for(n_adjacency, 256), 256>>>(d_stream, n_adjacency, d_tab, (uint32_t)(slots - 1));
+            HC_CU(cudaGetLastError());
         }
-        FCU(hc_copy_h2d_on(d_text, text, cut[1] - cut[0], s_copy));
-        FCU(cudaEventRecord(ev_in[0], s_copy));
+        HC_CU(hc_copy_h2d_on(d_text, text, cut[1] - cut[0], s_copy));
+        HC_CU(cudaEventRecord(ev_in[0], s_copy));
     }
     for (size_t i = 0; i < n_pieces; i++) {
         const int b = (int)(i & 1);
         if (i + 1 < n_pieces) {   // buffer b ^ 1 held piece i - 1, whose work has completed (the kept count below is read back)
-            FCU(hc_copy_h2d_on(d_text + (size_t)(b ^ 1) * tbytes, text + cut[i + 1], cut[i + 2] - cut[i + 1], s_copy));
-            FCU(cudaEventRecord(ev_in[b ^ 1], s_copy));
+            HC_CU(hc_copy_h2d_on(d_text + (size_t)(b ^ 1) * tbytes, text + cut[i + 1], cut[i + 2] - cut[i + 1], s_copy));
+            HC_CU(cudaEventRecord(ev_in[b ^ 1], s_copy));
         }
-        FCU(cudaStreamWaitEvent(0, ev_in[b], 0));
+        HC_CU(cudaStreamWaitEvent(0, ev_in[b], 0));
         hc_ingest_stats st;
         rc = hc_ingest_device(m, d_text + (size_t)b * tbytes, cut[i + 1] - cut[i], &ip, d_cand, nullptr, cap, nullptr, nullptr, 0,
                               &st, 0, 0, true);
@@ -1014,31 +1006,27 @@ static int fno1_nonedge_stream(const hc_idmap* m, const hc_fno_edge* head, uint6
         }
         lines += st.n_lines;
         if (st.n_scored) {
-            const int pb = (int)std::min<u64>((st.n_scored + 255) / 256, 148 * 16);
+            const int pb = grid_for(st.n_scored, 256);
             nonedge_probe<<<pb, 256>>>(d_cand, st.n_scored, d_tab, (uint32_t)(slots - 1), d_stream, d_keep);
             hc_scan::exclusive_u32(d_keep, st.n_scored, d_pos, d_total, d_bsum, 0);
             nonedge_scatter<<<pb, 256>>>(d_cand, d_keep, d_pos, st.n_scored, d_stream + n_head + kept);
-            FCU(cudaGetLastError());
-            FCU(cudaMemcpy(&total, d_total, sizeof(u64), cudaMemcpyDeviceToHost));
+            HC_CU(cudaGetLastError());
+            HC_CU(cudaMemcpy(&total, d_total, sizeof(u64), cudaMemcpyDeviceToHost));
             kept += total;
         }
     }
-    FCU(hc_copy_h2d(d_stream + n_head + kept, tail, n_tail * sizeof(hc_fno_edge)));
-    FCU(cudaEventRecord(t1, 0));
-    FCU(cudaEventSynchronize(t1));
-    FCU(cudaEventElapsedTime(&stats->device_ms, t0, t1));
+    HC_CU(hc_copy_h2d(d_stream + n_head + kept, tail, n_tail * sizeof(hc_fno_edge)));
+    HC_CU(cudaEventRecord(t1, 0));
+    HC_CU(cudaEventSynchronize(t1));
+    HC_CU(cudaEventElapsedTime(&stats->device_ms, t0, t1));
     stats->n_lines = lines;
     stats->n_nonedges = kept;
     stats->n_stream = n_head + kept + n_tail;
-    *d_stream_out = d_stream;
-    d_stream = nullptr;
 done:
     if (s_copy) { cudaStreamSynchronize(s_copy); cudaStreamDestroy(s_copy); }
     for (int k = 0; k < 2; k++) if (ev_in[k]) cudaEventDestroy(ev_in[k]);
     if (t0) cudaEventDestroy(t0);
     if (t1) cudaEventDestroy(t1);
-    hc_scratch_free(d_stream); hc_scratch_free(d_text); hc_scratch_free(d_cand); hc_scratch_free(d_keep); hc_scratch_free(d_pos);
-    hc_scratch_free(d_total); hc_scratch_free(d_bsum); hc_scratch_free(d_tab);
     return rc;
 }
 
@@ -1064,11 +1052,11 @@ extern "C" int hc_fno1_text_nonedges(const hc_fno_input* in, const hc_idmap* m, 
     if (!fno_edges_in_range(head, n_head, V, who) || !fno_edges_in_range(tail, n_tail, V, who)) return HC_ERR_ARG;
     int rc = fno1_check_input(in, who);
     if (rc != HC_OK) return rc;
-    hc_fno_edge* d_stream = nullptr;
-    FCU(cudaSetDevice(device));
+    ScratchBuf<hc_fno_edge> d_stream;              // filled by fno1_nonedge_stream
+    HC_CU(cudaSetDevice(device));
     {
         FnoPhase ph(who);
-        rc = fno1_nonedge_stream(m, head, n_head, n_adjacency, nonedge_text, nonedge_bytes, tail, n_tail, &d_stream, stats, who);
+        rc = fno1_nonedge_stream(m, head, n_head, n_adjacency, nonedge_text, nonedge_bytes, tail, n_tail, d_stream, stats, who);
         if (rc != HC_OK) goto done;
         ph.mark("stream with non-edge lines");
     }
@@ -1079,7 +1067,6 @@ extern "C" int hc_fno1_text_nonedges(const hc_fno_input* in, const hc_idmap* m, 
         if (n_records) *n_records = records;
     }
 done:
-    hc_scratch_free(d_stream);
     return rc;
 }
 

@@ -10,8 +10,8 @@
 //   * a %d field x: negatives first ('-' < '0'), among them by K(|x|) ("-1" < "-10" < "-2"): x < 0 ? K(|x|) : 2^37 + K(x);
 //   * a one-byte field (ord, ori1, ori2, type1, type2) compares as an unsigned byte at a fixed position.
 // The records are sorted by (K(id1), K(id2)) with the LSD radix sort of hc_radix.cuh (stable, so a run of equal ids keeps
-// record order), each run of equal ids is then ordered by the remaining fields by one thread (insertion sort up to 32
-// entries, heap sort beyond, as adj_sort_groups), and a line is kept when its fields differ from its predecessor's.
+// record order), each run of equal ids is then ordered by the remaining fields by one thread (hc_radix::sort_run), and a
+// line is kept when its fields differ from its predecessor's.
 // FNO3 keeps every record in record order (discovery order, src/FindNextOverlaps3.cpp:139-166).
 //
 // Byte offsets are the exclusive scan of the kept lines' lengths; the format kernel writes a block's lines into shared
@@ -28,7 +28,6 @@ typedef unsigned long long u64;
 
 constexpr int MAX_LINE = 2 * 10 + 6 * 11 + 5 + 12 + 1;     // two ids < 2^32, six %d fields, five bytes, 12 tabs, '\n'
 constexpr int FMT_THREADS = 256;                            // lines per block of the format kernel
-constexpr int INSERTION_MAX = 32;
 
 __device__ __forceinline__ hc_fno_overlap fields_of(const hc_fno_overlap& r) { return r; }
 __device__ __forceinline__ hc_fno_overlap fields_of(const hc_fno_overlap_small& r) {
@@ -104,19 +103,10 @@ __global__ void text_keys(const R* __restrict__ rec, u64 n, uint32_t* __restrict
 }
 
 template <class R>
-__device__ __forceinline__ bool rec_less(const R* rec, uint32_t a, uint32_t b) { return cmp_rest(fields_of(rec[a]), fields_of(rec[b])) < 0; }
-
-template <class R>
-__device__ void sift_down(const R* rec, uint32_t* v, uint32_t root, uint32_t m) {
-    while (true) {
-        uint32_t c = 2 * root + 1;
-        if (c >= m) return;
-        if (c + 1 < m && rec_less(rec, v[c], v[c + 1])) c++;
-        if (!rec_less(rec, v[root], v[c])) return;
-        const uint32_t t = v[root]; v[root] = v[c]; v[c] = t;
-        root = c;
-    }
-}
+struct RestLess {                                           // record indices by the fields after id1 / id2
+    const R* rec;
+    __device__ bool operator()(uint32_t a, uint32_t b) const { return cmp_rest(fields_of(rec[a]), fields_of(rec[b])) < 0; }
+};
 
 // one thread per run of equal (id1, id2): order the run's record indices by the remaining fields
 template <class R>
@@ -126,24 +116,7 @@ __global__ void text_runs(const ulonglong2* __restrict__ key, uint32_t* __restri
         if (i > 0) { const ulonglong2 p = key[i - 1]; if (p.x == k.x && p.y == k.y) continue; }
         u64 j = i + 1;
         while (j < n) { const ulonglong2 q = key[j]; if (q.x != k.x || q.y != k.y) break; j++; }
-        const uint32_t m = (uint32_t)(j - i);
-        if (m < 2) continue;
-        uint32_t* v = idx + i;
-        if (m <= INSERTION_MAX) {
-            for (uint32_t a = 1; a < m; a++) {
-                const uint32_t x = v[a];
-                const hc_fno_overlap ox = fields_of(rec[x]);
-                uint32_t b = a;
-                while (b > 0 && cmp_rest(fields_of(rec[v[b - 1]]), ox) > 0) { v[b] = v[b - 1]; b--; }
-                v[b] = x;
-            }
-        } else {
-            for (uint32_t r = m / 2; r-- > 0;) sift_down(rec, v, r, m);
-            for (uint32_t e = m - 1; e > 0; e--) {
-                const uint32_t t = v[0]; v[0] = v[e]; v[e] = t;
-                sift_down(rec, v, 0, e);
-            }
-        }
+        hc_radix::sort_run(idx + i, (uint32_t)(j - i), RestLess<R>{rec});
     }
 }
 
@@ -218,8 +191,6 @@ __global__ void __launch_bounds__(FMT_THREADS) text_format(const R* __restrict__
     }
 }
 
-inline int grid_for(u64 n, int threads) { const u64 b = (n + threads - 1) / threads; return (int)(b < 148 * 16 ? (b ? b : 1) : 148 * 16); }
-
 }  // namespace
 
 template <class R>
@@ -233,37 +204,39 @@ int fno_text(const R* d_rec, uint64_t n, const FnoText& t, FnoPhase& ph, const c
         return HC_ERR_ARG;
     }
     const int threads = 256, blocks = grid_for(n, threads);
-    uint32_t *d_len = nullptr, *d_klen = nullptr, *d_idx = nullptr, *d_idx2 = nullptr, *d_order = nullptr;
-    ulonglong2 *d_key = nullptr, *d_key2 = nullptr, *d_sorted = nullptr;
-    u64 *d_off = nullptr, *d_total = nullptr, *d_bsum = nullptr, *d_lines = nullptr;
-    char* d_text = nullptr;
+    ScratchBuf<uint32_t> d_len, d_klen, d_idx, d_idx2;
+    ScratchBuf<ulonglong2> d_key, d_key2;
+    ScratchBuf<u64> d_off, d_total, d_bsum, d_lines;
+    ScratchBuf<char> d_text;
+    uint32_t* d_order = nullptr;
+    ulonglong2* d_sorted = nullptr;
     u64 bytes = 0, lines = n;
-    FCU(hc_scratch_alloc((void**)&d_len, n * sizeof(uint32_t)));
-    FCU(hc_scratch_alloc((void**)&d_off, n * sizeof(u64)));
-    FCU(hc_scratch_alloc((void**)&d_total, sizeof(u64)));
-    FCU(hc_scratch_alloc((void**)&d_bsum, hc_scan::blocks_for(n) * sizeof(u64)));
+    HC_CU(d_len.alloc(n));
+    HC_CU(d_off.alloc(n));
+    HC_CU(d_total.alloc(1));
+    HC_CU(d_bsum.alloc(hc_scan::blocks_for(n)));
     if (t.sort_unique) {
-        FCU(hc_scratch_alloc((void**)&d_key, n * sizeof(ulonglong2))); FCU(hc_scratch_alloc((void**)&d_key2, n * sizeof(ulonglong2)));
-        FCU(hc_scratch_alloc((void**)&d_idx, n * sizeof(uint32_t))); FCU(hc_scratch_alloc((void**)&d_idx2, n * sizeof(uint32_t)));
-        FCU(hc_scratch_alloc((void**)&d_klen, n * sizeof(uint32_t))); FCU(hc_scratch_alloc((void**)&d_lines, sizeof(u64)));
+        HC_CU(d_key.alloc(n)); HC_CU(d_key2.alloc(n));
+        HC_CU(d_idx.alloc(n)); HC_CU(d_idx2.alloc(n));
+        HC_CU(d_klen.alloc(n)); HC_CU(d_lines.alloc(1));
         text_keys<R, true><<<blocks, threads>>>(d_rec, n, d_len, d_key, d_idx);
-        FCU(cudaGetLastError());
+        HC_CU(cudaGetLastError());
         ph.mark("text: keys + lengths");
-        FCU(hc_radix::sort_pairs(d_key, d_idx, d_key2, d_idx2, n, &d_sorted, &d_order));
+        HC_CU(hc_radix::sort_pairs(d_key, d_idx, d_key2, d_idx2, n, &d_sorted, &d_order));
         ph.mark("text: radix sort of the ids");
         text_runs<R><<<blocks, threads>>>(d_sorted, d_order, n, d_rec);
-        FCU(cudaMemsetAsync(d_lines, 0, sizeof(u64)));
+        HC_CU(cudaMemsetAsync(d_lines, 0, sizeof(u64)));
         text_marks<R><<<blocks, threads>>>(d_order, n, d_rec, d_len, d_klen, d_lines);
-        FCU(cudaGetLastError());
-        FCU(cudaMemcpy(&lines, d_lines, sizeof(u64), cudaMemcpyDeviceToHost));
+        HC_CU(cudaGetLastError());
+        HC_CU(cudaMemcpy(&lines, d_lines, sizeof(u64), cudaMemcpyDeviceToHost));
         ph.mark("text: runs sorted, repeats marked");
     } else {
         text_keys<R, false><<<blocks, threads>>>(d_rec, n, d_len, nullptr, nullptr);
-        FCU(cudaGetLastError());
+        HC_CU(cudaGetLastError());
         ph.mark("text: lengths");
     }
     hc_scan::exclusive_u32(t.sort_unique ? d_klen : d_len, n, d_off, d_total, d_bsum, 0);
-    FCU(cudaMemcpy(&bytes, d_total, sizeof(u64), cudaMemcpyDeviceToHost));
+    HC_CU(cudaMemcpy(&bytes, d_total, sizeof(u64), cudaMemcpyDeviceToHost));
     ph.mark("text: scan of line lengths");
     *t.n_bytes = bytes;
     *t.n_lines = lines;
@@ -272,17 +245,14 @@ int fno_text(const R* d_rec, uint64_t n, const FnoText& t, FnoPhase& ph, const c
         rc = HC_ERR_CAPACITY;
         goto done;
     }
-    FCU(hc_scratch_alloc((void**)&d_text, bytes));
+    HC_CU(d_text.alloc(bytes));
     text_format<R><<<(unsigned)((n + FMT_THREADS - 1) / FMT_THREADS), FMT_THREADS>>>(d_rec, t.sort_unique ? d_order : nullptr,
                                                                                     t.sort_unique ? d_klen : d_len, d_off, d_total, n, d_text);
-    FCU(cudaGetLastError());
+    HC_CU(cudaGetLastError());
     ph.mark("text: format");
-    FCU(hc_copy_d2h(t.text, d_text, bytes));
+    HC_CU(hc_copy_d2h(t.text, d_text, bytes));
     ph.mark("text: copy out");
 done:
-    hc_scratch_free(d_len); hc_scratch_free(d_klen); hc_scratch_free(d_idx); hc_scratch_free(d_idx2); hc_scratch_free(d_key);
-    hc_scratch_free(d_key2); hc_scratch_free(d_off); hc_scratch_free(d_total); hc_scratch_free(d_bsum); hc_scratch_free(d_lines);
-    hc_scratch_free(d_text);
     return rc;
 }
 

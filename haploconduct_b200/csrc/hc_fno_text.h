@@ -1,37 +1,24 @@
-// hc_fno_text.h -- what hc_fno.cu and hc_fno_text.cu share: the phase timer, the CUDA error macro, and the text stage
-// that turns the compacted FNO records (still in HBM) into the bytes of overlaps.txt.
+// hc_fno_text.h -- what hc_fno.cu and hc_fno_text.cu share: the phase timer and the text stage that turns the compacted
+// FNO records (still in HBM) into the bytes of overlaps.txt.
 #ifndef HC_FNO_TEXT_H_
 #define HC_FNO_TEXT_H_
 #include <cstdio>
 #include <cstdlib>
 #include <string>
-#include <time.h>
 #include <cuda_runtime.h>
 #include "../../include/hc_b200.h"
-
-void hc_set_last_error(const char* msg);   // hc_api.cu
-
-#define FCU(call)                                                                         \
-    do {                                                                                  \
-        cudaError_t _e = (call);                                                          \
-        if (_e != cudaSuccess) {                                                          \
-            hc_set_last_error((std::string(#call) + ": " + cudaGetErrorString(_e)).c_str()); \
-            rc = HC_ERR_CUDA;                                                             \
-            goto done;                                                                    \
-        }                                                                                 \
-    } while (0)
+#include "hc_stage.h"
 
 // HC_FNO_TIMING=1: phase times on stderr (synchronises the device at every mark)
 struct FnoPhase {
     bool on;
     double t0;
     const char* who;
-    static double now() { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6; }
-    explicit FnoPhase(const char* w) : on(getenv("HC_FNO_TIMING") != nullptr), t0(0), who(w) { if (on) t0 = now(); }
+    explicit FnoPhase(const char* w) : on(getenv("HC_FNO_TIMING") != nullptr), t0(0), who(w) { if (on) t0 = hc_now_ms(); }
     void mark(const char* what) {
         if (!on) return;
         cudaDeviceSynchronize();
-        const double t = now();
+        const double t = hc_now_ms();
         fprintf(stderr, "[%s] %-28s %8.2f ms\n", who, what, t - t0);
         t0 = t;
     }

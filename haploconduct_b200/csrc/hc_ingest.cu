@@ -13,8 +13,6 @@
 #include "../../include/hc_b200.h"
 #include "hc_ingest.h"
 
-void hc_set_last_error(const char* msg);   // hc_api.cu
-
 cudaError_t hc_idmap_ws(hc_idmap* m, int k, size_t bytes, void** out) {
     if (bytes > m->ws_cap[k]) {
         cudaFree(m->ws[k]);
@@ -282,16 +280,6 @@ __global__ void __launch_bounds__(LINES_PER_BLOCK) ing_scatter(const uint8_t* st
 
 }  // namespace
 
-#define ICU(call)                                                                            \
-    do {                                                                                     \
-        cudaError_t _e = (call);                                                             \
-        if (_e != cudaSuccess) {                                                             \
-            hc_set_last_error((std::string(#call) + ": " + cudaGetErrorString(_e)).c_str()); \
-            rc = HC_ERR_CUDA;                                                                \
-            goto done;                                                                       \
-        }                                                                                    \
-    } while (0)
-
 extern "C" void hc_idmap_destroy(hc_idmap* m);
 
 extern "C" hc_idmap* hc_idmap_create(const uint64_t* ids, uint64_t n_reads, int device) {
@@ -312,36 +300,37 @@ extern "C" hc_idmap* hc_idmap_create(const uint64_t* ids, uint64_t n_reads, int 
     }
     const bool dense = n_reads > 0 && max_id < 4 * n_reads + 1024;     // rename_fas.py numbers the reads 0..n-1
     int rc = HC_OK;
+    const char* who = "hc_idmap_create";
     u64* d_ids = nullptr;
     const int blocks = (int)std::min<u64>((n_reads + 255) / 256 + 1, 148 * 16);
-    ICU(cudaSetDevice(device));
+    HC_CU(cudaSetDevice(device));
     if (n_reads) {
-        ICU(cudaMalloc(&d_ids, n_reads * sizeof(u64)));
-        ICU(cudaMemcpy(d_ids, ids, n_reads * sizeof(u64), cudaMemcpyHostToDevice));
+        HC_CU(cudaMalloc(&d_ids, n_reads * sizeof(u64)));
+        HC_CU(cudaMemcpy(d_ids, ids, n_reads * sizeof(u64), cudaMemcpyHostToDevice));
     }
     if (dense) {
         m->direct_n = max_id + 1;
-        ICU(cudaMalloc(&m->direct, m->direct_n * sizeof(uint32_t)));
-        ICU(cudaMemset(m->direct, 0xff, m->direct_n * sizeof(uint32_t)));
+        HC_CU(cudaMalloc(&m->direct, m->direct_n * sizeof(uint32_t)));
+        HC_CU(cudaMemset(m->direct, 0xff, m->direct_n * sizeof(uint32_t)));
         idmap_insert_direct<<<blocks, 256>>>(d_ids, n_reads, m->direct);
     } else {
         u64 cap = 64;
         while (cap < 2 * n_reads + 2) cap <<= 1;
         m->mask = cap - 1;
-        ICU(cudaMalloc(&m->slots, cap * sizeof(ulonglong2)));
-        ICU(cudaMemset(m->slots, 0xff, cap * sizeof(ulonglong2)));
+        HC_CU(cudaMalloc(&m->slots, cap * sizeof(ulonglong2)));
+        HC_CU(cudaMemset(m->slots, 0xff, cap * sizeof(ulonglong2)));
         if (n_reads) idmap_insert<<<blocks, 256>>>(d_ids, n_reads, m->slots, m->mask);
     }
-    ICU(cudaGetLastError());
-    ICU(cudaDeviceSynchronize());
-    ICU(cudaEventCreate(&m->e0));
-    ICU(cudaEventCreate(&m->e1));
-    ICU(cudaStreamCreateWithFlags(&m->s_main, cudaStreamNonBlocking));
-    ICU(cudaStreamCreateWithFlags(&m->s_copy, cudaStreamNonBlocking));
-    ICU(cudaStreamCreateWithFlags(&m->s_out, cudaStreamNonBlocking));
+    HC_CU(cudaGetLastError());
+    HC_CU(cudaDeviceSynchronize());
+    HC_CU(cudaEventCreate(&m->e0));
+    HC_CU(cudaEventCreate(&m->e1));
+    HC_CU(cudaStreamCreateWithFlags(&m->s_main, cudaStreamNonBlocking));
+    HC_CU(cudaStreamCreateWithFlags(&m->s_copy, cudaStreamNonBlocking));
+    HC_CU(cudaStreamCreateWithFlags(&m->s_out, cudaStreamNonBlocking));
     for (int k = 0; k < 2; k++) {
-        ICU(cudaEventCreateWithFlags(&m->ev_in[k], cudaEventDisableTiming));
-        ICU(cudaEventCreateWithFlags(&m->ev_out[k], cudaEventDisableTiming));
+        HC_CU(cudaEventCreateWithFlags(&m->ev_in[k], cudaEventDisableTiming));
+        HC_CU(cudaEventCreateWithFlags(&m->ev_out[k], cudaEventDisableTiming));
     }
 done:
     cudaFree(d_ids);
@@ -370,6 +359,7 @@ int hc_ingest_device(const hc_idmap* cm, const char* d_text, uint64_t n_bytes, c
                      hc_ingest_stats* st, cudaStream_t stream, uint64_t line_base, bool all_lines) {
     hc_idmap* m = const_cast<hc_idmap*>(cm);     // the workspace is the only thing a call changes
     int rc = HC_OK;
+    const char* who = "hc_ingest_device";
     const u64 n_tiles = (n_bytes + TILE - 1) / TILE;
     uint32_t *d_tcnt = nullptr, *d_cs = nullptr, *d_cf = nullptr;
     u64 *d_toff = nullptr, *d_tot = nullptr, *d_ls = nullptr, *d_os = nullptr, *d_of = nullptr, *d_misc = nullptr;
@@ -382,32 +372,32 @@ int hc_ingest_device(const hc_idmap* cm, const char* d_text, uint64_t n_bytes, c
     memset(st, 0, sizeof(*st));
     st->first_error_line = EMPTY;
     if (n_bytes == 0) return HC_OK;
-    ICU(hc_idmap_ws(m, 0, n_tiles * sizeof(uint32_t), (void**)&d_tcnt));
-    ICU(hc_idmap_ws(m, 1, n_tiles * sizeof(u64), (void**)&d_toff));
-    ICU(hc_idmap_ws(m, 2, (8 + hc_scan::blocks_for(n_tiles)) * sizeof(u64), (void**)&d_tot));
+    HC_CU(hc_idmap_ws(m, 0, n_tiles * sizeof(uint32_t), (void**)&d_tcnt));
+    HC_CU(hc_idmap_ws(m, 1, n_tiles * sizeof(u64), (void**)&d_toff));
+    HC_CU(hc_idmap_ws(m, 2, (8 + hc_scan::blocks_for(n_tiles)) * sizeof(u64), (void**)&d_tot));
     d_misc = d_tot + 2;
-    ICU(cudaEventRecord(m->e0, stream));
+    HC_CU(cudaEventRecord(m->e0, stream));
     nl_count<<<(unsigned)n_tiles, 256, 0, stream>>>(d_text, n_bytes, d_tcnt);
     hc_scan::exclusive_u32(d_tcnt, n_tiles, d_toff, d_tot, d_tot + 8, stream);
-    ICU(cudaMemcpyAsync(&n_nl, d_tot, sizeof(u64), cudaMemcpyDeviceToHost, stream));
-    ICU(cudaMemcpyAsync(&last, d_text + n_bytes - 1, 1, cudaMemcpyDeviceToHost, stream));
-    ICU(cudaStreamSynchronize(stream));
+    HC_CU(cudaMemcpyAsync(&n_nl, d_tot, sizeof(u64), cudaMemcpyDeviceToHost, stream));
+    HC_CU(cudaMemcpyAsync(&last, d_text + n_bytes - 1, 1, cudaMemcpyDeviceToHost, stream));
+    HC_CU(cudaStreamSynchronize(stream));
     n_lines = n_nl + (last != '\n' ? 1 : 0);          // getline also returns an unterminated last line
-    ICU(hc_idmap_ws(m, 3, (n_nl + 2) * sizeof(u64), (void**)&d_ls));
-    ICU(cudaMemsetAsync(d_ls, 0, sizeof(u64), stream));
+    HC_CU(hc_idmap_ws(m, 3, (n_nl + 2) * sizeof(u64), (void**)&d_ls));
+    HC_CU(cudaMemsetAsync(d_ls, 0, sizeof(u64), stream));
     nl_mark<<<(unsigned)n_tiles, 256, 0, stream>>>(d_text, n_bytes, d_toff, d_ls);
     if (n_lines > p->max_overlaps) n_lines = p->max_overlaps;   // while (getline(...) && i < max_overlaps), :581
     st->n_lines = n_lines;
-    if (n_lines == 0) { ICU(cudaStreamSynchronize(stream)); goto done; }
+    if (n_lines == 0) { HC_CU(cudaStreamSynchronize(stream)); goto done; }
     n_blocks = (n_lines + LINES_PER_BLOCK - 1) / LINES_PER_BLOCK;
-    ICU(hc_idmap_ws(m, 4, n_lines * sizeof(hc_candidate), (void**)&d_tmp_c));
-    if (!all_lines) ICU(hc_idmap_ws(m, 5, n_lines * sizeof(hc_overlap_rec), (void**)&d_tmp_f));   // all_lines files no line as a non-edge
-    ICU(hc_idmap_ws(m, 6, n_lines, (void**)&d_status));
-    ICU(hc_idmap_ws(m, 7, n_blocks * sizeof(uint32_t), (void**)&d_cs));
-    ICU(hc_idmap_ws(m, 8, n_blocks * sizeof(uint32_t), (void**)&d_cf));
-    ICU(hc_idmap_ws(m, 9, n_blocks * sizeof(u64), (void**)&d_os));
-    ICU(hc_idmap_ws(m, 10, n_blocks * sizeof(u64), (void**)&d_of));
-    ICU(cudaMemcpyAsync(d_misc, misc, sizeof(misc), cudaMemcpyHostToDevice, stream));
+    HC_CU(hc_idmap_ws(m, 4, n_lines * sizeof(hc_candidate), (void**)&d_tmp_c));
+    if (!all_lines) HC_CU(hc_idmap_ws(m, 5, n_lines * sizeof(hc_overlap_rec), (void**)&d_tmp_f));   // all_lines files no line as a non-edge
+    HC_CU(hc_idmap_ws(m, 6, n_lines, (void**)&d_status));
+    HC_CU(hc_idmap_ws(m, 7, n_blocks * sizeof(uint32_t), (void**)&d_cs));
+    HC_CU(hc_idmap_ws(m, 8, n_blocks * sizeof(uint32_t), (void**)&d_cf));
+    HC_CU(hc_idmap_ws(m, 9, n_blocks * sizeof(u64), (void**)&d_os));
+    HC_CU(hc_idmap_ws(m, 10, n_blocks * sizeof(u64), (void**)&d_of));
+    HC_CU(cudaMemcpyAsync(d_misc, misc, sizeof(misc), cudaMemcpyHostToDevice, stream));
     D.text = d_text; D.n_bytes = n_bytes; D.line_start = d_ls; D.n_lines = n_lines; D.n_newlines = n_nl;
     D.ids.slots = m->slots; D.ids.mask = m->mask; D.ids.direct = m->direct; D.ids.direct_n = m->direct_n;
     D.min_overlap_len = p->min_overlap_len; D.min_overlap_perc = p->min_overlap_perc; D.relax = p->relax_PE_edges != 0;
@@ -417,17 +407,17 @@ int hc_ingest_device(const hc_idmap* cm, const char* d_text, uint64_t n_bytes, c
     ing_count<<<(unsigned)n_blocks, LINES_PER_BLOCK, 0, stream>>>(d_status, n_lines, d_cs, d_cf, d_misc);
     scan_counts<<<1, 1024, 0, stream>>>(d_cs, n_blocks, d_os, d_tot);
     scan_counts<<<1, 1024, 0, stream>>>(d_cf, n_blocks, d_of, d_tot + 1);
-    ICU(cudaMemcpyAsync(misc, d_misc, sizeof(misc), cudaMemcpyDeviceToHost, stream));
-    ICU(cudaMemcpyAsync(&tot_s, d_tot, sizeof(u64), cudaMemcpyDeviceToHost, stream));
-    ICU(cudaMemcpyAsync(&tot_f, d_tot + 1, sizeof(u64), cudaMemcpyDeviceToHost, stream));
-    ICU(cudaStreamSynchronize(stream));
+    HC_CU(cudaMemcpyAsync(misc, d_misc, sizeof(misc), cudaMemcpyDeviceToHost, stream));
+    HC_CU(cudaMemcpyAsync(&tot_s, d_tot, sizeof(u64), cudaMemcpyDeviceToHost, stream));
+    HC_CU(cudaMemcpyAsync(&tot_f, d_tot + 1, sizeof(u64), cudaMemcpyDeviceToHost, stream));
+    HC_CU(cudaStreamSynchronize(stream));
     st->n_scored = tot_s; st->n_filtered = tot_f; st->n_skipped = misc[0]; st->n_dropped = misc[1];
     st->first_error_line = misc[2];
     if (misc[2] != EMPTY) {
         uint8_t es = 0;
         u64 off[2] = {0, 0};
-        ICU(cudaMemcpy(&es, d_status + misc[2], 1, cudaMemcpyDeviceToHost));
-        ICU(cudaMemcpy(off, d_ls + misc[2], (misc[2] < n_nl ? 2 : 1) * sizeof(u64), cudaMemcpyDeviceToHost));
+        HC_CU(cudaMemcpy(&es, d_status + misc[2], 1, cudaMemcpyDeviceToHost));
+        HC_CU(cudaMemcpy(off, d_ls + misc[2], (misc[2] < n_nl ? 2 : 1) * sizeof(u64), cudaMemcpyDeviceToHost));
         st->first_error_status = es;
         st->first_error_offset = off[0];
         st->first_error_length = (misc[2] < n_nl ? off[1] - 1 : n_bytes) - off[0];
@@ -440,10 +430,10 @@ int hc_ingest_device(const hc_idmap* cm, const char* d_text, uint64_t n_bytes, c
     ing_scatter<<<(unsigned)n_blocks, LINES_PER_BLOCK, 0, stream>>>(d_status, d_tmp_c, d_tmp_f, n_lines, d_os, d_of, d_cand,
                                                                     reinterpret_cast<u64*>(d_cand_line), d_filt,
                                                                     reinterpret_cast<u64*>(d_filt_line), line_base);
-    ICU(cudaEventRecord(m->e1, stream));
-    ICU(cudaStreamSynchronize(stream));
-    ICU(cudaGetLastError());
-    ICU(cudaEventElapsedTime(&st->device_ms, m->e0, m->e1));
+    HC_CU(cudaEventRecord(m->e1, stream));
+    HC_CU(cudaStreamSynchronize(stream));
+    HC_CU(cudaGetLastError());
+    HC_CU(cudaEventElapsedTime(&st->device_ms, m->e0, m->e1));
 done:
     return rc;
 }
@@ -490,6 +480,7 @@ static int ingest_pipelined(hc_idmap* m, const char* text, u64 n_bytes, const hc
                             uint64_t* cand_line, u64 cand_cap, hc_overlap_rec* filtered, uint64_t* filtered_line, u64 filtered_cap,
                             hc_ingest_stats* stats, u64 piece) {
     int rc = HC_OK;
+    const char* who = "hc_ingest_overlaps";
     const std::vector<uint64_t> cut = hc_ingest_cuts(text, n_bytes, piece);
     const size_t n_pieces = cut.size() - 1;
     u64 max_piece = 0;
@@ -503,23 +494,23 @@ static int ingest_pipelined(hc_idmap* m, const char* text, u64 n_bytes, const hc
     u64 lines = 0, ns = 0, nf = 0;
     bool overflow = false;
     hc_ingest_params pp = *p;
-    ICU(hc_idmap_ws(m, 11, 2 * tbytes, (void**)&d_text));
-    ICU(hc_idmap_ws(m, 12, 2 * rec_cap * sizeof(hc_candidate), (void**)&d_cand));
-    ICU(hc_idmap_ws(m, 13, 2 * rec_cap * sizeof(hc_overlap_rec), (void**)&d_filt));
-    if (cand_line) ICU(hc_idmap_ws(m, 14, 2 * rec_cap * sizeof(u64), (void**)&d_cl));
-    if (filtered_line) ICU(hc_idmap_ws(m, 15, 2 * rec_cap * sizeof(u64), (void**)&d_fl));
+    HC_CU(hc_idmap_ws(m, 11, 2 * tbytes, (void**)&d_text));
+    HC_CU(hc_idmap_ws(m, 12, 2 * rec_cap * sizeof(hc_candidate), (void**)&d_cand));
+    HC_CU(hc_idmap_ws(m, 13, 2 * rec_cap * sizeof(hc_overlap_rec), (void**)&d_filt));
+    if (cand_line) HC_CU(hc_idmap_ws(m, 14, 2 * rec_cap * sizeof(u64), (void**)&d_cl));
+    if (filtered_line) HC_CU(hc_idmap_ws(m, 15, 2 * rec_cap * sizeof(u64), (void**)&d_fl));
     // pageable text / result buffers (a file read into memory, a std::vector) go through the pinned ring of hc_stage.cu,
     // copied by several host threads; pinned ones are handed to the copy engine as they are
-    ICU(hc_copy_h2d_on(d_text, text, cut[1] - cut[0], m->s_copy));
-    ICU(cudaEventRecord(m->ev_in[0], m->s_copy));
+    HC_CU(hc_copy_h2d_on(d_text, text, cut[1] - cut[0], m->s_copy));
+    HC_CU(cudaEventRecord(m->ev_in[0], m->s_copy));
     for (size_t i = 0; i < n_pieces && lines < p->max_overlaps; i++) {
         const int b = (int)(i & 1);
         if (i + 1 < n_pieces) {   // buffer (i+1)&1 was read by piece i-1, whose kernels have completed (ingest_device returns synchronised)
-            ICU(hc_copy_h2d_on(d_text + (size_t)(b ^ 1) * tbytes, text + cut[i + 1], cut[i + 2] - cut[i + 1], m->s_copy));
-            ICU(cudaEventRecord(m->ev_in[b ^ 1], m->s_copy));
+            HC_CU(hc_copy_h2d_on(d_text + (size_t)(b ^ 1) * tbytes, text + cut[i + 1], cut[i + 2] - cut[i + 1], m->s_copy));
+            HC_CU(cudaEventRecord(m->ev_in[b ^ 1], m->s_copy));
         }
-        ICU(cudaStreamWaitEvent(m->s_main, m->ev_in[b], 0));
-        if (i >= 2) ICU(cudaEventSynchronize(m->ev_out[b]));          // output set b has been copied out
+        HC_CU(cudaStreamWaitEvent(m->s_main, m->ev_in[b], 0));
+        if (i >= 2) HC_CU(cudaEventSynchronize(m->ev_out[b]));          // output set b has been copied out
         hc_ingest_stats st;
         pp.max_overlaps = p->max_overlaps - lines;
         const u64 room_s = overflow ? 0 : std::min<u64>(rec_cap, cand_cap - ns), room_f = overflow ? 0 : std::min<u64>(rec_cap, filtered_cap - nf);
@@ -536,20 +527,20 @@ static int ingest_pipelined(hc_idmap* m, const char* text, u64 n_bytes, const hc
         }
         if (!overflow) {
             if (st.n_scored) {
-                ICU(hc_copy_d2h_on(cand + ns, d_cand + (size_t)b * rec_cap, st.n_scored * sizeof(hc_candidate), m->s_out, nullptr));
-                if (cand_line) ICU(hc_copy_d2h_on(cand_line + ns, d_cl + (size_t)b * rec_cap, st.n_scored * sizeof(u64), m->s_out, nullptr));
+                HC_CU(hc_copy_d2h_on(cand + ns, d_cand + (size_t)b * rec_cap, st.n_scored * sizeof(hc_candidate), m->s_out, nullptr));
+                if (cand_line) HC_CU(hc_copy_d2h_on(cand_line + ns, d_cl + (size_t)b * rec_cap, st.n_scored * sizeof(u64), m->s_out, nullptr));
             }
             if (st.n_filtered) {
-                ICU(hc_copy_d2h_on(filtered + nf, d_filt + (size_t)b * rec_cap, st.n_filtered * sizeof(hc_overlap_rec), m->s_out, nullptr));
-                if (filtered_line) ICU(hc_copy_d2h_on(filtered_line + nf, d_fl + (size_t)b * rec_cap, st.n_filtered * sizeof(u64), m->s_out, nullptr));
+                HC_CU(hc_copy_d2h_on(filtered + nf, d_filt + (size_t)b * rec_cap, st.n_filtered * sizeof(hc_overlap_rec), m->s_out, nullptr));
+                if (filtered_line) HC_CU(hc_copy_d2h_on(filtered_line + nf, d_fl + (size_t)b * rec_cap, st.n_filtered * sizeof(u64), m->s_out, nullptr));
             }
         }
-        ICU(cudaEventRecord(m->ev_out[b], m->s_out));
+        HC_CU(cudaEventRecord(m->ev_out[b], m->s_out));
         lines += st.n_lines; ns += st.n_scored; nf += st.n_filtered;
         stats->n_skipped += st.n_skipped; stats->n_dropped += st.n_dropped; stats->device_ms += st.device_ms;
     }
-    ICU(cudaStreamSynchronize(m->s_out));
-    ICU(cudaStreamSynchronize(m->s_copy));
+    HC_CU(cudaStreamSynchronize(m->s_out));
+    HC_CU(cudaStreamSynchronize(m->s_copy));
     stats->n_lines = lines; stats->n_scored = ns; stats->n_filtered = nf;
     if (overflow) {
         hc_set_last_error("hc_ingest_overlaps: output buffer too small (required sizes returned in stats)");
@@ -566,6 +557,7 @@ extern "C" int hc_ingest_overlaps(const hc_idmap* cm, const char* text, uint64_t
     if (!cm || !p || !stats || (n_bytes && !text)) { hc_set_last_error("hc_ingest_overlaps: NULL argument"); return HC_ERR_ARG; }
     hc_idmap* m = const_cast<hc_idmap*>(cm);
     int rc = HC_OK;
+    const char* who = "hc_ingest_overlaps";
     char* d_text = nullptr;
     hc_candidate* d_cand = nullptr;
     hc_overlap_rec* d_filt = nullptr;
@@ -573,25 +565,25 @@ extern "C" int hc_ingest_overlaps(const hc_idmap* cm, const char* text, uint64_t
     memset(stats, 0, sizeof(*stats));
     stats->first_error_line = EMPTY;
     if (n_bytes == 0) return HC_OK;
-    ICU(cudaSetDevice(m->device));
+    HC_CU(cudaSetDevice(m->device));
     {
         const u64 piece = hc_ingest_piece_bytes();
         if (n_bytes > piece + piece / 2)
             return ingest_pipelined(m, text, n_bytes, p, cand, cand_line, cand_cap, filtered, filtered_line, filtered_cap, stats, piece);
     }
-    ICU(hc_idmap_ws(m, 11, n_bytes + 16, (void**)&d_text));
-    ICU(hc_copy_h2d(d_text, text, n_bytes));
-    if (cand_cap) { ICU(hc_idmap_ws(m, 12, cand_cap * sizeof(hc_candidate), (void**)&d_cand)); if (cand_line) ICU(hc_idmap_ws(m, 14, cand_cap * sizeof(u64), (void**)&d_cl)); }
-    if (filtered_cap) { ICU(hc_idmap_ws(m, 13, filtered_cap * sizeof(hc_overlap_rec), (void**)&d_filt)); if (filtered_line) ICU(hc_idmap_ws(m, 15, filtered_cap * sizeof(u64), (void**)&d_fl)); }
+    HC_CU(hc_idmap_ws(m, 11, n_bytes + 16, (void**)&d_text));
+    HC_CU(hc_copy_h2d(d_text, text, n_bytes));
+    if (cand_cap) { HC_CU(hc_idmap_ws(m, 12, cand_cap * sizeof(hc_candidate), (void**)&d_cand)); if (cand_line) HC_CU(hc_idmap_ws(m, 14, cand_cap * sizeof(u64), (void**)&d_cl)); }
+    if (filtered_cap) { HC_CU(hc_idmap_ws(m, 13, filtered_cap * sizeof(hc_overlap_rec), (void**)&d_filt)); if (filtered_line) HC_CU(hc_idmap_ws(m, 15, filtered_cap * sizeof(u64), (void**)&d_fl)); }
     rc = hc_ingest_device(m, d_text, n_bytes, p, d_cand, d_cl, cand_cap, d_filt, d_fl, filtered_cap, stats, m->s_main);
     if (rc != HC_OK) goto done;
     if (stats->n_scored) {
-        ICU(hc_copy_d2h(cand, d_cand, stats->n_scored * sizeof(hc_candidate)));
-        if (cand_line) ICU(hc_copy_d2h(cand_line, d_cl, stats->n_scored * sizeof(u64)));
+        HC_CU(hc_copy_d2h(cand, d_cand, stats->n_scored * sizeof(hc_candidate)));
+        if (cand_line) HC_CU(hc_copy_d2h(cand_line, d_cl, stats->n_scored * sizeof(u64)));
     }
     if (stats->n_filtered) {
-        ICU(hc_copy_d2h(filtered, d_filt, stats->n_filtered * sizeof(hc_overlap_rec)));
-        if (filtered_line) ICU(hc_copy_d2h(filtered_line, d_fl, stats->n_filtered * sizeof(u64)));
+        HC_CU(hc_copy_d2h(filtered, d_filt, stats->n_filtered * sizeof(hc_overlap_rec)));
+        if (filtered_line) HC_CU(hc_copy_d2h(filtered_line, d_fl, stats->n_filtered * sizeof(u64)));
     }
 done:
     return rc;

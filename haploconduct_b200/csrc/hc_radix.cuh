@@ -90,6 +90,42 @@ __global__ void __launch_bounds__(THREADS) tile_scatter(const ulonglong2* __rest
     }
 }
 
+// ---- the stage behind the sort: one thread orders a run of equal keys by a finer order -------------------------------
+constexpr uint32_t RUN_INSERTION_MAX = 32;
+
+template <class T, class Less>
+__device__ void sift_down(T* v, uint32_t root, uint32_t m, Less lt) {
+    while (true) {
+        uint32_t c = 2 * root + 1;
+        if (c >= m) return;
+        if (c + 1 < m && lt(v[c], v[c + 1])) c++;
+        if (!lt(v[root], v[c])) return;
+        const T x = v[root]; v[root] = v[c]; v[c] = x;
+        root = c;
+    }
+}
+
+// v[0, m) in lt order: insertion sort up to RUN_INSERTION_MAX entries, heap sort beyond (linear on a run of equal entries).
+// Not stable, so where lt leaves entries equal this exact algorithm decides their order (hc_sfo.cu: which file line of a
+// repeated line is kept); tests/test_gpu_prims.py pins it.
+template <class T, class Less>
+__device__ void sort_run(T* v, uint32_t m, Less lt) {
+    if (m <= RUN_INSERTION_MAX) {
+        for (uint32_t a = 1; a < m; a++) {
+            const T x = v[a];
+            uint32_t c = a;
+            while (c > 0 && lt(x, v[c - 1])) { v[c] = v[c - 1]; c--; }
+            v[c] = x;
+        }
+        return;
+    }
+    for (uint32_t r = m / 2; r-- > 0;) sift_down(v, r, m, lt);
+    for (uint32_t e = m - 1; e > 0; e--) {
+        const T x = v[0]; v[0] = v[e]; v[e] = x;
+        sift_down(v, 0, e, lt);
+    }
+}
+
 // Sorts n pairs by key, stably.  The result is in (*kres, *vres): (keys, vals) or (ktmp, vtmp), each holding n entries.
 // Enqueued on the legacy default stream; synchronises once (to read which digit positions vary).
 inline cudaError_t sort_pairs(ulonglong2* keys, uint32_t* vals, ulonglong2* ktmp, uint32_t* vtmp, u64 n,
@@ -98,20 +134,20 @@ inline cudaError_t sort_pairs(ulonglong2* keys, uint32_t* vals, ulonglong2* ktmp
     if (n == 0) return cudaSuccess;
     const uint32_t nb = (uint32_t)((n + TILE - 1) / TILE);
     const u64 cells = (u64)THREADS * nb;
-    u64 *d_acc = nullptr, *d_start = nullptr, *d_total = nullptr, *d_bsum = nullptr;
-    uint32_t* d_counts = nullptr;
+    ScratchBuf<u64> d_acc, d_start, d_total, d_bsum;
+    ScratchBuf<uint32_t> d_counts;
     u64 acc[4] = {~0ull, ~0ull, 0, 0};
     cudaError_t e;
     ulonglong2 *ki = keys, *ko = ktmp;
     uint32_t *vi = vals, *vo = vtmp;
-    if ((e = hc_scratch_alloc((void**)&d_acc, sizeof(acc))) != cudaSuccess) goto done;
-    if ((e = hc_scratch_alloc((void**)&d_counts, cells * sizeof(uint32_t))) != cudaSuccess) goto done;
-    if ((e = hc_scratch_alloc((void**)&d_start, cells * sizeof(u64))) != cudaSuccess) goto done;
-    if ((e = hc_scratch_alloc((void**)&d_total, sizeof(u64))) != cudaSuccess) goto done;
-    if ((e = hc_scratch_alloc((void**)&d_bsum, hc_scan::blocks_for(cells) * sizeof(u64))) != cudaSuccess) goto done;
-    if ((e = cudaMemcpyAsync(d_acc, acc, sizeof(acc), cudaMemcpyHostToDevice)) != cudaSuccess) goto done;
+    if ((e = d_acc.alloc(4)) != cudaSuccess) return e;
+    if ((e = d_counts.alloc(cells)) != cudaSuccess) return e;
+    if ((e = d_start.alloc(cells)) != cudaSuccess) return e;
+    if ((e = d_total.alloc(1)) != cudaSuccess) return e;
+    if ((e = d_bsum.alloc(hc_scan::blocks_for(cells))) != cudaSuccess) return e;
+    if ((e = cudaMemcpyAsync(d_acc, acc, sizeof(acc), cudaMemcpyHostToDevice)) != cudaSuccess) return e;
     and_or<<<(unsigned)(nb < 148 * 8 ? nb : 148 * 8), THREADS>>>(keys, n, d_acc);
-    if ((e = cudaMemcpy(acc, d_acc, sizeof(acc), cudaMemcpyDeviceToHost)) != cudaSuccess) goto done;
+    if ((e = cudaMemcpy(acc, d_acc, sizeof(acc), cudaMemcpyDeviceToHost)) != cudaSuccess) return e;
     for (int p = 0; p < 16; p++) {
         const u64 diff = p < 8 ? acc[0] ^ acc[2] : acc[1] ^ acc[3];
         if (((diff >> (8 * (p & 7))) & 0xffu) == 0) continue;       // every key has the same digit here
@@ -120,12 +156,10 @@ inline cudaError_t sort_pairs(ulonglong2* keys, uint32_t* vals, ulonglong2* ktmp
         tile_scatter<<<nb, THREADS>>>(ki, vi, n, p, nb, d_start, ko, vo);
         ulonglong2* tk = ki; ki = ko; ko = tk;
         uint32_t* tv = vi; vi = vo; vo = tv;
-        if ((e = cudaGetLastError()) != cudaSuccess) goto done;
+        if ((e = cudaGetLastError()) != cudaSuccess) return e;
     }
     *kres = ki; *vres = vi;
-done:
-    hc_scratch_free(d_acc); hc_scratch_free(d_counts); hc_scratch_free(d_start); hc_scratch_free(d_total); hc_scratch_free(d_bsum);
-    return e;
+    return cudaSuccess;
 }
 
 }  // namespace

@@ -51,15 +51,12 @@
 #include <numeric>
 #include <string>
 #include <vector>
-#include <time.h>
 #include <cuda_runtime.h>
 #include "../../include/hc_b200.h"
 #include "hc_radix.cuh"
 #include "hc_scan.cuh"
 #include "hc_stage.h"
 #include "hc_text.cuh"
-
-void hc_set_last_error(const char* msg);   // hc_api.cu
 
 namespace {
 
@@ -95,22 +92,6 @@ __device__ __forceinline__ unsigned long long err_key(uint32_t file, uint32_t li
     return (unsigned long long)file << 34 | (unsigned long long)line << 2 | status;
 }
 
-// to_long (:41) of [b, e): 0 not a number, 1 ok, 2 more than 18 digits (the host's long may overflow)
-__device__ int to_long(const char* t, u64 b, u64 e, i64* v) {
-    if (b == e) return 0;
-    bool neg = false;
-    if (t[b] == '+' || t[b] == '-') { neg = t[b] == '-'; b++; }
-    if (b == e) return 0;
-    i64 x = 0;
-    for (u64 p = b; p < e; p++) {
-        const char c = t[p];
-        if (c < '0' || c > '9') return 0;
-        if (p - b < 18) x = x * 10 + (c - '0');
-    }
-    *v = neg ? -x : x;
-    return e - b > 18 ? 2 : 1;
-}
-
 __device__ __forceinline__ bool is_digit(char c) { return c >= '0' && c <= '9'; }
 
 // bytewise compare of two texts (std::string operator<=>)
@@ -130,13 +111,6 @@ __device__ int32_t lookup(const Names& N, const char* s, u64 l) {
         if (c < 0) lo = mid + 1; else hi = mid;
     }
     return -1;
-}
-
-__device__ __forceinline__ void line_span(const char* t, u64 n, const u64* ls, u64 n_nl, u64 k, u64* b, u64* le) {
-    *b = ls[k];
-    u64 e = k < n_nl ? ls[k + 1] : n;
-    if (e > *b && t[e - 1] == '\n') e--;
-    *le = e;
 }
 
 struct FileIn { const char* t; u64 base, n; const u64* ls; u64 n_nl, nl; uint32_t file; };
@@ -175,12 +149,12 @@ __global__ void sam_parse(FileIn F, u64 first, u64 g0, Names N, Aln* __restrict_
         i64 flag = 0, POS = 0, dummy;
         int r;
         if (nf < 11) die = 1;
-        if (!die) { r = to_long(t, fb[1], fe[1], &flag); die |= r == 0; decline |= r == 2; }
+        if (!die) { r = parse_long(t, fb[1], fe[1], &flag); die |= r == 0; decline |= r == 2; }
         if (!die && !decline && (flag & 4)) continue;                  // unmapped: nothing else is read
         if (!die && !decline) {
-            r = to_long(t, fb[3], fe[3], &POS); die |= r == 0; decline |= r == 2 || POS >= BIG || POS <= -BIG;
+            r = parse_long(t, fb[3], fe[3], &POS); die |= r == 0; decline |= r == 2 || POS >= BIG || POS <= -BIG;
             const int more[3] = {4, 7, 8};                             // MAPQ, PNEXT, TLEN: only their validity matters
-            for (int f : more) { r = to_long(t, fb[f], fe[f], &dummy); die |= r == 0; decline |= r == 2; }
+            for (int f : more) { r = parse_long(t, fb[f], fe[f], &dummy); die |= r == 0; decline |= r == 2; }
         }
         Aln a;
         uint32_t runs = 0, z = 0;
@@ -382,28 +356,6 @@ __global__ void sam_ref_info(const Rec* __restrict__ srec, u64 n, const i64* __r
     if (threadIdx.x == 0) info[r] = RefInfo{s_rb, s_re, s_np, (i64)s_max};
 }
 
-struct Sink {                                         // counts bytes; writes them too when p != nullptr
-    char* p;
-    u64 n;
-    __device__ void c(char x) { if (p) p[n] = x; n++; }
-    __device__ void num(i64 v) {
-        unsigned long long u = v < 0 ? 0ull - (unsigned long long)v : (unsigned long long)v;
-        int d = 1;
-        for (unsigned long long x = u; x >= 10; x /= 10) d++;
-        d += v < 0;
-        if (p) {
-            char* q = p + n;
-            if (v < 0) *q = '-';
-            for (int k = d - 1; k >= (v < 0); k--) { q[k] = (char)('0' + u % 10); u /= 10; }
-        }
-        n += d;
-    }
-    __device__ void str(const char* t, u64 b, u64 l) {
-        if (p) for (u64 i = 0; i < l; i++) p[n + i] = t[b + i];
-        n += l;
-    }
-};
-
 struct Ctx { const char* t; const Aln* aln; const u64* ops; i64 min_ov; };
 
 struct Ov { i64 pos, len; };
@@ -486,7 +438,7 @@ __device__ PairOut pair_overlap(const Ctx& X, const Rec& R, const Rec& C, Sink& 
     }
     const char o1 = R.paired ? (R.rc ? '-' : '+') : (Ra.rev ? '-' : '+');
     const char o2 = C.paired ? (C.rc ? '-' : '+') : (Ca.rev ? '-' : '+');
-    s.str(X.t, Ra.id_off, Ra.id_len); s.c('\t'); s.str(X.t, Ca.id_off, Ca.id_len); s.c('\t'); s.num(o.pos); s.c('\t');
+    s.str(X.t, Ra.id_off, Ra.id_off + Ra.id_len); s.c('\t'); s.str(X.t, Ca.id_off, Ca.id_off + Ca.id_len); s.c('\t'); s.num(o.pos); s.c('\t');
     s.num(v.pos); s.c('\t'); s.c(ord); s.c('\t'); s.c(o1); s.c('\t'); s.c(o2); s.c('\t'); s.num(perc1); s.c('\t');
     s.num(perc2); s.c('\t'); s.num(o.len); s.c('\t'); s.num(v.len); s.c('\t'); s.c(t1); s.c('\t'); s.c(t2); s.c('\n');
     out.line = 1;
@@ -576,22 +528,7 @@ __global__ void sam_ref_stats(const Rec* __restrict__ srec, const RecCnt* __rest
     }
 }
 
-inline int grid_for(u64 n, int threads) { const u64 b = (n + threads - 1) / threads; return (int)(b < 148 * 16 ? (b ? b : 1) : 148 * 16); }
-inline double now_ms() { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6; }
-
 }  // namespace
-
-// an allocation that fails is HC_ERR_NOMEM (the caller runs the host converter), anything else HC_ERR_CUDA
-#define SCU(call)                                                                                              \
-    do {                                                                                                       \
-        cudaError_t _e = (call);                                                                               \
-        if (_e != cudaSuccess) {                                                                               \
-            hc_set_last_error((std::string("hc_sam2overlaps: ") + #call + ": " + cudaGetErrorString(_e)).c_str()); \
-            rc = _e == cudaErrorMemoryAllocation ? HC_ERR_NOMEM : HC_ERR_CUDA;                                 \
-            if (rc == HC_ERR_NOMEM) cudaGetLastError();                                                        \
-            goto done;                                                                                         \
-        }                                                                                                      \
-    } while (0)
 
 extern "C" int hc_sam2overlaps(const char* sam_s, uint64_t n_s, const char* sam_p, uint64_t n_p, const char* ref_names,
                                const uint64_t* ref_name_off, const uint32_t* ref_name_idx, uint32_t n_names, const int64_t* ref_len,
@@ -627,20 +564,21 @@ extern "C" int hc_sam2overlaps(const char* sam_s, uint64_t n_s, const char* sam_
     int rc = HC_OK;
     const int T = 256;
     const u64 n_all = n_s + n_p, names_bytes = n_names ? ref_name_off[n_names] : 0;
-    char *d_text = nullptr, *d_names = nullptr, *d_out = nullptr;
-    u64 *d_ls[2] = {nullptr, nullptr}, *d_noff = nullptr, *d_tot = nullptr, *d_bsum = nullptr, *d_ooff = nullptr, *d_ops = nullptr,
-        *d_mpos = nullptr, *d_rx = nullptr, *d_apos = nullptr, *d_boff = nullptr;
-    uint32_t *d_perm = nullptr, *d_nidx = nullptr, *d_mapped = nullptr, *d_nops = nullptr, *d_rev = nullptr, *d_smidx = nullptr,
-             *d_pmidx = nullptr, *d_st = nullptr, *d_rfirst = nullptr, *d_acc = nullptr, *d_val = nullptr, *d_val2 = nullptr,
-             *d_ord = nullptr, *d_nb = nullptr, *d_ovf = nullptr;
-    unsigned long long* d_cnt = nullptr;      // [0..2] first error per stage, [3] header end, [4] discards, [5] reverse pairs
-    i64* d_rlen = nullptr;
-    Aln* d_aln = nullptr;
-    Rec *d_rec = nullptr, *d_srec = nullptr;
-    RefInfo* d_info = nullptr;
-    RecCnt* d_rc = nullptr;
-    hc_sam_ref_stats* d_rs = nullptr;
-    ulonglong2 *d_key = nullptr, *d_key2 = nullptr, *d_skey = nullptr;
+    const char* who = "hc_sam2overlaps";
+    ScratchBuf<char> d_text, d_names, d_out;
+    ScratchBuf<u64> d_noff, d_tot, d_bsum, d_ooff, d_ops, d_mpos, d_rx, d_apos, d_boff;
+    ScratchBuf<uint32_t> d_perm, d_nidx, d_mapped, d_nops, d_rev, d_smidx, d_pmidx, d_st, d_rfirst, d_acc, d_val, d_val2, d_nb, d_ovf;
+    ScratchBuf<unsigned long long> d_cnt;     // [0..2] first error per stage, [3] header end, [4] discards, [5] reverse pairs
+    ScratchBuf<i64> d_rlen;
+    ScratchBuf<Aln> d_aln;
+    ScratchBuf<Rec> d_rec, d_srec;
+    ScratchBuf<RefInfo> d_info;
+    ScratchBuf<RecCnt> d_rc;
+    ScratchBuf<hc_sam_ref_stats> d_rs;
+    ScratchBuf<ulonglong2> d_key, d_key2;
+    u64* d_ls[2] = {nullptr, nullptr};        // hc_line_index's (cudaMalloc)
+    uint32_t* d_ord = nullptr;
+    ulonglong2* d_skey = nullptr;
     u64 n_nl[2] = {0, 0}, nl[2] = {0, 0}, first[2] = {0, 0}, ng = 0, n_ops = 0, nsm = 0, nm = 0, nruns = 0, npairs = 0, nrec = 0,
         out_bytes = 0;
     unsigned long long cnt[6];
@@ -651,30 +589,30 @@ extern "C" int hc_sam2overlaps(const char* sam_s, uint64_t n_s, const char* sam_
     std::vector<hc_sam_ref_stats> rs(n_refs);
     const u64 nbytes[2] = {n_s, n_p};
     const i64 min_ov = min_overlap_len > MIN_OV_CLAMP ? MIN_OV_CLAMP : (min_overlap_len < -MIN_OV_CLAMP ? -MIN_OV_CLAMP : min_overlap_len);
-    SCU(cudaSetDevice(device));
-    t0 = now_ms();
-    SCU(hc_scratch_alloc((void**)&d_text, n_all + 16));
-    if (n_s) SCU(hc_copy_h2d(d_text, sam_s, n_s));
-    if (n_p) SCU(hc_copy_h2d(d_text + n_s, sam_p, n_p));
-    t1 = now_ms();
+    HC_CU(cudaSetDevice(device));
+    t0 = hc_now_ms();
+    HC_CU(d_text.alloc(n_all + 16));
+    if (n_s) HC_CU(hc_copy_h2d(d_text, sam_s, n_s));
+    if (n_p) HC_CU(hc_copy_h2d(d_text + n_s, sam_p, n_p));
+    t1 = hc_now_ms();
     stats->h2d_ms = (float)(t1 - t0);
     t0 = t1;
     // the names table (sorted here for the binary search) and the reference lengths
-    SCU(hc_scratch_alloc((void**)&d_names, names_bytes + 1));
-    SCU(hc_scratch_alloc((void**)&d_noff, (n_names + 1) * sizeof(u64)));
-    SCU(hc_scratch_alloc((void**)&d_perm, (n_names + 1) * sizeof(uint32_t)));
-    SCU(hc_scratch_alloc((void**)&d_nidx, (n_names + 1) * sizeof(uint32_t)));
-    SCU(hc_scratch_alloc((void**)&d_rlen, (n_refs + 1) * sizeof(i64)));
-    if (names_bytes) SCU(cudaMemcpy(d_names, ref_names, names_bytes, cudaMemcpyHostToDevice));
+    HC_CU(d_names.alloc(names_bytes + 1));
+    HC_CU(d_noff.alloc(n_names + 1));
+    HC_CU(d_perm.alloc(n_names + 1));
+    HC_CU(d_nidx.alloc(n_names + 1));
+    HC_CU(d_rlen.alloc(n_refs + 1));
+    if (names_bytes) HC_CU(cudaMemcpy(d_names, ref_names, names_bytes, cudaMemcpyHostToDevice));
     if (n_names) {
-        SCU(cudaMemcpy(d_noff, ref_name_off, (n_names + 1) * sizeof(u64), cudaMemcpyHostToDevice));
-        SCU(cudaMemcpy(d_perm, perm.data(), n_names * sizeof(uint32_t), cudaMemcpyHostToDevice));
-        SCU(cudaMemcpy(d_nidx, ref_name_idx, n_names * sizeof(uint32_t), cudaMemcpyHostToDevice));
+        HC_CU(cudaMemcpy(d_noff, ref_name_off, (n_names + 1) * sizeof(u64), cudaMemcpyHostToDevice));
+        HC_CU(cudaMemcpy(d_perm, perm.data(), n_names * sizeof(uint32_t), cudaMemcpyHostToDevice));
+        HC_CU(cudaMemcpy(d_nidx, ref_name_idx, n_names * sizeof(uint32_t), cudaMemcpyHostToDevice));
     }
-    if (n_refs) SCU(cudaMemcpy(d_rlen, ref_len, n_refs * sizeof(i64), cudaMemcpyHostToDevice));
+    if (n_refs) HC_CU(cudaMemcpy(d_rlen, ref_len, n_refs * sizeof(i64), cudaMemcpyHostToDevice));
     N = Names{d_names, d_noff, d_perm, d_nidx, n_names};
     // lines, header, parse
-    for (int f = 0; f < 2; f++) SCU(hc_line_index(d_text + (f ? n_s : 0), nbytes[f], &d_ls[f], &n_nl[f], &nl[f], 0));
+    for (int f = 0; f < 2; f++) HC_CU(hc_line_index(d_text + (f ? n_s : 0), nbytes[f], &d_ls[f], &n_nl[f], &nl[f], 0));
     if ((nl[0] + nl[1]) >> 32) {
         stats->first_error_file = nl[0] >> 32 ? 0 : 1;
         stats->first_error_line = 1ull << 32;
@@ -684,132 +622,132 @@ extern "C" int hc_sam2overlaps(const char* sam_s, uint64_t n_s, const char* sam_
         goto done;
     }
     for (int i = 0; i < 6; i++) cnt[i] = i < 3 ? NO_ERR : 0;
-    SCU(hc_scratch_alloc((void**)&d_cnt, sizeof(cnt)));
-    SCU(hc_scratch_alloc((void**)&d_ovf, sizeof(uint32_t)));
-    SCU(hc_scratch_alloc((void**)&d_tot, sizeof(u64)));
-    SCU(cudaMemset(d_ovf, 0, sizeof(uint32_t)));
+    HC_CU(d_cnt.alloc(6));
+    HC_CU(d_ovf.alloc(1));
+    HC_CU(d_tot.alloc(1));
+    HC_CU(cudaMemset(d_ovf, 0, sizeof(uint32_t)));
     for (int f = 0; f < 2; f++) {
         cnt[3] = nl[f];
-        SCU(cudaMemcpy(d_cnt + 3, &cnt[3], sizeof(u64), cudaMemcpyHostToDevice));
+        HC_CU(cudaMemcpy(d_cnt + 3, &cnt[3], sizeof(u64), cudaMemcpyHostToDevice));
         if (nl[f]) {
             FileIn F = {d_text + (f ? n_s : 0), f ? n_s : 0, nbytes[f], d_ls[f], n_nl[f], nl[f], (uint32_t)f};
             sam_header<<<grid_for(nl[f], T), T>>>(F, d_cnt + 3);
-            SCU(cudaGetLastError());
+            HC_CU(cudaGetLastError());
         }
-        SCU(cudaMemcpy(&first[f], d_cnt + 3, sizeof(u64), cudaMemcpyDeviceToHost));
+        HC_CU(cudaMemcpy(&first[f], d_cnt + 3, sizeof(u64), cudaMemcpyDeviceToHost));
     }
     cnt[3] = 0;
-    SCU(cudaMemcpy(d_cnt, cnt, sizeof(cnt), cudaMemcpyHostToDevice));
+    HC_CU(cudaMemcpy(d_cnt, cnt, sizeof(cnt), cudaMemcpyHostToDevice));
     ng = (nl[0] - first[0]) + (nl[1] - first[1]);
-    SCU(hc_scratch_alloc((void**)&d_aln, (ng + 1) * sizeof(Aln)));
-    SCU(hc_scratch_alloc((void**)&d_mapped, (ng + 1) * sizeof(uint32_t)));
-    SCU(hc_scratch_alloc((void**)&d_nops, (ng + 1) * sizeof(uint32_t)));
-    SCU(hc_scratch_alloc((void**)&d_rev, (ng + 1) * sizeof(uint32_t)));
-    SCU(hc_scratch_alloc((void**)&d_bsum, hc_scan::blocks_for(ng + 1) * sizeof(u64)));
+    HC_CU(d_aln.alloc(ng + 1));
+    HC_CU(d_mapped.alloc(ng + 1));
+    HC_CU(d_nops.alloc(ng + 1));
+    HC_CU(d_rev.alloc(ng + 1));
+    HC_CU(d_bsum.alloc(hc_scan::blocks_for(ng + 1)));
     for (int f = 0; f < 2; f++) {
         if (nl[f] == first[f]) continue;
         FileIn F = {d_text + (f ? n_s : 0), f ? n_s : 0, nbytes[f], d_ls[f], n_nl[f], nl[f], (uint32_t)f};
         sam_parse<<<grid_for(nl[f] - first[f], T), T>>>(F, first[f], f ? nl[0] - first[0] : 0, N, d_aln, d_mapped, d_nops, d_rev, d_cnt);
-        SCU(cudaGetLastError());
+        HC_CU(cudaGetLastError());
     }
-    SCU(cudaMemcpy(cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost));
+    HC_CU(cudaMemcpy(cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost));
     if (cnt[0] != NO_ERR || cnt[1] != NO_ERR) goto input_error;
     // the CIGAR runs
-    SCU(hc_scratch_alloc((void**)&d_ooff, (ng + 1) * sizeof(u64)));
+    HC_CU(d_ooff.alloc(ng + 1));
     hc_scan::exclusive_u32(d_nops, ng, d_ooff, d_tot, d_bsum, 0);
-    SCU(cudaMemcpy(&n_ops, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
-    SCU(hc_scratch_alloc((void**)&d_ops, (n_ops + 1) * sizeof(u64)));
+    HC_CU(cudaMemcpy(&n_ops, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
+    HC_CU(d_ops.alloc(n_ops + 1));
     sam_ops<<<grid_for(ng, T), T>>>(d_text, d_mapped, d_ooff, ng, d_aln, d_ops);
-    SCU(cudaGetLastError());
-    hc_scratch_free(d_ooff); d_ooff = nullptr;
+    HC_CU(cudaGetLastError());
+    d_ooff.reset();
     // singles: the mapped lines of the single-end file in file order; counts
-    SCU(hc_scratch_alloc((void**)&d_mpos, (ng + 1) * sizeof(u64)));
+    HC_CU(d_mpos.alloc(ng + 1));
     {
         const u64 n0 = nl[0] - first[0], n1 = nl[1] - first[1];
         hc_scan::exclusive_u32(d_mapped, n0, d_mpos, d_tot, d_bsum, 0);
-        SCU(cudaMemcpy(&nsm, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
-        SCU(hc_scratch_alloc((void**)&d_smidx, (nsm + 1) * sizeof(uint32_t)));
+        HC_CU(cudaMemcpy(&nsm, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
+        HC_CU(d_smidx.alloc(nsm + 1));
         sam_gather_mapped<<<grid_for(n0, T), T>>>(d_mapped, d_mpos, 0, n0, d_smidx);
         hc_scan::exclusive_u32(d_rev, n0, d_mpos, d_tot, d_bsum, 0);
-        SCU(cudaMemcpy(&stats->reverse_s, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
+        HC_CU(cudaMemcpy(&stats->reverse_s, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
         stats->unmapped_s = n0 - nsm;
         hc_scan::exclusive_u32(d_mapped + n0, n1, d_mpos, d_tot, d_bsum, 0);
-        SCU(cudaMemcpy(&nm, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
+        HC_CU(cudaMemcpy(&nm, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
         stats->unmapped_p = n1 - nm;
-        SCU(hc_scratch_alloc((void**)&d_pmidx, (nm + 1) * sizeof(uint32_t)));
+        HC_CU(d_pmidx.alloc(nm + 1));
         sam_gather_mapped<<<grid_for(n1, T), T>>>(d_mapped, d_mpos, n0, n1, d_pmidx);
-        SCU(cudaGetLastError());
+        HC_CU(cudaGetLastError());
     }
     // pairing
-    SCU(hc_scratch_alloc((void**)&d_st, (nm + 1) * sizeof(uint32_t)));
-    SCU(hc_scratch_alloc((void**)&d_rx, (nm + 1) * sizeof(u64)));
-    SCU(hc_scratch_alloc((void**)&d_acc, (nm + 1) * sizeof(uint32_t)));
-    SCU(hc_scratch_alloc((void**)&d_apos, (nm + 1) * sizeof(u64)));
+    HC_CU(d_st.alloc(nm + 1));
+    HC_CU(d_rx.alloc(nm + 1));
+    HC_CU(d_acc.alloc(nm + 1));
+    HC_CU(d_apos.alloc(nm + 1));
     sam_run_starts<<<grid_for(nm, T), T>>>(d_text, d_aln, d_pmidx, nm, d_st);
     hc_scan::exclusive_u32(d_st, nm, d_rx, d_tot, d_bsum, 0);
-    SCU(cudaGetLastError());
-    SCU(cudaMemcpy(&nruns, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
-    SCU(hc_scratch_alloc((void**)&d_rfirst, (nruns + 1) * sizeof(uint32_t)));
+    HC_CU(cudaGetLastError());
+    HC_CU(cudaMemcpy(&nruns, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
+    HC_CU(d_rfirst.alloc(nruns + 1));
     sam_run_first<<<grid_for(nm, T), T>>>(d_st, d_rx, nm, d_rfirst);
     sam_pairs<<<grid_for(nm, T), T>>>(d_aln, d_pmidx, d_st, d_rx, d_rfirst, nm, d_acc, d_cnt + 4, d_cnt);
     hc_scan::exclusive_u32(d_acc, nm, d_apos, d_tot, d_bsum, 0);
-    SCU(cudaGetLastError());
-    SCU(cudaMemcpy(&npairs, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
-    SCU(cudaMemcpy(cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost));
+    HC_CU(cudaGetLastError());
+    HC_CU(cudaMemcpy(&npairs, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
+    HC_CU(cudaMemcpy(cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost));
     if (cnt[1] != NO_ERR) goto input_error;
     stats->discarded = cnt[4];
     stats->reverse_p = cnt[5];
     // records in (reference, position, singles first) order
     nrec = nsm + npairs;
     stats->total_alns = nrec;
-    SCU(hc_scratch_alloc((void**)&d_rec, (nrec + 1) * sizeof(Rec)));
-    SCU(hc_scratch_alloc((void**)&d_key, (nrec + 1) * sizeof(ulonglong2)));
-    SCU(hc_scratch_alloc((void**)&d_key2, (nrec + 1) * sizeof(ulonglong2)));
-    SCU(hc_scratch_alloc((void**)&d_val, (nrec + 1) * sizeof(uint32_t)));
-    SCU(hc_scratch_alloc((void**)&d_val2, (nrec + 1) * sizeof(uint32_t)));
+    HC_CU(d_rec.alloc(nrec + 1));
+    HC_CU(d_key.alloc(nrec + 1));
+    HC_CU(d_key2.alloc(nrec + 1));
+    HC_CU(d_val.alloc(nrec + 1));
+    HC_CU(d_val2.alloc(nrec + 1));
     sam_records<<<grid_for(nsm + nm, T), T>>>(d_aln, d_smidx, nsm, d_pmidx, d_acc, d_apos, nm, d_rec, d_key, d_val);
-    SCU(cudaGetLastError());
-    SCU(hc_radix::sort_pairs(d_key, d_val, d_key2, d_val2, nrec, &d_skey, &d_ord));
-    SCU(hc_scratch_alloc((void**)&d_srec, (nrec + 1) * sizeof(Rec)));
+    HC_CU(cudaGetLastError());
+    HC_CU(hc_radix::sort_pairs(d_key, d_val, d_key2, d_val2, nrec, &d_skey, &d_ord));
+    HC_CU(d_srec.alloc(nrec + 1));
     sam_gather<<<grid_for(nrec, T), T>>>(d_ord, nrec, d_rec, d_srec);
-    SCU(cudaGetLastError());
-    hc_scratch_free(d_rec); d_rec = nullptr;
-    hc_scratch_free(d_key); d_key = nullptr;
-    hc_scratch_free(d_key2); d_key2 = nullptr;
-    SCU(hc_scratch_alloc((void**)&d_info, (n_refs + 1) * sizeof(RefInfo)));
+    HC_CU(cudaGetLastError());
+    d_rec.reset();
+    d_key.reset();
+    d_key2.reset();
+    HC_CU(d_info.alloc(n_refs + 1));
     if (n_refs) sam_ref_info<<<n_refs, T>>>(d_srec, nrec, d_rlen, d_info);
-    SCU(cudaGetLastError());
+    HC_CU(cudaGetLastError());
     // the sweep: count, scan, write
     S.X = Ctx{d_text, d_aln, d_ops, min_ov};
     S.srec = d_srec; S.info = d_info; S.n = nrec;
-    SCU(hc_scratch_alloc((void**)&d_nb, (nrec + 1) * sizeof(uint32_t)));
-    SCU(hc_scratch_alloc((void**)&d_rc, (nrec + 1) * sizeof(RecCnt)));
-    SCU(hc_scratch_alloc((void**)&d_boff, (nrec + 1) * sizeof(u64)));
-    hc_scratch_free(d_bsum); d_bsum = nullptr;
-    SCU(hc_scratch_alloc((void**)&d_bsum, hc_scan::blocks_for(nrec + 1) * sizeof(u64)));
+    HC_CU(d_nb.alloc(nrec + 1));
+    HC_CU(d_rc.alloc(nrec + 1));
+    HC_CU(d_boff.alloc(nrec + 1));
+    d_bsum.reset();
+    HC_CU(d_bsum.alloc(hc_scan::blocks_for(nrec + 1)));
     sam_count<<<grid_for(nrec, T), T>>>(S, d_nb, d_rc, d_ovf, d_cnt);
-    SCU(cudaGetLastError());
-    SCU(cudaMemcpy(cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost));
-    SCU(cudaMemcpy(&ovf, d_ovf, sizeof(uint32_t), cudaMemcpyDeviceToHost));
+    HC_CU(cudaGetLastError());
+    HC_CU(cudaMemcpy(cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost));
+    HC_CU(cudaMemcpy(&ovf, d_ovf, sizeof(uint32_t), cudaMemcpyDeviceToHost));
     if (cnt[2] != NO_ERR) goto input_error;
     if (ovf) goto too_big;
     hc_scan::exclusive_u32(d_nb, nrec, d_boff, d_tot, d_bsum, 0);
-    SCU(cudaMemcpy(&out_bytes, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
-    SCU(hc_scratch_alloc((void**)&d_rs, (n_refs + 1) * sizeof(hc_sam_ref_stats)));
+    HC_CU(cudaMemcpy(&out_bytes, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
+    HC_CU(d_rs.alloc(n_refs + 1));
     if (n_refs) sam_ref_stats<<<n_refs, T>>>(d_srec, d_rc, d_info, d_rs);
-    SCU(cudaGetLastError());
-    if (n_refs) SCU(cudaMemcpy(rs.data(), d_rs, n_refs * sizeof(hc_sam_ref_stats), cudaMemcpyDeviceToHost));
+    HC_CU(cudaGetLastError());
+    if (n_refs) HC_CU(cudaMemcpy(rs.data(), d_rs, n_refs * sizeof(hc_sam_ref_stats), cudaMemcpyDeviceToHost));
     for (uint32_t r = 0; r < n_refs; r++) stats->n_out_lines += rs[r].n_overlaps;
     *n_text_bytes = out_bytes;
     if (out_bytes > text_cap) goto capacity;
-    SCU(hc_scratch_alloc((void**)&d_out, out_bytes + 1));
+    HC_CU(d_out.alloc(out_bytes + 1));
     sam_format<<<grid_for(nrec, T), T>>>(S, d_boff, d_out);
-    SCU(cudaGetLastError());
-    SCU(cudaDeviceSynchronize());
-    t1 = now_ms();
+    HC_CU(cudaGetLastError());
+    HC_CU(cudaDeviceSynchronize());
+    t1 = hc_now_ms();
     stats->device_ms = (float)(t1 - t0);
-    if (out_bytes) SCU(hc_copy_d2h(text, d_out, out_bytes));
-    stats->d2h_ms = (float)(now_ms() - t1);
+    if (out_bytes) HC_CU(hc_copy_d2h(text, d_out, out_bytes));
+    stats->d2h_ms = (float)(hc_now_ms() - t1);
     if (ref_stats && n_refs) memcpy(ref_stats, rs.data(), n_refs * sizeof(hc_sam_ref_stats));
     goto done;
 input_error:
@@ -820,7 +758,7 @@ input_error:
         stats->first_error_line = (e >> 2) & 0xffffffffull;
         stats->first_error_status = (uint32_t)(e & 3);
         u64 se[2] = {0, nbytes[f]};
-        SCU(cudaMemcpy(se, d_ls[f] + stats->first_error_line, (stats->first_error_line < n_nl[f] ? 2 : 1) * sizeof(u64), cudaMemcpyDeviceToHost));
+        HC_CU(cudaMemcpy(se, d_ls[f] + stats->first_error_line, (stats->first_error_line < n_nl[f] ? 2 : 1) * sizeof(u64), cudaMemcpyDeviceToHost));
         stats->first_error_offset = se[0];
         stats->first_error_length = se[1] - se[0];
     }
@@ -840,13 +778,5 @@ capacity:
     rc = HC_ERR_CAPACITY;
 done:
     cudaFree(d_ls[0]); cudaFree(d_ls[1]);
-    hc_scratch_free(d_text); hc_scratch_free(d_names); hc_scratch_free(d_out); hc_scratch_free(d_noff); hc_scratch_free(d_tot);
-    hc_scratch_free(d_bsum); hc_scratch_free(d_ooff); hc_scratch_free(d_ops); hc_scratch_free(d_mpos); hc_scratch_free(d_rx);
-    hc_scratch_free(d_apos); hc_scratch_free(d_boff); hc_scratch_free(d_perm); hc_scratch_free(d_nidx); hc_scratch_free(d_mapped);
-    hc_scratch_free(d_nops); hc_scratch_free(d_rev); hc_scratch_free(d_smidx); hc_scratch_free(d_pmidx); hc_scratch_free(d_st);
-    hc_scratch_free(d_rfirst); hc_scratch_free(d_acc); hc_scratch_free(d_val); hc_scratch_free(d_val2); hc_scratch_free(d_nb);
-    hc_scratch_free(d_ovf); hc_scratch_free(d_cnt); hc_scratch_free(d_rlen); hc_scratch_free(d_aln);
-    hc_scratch_free(d_rec); hc_scratch_free(d_srec); hc_scratch_free(d_info); hc_scratch_free(d_rc); hc_scratch_free(d_rs);
-    hc_scratch_free(d_key); hc_scratch_free(d_key2);
     return rc;
 }

@@ -30,7 +30,6 @@
 #include <cmath>
 #include <cstring>
 #include <string>
-#include <time.h>
 #include <cuda_runtime.h>
 #include "../../include/hc_b200.h"
 #include "hc_radix.cuh"
@@ -38,13 +37,10 @@
 #include "hc_stage.h"
 #include "hc_text.cuh"
 
-void hc_set_last_error(const char* msg);   // hc_api.cu
-
 namespace {
 
 typedef long long i64;
 
-constexpr int INSERTION_MAX = 32;
 constexpr i64 BIG = 1ll << 40;             // |OHA|, |OHB|, |OLA|, |OLB| below this: no sum or product of them overflows
 
 struct SfoRec {                            // a temporary line's numbers (host Rec :44)
@@ -75,57 +71,6 @@ __device__ int split8(const char* t, u64 b, u64 e, u64* fb, u64* fe) {
     return n;
 }
 
-// parse_long (:59); *nd = digits after the sign (more than 18: the host's long may overflow, the value is not used)
-__device__ bool parse_num(const char* t, u64 b, u64 e, i64* v, int* nd) {
-    if (b == e) return false;
-    bool neg = false;
-    if (t[b] == '+' || t[b] == '-') { neg = t[b] == '-'; b++; }
-    if (b == e) return false;
-    *nd = (int)(e - b < 100 ? e - b : 100);
-    i64 x = 0;
-    for (u64 p = b; p < e; p++) {
-        const char c = t[p];
-        if (c < '0' || c > '9') return false;
-        if (*nd <= 18) x = x * 10 + (c - '0');
-    }
-    *v = neg ? -x : x;
-    return true;
-}
-
-__device__ __forceinline__ int dec_len(i64 v) {       // bytes put_long (:133) writes
-    unsigned long long u = v < 0 ? 0ull - (unsigned long long)v : (unsigned long long)v;
-    int d = 1;
-    while (u >= 10) { u /= 10; d++; }
-    return d + (v < 0);
-}
-
-struct Sink {                                         // counts bytes; writes them too when p != nullptr
-    char* p;
-    u64 n;
-    __device__ void c(char x) { if (p) p[n] = x; n++; }
-    __device__ void num(i64 v) {
-        const int d = dec_len(v);
-        if (p) {
-            unsigned long long u = v < 0 ? 0ull - (unsigned long long)v : (unsigned long long)v;
-            char* q = p + n;
-            if (v < 0) *q = '-';
-            for (int k = d - 1; k >= (v < 0); k--) { q[k] = (char)('0' + u % 10); u /= 10; }
-        }
-        n += d;
-    }
-    __device__ void str(const char* t, u64 b, u64 e) {
-        if (p) for (u64 i = b; i < e; i++) p[n + (i - b)] = t[i];
-        n += e - b;
-    }
-};
-
-__device__ __forceinline__ void line_span(const char* t, u64 n, const u64* ls, u64 n_nl, u64 k, u64* b, u64* le) {
-    *b = ls[k];
-    u64 e = k < n_nl ? ls[k + 1] : n;
-    while (e > *b && t[e - 1] == '\n') e--;
-    *le = e;
-}
-
 // the temporary line (:328-342) into s; fb / fe: the 8 fields
 __device__ void temp_line(Sink& s, const char* t, u64 b, u64 le, const u64* fb, const u64* fe, const SfoRec& r) {
     s.num(r.idA); s.c('\t'); s.num(r.idB); s.c('\t');
@@ -145,13 +90,13 @@ __global__ void sfo_parse(const char* __restrict__ t, u64 n, const u64* __restri
         line_span(t, n, ls, n_nl, k, &b, &le);
         const int nf = split8(t, b, le, fb, fe);
         i64 v[7] = {0, 0, 0, 0, 0, 0, 0};
-        int nd[7] = {0, 0, 0, 0, 0, 0, 0};
+        int pr[7] = {1, 1, 1, 1, 1, 1, 1};
         uint32_t status = 0;
         if (nf != 8) status = HC_SFO_DIES;
+        for (int f = 0; f < 7 && !status; f++)          // parse_long (:59): any field that fails dies before any decline
+            if (f != 2 && (pr[f] = parse_long(t, fb[f], fe[f], &v[f])) == 0) status = HC_SFO_DIES;
         for (int f = 0; f < 7 && !status; f++)
-            if (f != 2 && !parse_num(t, fb[f], fe[f], &v[f], &nd[f])) status = HC_SFO_DIES;
-        for (int f = 0; f < 7 && !status; f++)
-            if (f != 2 && nd[f] > 18) status = HC_SFO_DECLINED;
+            if (pr[f] == 2) status = HC_SFO_DECLINED;
         const i64 sa = v[0], sb = v[1];
         if (!status && P.np > 0 && !(sa >= 0 && sa < P.lim && sb >= 0 && sb < P.lim)) status = HC_SFO_DIES;
         const i64 na = P.np == 0 ? sa : (sa < P.ns + P.np ? sa : sa - P.np);
@@ -211,44 +156,17 @@ struct TextLess {
     __device__ bool operator()(uint32_t a, uint32_t b) const { return tcmp(tmp, toff, rec, a, b) < 0; }
 };
 
-__device__ void sift_down(const TextLess& lt, uint32_t* v, uint32_t root, uint32_t m) {
-    while (true) {
-        uint32_t c = 2 * root + 1;
-        if (c >= m) return;
-        if (c + 1 < m && lt(v[c], v[c + 1])) c++;
-        if (!lt(v[root], v[c])) return;
-        const uint32_t x = v[root]; v[root] = v[c]; v[c] = x;
-        root = c;
-    }
-}
-
 __device__ __forceinline__ bool same_key(const ulonglong2& a, const ulonglong2& b) { return a.x == b.x && a.y == b.y; }
 
-// one thread per run of equal keys: the run's lines in text order (insertion sort up to 32, heap sort beyond; on a run of
-// identical lines the heap sort is linear)
+// one thread per run of equal keys: the run's lines in text order (hc_radix::sort_run, whose order of equal texts decides
+// which file line of a repeated line is kept)
 __global__ void sfo_runs(const ulonglong2* __restrict__ key, uint32_t* __restrict__ ord, u64 n, TextLess lt) {
     for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x) {
         const ulonglong2 k = key[i];
         if (i > 0 && same_key(key[i - 1], k)) continue;
         u64 j = i + 1;
         while (j < n && same_key(key[j], k)) j++;
-        const uint32_t m = (uint32_t)(j - i);
-        if (m < 2) continue;
-        uint32_t* v = ord + i;
-        if (m <= INSERTION_MAX) {
-            for (uint32_t a = 1; a < m; a++) {
-                const uint32_t x = v[a];
-                uint32_t c = a;
-                while (c > 0 && lt(x, v[c - 1])) { v[c] = v[c - 1]; c--; }
-                v[c] = x;
-            }
-        } else {
-            for (uint32_t r = m / 2; r-- > 0;) sift_down(lt, v, r, m);
-            for (uint32_t e = m - 1; e > 0; e--) {
-                const uint32_t x = v[0]; v[0] = v[e]; v[e] = x;
-                sift_down(lt, v, 0, e);
-            }
-        }
+        hc_radix::sort_run(ord + i, (uint32_t)(j - i), lt);
     }
 }
 
@@ -491,22 +409,7 @@ __global__ void sfo_out_compact(const char* __restrict__ out, const u64* __restr
     }
 }
 
-inline int grid_for(u64 n, int threads) { const u64 b = (n + threads - 1) / threads; return (int)(b < 148 * 16 ? (b ? b : 1) : 148 * 16); }
-inline double now_ms() { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6; }
-
 }  // namespace
-
-// an allocation that fails is HC_ERR_NOMEM (the caller runs the host converter), anything else HC_ERR_CUDA
-#define SCU(call)                                                                                              \
-    do {                                                                                                       \
-        cudaError_t _e = (call);                                                                               \
-        if (_e != cudaSuccess) {                                                                               \
-            hc_set_last_error((std::string("hc_sfo2overlaps: ") + #call + ": " + cudaGetErrorString(_e)).c_str()); \
-            rc = _e == cudaErrorMemoryAllocation ? HC_ERR_NOMEM : HC_ERR_CUDA;                                 \
-            if (rc == HC_ERR_NOMEM) cudaGetLastError();                                                        \
-            goto done;                                                                                         \
-        }                                                                                                      \
-    } while (0)
 
 extern "C" int hc_sfo2overlaps(const char* sfo, uint64_t n_bytes, int64_t num_singles, int64_t num_pairs, char* text,
                                uint64_t text_cap, uint64_t* n_text_bytes, hc_sfo_stats* stats, int device) {
@@ -526,31 +429,32 @@ extern "C" int hc_sfo2overlaps(const char* sfo, uint64_t n_bytes, int64_t num_si
     Params P;
     P.ns = num_singles; P.np = num_pairs;
     P.lim = (num_singles >= (1ll << 61) || num_pairs >= (1ll << 60)) ? (1ll << 62) : num_singles + 2 * num_pairs;
-    char *d_text = nullptr, *d_tmp = nullptr, *d_out = nullptr, *d_dst = nullptr;
-    u64 *d_ls = nullptr, *d_toff = nullptr, *d_tot = nullptr, *d_bsum = nullptr, *d_pos = nullptr, *d_gx = nullptr, *d_rbx = nullptr,
-        *d_rcx = nullptr, *d_soff = nullptr, *d_loff = nullptr, *d_lsout = nullptr, *d_koff = nullptr;
-    unsigned long long* d_cnt = nullptr;        // [0] first error, [1] ss count, [2] kept output lines
-    uint32_t *d_ovf = nullptr, *d_idx = nullptr, *d_idx2 = nullptr, *d_tlen = nullptr, *d_keep = nullptr, *d_uq = nullptr, *d_gf = nullptr,
-             *d_gstart = nullptr, *d_sb = nullptr, *d_rb = nullptr, *d_rc = nullptr, *d_sl = nullptr, *d_sc = nullptr, *d_klen = nullptr;
-    uint32_t *d_order = nullptr, ovf = 0;
-    ulonglong2 *d_key = nullptr, *d_key2 = nullptr, *d_sorted = nullptr;
-    SfoRec *d_rec = nullptr, *d_srec = nullptr;
+    const char* who = "hc_sfo2overlaps";
+    ScratchBuf<char> d_text, d_tmp, d_out, d_dst;
+    ScratchBuf<u64> d_toff, d_tot, d_bsum, d_pos, d_gx, d_rbx, d_rcx, d_soff, d_loff, d_lsout, d_koff;
+    ScratchBuf<unsigned long long> d_cnt;       // [0] first error, [1] ss count, [2] kept output lines
+    ScratchBuf<uint32_t> d_ovf, d_idx, d_idx2, d_tlen, d_gf, d_gstart, d_sb, d_rb, d_rc, d_sl, d_sc, d_klen;
+    ScratchBuf<ulonglong2> d_key, d_key2;
+    ScratchBuf<SfoRec> d_rec, d_srec;
+    u64* d_ls = nullptr;                        // hc_line_index's (cudaMalloc)
+    uint32_t *d_keep = nullptr, *d_uq = nullptr, *d_order = nullptr, ovf = 0;
+    ulonglong2* d_sorted = nullptr;
     u64 n_nl = 0, nl = 0, tbytes = 0, nu = 0, ng = 0, pre_bytes = 0, pre_lines = 0, out_bytes = 0;
     unsigned long long cnt[3] = {~0ull, 0, 0};
     double t0 = 0, t1 = 0;
     TextLess lt;
     Groups G;
-    SCU(cudaSetDevice(device));
-    t0 = now_ms();
+    HC_CU(cudaSetDevice(device));
+    t0 = hc_now_ms();
     if (n_bytes) {
-        SCU(hc_scratch_alloc((void**)&d_text, n_bytes + 16));
-        SCU(hc_copy_h2d(d_text, sfo, n_bytes));
+        HC_CU(d_text.alloc(n_bytes + 16));
+        HC_CU(hc_copy_h2d(d_text, sfo, n_bytes));
     }
-    t1 = now_ms();
+    t1 = hc_now_ms();
     stats->h2d_ms = (float)(t1 - t0);
     t0 = t1;
     if (n_bytes == 0) goto finish;
-    SCU(hc_line_index(d_text, n_bytes, &d_ls, &n_nl, &nl, 0));
+    HC_CU(hc_line_index(d_text, n_bytes, &d_ls, &n_nl, &nl, 0));
     stats->n_lines = nl;
     if (nl >> 32) {
         stats->first_error_line = 1ull << 32;
@@ -559,127 +463,127 @@ extern "C" int hc_sfo2overlaps(const char* sfo, uint64_t n_bytes, int64_t num_si
         rc = HC_ERR_INPUT;
         goto done;
     }
-    SCU(hc_scratch_alloc((void**)&d_cnt, sizeof(cnt)));
-    SCU(hc_scratch_alloc((void**)&d_ovf, sizeof(uint32_t)));
-    SCU(cudaMemcpy(d_cnt, cnt, sizeof(cnt), cudaMemcpyHostToDevice));
-    SCU(cudaMemset(d_ovf, 0, sizeof(uint32_t)));
-    SCU(hc_scratch_alloc((void**)&d_rec, nl * sizeof(SfoRec)));
-    SCU(hc_scratch_alloc((void**)&d_key, nl * sizeof(ulonglong2)));
-    SCU(hc_scratch_alloc((void**)&d_key2, nl * sizeof(ulonglong2)));
-    SCU(hc_scratch_alloc((void**)&d_idx, nl * sizeof(uint32_t)));
-    SCU(hc_scratch_alloc((void**)&d_idx2, nl * sizeof(uint32_t)));
-    SCU(hc_scratch_alloc((void**)&d_tlen, nl * sizeof(uint32_t)));
-    SCU(hc_scratch_alloc((void**)&d_toff, nl * sizeof(u64)));
-    SCU(hc_scratch_alloc((void**)&d_tot, sizeof(u64)));
-    SCU(hc_scratch_alloc((void**)&d_bsum, hc_scan::blocks_for(nl) * sizeof(u64)));
+    HC_CU(d_cnt.alloc(3));
+    HC_CU(d_ovf.alloc(1));
+    HC_CU(cudaMemcpy(d_cnt, cnt, sizeof(cnt), cudaMemcpyHostToDevice));
+    HC_CU(cudaMemset(d_ovf, 0, sizeof(uint32_t)));
+    HC_CU(d_rec.alloc(nl));
+    HC_CU(d_key.alloc(nl));
+    HC_CU(d_key2.alloc(nl));
+    HC_CU(d_idx.alloc(nl));
+    HC_CU(d_idx2.alloc(nl));
+    HC_CU(d_tlen.alloc(nl));
+    HC_CU(d_toff.alloc(nl));
+    HC_CU(d_tot.alloc(1));
+    HC_CU(d_bsum.alloc(hc_scan::blocks_for(nl)));
     sfo_parse<<<grid_for(nl, T), T>>>(d_text, n_bytes, d_ls, n_nl, nl, P, d_rec, d_key, d_idx, d_tlen, d_cnt);
-    SCU(cudaGetLastError());
-    SCU(cudaMemcpy(cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost));
+    HC_CU(cudaGetLastError());
+    HC_CU(cudaMemcpy(cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost));
     if (cnt[0] != ~0ull) goto input_error;
     hc_scan::exclusive_u32(d_tlen, nl, d_toff, d_tot, d_bsum, 0);
-    SCU(cudaMemcpy(&tbytes, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
-    SCU(hc_scratch_alloc((void**)&d_tmp, tbytes + 16));
+    HC_CU(cudaMemcpy(&tbytes, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
+    HC_CU(d_tmp.alloc(tbytes + 16));
     sfo_temp<<<grid_for(nl, T), T>>>(d_text, n_bytes, d_ls, n_nl, nl, d_rec, d_toff, d_tmp);
-    SCU(cudaGetLastError());
-    hc_scratch_free(d_text); d_text = nullptr;
+    HC_CU(cudaGetLastError());
+    d_text.reset();
     // sort | uniq
-    SCU(hc_radix::sort_pairs(d_key, d_idx, d_key2, d_idx2, nl, &d_sorted, &d_order));
+    HC_CU(hc_radix::sort_pairs(d_key, d_idx, d_key2, d_idx2, nl, &d_sorted, &d_order));
     lt.tmp = d_tmp; lt.toff = d_toff; lt.rec = d_rec;
     sfo_runs<<<grid_for(nl, T), T>>>(d_sorted, d_order, nl, lt);
     d_keep = d_tlen;                                   // the lengths are in d_toff now
     sfo_marks<<<grid_for(nl, T), T>>>(d_sorted, d_order, nl, lt, d_keep);
-    SCU(cudaGetLastError());
-    SCU(hc_scratch_alloc((void**)&d_pos, nl * sizeof(u64)));
+    HC_CU(cudaGetLastError());
+    HC_CU(d_pos.alloc(nl));
     hc_scan::exclusive_u32(d_keep, nl, d_pos, d_tot, d_bsum, 0);
-    SCU(cudaMemcpy(&nu, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
+    HC_CU(cudaMemcpy(&nu, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
     stats->n_unique = nu;
-    d_uq = (d_order == d_idx) ? d_idx2 : d_idx;        // the buffer the sort did not leave its result in
+    d_uq = (d_order == d_idx.get()) ? d_idx2.get() : d_idx.get();        // the buffer the sort did not leave its result in
     sfo_compact<<<grid_for(nl, T), T>>>(d_order, d_keep, d_pos, nl, d_uq);
-    SCU(cudaGetLastError());
-    hc_scratch_free(d_pos); d_pos = nullptr;
-    hc_scratch_free(d_key); d_key = nullptr;
-    hc_scratch_free(d_key2); d_key2 = nullptr;
-    hc_scratch_free(d_tmp); d_tmp = nullptr;
-    SCU(hc_scratch_alloc((void**)&d_srec, nu * sizeof(SfoRec)));
+    HC_CU(cudaGetLastError());
+    d_pos.reset();
+    d_key.reset();
+    d_key2.reset();
+    d_tmp.reset();
+    HC_CU(d_srec.alloc(nu));
     sfo_gather<<<grid_for(nu, T), T>>>(d_uq, nu, d_rec, d_srec);
-    SCU(cudaGetLastError());
-    hc_scratch_free(d_rec); d_rec = nullptr;
+    HC_CU(cudaGetLastError());
+    d_rec.reset();
     // groups
-    SCU(hc_scratch_alloc((void**)&d_gf, nu * sizeof(uint32_t)));
-    SCU(hc_scratch_alloc((void**)&d_gx, nu * sizeof(u64)));
+    HC_CU(d_gf.alloc(nu));
+    HC_CU(d_gx.alloc(nu));
     sfo_group_firsts<<<grid_for(nu, T), T>>>(d_srec, nu, P, d_gf);
     hc_scan::exclusive_u32(d_gf, nu, d_gx, d_tot, d_bsum, 0);
-    SCU(cudaGetLastError());
-    SCU(cudaMemcpy(&ng, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
-    SCU(hc_scratch_alloc((void**)&d_gstart, (ng + 1) * sizeof(uint32_t)));
+    HC_CU(cudaGetLastError());
+    HC_CU(cudaMemcpy(&ng, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
+    HC_CU(d_gstart.alloc(ng + 1));
     sfo_group_starts<<<grid_for(nu, T), T>>>(d_gf, d_gx, nu, d_gstart);
     // items: sizes, places, text
     G.uq = d_uq; G.nu = nu; G.rec = d_srec; G.P = P; G.gf = d_gf; G.gx = d_gx; G.gstart = d_gstart; G.ng = ng;
-    SCU(hc_scratch_alloc((void**)&d_sb, nu * sizeof(uint32_t)));
-    SCU(hc_scratch_alloc((void**)&d_rb, nu * sizeof(uint32_t)));
-    SCU(hc_scratch_alloc((void**)&d_rc, nu * sizeof(uint32_t)));
+    HC_CU(d_sb.alloc(nu));
+    HC_CU(d_rb.alloc(nu));
+    HC_CU(d_rc.alloc(nu));
     sfo_count<<<grid_for(nu, T), T>>>(G, d_sb, d_rb, d_rc, d_cnt, d_cnt + 1, d_ovf);
-    SCU(cudaGetLastError());
-    SCU(cudaMemcpy(cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost));
-    SCU(cudaMemcpy(&ovf, d_ovf, sizeof(uint32_t), cudaMemcpyDeviceToHost));
+    HC_CU(cudaGetLastError());
+    HC_CU(cudaMemcpy(cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost));
+    HC_CU(cudaMemcpy(&ovf, d_ovf, sizeof(uint32_t), cudaMemcpyDeviceToHost));
     if (cnt[0] != ~0ull) goto input_error;
     stats->s_s_count = cnt[1];
     if (ovf) goto too_big;
-    SCU(hc_scratch_alloc((void**)&d_rbx, (nu + 1) * sizeof(u64)));
-    SCU(hc_scratch_alloc((void**)&d_rcx, (nu + 1) * sizeof(u64)));
+    HC_CU(d_rbx.alloc(nu + 1));
+    HC_CU(d_rcx.alloc(nu + 1));
     hc_scan::exclusive_u32(d_rb, nu, d_rbx, d_tot, d_bsum, 0);
     hc_scan::exclusive_u32(d_rc, nu, d_rcx, d_tot, d_bsum, 0);
-    SCU(cudaMemcpy(&stats->p_count, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
-    SCU(hc_scratch_alloc((void**)&d_sl, nu * sizeof(uint32_t)));
-    SCU(hc_scratch_alloc((void**)&d_sc, nu * sizeof(uint32_t)));
+    HC_CU(cudaMemcpy(&stats->p_count, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
+    HC_CU(d_sl.alloc(nu));
+    HC_CU(d_sc.alloc(nu));
     sfo_slots<<<grid_for(nu, T), T>>>(G, d_sb, d_rbx, d_rcx, d_sl, d_sc, d_ovf);
-    SCU(cudaGetLastError());
-    SCU(cudaMemcpy(&ovf, d_ovf, sizeof(uint32_t), cudaMemcpyDeviceToHost));
+    HC_CU(cudaGetLastError());
+    HC_CU(cudaMemcpy(&ovf, d_ovf, sizeof(uint32_t), cudaMemcpyDeviceToHost));
     if (ovf) goto too_big;
-    SCU(hc_scratch_alloc((void**)&d_soff, nu * sizeof(u64)));
-    SCU(hc_scratch_alloc((void**)&d_loff, nu * sizeof(u64)));
+    HC_CU(d_soff.alloc(nu));
+    HC_CU(d_loff.alloc(nu));
     hc_scan::exclusive_u32(d_sl, nu, d_soff, d_tot, d_bsum, 0);
-    SCU(cudaMemcpy(&pre_bytes, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
+    HC_CU(cudaMemcpy(&pre_bytes, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
     hc_scan::exclusive_u32(d_sc, nu, d_loff, d_tot, d_bsum, 0);
-    SCU(cudaMemcpy(&pre_lines, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
+    HC_CU(cudaMemcpy(&pre_lines, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
     if (pre_lines == 0) goto finish;
-    SCU(hc_scratch_alloc((void**)&d_out, pre_bytes));
-    SCU(hc_scratch_alloc((void**)&d_lsout, (pre_lines + 1) * sizeof(u64)));
-    SCU(cudaMemcpy(d_lsout + pre_lines, &pre_bytes, sizeof(u64), cudaMemcpyHostToDevice));
+    HC_CU(d_out.alloc(pre_bytes));
+    HC_CU(d_lsout.alloc(pre_lines + 1));
+    HC_CU(cudaMemcpy(d_lsout + pre_lines, &pre_bytes, sizeof(u64), cudaMemcpyHostToDevice));
     sfo_format<<<grid_for(nu, T), T>>>(G, d_sb, d_rb, d_rbx, d_rcx, d_sl, d_sc, d_soff, d_loff, d_out, d_lsout);
-    SCU(cudaGetLastError());
+    HC_CU(cudaGetLastError());
     // final uniq
-    hc_scratch_free(d_bsum); d_bsum = nullptr;
-    SCU(hc_scratch_alloc((void**)&d_bsum, hc_scan::blocks_for(pre_lines) * sizeof(u64)));
-    SCU(hc_scratch_alloc((void**)&d_klen, pre_lines * sizeof(uint32_t)));
-    SCU(hc_scratch_alloc((void**)&d_koff, pre_lines * sizeof(u64)));
+    d_bsum.reset();
+    HC_CU(d_bsum.alloc(hc_scan::blocks_for(pre_lines)));
+    HC_CU(d_klen.alloc(pre_lines));
+    HC_CU(d_koff.alloc(pre_lines));
     sfo_out_marks<<<grid_for(pre_lines, T), T>>>(d_out, d_lsout, pre_lines, d_klen, d_cnt + 2);
     hc_scan::exclusive_u32(d_klen, pre_lines, d_koff, d_tot, d_bsum, 0);
-    SCU(cudaGetLastError());
-    SCU(cudaMemcpy(&out_bytes, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
-    SCU(cudaMemcpy(cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost));
+    HC_CU(cudaGetLastError());
+    HC_CU(cudaMemcpy(&out_bytes, d_tot, sizeof(u64), cudaMemcpyDeviceToHost));
+    HC_CU(cudaMemcpy(cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost));
     stats->n_out_lines = cnt[2];
     *n_text_bytes = out_bytes;
     if (out_bytes > text_cap) goto capacity;
-    SCU(hc_scratch_alloc((void**)&d_dst, out_bytes));
+    HC_CU(d_dst.alloc(out_bytes));
     sfo_out_compact<<<grid_for(pre_lines, T), T>>>(d_out, d_lsout, d_klen, d_koff, pre_lines, d_dst);
-    SCU(cudaGetLastError());
-    SCU(cudaDeviceSynchronize());
-    t1 = now_ms();
+    HC_CU(cudaGetLastError());
+    HC_CU(cudaDeviceSynchronize());
+    t1 = hc_now_ms();
     stats->device_ms = (float)(t1 - t0);
-    SCU(hc_copy_d2h(text, d_dst, out_bytes));
-    stats->d2h_ms = (float)(now_ms() - t1);
+    HC_CU(hc_copy_d2h(text, d_dst, out_bytes));
+    stats->d2h_ms = (float)(hc_now_ms() - t1);
     goto done;
 finish:                                                 // no output line
-    SCU(cudaDeviceSynchronize());
-    stats->device_ms = (float)(now_ms() - t0);
+    HC_CU(cudaDeviceSynchronize());
+    stats->device_ms = (float)(hc_now_ms() - t0);
     goto done;
 input_error:
     stats->first_error_line = cnt[0] >> 2;
     stats->first_error_status = (uint32_t)(cnt[0] & 3);
     {
         u64 se[2] = {0, n_bytes};
-        SCU(cudaMemcpy(se, d_ls + stats->first_error_line, (stats->first_error_line < n_nl ? 2 : 1) * sizeof(u64), cudaMemcpyDeviceToHost));
+        HC_CU(cudaMemcpy(se, d_ls + stats->first_error_line, (stats->first_error_line < n_nl ? 2 : 1) * sizeof(u64), cudaMemcpyDeviceToHost));
         stats->first_error_offset = se[0];
         stats->first_error_length = se[1] - se[0];
     }
@@ -696,12 +600,5 @@ capacity:
     rc = HC_ERR_CAPACITY;
 done:
     cudaFree(d_ls);
-    hc_scratch_free(d_text); hc_scratch_free(d_tmp); hc_scratch_free(d_out); hc_scratch_free(d_dst);
-    hc_scratch_free(d_toff); hc_scratch_free(d_tot); hc_scratch_free(d_bsum); hc_scratch_free(d_pos); hc_scratch_free(d_gx);
-    hc_scratch_free(d_rbx); hc_scratch_free(d_rcx); hc_scratch_free(d_soff); hc_scratch_free(d_loff); hc_scratch_free(d_lsout);
-    hc_scratch_free(d_koff); hc_scratch_free(d_cnt); hc_scratch_free(d_ovf); hc_scratch_free(d_idx); hc_scratch_free(d_idx2);
-    hc_scratch_free(d_tlen); hc_scratch_free(d_gf); hc_scratch_free(d_gstart); hc_scratch_free(d_sb); hc_scratch_free(d_rb);
-    hc_scratch_free(d_rc); hc_scratch_free(d_sl); hc_scratch_free(d_sc); hc_scratch_free(d_klen); hc_scratch_free(d_key);
-    hc_scratch_free(d_key2); hc_scratch_free(d_rec); hc_scratch_free(d_srec);
     return rc;
 }

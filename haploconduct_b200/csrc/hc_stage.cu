@@ -1,11 +1,13 @@
 // hc_stage.cu -- see hc_stage.h
 #include "hc_stage.h"
+#include "../../include/hc_b200.h"
 
 #include <omp.h>
 #include <stdlib.h>
 #include <string.h>
 
 #include <mutex>
+#include <string>
 #include <unistd.h>
 #include <stdio.h>
 #include <time.h>
@@ -299,8 +301,21 @@ void hc_scratch_free_on(void* p, cudaStream_t st) {
     if (p) cudaFreeAsync(p, st);
 }
 
+int hc_cuda_fail(const char* who, const char* call, cudaError_t e) {
+    hc_set_last_error((std::string(who) + ": " + call + ": " + cudaGetErrorString(e)).c_str());
+    if (e != cudaErrorMemoryAllocation) return HC_ERR_CUDA;
+    cudaGetLastError();
+    return HC_ERR_NOMEM;
+}
+
+double hc_now_ms() {
+    timespec ts;
+    clock_gettime(CLOCK_MONOTONIC, &ts);
+    return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6;
+}
+
 // ---- pinned host memory for callers of the host-buffer entry points (include/hc_b200.h) -----------------------------------
-extern "C" void* hc_host_alloc(unsigned long long bytes, int write_combined) {
+extern "C" void* hc_host_alloc(uint64_t bytes, int write_combined) {
     void* p = nullptr;
     const unsigned flags = cudaHostAllocPortable | (write_combined ? cudaHostAllocWriteCombined : 0u);
     if (cudaHostAlloc(&p, bytes ? (size_t)bytes : 1, flags) != cudaSuccess) { cudaGetLastError(); return nullptr; }

@@ -1,5 +1,6 @@
-// hc_text.cuh -- text primitives shared by the ingestion kernels (hc_ingest.cu: overlaps file, hc_pack.cu: FASTQ):
-// newline index of a device buffer (count -> scan -> mark) and the glibc number parsers the reference calls.
+// hc_text.cuh -- text primitives shared by the ingestion kernels (hc_ingest.cu: overlaps file, hc_pack.cu: FASTQ) and the
+// converters (hc_sfo.cu, hc_sam.cu): newline index of a device buffer (count -> scan -> mark), the lines it delimits, the
+// glibc number parsers the reference calls, the converters' number parser and their count-then-write output sink.
 #ifndef HC_TEXT_CUH_
 #define HC_TEXT_CUH_
 #include <cstdint>
@@ -145,6 +146,56 @@ __device__ u64 dev_strtoul0(const char* t, u64 p, u64 q) {
     return neg ? 0ull - v : v;
 }
 
+// parse_long of both host converters on [b, e): an optional sign, then decimal digits only.  0: not a number; 1: ok, *v set;
+// 2: more than 18 digits (the host's long may overflow; *v holds the first 18 and the caller declines the field).
+__device__ int parse_long(const char* t, u64 b, u64 e, long long* v) {
+    if (b == e) return 0;
+    bool neg = false;
+    if (t[b] == '+' || t[b] == '-') { neg = t[b] == '-'; b++; }
+    if (b == e) return 0;
+    long long x = 0;
+    for (u64 p = b; p < e; p++) {
+        const char c = t[p];
+        if (c < '0' || c > '9') return 0;
+        if (p - b < 18) x = x * 10 + (c - '0');
+    }
+    *v = neg ? -x : x;
+    return e - b > 18 ? 2 : 1;
+}
+
+// ---- lines and output ----------------------------------------------------------------------------
+// Line k of a text with the newline index ls (n_nl newlines, hc_line_index): [*b, *le) without its '\n'.  The span up to
+// the next line start ends in its only newline, so one strip is all there is.
+__device__ __forceinline__ void line_span(const char* t, u64 n, const u64* ls, u64 n_nl, u64 k, u64* b, u64* le) {
+    *b = ls[k];
+    u64 e = k < n_nl ? ls[k + 1] : n;
+    if (e > *b && t[e - 1] == '\n') e--;
+    *le = e;
+}
+
+// A thread's output text: counts the bytes, and writes them too when p != nullptr (the converters size every line with
+// one pass, scan the sizes and write with a second)
+struct Sink {
+    char* p;
+    u64 n;
+    __device__ void c(char x) { if (p) p[n] = x; n++; }
+    __device__ void num(long long v) {                   // printf("%ld")
+        unsigned long long u = v < 0 ? 0ull - (unsigned long long)v : (unsigned long long)v;
+        int d = 1;
+        for (unsigned long long x = u; x >= 10; x /= 10) d++;
+        d += v < 0;
+        if (p) {
+            char* q = p + n;
+            if (v < 0) *q = '-';
+            for (int k = d - 1; k >= (v < 0); k--) { q[k] = (char)('0' + u % 10); u /= 10; }
+        }
+        n += d;
+    }
+    __device__ void str(const char* t, u64 b, u64 e) {   // the bytes t[b, e)
+        if (p) for (u64 i = b; i < e; i++) p[n + (i - b)] = t[i];
+        n += e - b;
+    }
+};
 
 // Newline index of d_text[0, n): *d_line_start (cudaMalloc'ed here, n_newlines + 2 entries) holds the offset of every
 // line start, entry 0 = 0.  n_lines counts an unterminated last line too (std::getline returns it).

@@ -16,10 +16,20 @@
         if (e != cudaSuccess) goto done;                \
     } while (0)
 
+namespace {
+struct KeyLess {
+    const uint64_t* key;
+    __device__ bool operator()(uint32_t a, uint32_t b) const { return key[a] < key[b]; }
+};
+
+__global__ void sort_run_kernel(const uint64_t* key, uint32_t* idx, uint32_t m) { hc_radix::sort_run(idx, m, KeyLess{key}); }
+}  // namespace
+
 extern "C" {
 
 // The sizes the primitives are built for: [hc_scan::THREADS, hc_scan::PER_BLOCK, hc_radix::THREADS, hc_radix::TILE,
-// newline TILE of hc_text.cuh, scan_counts' block].  The tests derive their boundary sizes from these.
+// newline TILE of hc_text.cuh, scan_counts' block, hc_radix::RUN_INSERTION_MAX].  The tests derive their boundary sizes
+// from these.
 void hcp_constants(uint64_t* out) {
     out[0] = hc_scan::THREADS;
     out[1] = hc_scan::PER_BLOCK;
@@ -27,6 +37,7 @@ void hcp_constants(uint64_t* out) {
     out[3] = hc_radix::TILE;
     out[4] = TILE;
     out[5] = 1024;
+    out[6] = hc_radix::RUN_INSERTION_MAX;
 }
 
 uint64_t hcp_blocks_for(uint64_t n) { return hc_scan::blocks_for(n); }
@@ -81,6 +92,25 @@ int hcp_sort_pairs(uint64_t* keys, uint32_t* vals, uint64_t n, int* in_tmp) {
     SCU(cudaMemcpy(vals, vres, n * sizeof(uint32_t), cudaMemcpyDeviceToHost));
 done:
     cudaFree(d_k); cudaFree(d_kt); cudaFree(d_v); cudaFree(d_vt);
+    return (int)e;
+}
+
+// hc_radix::sort_run of the indices 0..m-1 of one run, ordered by key[index], on one thread; idx gets the permutation.
+int hcp_sort_run(const uint64_t* keys, uint32_t m, uint32_t* idx) {
+    uint64_t* d_k = nullptr;
+    uint32_t* d_i = nullptr;
+    cudaError_t e = cudaSuccess;
+    for (uint32_t i = 0; i < m; i++) idx[i] = i;
+    SCU(cudaMalloc(&d_k, (m ? m : 1) * sizeof(uint64_t)));
+    SCU(cudaMalloc(&d_i, (m ? m : 1) * sizeof(uint32_t)));
+    SCU(cudaMemcpy(d_k, keys, m * sizeof(uint64_t), cudaMemcpyHostToDevice));
+    SCU(cudaMemcpy(d_i, idx, m * sizeof(uint32_t), cudaMemcpyHostToDevice));
+    sort_run_kernel<<<1, 1>>>(d_k, d_i, m);
+    SCU(cudaGetLastError());
+    SCU(cudaDeviceSynchronize());
+    SCU(cudaMemcpy(idx, d_i, m * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+done:
+    cudaFree(d_k); cudaFree(d_i);
     return (int)e;
 }
 

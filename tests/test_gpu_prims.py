@@ -1,5 +1,6 @@
 """GPU suite: the multi-block primitives every ordered output rests on -- hc_scan::exclusive_u32, hc_radix::sort_pairs and
-hc_line_index (hc_text.cuh) -- compared exactly with numpy through the test-only C entry points of
+hc_line_index (hc_text.cuh) -- compared exactly with numpy, and the one-thread run sort behind the radix sort
+(hc_radix::sort_run) with a restatement of its algorithm, through the test-only C entry points of
 tests/cuda/hc_prims_shim.cu.  Each primitive has a second, carry-propagating loop in a single-block kernel that only runs
 past a fixed size: more than 1024 block sums (scan_block_sums), more than 16384 sort tiles (the digit-matrix scan of
 sort_pairs, 256 cells per tile) and more than 1024 text tiles (scan_counts).  The size lists below straddle those sizes;
@@ -14,6 +15,7 @@ import pytest
 SCAN_THREADS, SCAN_PER_BLOCK = 1024, 4096             # hc_scan::THREADS, hc_scan::PER_BLOCK
 RADIX_DIGITS, RADIX_TILE = 256, 2048                  # hc_radix::THREADS (= digit values), hc_radix::TILE
 TEXT_TILE, COUNTS_BLOCK = 4096, 1024                  # newline TILE of hc_text.cuh, threads of scan_counts
+RUN_INSERTION_MAX = 32                                # hc_radix::sort_run: insertion sort up to this, heap sort beyond
 SCAN_CARRY = SCAN_THREADS * SCAN_PER_BLOCK            # inputs above this: scan_block_sums carries between its passes
 SORT_CARRY = SCAN_CARRY // RADIX_DIGITS * RADIX_TILE  # records above this: the digit-matrix scan carries
 TEXT_CARRY = COUNTS_BLOCK * TEXT_TILE                 # text bytes above this: scan_counts carries
@@ -78,14 +80,15 @@ def shim():
     L.hcp_exclusive_u32.argtypes, L.hcp_exclusive_u32.restype = [P, u64, P, u64, P, P, u64], ctypes.c_int
     L.hcp_sort_pairs.argtypes, L.hcp_sort_pairs.restype = [P, P, u64, P], ctypes.c_int
     L.hcp_line_index.argtypes, L.hcp_line_index.restype = [P, u64, u64, P, u64, P, P], ctypes.c_int
+    L.hcp_sort_run.argtypes, L.hcp_sort_run.restype = [P, ctypes.c_uint32, P], ctypes.c_int
     return L
 
 
 @pytest.mark.gpu
 def test_shim_constants(shim):
-    c = np.zeros(6, dtype=np.uint64)
+    c = np.zeros(7, dtype=np.uint64)
     shim.hcp_constants(c.ctypes.data)
-    assert c.tolist() == [SCAN_THREADS, SCAN_PER_BLOCK, RADIX_DIGITS, RADIX_TILE, TEXT_TILE, COUNTS_BLOCK]
+    assert c.tolist() == [SCAN_THREADS, SCAN_PER_BLOCK, RADIX_DIGITS, RADIX_TILE, TEXT_TILE, COUNTS_BLOCK, RUN_INSERTION_MAX]
     for n in SCAN_SIZES:
         assert shim.hcp_blocks_for(n) == blocks_for(n)
 
@@ -252,3 +255,63 @@ def test_sort_pairs_past_the_cell_scan(shim, n, pattern):
     """16384 tiles are 4,194,304 digit-matrix cells, one full pass of scan_block_sums; one record more needs a second."""
     assert scan_blocks(sort_cells(n)) >= SCAN_THREADS
     check_sort(shim, n, pattern)
+
+
+# ---- hc_radix::sort_run ---------------------------------------------------------------------------------------------
+def sort_run_reference(key):
+    """sort_run's algorithm restated: the permutation of 0..m-1 it leaves, ties included.  It is not stable, and the order
+    of equal keys decides which file line of a repeated line hc_sfo2overlaps keeps (and so which line an error names)."""
+    v = list(range(len(key)))
+    m = len(v)
+    less = lambda a, b: key[a] < key[b]
+    if m <= RUN_INSERTION_MAX:
+        for a in range(1, m):
+            x, c = v[a], a
+            while c > 0 and less(x, v[c - 1]):
+                v[c] = v[c - 1]
+                c -= 1
+            v[c] = x
+        return v
+
+    def sift_down(root, end):
+        while True:
+            c = 2 * root + 1
+            if c >= end:
+                return
+            if c + 1 < end and less(v[c], v[c + 1]):
+                c += 1
+            if not less(v[root], v[c]):
+                return
+            v[root], v[c] = v[c], v[root]
+            root = c
+
+    for r in range(m // 2 - 1, -1, -1):
+        sift_down(r, m)
+    for e in range(m - 1, 0, -1):
+        v[0], v[e] = v[e], v[0]
+        sift_down(0, e)
+    return v
+
+
+def run_keys(m, pattern):
+    rng = np.random.default_rng(31 * m + len(pattern))
+    if pattern == "distinct":
+        return rng.permutation(m).astype(np.uint64) * np.uint64(0x9E3779B97F4A7C15)
+    if pattern == "equal":
+        return np.full(m, 7, dtype=np.uint64)
+    if pattern == "three":
+        return rng.integers(0, 3, m).astype(np.uint64)
+    assert pattern == "descending"
+    return np.arange(m, dtype=np.uint64)[::-1].copy()
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("pattern", ["distinct", "equal", "three", "descending"])
+@pytest.mark.parametrize("m", [0, 1, 2, RUN_INSERTION_MAX - 1, RUN_INSERTION_MAX, RUN_INSERTION_MAX + 1, 64, 1000])
+def test_sort_run(shim, m, pattern):
+    key = run_keys(m, pattern)
+    idx = np.full(m + 1, 0xFFFFFFFF, dtype=np.uint32)
+    assert shim.hcp_sort_run(key.ctypes.data, m, idx.ctypes.data) == 0
+    want = sort_run_reference(key.tolist())
+    assert idx[:m].tolist() == want
+    assert idx[m] == 0xFFFFFFFF
