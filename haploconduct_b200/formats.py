@@ -29,9 +29,10 @@ CANDIDATE_COMPACT = np.dtype([("idx1", "<u4"), ("idx2", "<u4"), ("pos1_flags", "
 
 def compact_candidates(c: np.ndarray) -> np.ndarray:
     """hc_candidate -> hc_candidate_compact (POS1 must fit 28 bits)."""
+    if len(c) and int(c["pos1"].max()) >= (1 << 28):      # a wider POS1 would spill into the ORI / ORD bits
+        raise ValueError("POS1 does not fit the 16-byte candidate record")
     out = np.zeros(len(c), dtype=CANDIDATE_COMPACT)
     out["idx1"], out["idx2"], out["pos2"] = c["idx1"], c["idx2"], c["pos2"]
-    assert (c["pos1"] < (1 << 28)).all()
     ordc = np.where(c["ord"] == ord("1"), 1, np.where(c["ord"] == ord("2"), 2, 0)).astype(np.uint32)
     out["pos1_flags"] = c["pos1"] | ((c["ori1"] != 0).astype(np.uint32) << 28) | ((c["ori2"] != 0).astype(np.uint32) << 29) | (ordc << 30)
     return out
